@@ -4,9 +4,13 @@ operands) on N B200s of one node, plus the CPU reference arm.
     python bench.py [--gpus N] [--steps K] [--warmup W]            # candidate (this repo's CUDA path)
     python bench.py --impl reference [--gpus N] --steps K --warmup W   # reference algorithm on the host CPU cores
     torchrun --nproc-per-node N ... bench.py --gpus N ...             # N > 1: one rank per GPU, batch-sharded
+    python bench.py ... --dump-outputs DIR                            # + the last timed step's outputs as DIR/*.npy
 
 A step = one `forward_with_guidance` call over one batch of 32 synthetic 518x518 images per GPU
 (BASELINE.json configs[1]), cycling through the 9 instructions.  Prints ONE JSON line on rank 0.
+
+Weights and inputs are seeded, so two runs with the same arguments see the same inputs: `--dump-outputs` lets two
+builds of the project be compared output for output (rank 0's shard when N > 1).
 """
 from __future__ import annotations
 
@@ -34,6 +38,22 @@ ALGO_GFLOP_BY_SIZE = {224: 48.4, 518: 321.5, 1036: 2218.0}
 ALGO_GFLOP_BACKBONE = {224: 46.32, 518: 303.15, 1036: 2041.0}  # --workload backbone (BASELINE.json configs[2])
 ALGO_GFLOP_PER_IMAGE = 321.5
 METRIC = "images/sec at 518x518 bf16"
+DUMP_MAX_BYTES = 64 * 10**6  # --dump-outputs: all .npy files together
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Write each tensor as `out_dir/<name>.npy` in float32.  When together they would exceed DUMP_MAX_BYTES, each is
+    replaced by the same share of its (flattened) elements, picked by a fixed seed, so runs stay comparable."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_MAX_BYTES - 1024 * len(arrays)  # room for the .npy headers
+    for name, a in arrays.items():
+        if total > budget:
+            keep = a.size * budget // total
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def _peaks():
@@ -107,12 +127,13 @@ def cpu_reference(steps: int, warmup: int, images_per_step: int):
     for i in range(warmup + steps):
         torch.manual_seed(11)
         t0 = time.perf_counter()
-        orc.forward_with_guidance(sd, x, ex, INSTRUCTIONS[i % 9], update_history=False)
+        out = orc.forward_with_guidance(sd, x, ex, INSTRUCTIONS[i % 9], update_history=False)
         if i >= warmup:
             times.append(time.perf_counter() - t0)
     total = sum(times)
     return {"value": images_per_step * len(times) / total, "ms_per_step": 1e3 * total / len(times),
-            "cores": torch.get_num_threads(), "images_per_step": images_per_step}
+            "cores": torch.get_num_threads(), "images_per_step": images_per_step,
+            "outputs": {"depth": out["depth"], "confidence": out["confidence"], "attention": out["heatmap"]}}
 
 
 def run_reference(args):
@@ -121,6 +142,8 @@ def run_reference(args):
         return
     ips = 2
     r = cpu_reference(args.steps, args.warmup, ips)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["outputs"])
     sample = f"{ips} synthetic 518x518 images per step, oracle port of reference forward_with_guidance, fp32, {r['cores']} threads"
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "images/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
@@ -381,12 +404,16 @@ def run_candidate(args):
     barrier()
     e0.record()
     for i in range(args.steps):
-        step(i, dev_imgs[i % n_sets])
+        out = step(i, dev_imgs[i % n_sets])
     e1.record()
     barrier()
     launches, _ = ops.trace_stop()
     clocks = sampler.stop() if rank == 0 else None
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        # written before the next pass: the backbone's CLS rows are a view of a workspace that it overwrites
+        names = ("cls_tokens",) if backbone_only else ("depth", "confidence", "attention")
+        dump_outputs(args.dump_outputs, dict(zip(names, out)))
 
     # ---- per-kernel device times: a second pass of the same K steps, launched eagerly with a CUDA-event pair around
     # every launch on the launching stream (graph replay hides individual launches from events) ----
@@ -525,6 +552,8 @@ def main():
                     help="sweep configs of BASELINE.json (224 / 1036); the headline metric is quoted at 518")
     ap.add_argument("--workload", default="guided", choices=["guided", "backbone"],
                     help="guided = configs[1] (default, the headline); backbone = configs[2] (DINOv2 tokens only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     global S, ALGO_GFLOP_PER_IMAGE, METRIC
     S = args.image_size

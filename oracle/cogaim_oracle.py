@@ -23,6 +23,7 @@ those outputs are committed under `tests/golden/` and checked by `tests/test_ora
 """
 from __future__ import annotations
 
+import hashlib
 import math
 from typing import Dict, Optional
 
@@ -180,6 +181,26 @@ def build_state_dict(seed: int = 0, num_cameras: int = 71, curiosity_guided: boo
 def state_dict_digest(sd: SD) -> Dict[str, float]:
     """Cheap fingerprint used by the golden fixtures: per-tensor fp64 sum and abs-sum."""
     return {k: (float(v.double().sum()), float(v.double().abs().sum())) for k, v in sd.items()}
+
+
+def matches_digest(v: torch.Tensor, digest) -> bool:
+    """`v` against its `state_dict_digest` entry (sum, abs-sum), up to the order of the fp64 additions: torch splits a
+    CPU sum across its threads, so the order depends on the host's core count, and two orders of n additions differ by
+    at most 2 n 2^-53 sum|x|.  Bit-exactness is `state_dict_sha256`'s job."""
+    s, a = digest
+    v = v.double()
+    tol = 2 * v.numel() * 2.0 ** -53 * a
+    return abs(float(v.sum()) - s) <= tol and abs(float(v.abs().sum()) - a) <= tol
+
+
+def state_dict_sha256(sd: SD) -> str:
+    """Bit-exact fingerprint of a whole state_dict: names, dtypes, shapes and bytes, in order."""
+    h = hashlib.sha256()
+    for k, v in sd.items():
+        v = v.detach().cpu().contiguous()
+        h.update(f"{k}:{v.dtype}:{tuple(v.shape)};".encode())
+        h.update(v.numpy().tobytes())
+    return h.hexdigest()
 
 
 # --------------------------------------------------------------------------------------------------

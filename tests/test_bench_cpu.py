@@ -24,6 +24,41 @@ def test_reference_arm_prints_one_contract_line():
     assert "workload" in d["config"]
 
 
+def test_reference_arm_dumps_the_same_outputs_on_every_run(tmp_path):
+    import numpy as np
+    dumps = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
+                              "--warmup", "0", "--image-size", "224", "--dump-outputs", str(tmp_path / run)],
+                             capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+        assert sorted(os.listdir(tmp_path / run)) == ["attention.npy", "confidence.npy", "depth.npy"]
+        dumps.append({n: np.load(tmp_path / run / f"{n}.npy") for n in ("depth", "confidence", "attention")})
+    a, b = dumps
+    assert a["depth"].shape == a["confidence"].shape == (2, 1) and a["attention"].shape == (2, 256)
+    for n in a:
+        assert a[n].dtype == np.float32 and np.isfinite(a[n]).all()
+        assert np.array_equal(a[n], b[n]), n
+
+
+def test_dump_outputs_samples_what_exceeds_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 64 * 1024)
+    big = {"a": torch.arange(40000, dtype=torch.float64), "b": torch.ones(3, 2)}
+    bench.dump_outputs(str(tmp_path / "x"), big)
+    bench.dump_outputs(str(tmp_path / "y"), big)
+    sizes = sum(os.path.getsize(tmp_path / "x" / f) for f in os.listdir(tmp_path / "x"))
+    assert sizes <= 64 * 1024
+    a = np.load(tmp_path / "x" / "a.npy")
+    assert a.dtype == np.float32 and 0 < a.size < 40000 and (np.diff(a) > 0).all()   # a sorted subset of the elements
+    assert np.array_equal(a, np.load(tmp_path / "y" / "a.npy"))                        # ... the same one every time
+    small = {"c": torch.ones(4, 5)}
+    bench.dump_outputs(str(tmp_path / "z"), small)
+    assert np.load(tmp_path / "z" / "c.npy").shape == (4, 5)                         # under the limit: whole
+
+
 def test_candidate_arm_refuses_to_run_without_a_gpu():
     import torch
     if torch.cuda.is_available():

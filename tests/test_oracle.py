@@ -15,6 +15,16 @@ from oracle import cogaim_oracle as orc
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
+def _assert_reference_init(sd, gold_file):
+    """Digests recorded from the reference (up to fp64 summation order) and the state_dict's SHA-256 (every bit)."""
+    gold = json.load(open(os.path.join(GOLD, gold_file)))
+    assert list(sd.keys()) == gold["names"]
+    for k, v in sd.items():
+        assert list(v.shape) == gold["shapes"][k], k
+        assert orc.matches_digest(v, gold["digest"][k]), k
+    assert orc.state_dict_sha256(sd) == json.load(open(os.path.join(GOLD, "state_dict_seed0_sha256.json")))[gold_file]
+
+
 @pytest.fixture(scope="module")
 def sd():
     return orc.build_state_dict(0)
@@ -26,14 +36,9 @@ def tokens224(sd):
 
 
 def test_state_dict_matches_reference_init(sd):
-    """Same seed + same construction order => the reference's 319 tensors, bit for bit (digest compare)."""
-    gold = json.load(open(os.path.join(GOLD, "state_dict_seed0.json")))
-    assert list(sd.keys()) == gold["names"]
+    """Same seed + same construction order => the reference's 319 tensors, bit for bit."""
     assert len(sd) == 319
-    for k, v in sd.items():
-        assert list(v.shape) == gold["shapes"][k], k
-        s, a = gold["digest"][k]
-        assert float(v.double().sum()) == s and float(v.double().abs().sum()) == a, k
+    _assert_reference_init(sd, "state_dict_seed0.json")
 
 
 def test_backbone_restated_vs_hf(sd, tokens224):
@@ -205,12 +210,9 @@ def test_curiosity_rewards_and_ring_buffer(sd, tokens224):
 
 def test_curiosity_guided_state_dict_and_forward():
     """Top-level `curiosity_guided_attention: {enabled: true}` (src/model.py:854): 335 tensors, modulated attention."""
-    gold_sd = json.load(open(os.path.join(GOLD, "state_dict_seed0_curiosity_guided.json")))
     sd = orc.build_state_dict(0, curiosity_guided=True)
-    assert list(sd.keys()) == gold_sd["names"] and len(sd) == 335
-    for k, v in sd.items():
-        s, a = gold_sd["digest"][k]
-        assert float(v.double().sum()) == s and float(v.double().abs().sum()) == a, k
+    assert len(sd) == 335
+    _assert_reference_init(sd, "state_dict_seed0_curiosity_guided.json")
     tokens = orc.dinov2_tokens(sd, orc.synthetic_images(2, 224))
     gold = np.load(os.path.join(GOLD, "curiosity_guided.npz"))
     _curiosity_sequence(dict(sd), tokens, gold, check_outputs=True)
@@ -225,12 +227,9 @@ def test_curiosity_guided_state_dict_and_forward():
 def test_lora_is_built_saved_and_ignored_by_the_reference():
     """Top-level `use_lora: true` (src/model.py:822-831): 24 more tensors, bit-identical init, and a forward that never
     reads them — the fixture was recorded with non-zero lora_B; the oracle, which has no LoRA code at all, reproduces it."""
-    gold_sd = json.load(open(os.path.join(GOLD, "state_dict_seed0_lora.json")))
     sd = orc.build_state_dict(0, use_lora=True)
-    assert list(sd.keys()) == gold_sd["names"] and len(sd) == 343
-    for k, v in sd.items():
-        s, a = gold_sd["digest"][k]
-        assert float(v.double().sum()) == s and float(v.double().abs().sum()) == a, k
+    assert len(sd) == 343
+    _assert_reference_init(sd, "state_dict_seed0_lora.json")
     assert float(sd["lora_layers.0.lora_B"].abs().sum()) == 0.0
     gold = np.load(os.path.join(GOLD, "lora.npz"))
     torch.manual_seed(11)
