@@ -36,7 +36,7 @@ class HeadsInputs(C.Structure):
     _fields_ = [("tokens", C.c_void_p), ("tokens_per_img", C.c_int), ("focal_feat", C.c_void_p),
                 ("pool_partial", C.c_void_p), ("pool_splits", C.c_int), ("tmp_w", C.c_void_p), ("tmp_b", C.c_void_p),
                 ("pooled_out", C.c_void_p), ("exif", C.c_void_p), ("camera_idx", C.c_void_p),
-                ("num_cameras", C.c_int), ("fault", C.c_void_p)]
+                ("num_cameras", C.c_int), ("fault", C.c_void_p), ("sweep_images", C.c_int)]
 
 
 class FocalValueArgs(C.Structure):
@@ -92,6 +92,16 @@ class ForwardCall(C.Structure):
                 ("use_graph", C.c_int)]
 
 
+SWEEP_MAX_K = 16  # CA_SWEEP_MAX_K (include/cogaim_b200.h)
+
+
+class SweepCall(C.Structure):
+    """ca_sweep_call (include/cogaim_b200.h)."""
+    _fields_ = [("K", C.c_int), ("instructions", C.POINTER(C.c_char_p)), ("masks", C.c_void_p), ("tmp_w", C.c_void_p),
+                ("tmp_b", C.c_void_p), ("eps", C.c_void_p), ("noise", C.c_void_p), ("depth", C.c_void_p),
+                ("conf", C.c_void_p), ("attention", C.c_void_p), ("argmax", C.c_void_p)]
+
+
 # name -> (argtypes); every function returns int status except where noted
 _SIGNATURES = {
     "ca_version": [],
@@ -127,12 +137,17 @@ _SIGNATURES = {
     "ca_focus_map": [c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr],
     "ca_guided_softmax": [c_ptr, c_ptr, C.c_longlong, c_ptr, c_ptr, C.c_int, C.c_int, C.c_float, C.c_float, c_ptr],
     "ca_weighted_pool": [c_ptr, C.c_longlong, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr],
+    "ca_guided_softmax_sweep": [c_ptr, C.c_longlong, c_ptr, C.c_longlong, C.c_longlong, c_ptr, c_ptr, C.c_int, C.c_int,
+                                C.c_int, C.c_float, C.c_float, c_ptr],
+    "ca_weighted_pool_sweep": [c_ptr, C.c_longlong, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                               c_ptr],
     "ca_heads": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, c_ptr, C.c_int, c_ptr],
     "ca_focal_value": [C.POINTER(FocalValueArgs), C.c_int, c_ptr],
     "ca_focal_fusion": [c_ptr, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr],
     "ca_create": [C.POINTER(C.c_void_p), C.POINTER(ModelWeights), C.c_int],
     "ca_destroy": [c_ptr],
     "ca_forward_guided": [c_ptr, C.POINTER(ForwardCall), c_ptr],
+    "ca_forward_guided_sweep": [c_ptr, C.POINTER(ForwardCall), C.POINTER(SweepCall), c_ptr],
     "ca_forward": [c_ptr, C.POINTER(ForwardCall), c_ptr],
     "ca_backbone": [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr],
     "ca_last_launch_count": [c_ptr],

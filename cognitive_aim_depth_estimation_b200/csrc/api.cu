@@ -187,6 +187,19 @@ int ca_weighted_pool(const float* src, long long src_batch_stride, int row_offse
                                   static_cast<cudaStream_t>(stream));
 }
 
+int ca_guided_softmax_sweep(const float* base, long long base_k_stride, const float* mask, long long mask_k_stride,
+                            long long mask_batch_stride, float* heat, int32_t* argmax, int K, int B, int N, float alpha,
+                            float temperature, void* stream) {
+  return ca::guided_softmax_sweep_launch(base, base_k_stride, mask, mask_k_stride, mask_batch_stride, heat, argmax, K, B, N,
+                                         alpha, temperature, static_cast<cudaStream_t>(stream));
+}
+
+int ca_weighted_pool_sweep(const float* src, long long src_batch_stride, int row_offset, const float* w, float* partial,
+                           int K, int B, int N, int D, int splits, void* stream) {
+  return ca::weighted_pool_sweep_launch(src, src_batch_stride, row_offset, w, partial, K, B, N, D, splits,
+                                        static_cast<cudaStream_t>(stream));
+}
+
 int ca_heads(const ca_heads_weights* w, const ca_heads_inputs* in, float* depth, float* conf, float* fused_out, int B,
              void* stream) {
   if (!w || !in) return ca::invalid("heads: null argument struct");

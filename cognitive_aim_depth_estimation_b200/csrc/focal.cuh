@@ -17,4 +17,12 @@ int guided_softmax_launch(const float* base, const float* mask, long long mask_b
 int weighted_pool_launch(const float* src, long long src_batch_stride, int row_offset, const float* w, const float* w2,
                          float* partial, int B, int N, int D, int splits, cudaStream_t stream);
 
+// Instruction sweeps (include/cogaim_b200.h, CA_SWEEP_MAX_K): K guidance rows per image in one launch.
+constexpr int kSweepMaxK = 16;
+int guided_softmax_sweep_launch(const float* base, long long base_k_stride, const float* mask, long long mask_k_stride,
+                                long long mask_batch_stride, float* heat, int* argmax, int K, int B, int N, float alpha,
+                                float temperature, cudaStream_t stream);
+int weighted_pool_sweep_launch(const float* src, long long src_batch_stride, int row_offset, const float* w, float* partial,
+                               int K, int B, int N, int D, int splits, cudaStream_t stream);
+
 }  // namespace ca

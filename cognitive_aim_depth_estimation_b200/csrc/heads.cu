@@ -21,7 +21,11 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_kernel(const HeadsWeights
   __shared__ __align__(16) float s_b[256];
   __shared__ __align__(16) float s_cat[192];
   __shared__ __align__(16) float s_f[192];
-  const int b = blockIdx.x;
+  // r: output row; b: image.  In an instruction sweep r = k * B + b (k = call, sweep_images = B), otherwise r = b.
+  const int r = blockIdx.x;
+  const int nb = in.sweep_images > 0 ? in.sweep_images : gridDim.x;
+  const int b = r % nb;
+  const size_t k = r / nb;
   const int tid = threadIdx.x;
 
   // ---- ambient stream on the CLS token ----
@@ -40,12 +44,12 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_kernel(const HeadsWeights
     for (int i = tid; i < 768; i += kHeadsThreads) {
       float acc = 0.f;
       for (int s = 0; s < in.pool_splits; ++s)
-        acc += in.pool_partial[(static_cast<size_t>(b) * in.pool_splits + s) * 768 + i];
+        acc += in.pool_partial[(static_cast<size_t>(r) * in.pool_splits + s) * 768 + i];
       s_in[i] = acc;
-      if (in.pooled_out) in.pooled_out[static_cast<size_t>(b) * 768 + i] = acc;
+      if (in.pooled_out) in.pooled_out[static_cast<size_t>(r) * 768 + i] = acc;
     }
     __syncthreads();
-    dense(in.tmp_w, in.tmp_b, s_in, s_cat + 64, 768, 64, false);
+    dense(in.tmp_w + k * 64 * 768, in.tmp_b + k * 64, s_in, s_cat + 64, 768, 64, false);
   }
 
   // ---- EXIF prior (zero slot when EXIF is absent: the reference zero-pads, src/model.py:1035-1039) ----
@@ -78,7 +82,7 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_kernel(const HeadsWeights
   // ---- fusion + heads ----
   dense(wt.fus_w, wt.fus_b, s_cat, s_f, 192, 192, true);
   if (fused_out)
-    for (int i = tid; i < 192; i += kHeadsThreads) fused_out[static_cast<size_t>(b) * 192 + i] = s_f[i];
+    for (int i = tid; i < 192; i += kHeadsThreads) fused_out[static_cast<size_t>(r) * 192 + i] = s_f[i];
   if (warp_id() < 2) {
     const float* w = warp_id() == 0 ? wt.dec_w : wt.conf_w0;
     float acc = 0.f;
@@ -87,11 +91,11 @@ __global__ void __launch_bounds__(kHeadsThreads) heads_kernel(const HeadsWeights
     if (lane_id() == 0) {
       if (warp_id() == 0) {
         const float z = acc + wt.dec_b[0];
-        depth[b] = z > 20.0f ? z : log1pf(expf(z));  // Softplus(beta=1, threshold=20)
+        depth[r] = z > 20.0f ? z : log1pf(expf(z));  // Softplus(beta=1, threshold=20)
       } else {
         const float c = fmaxf(acc + wt.conf_b0[0], 0.f);
         const float z = c * wt.conf_w2[0] + wt.conf_b2[0];
-        conf[b] = 1.0f / (1.0f + expf(-z));
+        conf[r] = 1.0f / (1.0f + expf(-z));
       }
     }
   }
@@ -147,6 +151,8 @@ int heads_launch(const HeadsWeights& w, const HeadsInputs& in, float* depth, flo
   CA_REQUIRE(in.focal_feat || (in.pool_partial && in.tmp_w && in.tmp_b && in.pool_splits > 0),
              "heads: neither focal features nor pooled partials + projection given");
   CA_REQUIRE(in.exif == nullptr || in.camera_idx != nullptr, "heads: EXIF given without camera_idx");
+  CA_REQUIRE(in.sweep_images >= 0 && (in.sweep_images == 0 || (in.focal_feat == nullptr && B % in.sweep_images == 0)),
+             "heads: an instruction sweep is guided only and needs B = K * sweep_images rows");
   CA_TRY(launch_kernel(heads_kernel, dim3(B), dim3(kHeadsThreads), 0, stream, w, in, depth, conf, fused_out));
   CA_CUDA(cudaGetLastError());
   return 0;

@@ -54,7 +54,21 @@ struct Workspace {
   int P = 0, lde = 0;
   std::map<int, std::pair<cudaGraphExec_t, int>> graphs;  // path key -> (executable graph, launches)
   std::map<int, int> seen;                                // path key -> calls so far
+  // instruction sweeps: the per-call buffers of K calls (rows k * B + b), one arena per K; the backbone and focal
+  // buffers above are shared with the single-call paths
+  struct Sweep {
+    void* arena = nullptr;
+    float *mask_in, *heat, *pool, *depth, *conf, *tmpw, *tmpb, *cur_eps, *cur_noise, *cur_raw, *cur_reward;
+    int* argmax;
+  };
+  std::map<int, Sweep> sweeps;  // K -> buffers
 };
+
+void free_workspace(Workspace& w) {
+  for (auto& g : w.graphs) cudaGraphExecDestroy(g.second.first);
+  for (auto& s : w.sweeps) cudaFree(s.second.arena);
+  cudaFree(w.arena);
+}
 
 struct PinnedSlot {
   float* buf = nullptr;
@@ -253,8 +267,7 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   }
   if (h->ws.size() >= 4) {  // keep the cache bounded: drop the oldest entry
     auto old = h->ws.begin();
-    for (auto& g : old->second.graphs) cudaGraphExecDestroy(g.second.first);
-    cudaFree(old->second.arena);
+    free_workspace(old->second);
     h->ws.erase(old);
   }
   Workspace w;
@@ -316,6 +329,38 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   CA_CUDA(cudaMemset(w.exif_in, 0, B * 3 * 4));
   CA_CUDA(cudaMemset(w.cam_in, 0, B * 8));
   *out = &h->ws.emplace(key, w).first->second;
+  return 0;
+}
+
+int get_sweep(Workspace& w, int K, Workspace::Sweep** out) {
+  auto it = w.sweeps.find(K);
+  if (it == w.sweeps.end()) {
+    const int g = w.S / 14;
+    const size_t N = static_cast<size_t>(g) * g, KB = static_cast<size_t>(K) * w.B;
+    size_t off = 0;
+    std::vector<std::pair<void**, size_t>> slots;
+    Workspace::Sweep s;
+    auto want = [&](auto** p, size_t bytes) {
+      slots.push_back({reinterpret_cast<void**>(p), off});
+      off += (bytes + 255) & ~static_cast<size_t>(255);
+    };
+    want(&s.mask_in, K * N * 4);
+    want(&s.heat, KB * N * 4);
+    want(&s.argmax, KB * 4);
+    want(&s.pool, KB * kPoolSplits * kD * 4);
+    want(&s.depth, KB * 4);
+    want(&s.conf, KB * 4);
+    want(&s.tmpw, static_cast<size_t>(K) * 64 * kD * 4);
+    want(&s.tmpb, static_cast<size_t>(K) * 64 * 4);
+    want(&s.cur_eps, KB * 192 * 4);
+    want(&s.cur_noise, KB * kD * 4);
+    want(&s.cur_raw, KB * 4);
+    want(&s.cur_reward, KB * 4);
+    CA_CUDA(cudaMalloc(&s.arena, off));
+    for (auto& sl : slots) *sl.first = static_cast<char*>(s.arena) + sl.second;
+    it = w.sweeps.emplace(K, s).first;
+  }
+  *out = &it->second;
   return 0;
 }
 
@@ -480,14 +525,16 @@ int focal_iterations(ca_handle* h, Workspace& w, const Tables& tb, bool want_fea
 // CuriosityModule runs of one call on the side stream (forked here, joined by curiosity_join): output-dead under the
 // shipped configurations and latency-bound, so it runs under the focal stream's GEMMs.  The fork / join are stream
 // dependencies: during capture they become a parallel branch of the graph.
-int curiosity_fork(ca_handle* h, Workspace& w, int runs, cudaStream_t st) {
+// eps / noise / raw / reward: [runs, B, ...] buffers of the runs (the workspace's, or an instruction sweep's).
+int curiosity_fork(ca_handle* h, Workspace& w, int runs, const float* eps, const float* noise, float* raw, float* reward,
+                   cudaStream_t st) {
   const int B = w.B, g = w.S / 14, T = g * g + 1;
   CA_CUDA(cudaEventRecord(h->fork, st));
   CA_CUDA(cudaStreamWaitEvent(h->side, h->fork, 0));
   for (int j = 0; j < runs; ++j) {
-    CA_TRY(ca::curiosity_launch(h->w.curiosity, w.tokens, T, w.cur_eps + static_cast<size_t>(j) * B * 192,
-                                w.cur_noise + static_cast<size_t>(j) * B * kD, w.cur_raw + static_cast<size_t>(j) * B,
-                                w.cur_reward + static_cast<size_t>(j) * B, h->w.exploration_history, h->w.history_len,
+    CA_TRY(ca::curiosity_launch(h->w.curiosity, w.tokens, T, eps + static_cast<size_t>(j) * B * 192,
+                                noise + static_cast<size_t>(j) * B * kD, raw + static_cast<size_t>(j) * B,
+                                reward + static_cast<size_t>(j) * B, h->w.exploration_history, h->w.history_len,
                                 h->w.history_pointer, B, h->side));
     h->launches += h->w.exploration_history ? 2 : 1;
   }
@@ -523,10 +570,8 @@ int heads(ca_handle* h, Workspace& w, bool guided, bool has_exif, int* fault, cu
 }
 
 // per-call HOST inputs -> pinned staging slot -> fixed device buffers (SM-side reads of the pinned memory)
-int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, bool guided, int runs, cudaStream_t st) {
-  const size_t B = w.B;
-  const size_t n_w = guided ? 64 * kD + 64 : 0;
-  const size_t need = n_w + static_cast<size_t>(runs) * B * (192 + kD);
+// next slot of the pinned ring, holding at least `need` floats
+int pinned_slot(ca_handle* h, size_t need, PinnedSlot** out) {
   PinnedSlot& s = h->ring[h->ring_next];
   h->ring_next = (h->ring_next + 1) % 4;
   if (s.done) CA_CUDA(cudaEventSynchronize(s.done));  // the reads of four calls ago (normally long finished)
@@ -536,6 +581,17 @@ int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, bool
     s.cap = need;
   }
   if (!s.done) CA_CUDA(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+  *out = &s;
+  return 0;
+}
+
+int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, bool guided, int runs, cudaStream_t st) {
+  const size_t B = w.B;
+  const size_t n_w = guided ? 64 * kD + 64 : 0;
+  const size_t need = n_w + static_cast<size_t>(runs) * B * (192 + kD);
+  PinnedSlot* sp = nullptr;
+  CA_TRY(pinned_slot(h, need, &sp));
+  PinnedSlot& s = *sp;
   float* p = s.buf;
   if (guided) {
     memcpy(p, c.tmp_w, 64 * kD * sizeof(float));
@@ -551,6 +607,26 @@ int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, bool
   CA_TRY(ca::fetch_pinned_launch(w.cur_noise, p + static_cast<size_t>(runs) * B * 192, static_cast<size_t>(runs) * B * kD, st));
   h->launches += 2;
   CA_CUDA(cudaEventRecord(s.done, st));
+  return 0;
+}
+
+// the K calls' projections and curiosity draws (HOST) -> one pinned slot sized for K -> the sweep's device buffers
+int stage_sweep_inputs(ca_handle* h, Workspace& w, Workspace::Sweep& s, const ca_sweep_call& c, cudaStream_t st) {
+  const size_t K = c.K, B = w.B;
+  const size_t n_tw = K * 64 * kD, n_tb = K * 64, n_eps = K * B * 192, n_noise = K * B * kD;
+  PinnedSlot* slot = nullptr;
+  CA_TRY(pinned_slot(h, n_tw + n_tb + n_eps + n_noise, &slot));
+  float* p = slot->buf;
+  memcpy(p, c.tmp_w, n_tw * sizeof(float));
+  memcpy(p + n_tw, c.tmp_b, n_tb * sizeof(float));
+  memcpy(p + n_tw + n_tb, c.eps, n_eps * sizeof(float));
+  memcpy(p + n_tw + n_tb + n_eps, c.noise, n_noise * sizeof(float));
+  CA_TRY(ca::fetch_pinned_launch(s.tmpw, p, n_tw, st));
+  CA_TRY(ca::fetch_pinned_launch(s.tmpb, p + n_tw, n_tb, st));
+  CA_TRY(ca::fetch_pinned_launch(s.cur_eps, p + n_tw + n_tb, n_eps, st));
+  CA_TRY(ca::fetch_pinned_launch(s.cur_noise, p + n_tw + n_tb + n_eps, n_noise, st));
+  h->launches += 4;
+  CA_CUDA(cudaEventRecord(slot->done, st));
   return 0;
 }
 
@@ -648,10 +724,7 @@ int ca_destroy(ca_handle* h) {
   if (!h) return 0;
   DeviceGuard guard(h->device);
   cudaDeviceSynchronize();
-  for (auto& kv : h->ws) {
-    for (auto& g : kv.second.graphs) cudaGraphExecDestroy(g.second.first);
-    cudaFree(kv.second.arena);
-  }
+  for (auto& kv : h->ws) free_workspace(kv.second);
   for (auto& kv : h->tables) {
     cudaFree(kv.second.pos);
     cudaFree(kv.second.pe);
@@ -724,7 +797,7 @@ int ca_forward_guided(ca_handle* h, const ca_forward_call* c, void* stream) {
   const int key = 100 + (mstride ? 1 : 0);
   CA_TRY(run_sequence(h, w, key, c->use_graph != 0, st, [&]() -> int {
     CA_TRY(backbone_layers(h, w, *tb, st));
-    CA_TRY(curiosity_fork(h, w, 1, st));
+    CA_TRY(curiosity_fork(h, w, 1, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st));
     float* base = nullptr;
     CA_TRY(focal_iterations(h, w, *tb, false, st, &base));
     LAUNCH(ca::guided_softmax_launch(base, w.mask_in, mstride ? N : 0, w.heat, w.argmax, B, N, 0.7f, 0.05f, st));
@@ -737,6 +810,84 @@ int ca_forward_guided(ca_handle* h, const ca_forward_call* c, void* stream) {
   CA_CUDA(cudaMemcpyAsync(c->conf, w.conf, B * 4, cudaMemcpyDeviceToDevice, st));
   CA_CUDA(cudaMemcpyAsync(c->attention, w.heat, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
   if (c->argmax) CA_CUDA(cudaMemcpyAsync(c->argmax, w.argmax, B * 4, cudaMemcpyDeviceToDevice, st));
+  h->last_launches = h->launches;
+  return 0;
+}
+
+int ca_forward_guided_sweep(ca_handle* h, const ca_forward_call* c, const ca_sweep_call* sw, void* stream) {
+  CA_REQUIRE(h && c && sw, "forward_guided_sweep: null handle / call / sweep");
+  CA_REQUIRE(c->images && c->B > 0, "forward_guided_sweep: null images or empty batch");
+  CA_REQUIRE(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260,
+             "forward_guided_sweep: image side must be a multiple of 14 in [56, 1260]");
+  CA_REQUIRE(c->exif && c->camera_idx, "forward_guided_sweep: EXIF inputs are required (without them the reference falls "
+                                       "back to forward(): call ca_forward)");
+  CA_REQUIRE(!c->instruction && !c->mask && !c->tmp_w && !c->tmp_b && !c->eps && !c->noise && !c->depth && !c->conf &&
+                 !c->attention && !c->argmax && !c->fused,
+             "forward_guided_sweep: the per-call fields of ca_forward_call must be NULL (they go in ca_sweep_call)");
+  const int K = sw->K;
+  CA_REQUIRE(K >= 1 && K <= CA_SWEEP_MAX_K, "forward_guided_sweep: K must be in 1..CA_SWEEP_MAX_K (16)");
+  CA_REQUIRE((sw->instructions != nullptr) != (sw->masks != nullptr), "forward_guided_sweep: give instructions OR masks");
+  if (sw->instructions)
+    for (int k = 0; k < K; ++k) CA_REQUIRE(sw->instructions[k], "forward_guided_sweep: null instruction string");
+  CA_REQUIRE(sw->tmp_w && sw->tmp_b && sw->eps && sw->noise,
+             "forward_guided_sweep: null per-call projections or CuriosityModule draws (HOST pointers)");
+  CA_REQUIRE(sw->depth && sw->conf && sw->attention, "forward_guided_sweep: null output");
+  DeviceGuard guard(h->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int B = c->B, S = c->S, g = S / 14, N = g * g, T = N + 1;
+  Workspace* wp = nullptr;
+  Tables* tb = nullptr;
+  Workspace::Sweep* sp = nullptr;
+  CA_TRY(get_workspace(h, B, S, &wp));
+  CA_TRY(get_tables(h, g, &tb));
+  Workspace& w = *wp;
+  CA_TRY(get_sweep(w, K, &sp));
+  Workspace::Sweep& s = *sp;
+  h->launches = 0;
+  // mask set [K, N], one row per call, shared by the batch (mask stride per image 0)
+  if (sw->instructions) {
+    for (int k = 0; k < K; ++k) {
+      float* m = nullptr;
+      CA_TRY(get_mask(tb, sw->instructions[k], g, &m));
+      CA_CUDA(cudaMemcpyAsync(s.mask_in + static_cast<size_t>(k) * N, m, static_cast<size_t>(N) * 4, cudaMemcpyDeviceToDevice, st));
+    }
+  } else {
+    CA_CUDA(cudaMemcpyAsync(s.mask_in, sw->masks, static_cast<size_t>(K) * N * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  CA_TRY(stage_sweep_inputs(h, w, s, *sw, st));
+  CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
+  CA_TRY(patch_rows(h, w, c->images, c->images_u8, st));
+  int* fault = c->fault;
+  CA_TRY(run_sequence(h, w, 300 + K, c->use_graph != 0, st, [&]() -> int {
+    CA_TRY(backbone_layers(h, w, *tb, st));
+    CA_TRY(curiosity_fork(h, w, K, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st));
+    float* base = nullptr;
+    CA_TRY(focal_iterations(h, w, *tb, false, st, &base));  // shared by the K calls: it does not read the instruction
+    LAUNCH(ca::guided_softmax_sweep_launch(base, 0, s.mask_in, N, 0, s.heat, s.argmax, K, B, N, 0.7f, 0.05f, st));
+    LAUNCH(ca::weighted_pool_sweep_launch(w.tokens, static_cast<long long>(T) * kD, 1, s.heat, s.pool, K, B, N, kD,
+                                          kPoolSplits, st));
+    ca_heads_inputs in{};
+    in.tokens = w.tokens;
+    in.tokens_per_img = T;
+    in.pool_partial = s.pool;
+    in.pool_splits = kPoolSplits;
+    in.tmp_w = s.tmpw;
+    in.tmp_b = s.tmpb;
+    in.exif = w.exif_in;
+    in.camera_idx = w.cam_in;
+    in.num_cameras = h->w.num_cameras;
+    in.fault = fault;
+    in.sweep_images = B;
+    LAUNCH(ca::heads_launch(h->w.heads, in, s.depth, s.conf, nullptr, K * B, st));
+    CA_TRY(curiosity_join(h, st));
+    return 0;
+  }));
+  const size_t KB = static_cast<size_t>(K) * B;
+  CA_CUDA(cudaMemcpyAsync(sw->depth, s.depth, KB * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(sw->conf, s.conf, KB * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(sw->attention, s.heat, KB * N * 4, cudaMemcpyDeviceToDevice, st));
+  if (sw->argmax) CA_CUDA(cudaMemcpyAsync(sw->argmax, s.argmax, KB * 4, cudaMemcpyDeviceToDevice, st));
   h->last_launches = h->launches;
   return 0;
 }
@@ -767,7 +918,7 @@ int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
   const int key = 200 + (has_exif ? 1 : 0) + 2 * runs;
   CA_TRY(run_sequence(h, w, key, c->use_graph != 0, st, [&]() -> int {
     CA_TRY(backbone_layers(h, w, *tb, st));
-    CA_TRY(curiosity_fork(h, w, runs, st));
+    CA_TRY(curiosity_fork(h, w, runs, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st));
     CA_TRY(focal_iterations(h, w, *tb, true, st, &att));
     CA_TRY(heads(h, w, false, has_exif, fault, st));
     CA_TRY(curiosity_join(h, st));

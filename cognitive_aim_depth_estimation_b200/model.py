@@ -29,6 +29,7 @@ import torch
 import torch.nn as nn
 
 from . import ops, tables
+from ._lib import SWEEP_MAX_K as _SWEEP_MAX_K  # instructions per sweep: the sweep pool keeps one accumulator each
 from .config import DEFAULT_COGNITIVE_MODULES, EffectiveConfig, effective_config
 from .init import reference_init_
 
@@ -873,6 +874,133 @@ class CognitiveAimModel(nn.Module):
         self._last_argmax = ws["argmax"].clone()
         self._last_curiosity = ws["cur_reward"][0]
         depth, conf = ws["depth"].clone().unsqueeze(1), ws["conf"].clone().unsqueeze(1)
+        return (depth, conf, heat) if return_attention else (depth, conf)
+
+    def _sweep_draws(self, B: int, K: int):
+        """The host-side random draws of K successive guided calls, in the reference's order per call: the
+        CuriosityModule's randn(B,192), randn(B,768) (src/model.py:609,744), then the fresh nn.Linear(768, 64) (:1421).
+        Returns K tuples (eps [B,192], noise [B,768], projection weight [64,768], projection bias [64])."""
+        out = []
+        for _ in range(K):
+            eps, noise = self._curiosity_draw(B)
+            tmp = nn.Linear(_D, 64)
+            out.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
+        return out
+
+    def _sweep_buffers(self, ws, B: int, S: int, K: int):
+        """Per-call buffers of a K-instruction sweep (rows k * B + b), kept with the (B, S) workspace whose backbone and
+        focal buffers the sweep shares."""
+        sweeps = ws.setdefault("sweeps", {})
+        sw = sweeps.get(K)
+        if sw is None:
+            dev = self._device()
+            N = (S // 14) ** 2
+            fl = dict(device=dev, dtype=torch.float32)
+            iters = self.cfg.num_iterations
+            sw = {
+                "mask_in": torch.empty(K, B, N, **fl), "heat": torch.empty(K, B, N, **fl),
+                "argmax": torch.empty(K, B, device=dev, dtype=torch.int32),
+                "pool": torch.empty(K * B, _POOL_SPLITS, _D, **fl),
+                "depth": torch.empty(K, B, **fl), "conf": torch.empty(K, B, **fl),
+                "tmpw": torch.empty(K, 64, _D, **fl), "tmpb": torch.empty(K, 64, **fl),
+                "cur_eps": torch.zeros(K, B, 192, **fl), "cur_noise": torch.zeros(K, B, _D, **fl),
+                "cur_raw": torch.empty(K, B, **fl), "cur_reward": torch.empty(K, B, **fl),
+                "cur_weight": torch.empty(K, iters, B, **fl),
+                # curiosity-guided attention: one focal pass per call, its last-iteration attention kept per call
+                "base": torch.empty(K, B, N, **fl) if self.cfg.curiosity_guided else None,
+            }
+            if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
+                for t in sw.values():
+                    if torch.is_tensor(t) and t.is_floating_point():
+                        t.fill_(float("nan"))
+            sweeps[K] = sw
+        # the single-call buffers (tokens, focal workspace, EXIF, graphs) come from ws; the per-call ones from sw
+        return {**ws, **sw}
+
+    def _stage_sweep(self, sw, slot, draws, B: int, K: int):
+        """The K calls' draws -> pinned staging sized for (B, K) -> the sweep's device buffers (as _stage_draws)."""
+        bufs = slot.setdefault("sweep", {}).get((B, K))
+        if bufs is None:
+            bufs = slot["sweep"][(B, K)] = tuple(torch.empty(*s).pin_memory() for s in
+                                                 ((K, B, 192), (K, B, _D), (K, 64, _D), (K, 64)))
+        for k, d in enumerate(draws):
+            for buf, t in zip(bufs, d):
+                buf[k].copy_(t)
+        for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb"), bufs):
+            ops.fetch_pinned(sw[dst], buf)
+
+    @torch.no_grad()
+    @_on_own_device
+    def forward_with_guidance_sweep(self, images, exif_data, guidances, return_attention=False):
+        """K = len(guidances) guided calls over one batch in one pass: bit-identical to
+        `[forward_with_guidance(images, exif_data, g) for g in guidances]` from the same global-RNG state — outputs,
+        generator state, CuriosityModule ring buffer and `_last_*` state — with the backbone and (unless curiosity-guided
+        attention is enabled) the focal iterations run once instead of K times.  Each entry is what `attention_guidance`
+        accepts: an instruction string or alias, a guidance tensor [N'], or a list of B per-image instructions.
+        Returns depth [K, B, 1], confidence [K, B, 1] (and the heat maps [K, B, N] with `return_attention`)."""
+        self._raise_on_fault()
+        if not isinstance(guidances, (list, tuple)):
+            raise ValueError("guidances must be a list of K instructions / guidance tensors / per-image lists")
+        K = len(guidances)
+        if not 1 <= K <= _SWEEP_MAX_K:
+            raise ValueError(f"an instruction sweep takes 1..{_SWEEP_MAX_K} guidances, got {K}")
+        if any(gd is None for gd in guidances):
+            raise ValueError("a None guidance runs the un-guided focal path (src/model.py:1206-1212): use "
+                             "forward_with_guidance for it")
+        if exif_data is None or not self.use_exif:
+            raise ValueError("an instruction sweep needs EXIF data and a model with the EXIF prior (otherwise the "
+                             "reference falls back to forward(): use forward_with_guidance)")
+        B, S = self._check_images(images)
+        pk = self._pack()
+        g = S // 14
+        N, T = g * g, g * g + 1
+        masks = []
+        for gd in guidances:
+            m = self._mask(gd, g)
+            if m.dim() == 2 and m.shape[0] != B:
+                raise ValueError(f"{m.shape[0]} per-image instructions for a batch of {B}")
+            masks.append(m.expand(B, N))
+        mask = torch.stack(masks)  # [K, B, N]: strings and [N] guidance broadcast over the batch
+        exif, cam = self._exif_tensors(exif_data, B)
+        draws = self._sweep_draws(B, K)
+        ws = self._workspace(B, S)
+        sw = self._sweep_buffers(ws, B, S, K)
+        slot = self._pinned_slot()
+        self._stage_sweep(sw, slot, draws, B, K)
+        slot["event"].record()
+        sw["mask_in"].copy_(mask, non_blocking=True)
+        ws["exif_in"].copy_(exif, non_blocking=True)
+        ws["cam_in"].copy_(cam, non_blocking=True)
+        self._grid_tables(g)
+        patches, images = self._patch_rows(images, ws, S)
+        cg = self.cfg.curiosity_guided
+
+        def device_pass():
+            self._backbone_layers(ws, patches, B, S)
+            self._curiosity_runs(sw, B, T, ("guided",) * K)
+            if cg:
+                # each call's focal attention is modulated by its own curiosity score (src/model.py:264-276)
+                for k in range(K):
+                    sw["base"][k].copy_(self._focal_iterations(ws, B, g, want_features=False, cur_weight=sw["cur_weight"][k]))
+                base, base_k_stride = sw["base"], B * N
+            else:
+                base, base_k_stride = self._focal_iterations(ws, B, g, want_features=False), 0
+            ops.guided_softmax_sweep(base, base_k_stride, sw["mask_in"], sw["heat"], sw["argmax"], K, B, N)
+            ops.weighted_pool_sweep(ws["tokens"], T * _D, 1, sw["heat"], sw["pool"], K, B, N, _D, _POOL_SPLITS)
+            ops.heads(pk["heads"], tokens=ws["tokens"], tokens_per_img=T, depth=sw["depth"], conf=sw["conf"], B=K * B,
+                      pool_partial=sw["pool"], pool_splits=_POOL_SPLITS, tmp_w=sw["tmpw"], tmp_b=sw["tmpb"],
+                      exif=ws["exif_in"], camera_idx=ws["cam_in"], num_cameras=self.cfg.num_cameras,
+                      fault_ptr=self._fault_word().data_ptr(), sweep_images=B)
+            self._curiosity_join()
+
+        self._run(ws, ("sweep", K, self._curiosity_key()), device_pass)
+        self._keepalive = (exif, cam, mask, images)
+        heat = sw["heat"].clone()
+        # what the last of the K calls leaves behind
+        self._last_attention_weights = heat[K - 1]
+        self._last_argmax = sw["argmax"][K - 1].clone()
+        self._last_curiosity = sw["cur_reward"][K - 1]
+        depth, conf = sw["depth"].clone().unsqueeze(-1), sw["conf"].clone().unsqueeze(-1)
         return (depth, conf, heat) if return_attention else (depth, conf)
 
     @torch.no_grad()

@@ -198,6 +198,47 @@ class NativeModel:
         return out["depth"].unsqueeze(1), out["conf"].unsqueeze(1), out["heat"], out["argmax"]
 
     @torch.no_grad()
+    def forward_with_guidance_sweep(self, images, exif, guidances):
+        """K = len(guidances) `forward_with_guidance` calls in one native call (ca_forward_guided_sweep): the backbone and
+        the focal pass run once.  `guidances`: K instruction strings, or K guidance tensors [N].  Draws the K calls'
+        random numbers in the reference's order per call.  -> depth [K,B,1], confidence [K,B,1], heat maps [K,B,N],
+        arg-max cells [K,B]."""
+        K = len(guidances)
+        if not 1 <= K <= _lib.SWEEP_MAX_K:
+            raise ValueError(f"an instruction sweep takes 1..{_lib.SWEEP_MAX_K} guidances, got {K}")
+        c, held, B, S = self._call(images, exif)
+        N = (S // 14) ** 2
+        s = _lib.SweepCall()
+        s.K = K
+        if all(isinstance(g, str) for g in guidances):
+            names = (C.c_char_p * K)(*[g.encode() for g in guidances])
+            held.append(names)
+            s.instructions = C.cast(names, C.POINTER(C.c_char_p))
+        elif all(torch.is_tensor(g) and g.dim() == 1 and g.numel() == N for g in guidances):
+            m = torch.stack([g.to(self.device, torch.float32) for g in guidances]).contiguous()
+            held.append(m)
+            s.masks = m.data_ptr()
+        else:
+            raise ValueError(f"guidances must be K instruction strings or K guidance tensors of length {N}")
+        draws = []
+        for _ in range(K):
+            eps, noise = torch.randn(B, 192), torch.randn(B, _D)   # :609, :744 of call k
+            tmp = nn.Linear(_D, 64)                                # :1421 of call k
+            draws.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
+        eps, noise, tw, tb = (torch.stack([d[i] for d in draws]).contiguous() for i in range(4))
+        held += [eps, noise, tw, tb]
+        s.tmp_w, s.tmp_b, s.eps, s.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
+        out = {"depth": torch.empty(K, B, device=self.device), "conf": torch.empty(K, B, device=self.device),
+               "heat": torch.empty(K, B, N, device=self.device),
+               "argmax": torch.empty(K, B, device=self.device, dtype=torch.int32)}
+        s.depth, s.conf, s.attention, s.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ca_forward_guided_sweep(self._h, C.byref(c), C.byref(s), self._stream()),
+                       "ca_forward_guided_sweep")
+        self._held = held
+        return out["depth"].unsqueeze(-1), out["conf"].unsqueeze(-1), out["heat"], out["argmax"]
+
+    @torch.no_grad()
     def forward(self, images, exif: Optional[dict] = None, runs: int = 1):
         """-> depth [B,1], confidence [B,1], focal attention [B,N], fusion features [B,192] (src/model.py:1064-1155).
         `runs`: how often the reference would run its CuriosityModule in this call (1..3, :992, :1104, :1138)."""

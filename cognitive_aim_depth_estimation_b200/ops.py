@@ -300,6 +300,29 @@ def weighted_pool(src, src_batch_stride, row_offset, w, w2, partial, B, N, D, sp
     _end(e0, "pool", 1, float(B * N * D * 4))
 
 
+def guided_softmax_sweep(base, base_k_stride, mask, heat, argmax, K, B, N, alpha=0.7, temperature=0.05):
+    """K * B rows of `guided_softmax` (instruction sweep): mask [K, B, N], heat [K, B, N], argmax [K, B]; row k * B + b
+    reads base + k * base_k_stride + b * N (base_k_stride 0: one base attention [B, N] shared by every instruction)."""
+    _req(base, torch.float32, "base")
+    _req(mask, torch.float32, "mask")
+    _req(heat, torch.float32, "heat")
+    _req(argmax, torch.int32, "argmax")
+    if mask.shape != (K, B, N) or not mask.is_contiguous():
+        raise ValueError(f"sweep mask must be a contiguous [K, B, N] = [{K}, {B}, {N}] tensor, got {tuple(mask.shape)}")
+    e0 = _begin()
+    check(_lib.load().ca_guided_softmax_sweep(ptr(base), base_k_stride, ptr(mask), B * N, N, ptr(heat), ptr(argmax), K, B,
+                                              N, alpha, temperature, stream_ptr()), "ca_guided_softmax_sweep")
+    _end(e0, "small", 1)
+
+
+def weighted_pool_sweep(src, src_batch_stride, row_offset, w, partial, K, B, N, D, splits):
+    """`weighted_pool` for K weight vectors w [K, B, N] at once: partial [K * B, splits, D], the tokens read once."""
+    e0 = _begin()
+    check(_lib.load().ca_weighted_pool_sweep(ptr(src), src_batch_stride, row_offset, ptr(w), ptr(partial), K, B, N, D,
+                                             splits, stream_ptr()), "ca_weighted_pool_sweep")
+    _end(e0, "pool", 1, float(B * N * D * 4))
+
+
 def resize_u8(src, out_h, out_w):
     """uint8 [B, H0, W0, 3] -> uint8 [B, out_h, out_w, 3], bit-exact PIL.Image.resize(..., BILINEAR) (csrc/resize.cu)."""
     _req(src, torch.uint8, "src")
@@ -402,12 +425,15 @@ def make_heads_weights(named):
 
 def heads(weights, *, tokens, tokens_per_img, depth, conf, B, focal_feat=None, pool_partial=None, pool_splits=0,
           tmp_w=None, tmp_b=None, pooled_out=None, exif=None, camera_idx=None, fused_out=None, num_cameras=0,
-          fault_ptr=None):
+          fault_ptr=None, sweep_images=0):
     """`fault_ptr`: address of a device-visible int32 (pinned host memory) that receives bit 0 when a camera index lies
-    outside [0, num_cameras) — the range check of the embedding lookup, done on the device so the call never syncs."""
+    outside [0, num_cameras) — the range check of the embedding lookup, done on the device so the call never syncs.
+    `sweep_images` > 0: an instruction sweep of B / sweep_images calls over `sweep_images` images (rows k * images + b,
+    tmp_w [K, 64, 768], tmp_b [K, 64]; include/cogaim_b200.h ca_heads_inputs)."""
     import ctypes as C
     inp = _lib.HeadsInputs(_dp(tokens), tokens_per_img, _dp(focal_feat), _dp(pool_partial), pool_splits, _dp(tmp_w),
-                           _dp(tmp_b), _dp(pooled_out), _dp(exif), _dp(camera_idx), int(num_cameras), fault_ptr)
+                           _dp(tmp_b), _dp(pooled_out), _dp(exif), _dp(camera_idx), int(num_cameras), fault_ptr,
+                           int(sweep_images))
     e0 = _begin()
     check(_lib.load().ca_heads(C.byref(weights), C.byref(inp), ptr(depth), ptr(conf), ptr(fused_out), B, stream_ptr()),
           "ca_heads")

@@ -9,6 +9,8 @@ What demo.py does per image and what runs here instead:
     delattr(model, '_last_attention_weights')          -> the same                              (demo.py:334-335)
     model.forward_with_guidance(x, exif, instruction)  -> the same call                         (demo.py:344-346)
     numpy / scipy heat-map overlay                     -> model.focus_map((h, w)) on the GPU    (demo.py:530-563)
+`--instruction all` (demo_results/: one photograph under all nine instructions) runs ONE instruction sweep
+(`Predictor.predict_all`, model.forward_with_guidance_sweep) instead of nine calls, with the same printed results.
 Weights: random init (seed 0, the reference's own construction order) unless --checkpoint names a reference state_dict.
 """
 from __future__ import annotations
@@ -68,6 +70,29 @@ class Predictor:
             meta["overlay"] = self.model.focus_map(overlay_size)[0]
         return float(depth.squeeze()), float(conf.squeeze()), meta
 
+    @torch.no_grad()
+    def predict_all(self, jpeg_bytes: bytes, instructions, exif=None, overlay_size=None):
+        """`[predict(jpeg_bytes, ins, exif, overlay_size) for ins in instructions]` — demo_results/' one photograph under
+        every instruction — as ONE instruction sweep: the image is decoded and run through the backbone and the focal
+        stream once.  Same results, bit for bit, and the same model state afterwards."""
+        x = self.model.preprocess_jpeg([jpeg_bytes], self.image_size)
+        exif = exif if exif is not None else self.default_exif(1)
+        if hasattr(self.model, "_last_attention_weights"):
+            delattr(self.model, "_last_attention_weights")
+        depth, conf, heat = self.model.forward_with_guidance_sweep(x, exif, list(instructions), return_attention=True)
+        g = self.image_size // 14
+        out = []
+        for k, ins in enumerate(instructions):
+            cell = int(heat[k, 0].argmax())
+            meta = {"processed_size": (self.image_size, self.image_size), "instruction": ins,
+                    "attention_cell": (cell // g, cell % g),
+                    "model_status": {"ambient": self.model.use_ambient, "focal": self.model.use_focal,
+                                     "exif": self.model.use_exif}}
+            if overlay_size is not None:
+                meta["overlay"] = self.model.focus_map(overlay_size, attention=heat[k])[0]
+            out.append((float(depth[k].squeeze()), float(conf[k].squeeze()), meta))
+        return out
+
 
 def main():
     ap = argparse.ArgumentParser()
@@ -83,9 +108,12 @@ def main():
     torch.manual_seed(0)
     p = Predictor(sd, image_size=args.image_size)
     data = open(args.image, "rb").read()
-    todo = INSTRUCTIONS if args.instruction == "all" else [args.instruction]
-    for ins in todo:
-        depth, conf, meta = p.predict(data, ins, overlay_size=(480, 640) if args.overlay else None)
+    overlay_size = (480, 640) if args.overlay else None
+    if args.instruction == "all":  # every instruction in one sweep (backbone and focal pass once)
+        results = zip(INSTRUCTIONS, p.predict_all(data, INSTRUCTIONS, overlay_size=overlay_size))
+    else:
+        results = [(args.instruction, p.predict(data, args.instruction, overlay_size=overlay_size))]
+    for ins, (depth, conf, meta) in results:
         print(f"{str(ins):13s} depth {depth:.4f}  confidence {conf:.4f}  attention cell {meta['attention_cell']}")
     if args.overlay:
         import numpy as np

@@ -144,6 +144,23 @@ int ca_guided_softmax(const float* base, const float* mask, long long mask_batch
 int ca_weighted_pool(const float* src, long long src_batch_stride, int row_offset, const float* w, const float* w2,
                      float* partial, int B, int N, int D, int splits, void* stream);
 
+/* Instruction sweeps: K guidance instructions over the same batch (K successive forward_with_guidance calls that share
+ * the backbone and the focal pass).  Rows r = k * B + b, k-major.  K is at most CA_SWEEP_MAX_K: the sweep pool keeps one
+ * float4 accumulator per instruction in registers. */
+#define CA_SWEEP_MAX_K 16
+/* ca_guided_softmax for K * B rows: row r = k * B + b reads mask + k * mask_k_stride + b * mask_batch_stride and base +
+ * k * base_k_stride + b * N (base_k_stride 0: one focal pass shared by every instruction; B * N: one per instruction,
+ * curiosity-guided attention), writes heat [K * B, N] and argmax [K * B].  Each row is computed exactly as
+ * ca_guided_softmax computes it. */
+int ca_guided_softmax_sweep(const float* base, long long base_k_stride, const float* mask, long long mask_k_stride,
+                            long long mask_batch_stride, float* heat, int32_t* argmax, int K, int B, int N, float alpha,
+                            float temperature, void* stream);
+/* partial[k * B + b, s, :] = sum_{n in split s} w[k, b, n] * src[b*src_batch_stride + (row_offset+n)*D + :] for K weight
+ * vectors w [K, B, N]: the tokens are read once for all K.  Bit for bit what K ca_weighted_pool launches (w2 = NULL) with
+ * the same `splits` write.  D must be 768. */
+int ca_weighted_pool_sweep(const float* src, long long src_batch_stride, int row_offset, const float* w, float* partial,
+                           int K, int B, int N, int D, int splits, void* stream);
+
 /* Heads ------------------------------------------------------------------------------------------ */
 /* All members are DEVICE pointers to fp32 row-major [out, in] weights / [out] biases of the reference modules. */
 typedef struct ca_heads_weights {
@@ -169,6 +186,10 @@ typedef struct ca_heads_inputs {
   const long long* camera_idx;/* [B] */
   int num_cameras;            /* rows of cam_emb; an index outside [0, num_cameras) is clamped and reported in *fault */
   int* fault;                 /* optional device-visible word (e.g. pinned host memory): bit 0 set on a bad camera_idx */
+  int sweep_images;           /* 0: one CTA per image.  > 0 (instruction sweep, guided only): the B passed to ca_heads is
+                                 K * sweep_images; CTA r reads image b = r % sweep_images (CLS token, EXIF, camera index),
+                                 projection k = r / sweep_images of tmp_w [K, 64, 768] / tmp_b [K, 64], pool_partial row r,
+                                 and writes depth[r], conf[r] */
 } ca_heads_inputs;
 
 /* depth[B], conf[B] (and optionally fused_out[B,192]) from the backbone tokens + focal slot + EXIF.
@@ -347,6 +368,26 @@ int ca_create(ca_handle** out, const ca_model_weights* w, int device);
 int ca_destroy(ca_handle* h);
 /* forward_with_guidance(images, exif, instruction | guidance tensor) -> depth, confidence, heat map, arg-max cell. */
 int ca_forward_guided(ca_handle* h, const ca_forward_call* call, void* stream);
+/* Instruction sweep: K = 1..CA_SWEEP_MAX_K guided calls over one batch.  HOST pointers where marked, device otherwise. */
+typedef struct ca_sweep_call {
+  int K;
+  const char* const* instructions; /* HOST [K] instruction strings / aliases, or NULL when `masks` is given */
+  const float* masks;              /* [K, N] explicit guidance, one row per call, shared by the batch; or NULL */
+  const float* tmp_w;              /* HOST [K, 64, 768]: the per-call projections, in call order  src/model.py:1421 */
+  const float* tmp_b;              /* HOST [K, 64] */
+  const float* eps;                /* HOST [K, B, 192]: the CuriosityModule draw of :609 of each call */
+  const float* noise;              /* HOST [K, B, 768]: the draw of :744 of each call */
+  float* depth;                    /* out [K, B] */
+  float* conf;                     /* out [K, B] */
+  float* attention;                /* out [K, B, N] heat maps */
+  int* argmax;                     /* out [K, B] or NULL */
+} ca_sweep_call;
+/* K forward_with_guidance calls on the same images and EXIF, in one: the backbone and the focal iterations run once, the
+ * CuriosityModule K times (the ring buffer receives K runs of B entries in call order), the guidance, pooling and heads
+ * once for all K * B rows.  Bit-identical to K ca_forward_guided calls given the same per-call draws.  `call` supplies
+ * images, images_u8, B, S, exif, camera_idx, fault and use_graph; its per-call fields (instruction, mask, tmp_w, tmp_b,
+ * eps, noise, depth, conf, attention, argmax, fused) must be NULL. */
+int ca_forward_guided_sweep(ca_handle* h, const ca_forward_call* call, const ca_sweep_call* sweep, void* stream);
 /* forward(images, exif or none) -> depth, confidence, last-iteration focal attention, fusion features. */
 int ca_forward(ca_handle* h, const ca_forward_call* call, void* stream);
 /* DINOv2 tokens only: tokens_out fp32 [B, 1+N, 768] (BASELINE.json configs[2]). */
