@@ -89,10 +89,12 @@ class ForwardCall(C.Structure):
                 ("mask_batch_stride", C.c_longlong), ("tmp_w", C.c_void_p), ("tmp_b", C.c_void_p), ("eps", C.c_void_p),
                 ("noise", C.c_void_p), ("curiosity_runs", C.c_int), ("depth", C.c_void_p), ("conf", C.c_void_p),
                 ("attention", C.c_void_p), ("argmax", C.c_void_p), ("fused", C.c_void_p), ("fault", C.c_void_p),
-                ("use_graph", C.c_int)]
+                ("use_graph", C.c_int), ("image_list", C.POINTER(C.c_void_p)), ("image_hw", C.POINTER(C.c_int))]
 
 
 SWEEP_MAX_K = 16  # CA_SWEEP_MAX_K (include/cogaim_b200.h)
+RESIZE_MAX_SIDE = 16384  # CA_RESIZE_MAX_SIDE
+RESIZE_LIST_CHUNK = 128  # CA_RESIZE_LIST_CHUNK
 
 
 class SweepCall(C.Structure):
@@ -102,7 +104,7 @@ class SweepCall(C.Structure):
                 ("conf", C.c_void_p), ("attention", C.c_void_p), ("argmax", C.c_void_p)]
 
 
-# name -> (argtypes); every function returns int status except where noted
+# name -> (argtypes); every function returns int status except where noted in _RESTYPES
 _SIGNATURES = {
     "ca_version": [],
     "ca_device_check": [C.c_int],
@@ -130,6 +132,9 @@ _SIGNATURES = {
     "ca_curiosity_modulation": [C.POINTER(CuriosityModWeights), c_ptr, C.c_float, C.c_float, c_ptr, C.c_int, C.c_int,
                                 C.c_int, c_ptr],
     "ca_resize_u8": [c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr],
+    "ca_resize_u8_list_tmp_bytes": [C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int],
+    "ca_resize_u8_list": [C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.c_int, C.c_int, C.c_int, c_ptr, C.c_size_t, c_ptr,
+                          c_ptr],
     "ca_jpeg_info": [C.c_char_p, C.c_size_t, C.POINTER(C.c_int), C.POINTER(C.c_int)],
     "ca_jpeg_decode": [C.c_char_p, C.c_size_t, c_ptr, C.c_int, C.c_int, c_ptr],
     "ca_jpeg_decode_batch": [C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), C.c_int, C.POINTER(C.c_void_p),
@@ -150,8 +155,12 @@ _SIGNATURES = {
     "ca_forward_guided_sweep": [c_ptr, C.POINTER(ForwardCall), C.POINTER(SweepCall), c_ptr],
     "ca_forward": [c_ptr, C.POINTER(ForwardCall), c_ptr],
     "ca_backbone": [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr],
+    "ca_backbone_list": [c_ptr, C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.c_int, C.c_int, c_ptr, c_ptr],
     "ca_last_launch_count": [c_ptr],
 }
+
+
+_RESTYPES = {"ca_resize_u8_list_tmp_bytes": C.c_size_t}
 
 
 def exported_symbols():
@@ -173,7 +182,7 @@ def load():
     lib.ca_last_error.argtypes = []
     for name, argtypes in _SIGNATURES.items():
         fn = getattr(lib, name)
-        fn.restype = C.c_int
+        fn.restype = _RESTYPES.get(name, C.c_int)
         fn.argtypes = argtypes
     _lib = lib
     return lib
@@ -188,6 +197,14 @@ def check(status: int, what: str):
 def ptr(t):
     """Device pointer of a torch tensor (or None)."""
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+def image_arrays(images):
+    """HOST arrays (device pointers [B], (H, W) pairs [B, 2]) of a list of uint8 [H_i, W_i, 3] CUDA tensors, as the
+    list entry points (ca_resize_u8_list, ca_forward_call.image_list) take them."""
+    ptrs = (C.c_void_p * len(images))(*[t.data_ptr() for t in images])
+    hw = (C.c_int * (2 * len(images)))(*[int(d) for t in images for d in t.shape[:2]])
+    return ptrs, hw
 
 
 def stream_ptr():

@@ -236,6 +236,16 @@ int ca_resize_u8(const uint8_t* src, int B, int H0, int W0, int out_h, int out_w
   return ca::resize_u8_launch(src, B, H0, W0, out_h, out_w, tmp, out, static_cast<cudaStream_t>(stream));
 }
 
+size_t ca_resize_u8_list_tmp_bytes(const int* h_hw, int B, int out_h, int out_w) {
+  return ca::resize_list_tmp_bytes(h_hw, B, out_h, out_w);
+}
+
+int ca_resize_u8_list(const uint8_t* const* h_images, const int* h_hw, int B, int out_h, int out_w, uint8_t* tmp,
+                      size_t tmp_bytes, uint8_t* out, void* stream) {
+  return ca::resize_list_launch(h_images, h_hw, B, out_h, out_w, tmp, tmp_bytes, out, static_cast<cudaStream_t>(stream),
+                                nullptr);
+}
+
 int ca_jpeg_info(const uint8_t* h_data, size_t len, int* width, int* height) {
   return ca::jpeg_info(h_data, len, width, height, nullptr);
 }

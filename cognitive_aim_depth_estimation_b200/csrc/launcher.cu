@@ -28,6 +28,7 @@
 #include "gemm.cuh"
 #include "heads.cuh"
 #include "host.h"
+#include "resize.cuh"
 #include "rowops.cuh"
 
 namespace {
@@ -90,6 +91,10 @@ struct ca_handle {
   cudaEvent_t fork = nullptr, join = nullptr;
   int launches = 0;       // running count of the sequence being issued
   int last_launches = 0;  // of the last completed call
+  // photographs of individual sizes (ca_forward_call.image_list): the resized uint8 [B, S, S, 3] batch followed by the
+  // resize temporary, grow-only
+  uint8_t* resize_buf = nullptr;
+  size_t resize_cap = 0;
 };
 
 namespace {
@@ -630,9 +635,45 @@ int stage_sweep_inputs(ca_handle* h, Workspace& w, Workspace::Sweep& s, const ca
   return 0;
 }
 
-int patch_rows(ca_handle* h, Workspace& w, const void* images, int images_u8, cudaStream_t st) {
+// The images of one call: a uniform tensor (`images`, fp32 or uint8 at model resolution) or B photographs of
+// individual sizes (`list` / `hw`, HOST arrays).
+struct ImagesIn {
+  const void* images;
+  int u8;
+  const uint8_t* const* list;
+  const int* hw;
+};
+
+ImagesIn images_of(const ca_forward_call& c) { return {c.images, c.images_u8, c.image_list, c.image_hw}; }
+
+int check_images(const ImagesIn& in) {
+  CA_REQUIRE((in.images != nullptr) != (in.list != nullptr), "forward: give images OR image_list");
+  CA_REQUIRE(!in.list || in.hw, "forward: image_list needs image_hw");
+  return 0;
+}
+
+// Eager, in front of the (possibly replayed) graph: nothing here depends on a captured address except w.patches.
+int patch_rows(ca_handle* h, Workspace& w, const ImagesIn& in, cudaStream_t st) {
   static const float mean[3] = {0.485f, 0.456f, 0.406f}, stdv[3] = {0.229f, 0.224f, 0.225f};
-  if (images_u8)
+  const void* images = in.images;
+  if (in.list) {
+    const size_t out_bytes = (static_cast<size_t>(w.B) * w.S * w.S * 3 + 255) & ~static_cast<size_t>(255);
+    const size_t tmp_bytes = ca::resize_list_tmp_bytes(in.hw, w.B, w.S, w.S);
+    if (h->resize_cap < out_bytes + tmp_bytes) {
+      // cudaFree waits for the device: the previous batch's reads of the old buffer have finished
+      if (h->resize_buf) CA_CUDA(cudaFree(h->resize_buf));
+      h->resize_buf = nullptr;
+      h->resize_cap = 0;
+      CA_CUDA(cudaMalloc(&h->resize_buf, out_bytes + tmp_bytes));
+      h->resize_cap = out_bytes + tmp_bytes;
+    }
+    int n = 0;
+    CA_TRY(ca::resize_list_launch(in.list, in.hw, w.B, w.S, w.S, h->resize_buf + out_bytes, tmp_bytes, h->resize_buf, st,
+                                  &n));
+    h->launches += n;
+    images = h->resize_buf;
+  }
+  if (in.u8 || in.list)
     LAUNCH(ca::preprocess_u8_launch(static_cast<const uint8_t*>(images), w.patches, w.B, w.S, mean, stdv, st));
   else
     LAUNCH(ca::patchify_f32_launch(static_cast<const float*>(images), w.patches, w.B, w.S, st));
@@ -672,7 +713,8 @@ int run_sequence(ca_handle* h, Workspace& w, int key, bool use_graph, cudaStream
 
 int check_call(const ca_handle* h, const ca_forward_call* c) {
   CA_REQUIRE(h && c, "null handle / call");
-  CA_REQUIRE(c->images && c->B > 0, "forward: null images or empty batch");
+  CA_REQUIRE(c->B > 0, "forward: empty batch");
+  CA_TRY(check_images(images_of(*c)));
   CA_REQUIRE(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260, "forward: image side must be a multiple of 14 in [56, 1260]");
   CA_REQUIRE(c->depth && c->conf, "forward: null output");
   CA_REQUIRE(c->eps && c->noise, "forward: null CuriosityModule draws (HOST pointers, src/model.py:609,744)");
@@ -735,6 +777,7 @@ int ca_destroy(ca_handle* h) {
     if (s.buf) cudaFreeHost(s.buf);
     if (s.done) cudaEventDestroy(s.done);
   }
+  if (h->resize_buf) cudaFree(h->resize_buf);
   cudaStreamDestroy(h->side);
   cudaEventDestroy(h->fork);
   cudaEventDestroy(h->join);
@@ -744,8 +787,11 @@ int ca_destroy(ca_handle* h) {
 
 int ca_last_launch_count(const ca_handle* h) { return h ? h->last_launches : 0; }
 
-int ca_backbone(ca_handle* h, const void* images, int images_u8, int B, int S, float* tokens_out, void* stream) {
-  CA_REQUIRE(h && images && B > 0 && S >= 56 && S % 14 == 0, "ca_backbone: bad argument");
+namespace {
+
+int backbone(ca_handle* h, const ImagesIn& in, int B, int S, float* tokens_out, void* stream) {
+  CA_REQUIRE(h && B > 0 && S >= 56 && S % 14 == 0, "ca_backbone: bad argument");
+  CA_TRY(check_images(in));
   DeviceGuard guard(h->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   Workspace* w = nullptr;
@@ -753,7 +799,7 @@ int ca_backbone(ca_handle* h, const void* images, int images_u8, int B, int S, f
   CA_TRY(get_workspace(h, B, S, &w));
   CA_TRY(get_tables(h, S / 14, &tb));
   h->launches = 0;
-  CA_TRY(patch_rows(h, *w, images, images_u8, st));
+  CA_TRY(patch_rows(h, *w, in, st));
   CA_TRY(run_sequence(h, *w, 0, true, st, [&]() { return backbone_layers(h, *w, *tb, st); }));
   if (tokens_out) {
     const size_t g = S / 14;
@@ -761,6 +807,18 @@ int ca_backbone(ca_handle* h, const void* images, int images_u8, int B, int S, f
   }
   h->last_launches = h->launches;
   return 0;
+}
+
+}  // namespace
+
+int ca_backbone(ca_handle* h, const void* images, int images_u8, int B, int S, float* tokens_out, void* stream) {
+  return backbone(h, ImagesIn{images, images_u8, nullptr, nullptr}, B, S, tokens_out, stream);
+}
+
+int ca_backbone_list(ca_handle* h, const uint8_t* const* image_list, const int* image_hw, int B, int S, float* tokens_out,
+                     void* stream) {
+  CA_REQUIRE(image_list, "ca_backbone_list: null image list");
+  return backbone(h, ImagesIn{nullptr, 0, image_list, image_hw}, B, S, tokens_out, stream);
 }
 
 int ca_forward_guided(ca_handle* h, const ca_forward_call* c, void* stream) {
@@ -792,7 +850,7 @@ int ca_forward_guided(ca_handle* h, const ca_forward_call* c, void* stream) {
   CA_CUDA(cudaMemcpyAsync(w.mask_in, mask, static_cast<size_t>(mstride ? B : 1) * N * 4, cudaMemcpyDeviceToDevice, st));
   CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
   CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
-  CA_TRY(patch_rows(h, w, c->images, c->images_u8, st));
+  CA_TRY(patch_rows(h, w, images_of(*c), st));
   int* fault = c->fault;
   const int key = 100 + (mstride ? 1 : 0);
   CA_TRY(run_sequence(h, w, key, c->use_graph != 0, st, [&]() -> int {
@@ -816,7 +874,8 @@ int ca_forward_guided(ca_handle* h, const ca_forward_call* c, void* stream) {
 
 int ca_forward_guided_sweep(ca_handle* h, const ca_forward_call* c, const ca_sweep_call* sw, void* stream) {
   CA_REQUIRE(h && c && sw, "forward_guided_sweep: null handle / call / sweep");
-  CA_REQUIRE(c->images && c->B > 0, "forward_guided_sweep: null images or empty batch");
+  CA_REQUIRE(c->B > 0, "forward_guided_sweep: empty batch");
+  CA_TRY(check_images(images_of(*c)));
   CA_REQUIRE(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260,
              "forward_guided_sweep: image side must be a multiple of 14 in [56, 1260]");
   CA_REQUIRE(c->exif && c->camera_idx, "forward_guided_sweep: EXIF inputs are required (without them the reference falls "
@@ -857,7 +916,7 @@ int ca_forward_guided_sweep(ca_handle* h, const ca_forward_call* c, const ca_swe
   CA_TRY(stage_sweep_inputs(h, w, s, *sw, st));
   CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
   CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
-  CA_TRY(patch_rows(h, w, c->images, c->images_u8, st));
+  CA_TRY(patch_rows(h, w, images_of(*c), st));
   int* fault = c->fault;
   CA_TRY(run_sequence(h, w, 300 + K, c->use_graph != 0, st, [&]() -> int {
     CA_TRY(backbone_layers(h, w, *tb, st));
@@ -912,7 +971,7 @@ int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
     CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
     CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
   }
-  CA_TRY(patch_rows(h, w, c->images, c->images_u8, st));
+  CA_TRY(patch_rows(h, w, images_of(*c), st));
   int* fault = c->fault;
   float* att = nullptr;
   const int key = 200 + (has_exif ? 1 : 0) + 2 * runs;

@@ -29,6 +29,7 @@ import torch
 import torch.nn as nn
 
 from . import ops, tables
+from ._lib import RESIZE_MAX_SIDE as _RESIZE_MAX_SIDE  # largest photograph side the resize stages in shared memory
 from ._lib import SWEEP_MAX_K as _SWEEP_MAX_K  # instructions per sweep: the sweep pool keeps one accumulator each
 from .config import DEFAULT_COGNITIVE_MODULES, EffectiveConfig, effective_config
 from .init import reference_init_
@@ -543,10 +544,34 @@ class CognitiveAimModel(nn.Module):
         ops.fetch_pinned(ws["cur_eps"][:k], bufs[0][:k])
         ops.fetch_pinned(ws["cur_noise"][:k], bufs[1][:k])
 
+    @staticmethod
+    def _check_side(S):
+        if S < 56 or S % 14 != 0 or S > _MAX_SIDE:
+            raise ValueError(f"image side must be a multiple of 14 in [56, {_MAX_SIDE}] (got {S})")
+
+    def _check_list(self, images, S):
+        """B of a list of photographs of individual sizes (uint8 [H_i, W_i, 3], CPU or CUDA) resized to S x S."""
+        if len(images) == 0:
+            raise ValueError("empty list of images")
+        for i, t in enumerate(images):
+            if not torch.is_tensor(t) or t.dtype != torch.uint8 or t.dim() != 3 or t.shape[-1] != 3:
+                raise ValueError(f"image {i} of the list must be a uint8 [H, W, 3] tensor")
+            if not 0 < min(t.shape[0], t.shape[1]) <= max(t.shape[0], t.shape[1]) <= _RESIZE_MAX_SIDE:
+                raise ValueError(f"image {i} of the list is {t.shape[0]} x {t.shape[1]}: sides must be in "
+                                 f"[1, {_RESIZE_MAX_SIDE}]")
+        if S is None:
+            raise ValueError("a list of images is resized to model.input_size: set it (demo.py's dataset.image_size)")
+        self._check_side(S)
+        return len(images)
+
     def _check_images(self, images):
         """(B, S) of a forward input: float [B, 3, S, S] already normalised (what the reference's forward takes), or —
         an extension for the demo-shaped flow — uint8 [B, H, W, 3] straight from the decoder (demo.py:312-319 on the
-        GPU: Resize((input_size, input_size)) when the size differs, ToTensor, Normalize, fused with the patchify)."""
+        GPU: Resize((input_size, input_size)) when the size differs, ToTensor, Normalize, fused with the patchify), or a
+        list of uint8 [H_i, W_i, 3] photographs of individual sizes, all resized to input_size (demo.py:406-432
+        `predict_batch` over a folder)."""
+        if isinstance(images, (list, tuple)):
+            return self._check_list(images, self.input_size), self.input_size
         if torch.is_tensor(images) and images.dtype == torch.uint8:
             if images.dim() != 4 or images.shape[-1] != 3:
                 raise ValueError("uint8 images must be [B, H, W, 3]")
@@ -554,8 +579,7 @@ class CognitiveAimModel(nn.Module):
             S = self.input_size if self.input_size is not None else H
             if self.input_size is None and H != W:
                 raise ValueError("uint8 images must be square, or set model.input_size to resize like demo.py")
-            if S < 56 or S % 14 != 0 or S > _MAX_SIDE:
-                raise ValueError(f"image side must be a multiple of 14 in [56, {_MAX_SIDE}] (got {S})")
+            self._check_side(S)
             return B, S
         if not torch.is_tensor(images) or images.dim() != 4 or images.shape[1] != 3:
             raise ValueError("images must be a [B, 3, S, S] tensor")
@@ -567,8 +591,13 @@ class CognitiveAimModel(nn.Module):
         return B, H
 
     def _patch_rows(self, images, ws, S: int):
-        """im2col rows (bf16 [B*N, 592]) of the batch into ws['patches']; returns (patches, tensor to keep alive)."""
+        """im2col rows (bf16 [B*N, 592]) of the batch into ws['patches']; returns (patches, tensors to keep alive).
+        Runs eagerly in front of the (possibly replayed) graph, so lists of other sizes replay the same graph."""
         dev = self._device()
+        if isinstance(images, (list, tuple)):
+            src = [t.to(dev).contiguous() for t in images]
+            u8 = ops.resize_u8_list(src, S, S)  # demo.py:162-163 per image, the whole batch in one launch per pass
+            return ops.preprocess_u8(u8, ws["patches"]), (src, u8)
         if images.dtype == torch.uint8:
             u8 = images.to(dev).contiguous()
             if tuple(u8.shape[1:3]) != (S, S):
@@ -583,10 +612,10 @@ class CognitiveAimModel(nn.Module):
         `patches` (bf16 [B*N, 592] from `preprocess_u8`) may be given instead of images.
         The result is a BORROWED view of the (B, S) workspace: the next call at the same shape overwrites it — clone it to
         keep it (the forward passes return fresh tensors)."""
-        pk = self._pack()
-        dev = self._device()
         if patches is None:
             B, S = self._check_images(images)
+        pk = self._pack()
+        dev = self._device()
         g = S // 14
         N, T = g * g, g * g + 1
         ws = self._workspace(B, S)
@@ -712,6 +741,22 @@ class CognitiveAimModel(nn.Module):
             ops.focal_fusion(ws["feats"], iters, pk["ffw0"], pk["ffb0"], pk["ffw1"], pk["ffb1"], ws["focal_feat"], B)
         return ws["attn"][iters - 1]
 
+    @staticmethod
+    def _check_per_image(guidance, B: int):
+        if isinstance(guidance, (list, tuple)) and len(guidance) != B:
+            raise ValueError(f"{len(guidance)} per-image instructions for a batch of {B}")
+
+    def _check_exif(self, exif_data, B: int):
+        """The EXIF entry counts against the batch, before anything is drawn or launched (_exif_tensors converts)."""
+        if exif_data is None or not self.use_exif:
+            return
+        for key in ("focal_length", "aperture", "iso", "camera_idx"):
+            if key not in exif_data:
+                raise ValueError(f"exif_data is missing '{key}'")
+            n = exif_data[key].numel() if torch.is_tensor(exif_data[key]) else torch.as_tensor(exif_data[key]).numel()
+            if n != B:
+                raise ValueError(f"exif_data['{key}'] has {n} entries for a batch of {B}")
+
     def _exif_tensors(self, exif_data, B: int):
         if exif_data is None or not self.use_exif:
             return None, None
@@ -827,6 +872,8 @@ class CognitiveAimModel(nn.Module):
             return self._forward_impl(images, exif_data, return_attention, mode="guided_fallback",
                                       guidance=attention_guidance)
         B, S = self._check_images(images)
+        self._check_per_image(attention_guidance, B)
+        self._check_exif(exif_data, B)
         pk = self._pack()
         dev = self._device()
         g = S // 14
@@ -951,6 +998,9 @@ class CognitiveAimModel(nn.Module):
             raise ValueError("an instruction sweep needs EXIF data and a model with the EXIF prior (otherwise the "
                              "reference falls back to forward(): use forward_with_guidance)")
         B, S = self._check_images(images)
+        for gd in guidances:
+            self._check_per_image(gd, B)
+        self._check_exif(exif_data, B)
         pk = self._pack()
         g = S // 14
         N, T = g * g, g * g + 1
@@ -1020,6 +1070,8 @@ class CognitiveAimModel(nn.Module):
                            `fusion` and falls back to forward() (:1237-1240) with the guided attention already stored."""
         self._raise_on_fault()
         B, S = self._check_images(images)
+        self._check_per_image(guidance, B)
+        self._check_exif(exif_data, B)
         pk = self._pack()
         g = S // 14
         N, T = g * g, g * g + 1
@@ -1161,7 +1213,12 @@ class CognitiveAimModel(nn.Module):
         dev = self._device()
         if dev.type != "cuda":
             raise RuntimeError("preprocess runs only on a CUDA sm_100 device; there is no CPU fallback")
-        r = ops.resize_u8(images_hwc_u8.to(dev).contiguous(), size, size)
+        return self._normalise(ops.resize_u8(images_hwc_u8.to(dev).contiguous(), size, size), mean, std)
+
+    @staticmethod
+    def _normalise(r, mean, std):
+        """uint8 [B, S, S, 3] -> ToTensor -> Normalize: float32 [B, 3, S, S] (demo.py:164-166)."""
+        dev = r.device
         # ToTensor: a true division (a tensor divisor; dividing by a Python scalar multiplies by the reciprocal on CUDA)
         x = r.permute(0, 3, 1, 2).to(torch.float32) / torch.full((1,), 255.0, device=dev)
         m = torch.tensor(mean, device=dev).view(1, 3, 1, 1)
@@ -1173,26 +1230,31 @@ class CognitiveAimModel(nn.Module):
     def preprocess_jpeg(self, jpeg_files, size: int, mean=ops.IMAGENET_MEAN, std=ops.IMAGENET_STD):
         """demo.py:312-319 for a list of JPEG files given as bytes: decode (nvJPEG) -> Resize((size, size)) (exact Pillow
         arithmetic) -> ToTensor -> Normalize, all on the GPU.  Images may differ in size (each is resized on its own, as
-        `predict_batch` does, demo.py:406-432).  Returns float32 [B, 3, size, size]."""
+        `predict_batch` does, demo.py:406-432, in one resize for the whole list).  Returns float32 [B, 3, size, size]."""
         dev = self._device()
         if dev.type != "cuda":
             raise RuntimeError("preprocess_jpeg runs only on a CUDA sm_100 device; there is no CPU fallback")
         if len(jpeg_files) == 0:
             raise ValueError("empty list of JPEG files")
-        # one batched nvJPEG decode for all files; images of equal size come back as slices of one [n, H, W, 3] block and
-        # are resized + normalised as one tensor (one launch sequence per distinct source size, not per file)
-        imgs, groups = ops.jpeg_decode_batch(list(jpeg_files), dev, return_groups=True)
-        out = torch.empty(len(imgs), 3, size, size, device=dev, dtype=torch.float32)
-        for block, idx in groups:
-            out[idx] = self.preprocess(block, size, mean, std)
-        return out
+        # one batched nvJPEG decode for all files, one ragged resize, one normalisation: the launch count does not depend on
+        # the number of distinct source sizes
+        imgs = ops.jpeg_decode_batch(list(jpeg_files), dev)
+        return self._normalise(ops.resize_u8_list(imgs, size, size), mean, std)
 
     @torch.no_grad()
     @_on_own_device
-    def tokens_from_uint8(self, images_hwc_u8: torch.Tensor, size: Optional[int] = None):
+    def tokens_from_uint8(self, images_hwc_u8, size: Optional[int] = None):
         """uint8 [B, H, W, 3] -> backbone tokens: demo.py:162-166 on the GPU — Resize((size, size)) exactly as Pillow does
         it (skipped when the images already have that size or `size` is None), then ToTensor + Normalize + patchify
-        fused in one kernel."""
+        fused in one kernel.  A list of uint8 [H_i, W_i, 3] photographs of individual sizes is resized to `size` (or,
+        when it is None, model.input_size)."""
+        if isinstance(images_hwc_u8, (list, tuple)):
+            S = size if size is not None else self.input_size
+            B = self._check_list(images_hwc_u8, S)
+            self._pack()
+            ws = self._workspace(B, S)
+            patches, self._keepalive = self._patch_rows(images_hwc_u8, ws, S)
+            return self.backbone_tokens(None, patches=patches, B=B, S=S)
         if images_hwc_u8.dtype != torch.uint8 or images_hwc_u8.dim() != 4 or images_hwc_u8.shape[-1] != 3:
             raise ValueError("expected uint8 [B, H, W, 3]")
         if size is not None and tuple(images_hwc_u8.shape[1:3]) != (size, size):

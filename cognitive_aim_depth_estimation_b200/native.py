@@ -153,17 +153,32 @@ class NativeModel:
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
-    def _call(self, images, exif) -> _lib.ForwardCall:
+    def _image_list(self, images, S):
+        """A list of uint8 [H_i, W_i, 3] photographs -> (device tensors, HOST pointer array, HOST (H, W) array)."""
+        if S is None:
+            raise ValueError("a list of images needs S, the side they are resized to")
+        if len(images) == 0 or any(t.dtype != torch.uint8 or t.dim() != 3 or t.shape[-1] != 3 for t in images):
+            raise ValueError("expected a non-empty list of uint8 [H, W, 3] tensors")
+        imgs = [t.to(self.device).contiguous() for t in images]
+        ptrs, hw = _lib.image_arrays(imgs)
+        return imgs, C.cast(ptrs, C.POINTER(C.c_void_p)), C.cast(hw, C.POINTER(C.c_int)), [imgs, ptrs, hw]
+
+    def _call(self, images, exif, S=None) -> _lib.ForwardCall:
         c = _lib.ForwardCall()
-        if images.dtype == torch.uint8:
+        if isinstance(images, (list, tuple)):
+            imgs, c.image_list, c.image_hw, held = self._image_list(images, S)
+            B = len(imgs)
+            c.B, c.S = B, S
+        elif images.dtype == torch.uint8:
             B, S = images.shape[0], images.shape[1]
             c.images_u8 = 1
         else:
             B, S = images.shape[0], images.shape[-1]
             images = images.to(self.device, torch.float32)
-        images = images.to(self.device).contiguous()
-        c.images, c.B, c.S = images.data_ptr(), B, S
-        held = [images]
+        if not isinstance(images, (list, tuple)):
+            images = images.to(self.device).contiguous()
+            c.images, c.B, c.S = images.data_ptr(), B, S
+            held = [images]
         if exif is not None:
             cont = torch.stack([exif["focal_length"].reshape(-1), exif["aperture"].reshape(-1),
                                 exif["iso"].reshape(-1)], dim=1).to(self.device, torch.float32).contiguous()
@@ -174,9 +189,10 @@ class NativeModel:
         return c, held, B, S
 
     @torch.no_grad()
-    def forward_with_guidance(self, images, exif, guidance):
-        """-> depth [B,1], confidence [B,1], heat map [B,N], arg-max cell [B] (reference src/model.py:1157-1240)."""
-        c, held, B, S = self._call(images, exif)
+    def forward_with_guidance(self, images, exif, guidance, S=None):
+        """-> depth [B,1], confidence [B,1], heat map [B,N], arg-max cell [B] (reference src/model.py:1157-1240).
+        `images` may be a list of uint8 [H_i, W_i, 3] photographs of individual sizes: the library resizes them to S."""
+        c, held, B, S = self._call(images, exif, S)
         N = (S // 14) ** 2
         eps, noise = torch.randn(B, 192), torch.randn(B, _D)       # :609, :744 (CuriosityModule, before the projection)
         tmp = nn.Linear(_D, 64)                                    # :1421: same constructor => same generator draws
@@ -198,7 +214,7 @@ class NativeModel:
         return out["depth"].unsqueeze(1), out["conf"].unsqueeze(1), out["heat"], out["argmax"]
 
     @torch.no_grad()
-    def forward_with_guidance_sweep(self, images, exif, guidances):
+    def forward_with_guidance_sweep(self, images, exif, guidances, S=None):
         """K = len(guidances) `forward_with_guidance` calls in one native call (ca_forward_guided_sweep): the backbone and
         the focal pass run once.  `guidances`: K instruction strings, or K guidance tensors [N].  Draws the K calls'
         random numbers in the reference's order per call.  -> depth [K,B,1], confidence [K,B,1], heat maps [K,B,N],
@@ -206,7 +222,7 @@ class NativeModel:
         K = len(guidances)
         if not 1 <= K <= _lib.SWEEP_MAX_K:
             raise ValueError(f"an instruction sweep takes 1..{_lib.SWEEP_MAX_K} guidances, got {K}")
-        c, held, B, S = self._call(images, exif)
+        c, held, B, S = self._call(images, exif, S)
         N = (S // 14) ** 2
         s = _lib.SweepCall()
         s.K = K
@@ -239,10 +255,10 @@ class NativeModel:
         return out["depth"].unsqueeze(-1), out["conf"].unsqueeze(-1), out["heat"], out["argmax"]
 
     @torch.no_grad()
-    def forward(self, images, exif: Optional[dict] = None, runs: int = 1):
+    def forward(self, images, exif: Optional[dict] = None, runs: int = 1, S=None):
         """-> depth [B,1], confidence [B,1], focal attention [B,N], fusion features [B,192] (src/model.py:1064-1155).
         `runs`: how often the reference would run its CuriosityModule in this call (1..3, :992, :1104, :1138)."""
-        c, held, B, S = self._call(images, exif)
+        c, held, B, S = self._call(images, exif, S)
         N = (S // 14) ** 2
         draws = [(torch.randn(B, 192), torch.randn(B, _D)) for _ in range(runs)]
         eps = torch.stack([d[0] for d in draws]).contiguous()
@@ -257,7 +273,16 @@ class NativeModel:
         return out["depth"].unsqueeze(1), out["conf"].unsqueeze(1), out["att"], out["fused"]
 
     @torch.no_grad()
-    def backbone_tokens(self, images):
+    def backbone_tokens(self, images, S=None):
+        if isinstance(images, (list, tuple)):
+            imgs, ptrs, hw, held = self._image_list(images, S)
+            B, g = len(imgs), S // 14
+            tokens = torch.empty(B, g * g + 1, _D, device=self.device)
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.ca_backbone_list(self._h, ptrs, hw, B, S, tokens.data_ptr(), self._stream()),
+                           "ca_backbone_list")
+            self._held = held
+            return tokens
         u8 = images.dtype == torch.uint8
         B, S = (images.shape[0], images.shape[1]) if u8 else (images.shape[0], images.shape[-1])
         images = (images if u8 else images.to(torch.float32)).to(self.device).contiguous()

@@ -337,6 +337,40 @@ def resize_u8(src, out_h, out_w):
     return out
 
 
+def resize_u8_list(images, out_h, out_w):
+    """list of B uint8 [H_i, W_i, 3] CUDA tensors (individual sizes) -> uint8 [B, out_h, out_w, 3], each image bit-exact
+    PIL.Image.resize(..., BILINEAR); two launches for the whole batch whatever its mix of sizes (csrc/resize.cu)."""
+    import ctypes as C
+    if not isinstance(images, (list, tuple)) or len(images) == 0:
+        raise ValueError("resize_u8_list expects a non-empty list of images")
+    for t in images:
+        _req(t, torch.uint8, "images")
+        if t.dim() != 3 or t.shape[-1] != 3 or not t.is_contiguous():
+            raise ValueError("resize_u8_list expects contiguous uint8 [H, W, 3] tensors")
+        if not 0 < min(t.shape[0], t.shape[1]) <= max(t.shape[0], t.shape[1]) <= _lib.RESIZE_MAX_SIDE:
+            raise ValueError(f"image sides must be in [1, {_lib.RESIZE_MAX_SIDE}], got {tuple(t.shape[:2])}")
+    B = len(images)
+    dev = images[0].device
+    if any(t.device != dev for t in images):
+        raise ValueError("resize_u8_list expects every image on one device")
+    lib = _lib.load()
+    ptrs, hw = _lib.image_arrays(images)
+    tmp_bytes = int(lib.ca_resize_u8_list_tmp_bytes(hw, B, out_h, out_w))
+    out = torch.empty(B, out_h, out_w, 3, device=dev, dtype=torch.uint8)
+    tmp = torch.empty(tmp_bytes, device=dev, dtype=torch.uint8) if tmp_bytes else None
+    # kernels per chunk of images: one per pass that some image of the chunk needs (an image of the target size is copied)
+    n = 0
+    for c0 in range(0, B, _lib.RESIZE_LIST_CHUNK):
+        chunk = images[c0:c0 + _lib.RESIZE_LIST_CHUNK]
+        n += any(t.shape[1] != out_w for t in chunk) + any(t.shape[0] != out_h for t in chunk)
+    e0 = _begin()
+    with torch.cuda.device(dev):
+        check(lib.ca_resize_u8_list(ptrs, hw, B, out_h, out_w, ptr(tmp), tmp_bytes, ptr(out), stream_ptr()),
+              "ca_resize_u8_list")
+    _end(e0, "resize", n, float(sum(t.numel() for t in images) + out.numel()))
+    return out
+
+
 def jpeg_decode(data: bytes, device=None):
     """One JPEG file's bytes -> uint8 [H, W, 3] RGB CUDA tensor, decoded by nvJPEG on the current stream
     (csrc/jpeg.cu; reference demo.py:312 `Image.open(path).convert('RGB')`)."""
@@ -359,8 +393,7 @@ def jpeg_decode_batch(files, device=None, return_groups=False):
     """List of JPEG files (bytes) -> list of uint8 [H_i, W_i, 3] RGB CUDA tensors, decoded in ONE nvjpegDecodeBatched call
     (reference demo.py:406-432 `predict_batch` opens and decodes its files one at a time).  Images of equal size share
     one contiguous [k, H, W, 3] allocation (the returned tensors are its slices); `return_groups=True` also returns
-    [(block [k, H, W, 3], indices into the list)] so that same-sized photographs go to the resize / normalise kernels as
-    one tensor."""
+    [(block [k, H, W, 3], indices into the list)].  `resize_u8_list` takes the returned list whatever its sizes."""
     import ctypes as C
     if len(files) == 0:
         raise ValueError("empty list of JPEG files")

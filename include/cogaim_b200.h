@@ -258,6 +258,20 @@ int ca_curiosity_modulation(const ca_curiosity_mod_weights* w, const float* rewa
  * them and cached per (device, source size, target size) — the first call for a new size allocates and synchronises. */
 int ca_resize_u8(const uint8_t* src, int B, int H0, int W0, int out_h, int out_w, uint8_t* tmp, uint8_t* out,
                  void* stream);
+/* Largest source (and target) side the resize accepts: the horizontal pass stages 4 source rows of up to this many
+ * pixels in shared memory.  Larger images are rejected with CA_STATUS_INVALID. */
+#define CA_RESIZE_MAX_SIDE 16384
+/* Images per launch of each resize pass: the per-image descriptors travel as one kernel parameter.  Larger batches are
+ * resized in chunks of this many images. */
+#define CA_RESIZE_LIST_CHUNK 128
+/* B images of individual sizes -> uint8 [B, out_h, out_w, 3]; bit-exact PIL.Image.resize(..., BILINEAR) per image.
+ * h_images: HOST array of B device pointers (uint8 HWC, contiguous); h_hw: HOST [B, 2] (H0, W0).  Per image a pass runs
+ * only on an axis whose size changes (Pillow's semantics); an image of the target size is copied.  Each pass is one
+ * launch for the whole batch (per CA_RESIZE_LIST_CHUNK images), whatever its mix of sizes.  tmp: at least
+ * ca_resize_u8_list_tmp_bytes(h_hw, B, out_h, out_w) bytes (0 when no image changes both axes; tmp may then be NULL). */
+size_t ca_resize_u8_list_tmp_bytes(const int* h_hw, int B, int out_h, int out_w);
+int ca_resize_u8_list(const uint8_t* const* h_images, const int* h_hw, int B, int out_h, int out_w, uint8_t* tmp,
+                      size_t tmp_bytes, uint8_t* out, void* stream);
 
 /* ---- demo.py:312 `Image.open(path).convert('RGB')`: JPEG ingest through nvJPEG (CUDA toolkit; loaded lazily) ---------
  * h_data / len: one JPEG file's bytes in HOST memory.  ca_jpeg_info fills the decoded size; ca_jpeg_decode writes
@@ -361,6 +375,12 @@ typedef struct ca_forward_call {
   float* fused;                 /* out [B,192] fusion features (un-guided) or NULL */
   int* fault;                   /* optional device-visible word: bit 0 = camera_idx out of range */
   int use_graph;                /* 1: capture the launch sequence once per (path, B, S) and replay it */
+  /* Photographs of individual sizes (demo.py:406-432 `predict_batch` over a folder): when set, `images` must be NULL
+   * and the handle resizes each image to S x S (exactly as ca_resize_u8_list does) into a buffer it owns, then
+   * normalises and patchifies the batch.  The resize runs in front of the (possibly replayed) graph, so batches of
+   * other sizes at the same (B, S) replay the same graph.  Zero-initialised callers keep the `images` behaviour. */
+  const uint8_t* const* image_list; /* HOST [B]: device pointers to uint8 [H_i, W_i, 3] (contiguous) */
+  const int* image_hw;              /* HOST [B, 2]: (H_i, W_i), each side at most CA_RESIZE_MAX_SIDE */
 } ca_forward_call;
 
 /* `w` (HOST struct of device pointers) is copied; the weights themselves must outlive the handle. */
@@ -392,6 +412,10 @@ int ca_forward_guided_sweep(ca_handle* h, const ca_forward_call* call, const ca_
 int ca_forward(ca_handle* h, const ca_forward_call* call, void* stream);
 /* DINOv2 tokens only: tokens_out fp32 [B, 1+N, 768] (BASELINE.json configs[2]). */
 int ca_backbone(ca_handle* h, const void* images, int images_u8, int B, int S, float* tokens_out, void* stream);
+/* The same from B photographs of individual sizes (HOST arrays as in ca_forward_call.image_list / image_hw), resized to
+ * S x S by the handle. */
+int ca_backbone_list(ca_handle* h, const uint8_t* const* image_list, const int* image_hw, int B, int S, float* tokens_out,
+                     void* stream);
 /* kernels launched by the last ca_forward* / ca_backbone call of this handle (the launch-count claim of bench.py). */
 int ca_last_launch_count(const ca_handle* h);
 
