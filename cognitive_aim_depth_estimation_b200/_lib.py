@@ -93,6 +93,7 @@ class ForwardCall(C.Structure):
 
 
 SWEEP_MAX_K = 16  # CA_SWEEP_MAX_K (include/cogaim_b200.h)
+GUIDE_TAIL_MAX_B = 1  # CA_GUIDE_TAIL_MAX_B: guide calls of larger batches run the three-kernel chain
 RESIZE_MAX_SIDE = 16384  # CA_RESIZE_MAX_SIDE
 RESIZE_LIST_CHUNK = 128  # CA_RESIZE_LIST_CHUNK
 
@@ -102,6 +103,13 @@ class SweepCall(C.Structure):
     _fields_ = [("K", C.c_int), ("instructions", C.POINTER(C.c_char_p)), ("masks", C.c_void_p), ("tmp_w", C.c_void_p),
                 ("tmp_b", C.c_void_p), ("eps", C.c_void_p), ("noise", C.c_void_p), ("depth", C.c_void_p),
                 ("conf", C.c_void_p), ("attention", C.c_void_p), ("argmax", C.c_void_p)]
+
+
+class GuideCall(C.Structure):
+    """ca_guide_call (include/cogaim_b200.h)."""
+    _fields_ = [("instruction", C.c_char_p), ("mask", C.c_void_p), ("mask_batch_stride", C.c_longlong),
+                ("tmp_w", C.c_void_p), ("tmp_b", C.c_void_p), ("eps", C.c_void_p), ("noise", C.c_void_p),
+                ("depth", C.c_void_p), ("conf", C.c_void_p), ("attention", C.c_void_p), ("argmax", C.c_void_p)]
 
 
 # name -> (argtypes); every function returns int status except where noted in _RESTYPES
@@ -147,6 +155,8 @@ _SIGNATURES = {
     "ca_weighted_pool_sweep": [c_ptr, C.c_longlong, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                c_ptr],
     "ca_heads": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, c_ptr, C.c_int, c_ptr],
+    "ca_guide_tail": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, C.c_longlong, c_ptr, c_ptr, c_ptr,
+                      c_ptr, c_ptr, C.c_int, C.c_int, C.c_float, C.c_float, c_ptr],
     "ca_focal_value": [C.POINTER(FocalValueArgs), C.c_int, c_ptr],
     "ca_focal_fusion": [c_ptr, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr],
     "ca_create": [C.POINTER(C.c_void_p), C.POINTER(ModelWeights), C.c_int],
@@ -157,6 +167,10 @@ _SIGNATURES = {
     "ca_backbone": [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr],
     "ca_backbone_list": [c_ptr, C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.c_int, C.c_int, c_ptr, c_ptr],
     "ca_last_launch_count": [c_ptr],
+    "ca_encode": [c_ptr, C.POINTER(ForwardCall), C.POINTER(C.c_void_p), c_ptr],
+    "ca_guide": [c_ptr, c_ptr, C.POINTER(GuideCall), c_ptr],
+    "ca_guide_sweep": [c_ptr, c_ptr, C.POINTER(SweepCall), c_ptr],
+    "ca_scene_destroy": [c_ptr],
 }
 
 

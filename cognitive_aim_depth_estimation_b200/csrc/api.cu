@@ -206,6 +206,14 @@ int ca_heads(const ca_heads_weights* w, const ca_heads_inputs* in, float* depth,
   return ca::heads_launch(*w, *in, depth, conf, fused_out, B, static_cast<cudaStream_t>(stream));
 }
 
+int ca_guide_tail(const ca_heads_weights* w, const ca_heads_inputs* in, const float* base, const float* mask,
+                  long long mask_batch_stride, float* heat, int32_t* argmax, uint32_t* ticket, float* depth, float* conf,
+                  int B, int N, float alpha, float temperature, void* stream) {
+  if (!w || !in) return ca::invalid("guide_tail: null argument struct");
+  return ca::guide_tail_launch(*w, *in, base, mask, mask_batch_stride, heat, argmax, ticket, depth, conf, B, N, alpha,
+                               temperature, static_cast<cudaStream_t>(stream));
+}
+
 int ca_focal_value(const ca_focal_value_args* a, int B, void* stream) {
   if (!a) return ca::invalid("focal_value: null argument struct");
   return ca::focal_value_launch(*a, B, static_cast<cudaStream_t>(stream));

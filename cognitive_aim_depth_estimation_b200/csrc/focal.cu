@@ -3,11 +3,13 @@
 //   focal_finalize   : column sums of pass B -> mean + centre bias -> L1 norm -> clamp -> renorm (+ re-focus scale)
 //   guided_softmax   : softmax((0.7*mask + 0.3*a) / 0.05) and its argmax cell
 //   weighted_pool    : sum_n w[b,n] * tokens[b,1+n,:]  (bandwidth-bound, split over N, deterministic partials)
+//   guide_tail       : guided_softmax -> weighted_pool -> heads of one guided call in one launch
 // Reference: src/model.py:197-200,234-282 (FocalStream), :426 (re-focus), :1404-1414 (_guided_focal_stream).
 #include "common.cuh"
 #include "focal.cuh"
 
 #include <cuda_fp16.h>
+#include "heads_row.cuh"
 #include "host.h"
 
 namespace ca {
@@ -357,6 +359,133 @@ __global__ void __launch_bounds__(192) weighted_pool_sweep_kernel(const float* _
       reinterpret_cast<float4*>(partial + ((static_cast<size_t>(k) * B + b) * gridDim.x + split) * D)[threadIdx.x] = acc[k];
 }
 
+// The guided tail of one call in one launch: guided_softmax -> weighted_pool -> heads, bit for bit.
+// grid = (splits, B), kHeadsThreads threads.  Every CTA of image b recomputes the image's guided softmax (N <= 8192 logits
+// in shared memory) with threads 0..255 in guided_softmax_kernel's striding and reductions — both depend on the thread
+// count, so the other 768 threads only contribute the neutral elements a 256-thread block has in its idle lanes.  CTA
+// `split` then pools its rows of the tokens with threads 0..191 exactly as weighted_pool_kernel does and writes its
+// partial; the last CTA of the image (a per-image ticket, re-armed by that CTA, so nothing has to be cleared between
+// launches) runs the heads body on the 32 partials.  Split 0 writes the heat map and the argmax.
+constexpr int kTailSoftmaxThreads = 256;  // guided_softmax_kernel's block size
+constexpr int kTailPoolThreads = 192;     // weighted_pool_kernel's block size (D = 768 as float4)
+constexpr int kTailMaxN = kFinalizeThreads * kFinalizeCols;
+__global__ void __launch_bounds__(kHeadsThreads) guide_tail_kernel(const HeadsWeights wt, const HeadsInputs in,
+                                                                   const float* __restrict__ base,
+                                                                   const float* __restrict__ mask,
+                                                                   long long mask_batch_stride, float* __restrict__ heat,
+                                                                   int* __restrict__ argmax, float* partial,
+                                                                   unsigned int* __restrict__ ticket,
+                                                                   float* __restrict__ depth, float* __restrict__ conf,
+                                                                   int N, float alpha, float temperature) {
+  griddep_sync();  // PDL: nothing before this line reads or writes global memory
+  __shared__ float s_p[kTailMaxN];
+  __shared__ float red[32];
+  __shared__ int redi[32];
+  __shared__ bool s_last;
+  const int b = blockIdx.y;
+  const int split = blockIdx.x;
+  const int tid = threadIdx.x;
+  const bool soft = tid < kTailSoftmaxThreads;
+
+  // ---- guided softmax (guided_softmax_kernel, row b) ----
+  const float* mb = mask + static_cast<size_t>(b) * mask_batch_stride;
+  const float* bb = base + static_cast<size_t>(b) * N;
+  float mx = -INFINITY;
+  int mi = 0x7fffffff;
+  if (soft)
+    for (int j = tid; j < N; j += kTailSoftmaxThreads) {
+      const float t = (alpha * mb[j] + (1.0f - alpha) * bb[j]) / temperature;
+      s_p[j] = t;
+      if (t > mx) {
+        mx = t;
+        mi = j;
+      }
+    }
+  for (int o = 16; o > 0; o >>= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, mx, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, mi, o);
+    if (om > mx || (om == mx && oi < mi)) {
+      mx = om;
+      mi = oi;
+    }
+  }
+  const int w = warp_id(), l = lane_id();
+  if (l == 0) {
+    red[w] = mx;
+    redi[w] = mi;
+  }
+  __syncthreads();
+  // lanes of the idle warps hold (-inf, INT_MAX): what lanes >= 8 read in a 256-thread block
+  mx = red[l];
+  mi = redi[l];
+  for (int o = 16; o > 0; o >>= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, mx, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, mi, o);
+    if (om > mx || (om == mx && oi < mi)) {
+      mx = om;
+      mi = oi;
+    }
+  }
+  float local = 0.f;
+  if (soft)
+    for (int j = tid; j < N; j += kTailSoftmaxThreads) {
+      const float e = expf(s_p[j] - mx);
+      s_p[j] = e;
+      local += e;
+    }
+  const float tot = block_sum(local, red);  // idle warps add 0: the zero lanes of a 256-thread block_sum
+  float* hb = heat + static_cast<size_t>(b) * N;
+  if (soft)
+    for (int j = tid; j < N; j += kTailSoftmaxThreads) {
+      const float h = s_p[j] / tot;
+      s_p[j] = h;
+      if (split == 0) hb[j] = h;
+    }
+  if (split == 0 && tid == 0 && argmax) argmax[b] = mi;
+  __syncthreads();
+
+  // ---- weighted pool of this split's rows (weighted_pool_kernel, w2 = NULL, row offset 1) ----
+  if (tid < kTailPoolThreads) {
+    const int rps = (N + gridDim.x - 1) / gridDim.x;
+    const int n0 = split * rps;
+    const int n1 = min(N, n0 + rps);
+    const float4* s4 = reinterpret_cast<const float4*>(in.tokens + static_cast<size_t>(b) * in.tokens_per_img * 768 + 768);
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    constexpr int kBatch = 8;
+    for (int n = n0; n < n1; n += kBatch) {
+      float4 t[kBatch];
+      float g[kBatch];
+#pragma unroll
+      for (int u = 0; u < kBatch; ++u) {
+        const bool inr = n + u < n1;
+        t[u] = inr ? s4[static_cast<size_t>(n + u) * 192 + tid] : make_float4(0.f, 0.f, 0.f, 0.f);
+        g[u] = inr ? s_p[n + u] : 0.f;
+      }
+#pragma unroll
+      for (int u = 0; u < kBatch; ++u) {
+        acc.x = fmaf(g[u], t[u].x, acc.x);
+        acc.y = fmaf(g[u], t[u].y, acc.y);
+        acc.z = fmaf(g[u], t[u].z, acc.z);
+        acc.w = fmaf(g[u], t[u].w, acc.w);
+      }
+    }
+    reinterpret_cast<float4*>(partial + (static_cast<size_t>(b) * gridDim.x + split) * 768)[tid] = acc;
+  }
+
+  // ---- the last CTA of the image runs the heads ----
+  __threadfence();
+  __syncthreads();
+  if (tid == 0) {
+    const unsigned int t = atomicAdd(ticket + b, 1u);
+    s_last = t == gridDim.x - 1;
+    if (s_last) ticket[b] = 0u;  // every CTA of this image has taken its ticket: re-arm for the next launch
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  heads_row(wt, in, depth, conf, nullptr, b, gridDim.y);
+}
+
 }  // namespace
 
 int rowstats_merge_launch(const float* pm, const float* ps, const float* weight, float* rmax, float* rinv, float* wtab,
@@ -449,6 +578,23 @@ int weighted_pool_sweep_launch(const float* src, long long src_batch_stride, int
   else
     CA_TRY(launch_kernel(weighted_pool_sweep_kernel<kSweepMaxK>, grid, dim3(192), 0, stream, src, src_batch_stride,
                          row_offset, w, partial, K, B, N, D, rps));
+  CA_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int guide_tail_launch(const HeadsWeights& w, const HeadsInputs& in, const float* base, const float* mask,
+                      long long mask_batch_stride, float* heat, int* argmax, unsigned int* ticket, float* depth,
+                      float* conf, int B, int N, float alpha, float temperature, cudaStream_t stream) {
+  CA_REQUIRE(base && mask && heat && ticket && depth && conf && in.tokens, "guide_tail: null pointer");
+  CA_REQUIRE(in.focal_feat == nullptr && in.sweep_images == 0, "guide_tail: guided single calls only (no focal_feat, no sweep)");
+  CA_REQUIRE(in.pool_partial && in.tmp_w && in.tmp_b && in.pool_splits > 0, "guide_tail: pool partials and projection needed");
+  CA_REQUIRE(in.exif == nullptr || in.camera_idx != nullptr, "guide_tail: EXIF given without camera_idx");
+  CA_REQUIRE(B > 0 && N > 0 && N <= kTailMaxN, "guide_tail: B > 0 and 0 < N <= 8192");
+  CA_REQUIRE(in.tokens_per_img == N + 1, "guide_tail: tokens_per_img must be N + 1 (CLS + patch tokens)");
+  CA_REQUIRE(mask_batch_stride == 0 || mask_batch_stride >= N, "guide_tail: mask batch stride must be 0 or >= N");
+  CA_TRY(launch_kernel(guide_tail_kernel, dim3(in.pool_splits, B), dim3(kHeadsThreads), 0, stream, w, in, base, mask,
+                       mask_batch_stride, heat, argmax, const_cast<float*>(in.pool_partial), ticket, depth, conf, N, alpha,
+                       temperature));
   CA_CUDA(cudaGetLastError());
   return 0;
 }

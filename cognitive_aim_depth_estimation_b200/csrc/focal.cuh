@@ -3,6 +3,8 @@
 
 #include <cuda_runtime.h>
 
+#include "heads.cuh"
+
 namespace ca {
 
 int rowstats_merge_launch(const float* pm, const float* ps, const float* weight, float* rmax, float* rinv, float* wtab,
@@ -16,6 +18,11 @@ int guided_softmax_launch(const float* base, const float* mask, long long mask_b
                           int B, int N, float alpha, float temperature, cudaStream_t stream);
 int weighted_pool_launch(const float* src, long long src_batch_stride, int row_offset, const float* w, const float* w2,
                          float* partial, int B, int N, int D, int splits, cudaStream_t stream);
+// guided_softmax -> weighted_pool (in.pool_splits splits) -> heads in one launch, bit for bit; ticket: [B] zero-initialised
+// counters, left at zero by every launch.
+int guide_tail_launch(const HeadsWeights& w, const HeadsInputs& in, const float* base, const float* mask,
+                      long long mask_batch_stride, float* heat, int* argmax, unsigned int* ticket, float* depth,
+                      float* conf, int B, int N, float alpha, float temperature, cudaStream_t stream);
 
 // Instruction sweeps (include/cogaim_b200.h, CA_SWEEP_MAX_K): K guidance rows per image in one launch.
 constexpr int kSweepMaxK = 16;

@@ -17,7 +17,11 @@
 #include <math.h>
 #include <string.h>
 
+#include <atomic>
+
 #include <map>
+#include <mutex>
+#include <set>
 #include <string>
 #include <tuple>
 #include <vector>
@@ -45,12 +49,14 @@ struct Tables {
 
 struct Workspace {
   int B = 0, S = 0;
+  unsigned long long gen = 0;  // unique per allocation: a scene's graphs captured on another workspace are not replayed
   void* arena = nullptr;
   __nv_bfloat16 *patches, *h, *qkv, *att, *mlp, *xin, *qk;
   float *x, *tokens, *pm, *ps, *pc, *wtab, *attn, *cvec, *rowscale, *heat, *pool, *pool_pe, *pooled, *feats, *focal_feat,
       *fused, *depth, *conf, *mask_in, *tmpw, *tmpb, *exif_in, *cur_eps, *cur_noise, *cur_raw, *cur_reward, *ln_stats;
   void* E;
   int* argmax;
+  int* tail_ticket;  // [B] per-image tickets of the fused guide tail, zero when idle
   long long* cam_in;
   int P = 0, lde = 0;
   std::map<int, std::pair<cudaGraphExec_t, int>> graphs;  // path key -> (executable graph, launches)
@@ -95,6 +101,22 @@ struct ca_handle {
   // resize temporary, grow-only
   uint8_t* resize_buf = nullptr;
   size_t resize_cap = 0;
+  unsigned long long id = 0;  // unique per handle: scenes record it (a later handle may reuse the address)
+};
+
+// A scene (ca_encode): buffers it owns in one device allocation, the handle it belongs to (by id, never dereferenced
+// once that handle is gone), and the graphs of its guide calls, captured on its own buffers and one workspace.
+struct ca_scene {
+  unsigned long long handle_id = 0;
+  int device = 0, B = 0, S = 0;
+  void* arena = nullptr;
+  float *tokens = nullptr, *base = nullptr, *exif = nullptr;
+  long long* cam = nullptr;
+  int* fault = nullptr;
+  bool use_graph = false;
+  unsigned long long ws_gen = 0;                           // workspace the graphs below were captured on
+  std::map<int, std::pair<cudaGraphExec_t, int>> graphs;  // path key -> (executable graph, launches)
+  std::map<int, int> seen;                                // path key -> calls so far
 };
 
 namespace {
@@ -325,6 +347,7 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   want(&w.tmpb, 64 * 4);
   want(&w.exif_in, B * 3 * 4);
   want(&w.cam_in, B * 8);
+  want(&w.tail_ticket, B * 4);
   want(&w.cur_eps, static_cast<size_t>(kMaxRuns) * B * 192 * 4);
   want(&w.cur_noise, static_cast<size_t>(kMaxRuns) * B * kD * 4);
   want(&w.cur_raw, static_cast<size_t>(kMaxRuns) * B * 4);
@@ -333,6 +356,9 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   for (auto& s : slots) *s.p = static_cast<char*>(w.arena) + s.o;
   CA_CUDA(cudaMemset(w.exif_in, 0, B * 3 * 4));
   CA_CUDA(cudaMemset(w.cam_in, 0, B * 8));
+  CA_CUDA(cudaMemset(w.tail_ticket, 0, B * 4));
+  static std::atomic<unsigned long long> next_gen{1};
+  w.gen = next_gen.fetch_add(1);
   *out = &h->ws.emplace(key, w).first->second;
   return 0;
 }
@@ -532,12 +558,12 @@ int focal_iterations(ca_handle* h, Workspace& w, const Tables& tb, bool want_fea
 // dependencies: during capture they become a parallel branch of the graph.
 // eps / noise / raw / reward: [runs, B, ...] buffers of the runs (the workspace's, or an instruction sweep's).
 int curiosity_fork(ca_handle* h, Workspace& w, int runs, const float* eps, const float* noise, float* raw, float* reward,
-                   cudaStream_t st) {
+                   cudaStream_t st, const float* tokens = nullptr) {
   const int B = w.B, g = w.S / 14, T = g * g + 1;
   CA_CUDA(cudaEventRecord(h->fork, st));
   CA_CUDA(cudaStreamWaitEvent(h->side, h->fork, 0));
   for (int j = 0; j < runs; ++j) {
-    CA_TRY(ca::curiosity_launch(h->w.curiosity, w.tokens, T, eps + static_cast<size_t>(j) * B * 192,
+    CA_TRY(ca::curiosity_launch(h->w.curiosity, tokens ? tokens : w.tokens, T, eps + static_cast<size_t>(j) * B * 192,
                                 noise + static_cast<size_t>(j) * B * kD, raw + static_cast<size_t>(j) * B,
                                 reward + static_cast<size_t>(j) * B, h->w.exploration_history, h->w.history_len,
                                 h->w.history_pointer, B, h->side));
@@ -683,12 +709,13 @@ int patch_rows(ca_handle* h, Workspace& w, const ImagesIn& in, cudaStream_t st) 
 // Run `seq` eagerly the first time a path key is seen on this workspace, capture + instantiate it the second time, replay
 // the graph afterwards.
 template <class F>
-int run_sequence(ca_handle* h, Workspace& w, int key, bool use_graph, cudaStream_t st, F&& seq) {
-  const int calls = w.seen[key]++;
-  auto g = w.graphs.find(key);
+int run_captured(ca_handle* h, std::map<int, std::pair<cudaGraphExec_t, int>>& graphs, std::map<int, int>& seen, int key,
+                 bool use_graph, cudaStream_t st, F&& seq) {
+  const int calls = seen[key]++;
+  auto g = graphs.find(key);
   // (the legacy default stream cannot be captured: such callers get eager launches)
   if (!use_graph || calls == 0 || st == nullptr) return seq();
-  if (g == w.graphs.end()) {
+  if (g == graphs.end()) {
     const int before = h->launches;
     CA_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeRelaxed));
     const int status = seq();
@@ -703,11 +730,49 @@ int run_sequence(ca_handle* h, Workspace& w, int key, bool use_graph, cudaStream
     const cudaError_t ei = cudaGraphInstantiate(&exec, graph, 0);
     cudaGraphDestroy(graph);
     CA_CUDA(ei);
-    g = w.graphs.emplace(key, std::make_pair(exec, h->launches - before)).first;
+    g = graphs.emplace(key, std::make_pair(exec, h->launches - before)).first;
     h->launches = before;
   }
   CA_CUDA(cudaGraphLaunch(g->second.first, st));
   h->launches += g->second.second;
+  return 0;
+}
+
+template <class F>
+int run_sequence(ca_handle* h, Workspace& w, int key, bool use_graph, cudaStream_t st, F&& seq) {
+  return run_captured(h, w.graphs, w.seen, key, use_graph, st, static_cast<F&&>(seq));
+}
+
+// Live handles and scenes: a scene is only used while its handle lives, and a destroyed scene is never touched again.
+std::mutex g_live_mu;
+std::map<const ca_handle*, unsigned long long> g_live_handles;
+std::set<const ca_scene*> g_live_scenes;
+std::atomic<unsigned long long> g_next_handle_id{1};
+
+int check_scene(const ca_handle* h, const ca_scene* sc) {
+  std::lock_guard<std::mutex> lock(g_live_mu);
+  CA_REQUIRE(h && sc, "null handle / scene");
+  auto it = g_live_handles.find(h);
+  CA_REQUIRE(it != g_live_handles.end(), "the handle has been destroyed");
+  CA_REQUIRE(g_live_scenes.count(sc) != 0, "the scene has been destroyed");
+  CA_REQUIRE(sc->handle_id == it->second, "the scene belongs to another (possibly destroyed) handle");
+  return 0;
+}
+
+void drop_scene_graphs(ca_scene* sc) {
+  for (auto& g : sc->graphs) cudaGraphExecDestroy(g.second.first);
+  sc->graphs.clear();
+  sc->seen.clear();
+}
+
+// The workspace a guide call of `sc` runs on; the scene's graphs are dropped when it is not the one they were captured on.
+int scene_workspace(ca_handle* h, ca_scene* sc, Workspace** out, Tables** tb) {
+  CA_TRY(get_workspace(h, sc->B, sc->S, out));
+  CA_TRY(get_tables(h, sc->S / 14, tb));
+  if (sc->ws_gen != (*out)->gen) {
+    drop_scene_graphs(sc);
+    sc->ws_gen = (*out)->gen;
+  }
   return 0;
 }
 
@@ -758,12 +823,21 @@ int ca_create(ca_handle** out, const ca_model_weights* w, int device) {
     delete h;
     return ca::cuda_fail(cudaGetLastError(), "ca_create: stream / event creation", __FILE__, __LINE__);
   }
+  {
+    std::lock_guard<std::mutex> lock(g_live_mu);
+    h->id = g_next_handle_id.fetch_add(1);
+    g_live_handles[h] = h->id;
+  }
   *out = h;
   return 0;
 }
 
 int ca_destroy(ca_handle* h) {
   if (!h) return 0;
+  {
+    std::lock_guard<std::mutex> lock(g_live_mu);
+    g_live_handles.erase(h);  // its scenes are refused from now on
+  }
   DeviceGuard guard(h->device);
   cudaDeviceSynchronize();
   for (auto& kv : h->ws) free_workspace(kv.second);
@@ -989,6 +1063,215 @@ int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
   if (c->attention) CA_CUDA(cudaMemcpyAsync(c->attention, att, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
   if (c->fused) CA_CUDA(cudaMemcpyAsync(c->fused, w.fused, static_cast<size_t>(B) * 192 * 4, cudaMemcpyDeviceToDevice, st));
   h->last_launches = h->launches;
+  return 0;
+}
+
+
+int ca_encode(ca_handle* h, const ca_forward_call* c, ca_scene** out, void* stream) {
+  CA_REQUIRE(h && c && out, "encode: null handle / call / out");
+  {
+    std::lock_guard<std::mutex> lock(g_live_mu);
+    CA_REQUIRE(g_live_handles.count(h) != 0, "encode: the handle has been destroyed");
+  }
+  CA_REQUIRE(c->B > 0, "encode: empty batch");
+  CA_TRY(check_images(images_of(*c)));
+  CA_REQUIRE(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260, "encode: image side must be a multiple of 14 in [56, 1260]");
+  CA_REQUIRE(c->exif && c->camera_idx, "encode: EXIF inputs are required (without them the reference falls back to "
+                                       "forward(): call ca_forward)");
+  CA_REQUIRE(!c->instruction && !c->mask && !c->tmp_w && !c->tmp_b && !c->eps && !c->noise && !c->depth && !c->conf &&
+                 !c->attention && !c->argmax && !c->fused,
+             "encode: the per-call fields of ca_forward_call must be NULL (they go in ca_guide_call / ca_sweep_call)");
+  DeviceGuard guard(h->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int B = c->B, S = c->S, g = S / 14, N = g * g, T = N + 1;
+  Workspace* wp = nullptr;
+  Tables* tb = nullptr;
+  CA_TRY(get_workspace(h, B, S, &wp));
+  CA_TRY(get_tables(h, g, &tb));
+  Workspace& w = *wp;
+  h->launches = 0;
+  CA_TRY(patch_rows(h, w, images_of(*c), st));
+  float* base = nullptr;
+  CA_TRY(run_sequence(h, w, 400, c->use_graph != 0, st, [&]() -> int {
+    CA_TRY(backbone_layers(h, w, *tb, st));
+    return focal_iterations(h, w, *tb, false, st, &base);
+  }));
+  base = w.attn + static_cast<size_t>(h->w.n_focal - 1) * B * N;
+  const size_t tok = static_cast<size_t>(B) * T * kD * 4, bn = static_cast<size_t>(B) * N * 4;
+  const size_t o_base = (tok + 255) & ~size_t(255), o_exif = o_base + ((bn + 255) & ~size_t(255));
+  const size_t o_cam = o_exif + 256 * ((static_cast<size_t>(B) * 12 + 255) / 256);
+  ca_scene* sc = new ca_scene();
+  if (cudaMalloc(&sc->arena, o_cam + static_cast<size_t>(B) * 8) != cudaSuccess) {
+    delete sc;
+    return ca::cuda_fail(cudaGetLastError(), "encode: scene allocation", __FILE__, __LINE__);
+  }
+  char* a = static_cast<char*>(sc->arena);
+  sc->tokens = reinterpret_cast<float*>(a);
+  sc->base = reinterpret_cast<float*>(a + o_base);
+  sc->exif = reinterpret_cast<float*>(a + o_exif);
+  sc->cam = reinterpret_cast<long long*>(a + o_cam);
+  sc->handle_id = h->id;
+  sc->device = h->device;
+  sc->B = B;
+  sc->S = S;
+  sc->fault = c->fault;
+  sc->use_graph = c->use_graph != 0;
+  const int status = [&]() -> int {
+    CA_CUDA(cudaMemcpyAsync(sc->tokens, w.tokens, tok, cudaMemcpyDeviceToDevice, st));
+    CA_CUDA(cudaMemcpyAsync(sc->base, base, bn, cudaMemcpyDeviceToDevice, st));
+    CA_CUDA(cudaMemcpyAsync(sc->exif, c->exif, static_cast<size_t>(B) * 12, cudaMemcpyDeviceToDevice, st));
+    CA_CUDA(cudaMemcpyAsync(sc->cam, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
+    return 0;
+  }();
+  if (status != 0) {
+    cudaFree(sc->arena);
+    delete sc;
+    return status;
+  }
+  {
+    std::lock_guard<std::mutex> lock(g_live_mu);
+    g_live_scenes.insert(sc);
+  }
+  h->last_launches = h->launches;
+  *out = sc;
+  return 0;
+}
+
+int ca_guide(ca_handle* h, ca_scene* sc, const ca_guide_call* c, void* stream) {
+  CA_TRY(check_scene(h, sc));
+  CA_REQUIRE(c, "guide: null call");
+  CA_REQUIRE((c->instruction != nullptr) != (c->mask != nullptr), "guide: give an instruction OR a mask");
+  CA_REQUIRE(c->tmp_w && c->tmp_b && c->eps && c->noise,
+             "guide: null per-call projection or CuriosityModule draws (HOST pointers, src/model.py:609,744,1421)");
+  CA_REQUIRE(c->depth && c->conf && c->attention, "guide: null output");
+  DeviceGuard guard(h->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int B = sc->B, g = sc->S / 14, N = g * g, T = N + 1;
+  Workspace* wp = nullptr;
+  Tables* tb = nullptr;
+  CA_TRY(scene_workspace(h, sc, &wp, &tb));
+  Workspace& w = *wp;
+  h->launches = 0;
+  const float* mask = c->mask;
+  long long mstride = c->mask_batch_stride;
+  if (c->instruction) {
+    float* m = nullptr;
+    CA_TRY(get_mask(tb, c->instruction, g, &m));
+    mask = m;
+    mstride = 0;
+  }
+  CA_REQUIRE(mstride == 0 || mstride == N, "guide: mask batch stride must be 0 or N");
+  ca_forward_call staged{};
+  staged.tmp_w = c->tmp_w;
+  staged.tmp_b = c->tmp_b;
+  staged.eps = c->eps;
+  staged.noise = c->noise;
+  CA_TRY(stage_host_inputs(h, w, staged, true, 1, st));
+  CA_CUDA(cudaMemcpyAsync(w.mask_in, mask, static_cast<size_t>(mstride ? B : 1) * N * 4, cudaMemcpyDeviceToDevice, st));
+  CA_TRY(run_captured(h, sc->graphs, sc->seen, 1 + (mstride ? 1 : 0), sc->use_graph, st, [&]() -> int {
+    CA_TRY(curiosity_fork(h, w, 1, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st, sc->tokens));
+    ca_heads_inputs in{};
+    in.tokens = sc->tokens;
+    in.tokens_per_img = T;
+    in.pool_partial = w.pool;
+    in.pool_splits = kPoolSplits;
+    in.tmp_w = w.tmpw;
+    in.tmp_b = w.tmpb;
+    in.exif = sc->exif;
+    in.camera_idx = sc->cam;
+    in.num_cameras = h->w.num_cameras;
+    in.fault = sc->fault;
+    if (B <= CA_GUIDE_TAIL_MAX_B) {
+      LAUNCH(ca::guide_tail_launch(h->w.heads, in, sc->base, w.mask_in, mstride ? N : 0, w.heat, w.argmax, reinterpret_cast<unsigned int*>(w.tail_ticket),
+                                   w.depth, w.conf, B, N, 0.7f, 0.05f, st));
+    } else {
+      LAUNCH(ca::guided_softmax_launch(sc->base, w.mask_in, mstride ? N : 0, w.heat, w.argmax, B, N, 0.7f, 0.05f, st));
+      LAUNCH(ca::weighted_pool_launch(sc->tokens, static_cast<long long>(T) * kD, 1, w.heat, nullptr, w.pool, B, N, kD,
+                                      kPoolSplits, st));
+      LAUNCH(ca::heads_launch(h->w.heads, in, w.depth, w.conf, nullptr, B, st));
+    }
+    return curiosity_join(h, st);
+  }));
+  CA_CUDA(cudaMemcpyAsync(c->depth, w.depth, B * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c->conf, w.conf, B * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c->attention, w.heat, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
+  if (c->argmax) CA_CUDA(cudaMemcpyAsync(c->argmax, w.argmax, B * 4, cudaMemcpyDeviceToDevice, st));
+  h->last_launches = h->launches;
+  return 0;
+}
+
+int ca_guide_sweep(ca_handle* h, ca_scene* sc, const ca_sweep_call* sw, void* stream) {
+  CA_TRY(check_scene(h, sc));
+  CA_REQUIRE(sw, "guide_sweep: null sweep");
+  const int K = sw->K;
+  CA_REQUIRE(K >= 1 && K <= CA_SWEEP_MAX_K, "guide_sweep: K must be in 1..CA_SWEEP_MAX_K (16)");
+  CA_REQUIRE((sw->instructions != nullptr) != (sw->masks != nullptr), "guide_sweep: give instructions OR masks");
+  if (sw->instructions)
+    for (int k = 0; k < K; ++k) CA_REQUIRE(sw->instructions[k], "guide_sweep: null instruction string");
+  CA_REQUIRE(sw->tmp_w && sw->tmp_b && sw->eps && sw->noise,
+             "guide_sweep: null per-call projections or CuriosityModule draws (HOST pointers)");
+  CA_REQUIRE(sw->depth && sw->conf && sw->attention, "guide_sweep: null output");
+  DeviceGuard guard(h->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int B = sc->B, g = sc->S / 14, N = g * g, T = N + 1;
+  Workspace* wp = nullptr;
+  Tables* tb = nullptr;
+  CA_TRY(scene_workspace(h, sc, &wp, &tb));
+  Workspace& w = *wp;
+  Workspace::Sweep* sp = nullptr;
+  CA_TRY(get_sweep(w, K, &sp));
+  Workspace::Sweep& s = *sp;
+  h->launches = 0;
+  if (sw->instructions) {
+    for (int k = 0; k < K; ++k) {
+      float* m = nullptr;
+      CA_TRY(get_mask(tb, sw->instructions[k], g, &m));
+      CA_CUDA(cudaMemcpyAsync(s.mask_in + static_cast<size_t>(k) * N, m, static_cast<size_t>(N) * 4, cudaMemcpyDeviceToDevice, st));
+    }
+  } else {
+    CA_CUDA(cudaMemcpyAsync(s.mask_in, sw->masks, static_cast<size_t>(K) * N * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  CA_TRY(stage_sweep_inputs(h, w, s, *sw, st));
+  CA_TRY(run_captured(h, sc->graphs, sc->seen, 100 + K, sc->use_graph, st, [&]() -> int {
+    CA_TRY(curiosity_fork(h, w, K, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st, sc->tokens));
+    LAUNCH(ca::guided_softmax_sweep_launch(sc->base, 0, s.mask_in, N, 0, s.heat, s.argmax, K, B, N, 0.7f, 0.05f, st));
+    LAUNCH(ca::weighted_pool_sweep_launch(sc->tokens, static_cast<long long>(T) * kD, 1, s.heat, s.pool, K, B, N, kD,
+                                          kPoolSplits, st));
+    ca_heads_inputs in{};
+    in.tokens = sc->tokens;
+    in.tokens_per_img = T;
+    in.pool_partial = s.pool;
+    in.pool_splits = kPoolSplits;
+    in.tmp_w = s.tmpw;
+    in.tmp_b = s.tmpb;
+    in.exif = sc->exif;
+    in.camera_idx = sc->cam;
+    in.num_cameras = h->w.num_cameras;
+    in.fault = sc->fault;
+    in.sweep_images = B;
+    LAUNCH(ca::heads_launch(h->w.heads, in, s.depth, s.conf, nullptr, K * B, st));
+    return curiosity_join(h, st);
+  }));
+  const size_t KB = static_cast<size_t>(K) * B;
+  CA_CUDA(cudaMemcpyAsync(sw->depth, s.depth, KB * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(sw->conf, s.conf, KB * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(sw->attention, s.heat, KB * N * 4, cudaMemcpyDeviceToDevice, st));
+  if (sw->argmax) CA_CUDA(cudaMemcpyAsync(sw->argmax, s.argmax, KB * 4, cudaMemcpyDeviceToDevice, st));
+  h->last_launches = h->launches;
+  return 0;
+}
+
+int ca_scene_destroy(ca_scene* sc) {
+  if (!sc) return 0;
+  {
+    std::lock_guard<std::mutex> lock(g_live_mu);
+    CA_REQUIRE(g_live_scenes.count(sc) != 0, "scene_destroy: not a live scene (already destroyed?)");
+    g_live_scenes.erase(sc);
+  }
+  DeviceGuard guard(sc->device);
+  drop_scene_graphs(sc);
+  cudaFree(sc->arena);  // waits for the work that still reads it
+  delete sc;
   return 0;
 }
 

@@ -23,6 +23,7 @@ import contextlib
 import functools
 import math
 import os
+import weakref
 from typing import Dict, Optional
 
 import torch
@@ -30,6 +31,7 @@ import torch.nn as nn
 
 from . import ops, tables
 from ._lib import RESIZE_MAX_SIDE as _RESIZE_MAX_SIDE  # largest photograph side the resize stages in shared memory
+from ._lib import GUIDE_TAIL_MAX_B as _GUIDE_TAIL_MAX_B  # guide calls of larger batches run the three-kernel tail
 from ._lib import SWEEP_MAX_K as _SWEEP_MAX_K  # instructions per sweep: the sweep pool keeps one accumulator each
 from .config import DEFAULT_COGNITIVE_MODULES, EffectiveConfig, effective_config
 from .init import reference_init_
@@ -158,6 +160,24 @@ def _register(root: nn.Module, dotted: str, tensor: torch.Tensor, buffer: bool):
         mod.register_parameter(parts[-1], nn.Parameter(tensor, requires_grad=False))
 
 
+class Scene:
+    """The instruction-independent part of a guided call over one batch, kept for any number of later instructions
+    (`CognitiveAimModel.encode` -> `guide` / `guide_sweep`).  Owns its buffers: the backbone tokens [B, T, 768] fp32
+    (not the workspace the next forward overwrites), the last focal iteration's attention [B, N] (None with
+    curiosity-guided attention, where every call's focal pass depends on its own curiosity score), the EXIF and camera
+    indices on the device, and the CUDA graphs captured on these buffers.  Everything is released with the scene.
+    Valid for the model and weights it was encoded with: re-packed weights (`load_state_dict`, `.to()`,
+    `set_lora_adapters`) make it stale."""
+
+    def __init__(self, model, B: int, S: int, tokens, base, exif, cam):
+        self._model = weakref.ref(model)
+        self._stamp = model._weights_version
+        self.B, self.S, self.device = B, S, tokens.device
+        self.tokens, self.base, self.exif, self.camera_idx = tokens, base, exif, cam
+        self._graphs: Dict = {}
+        self._guided = 0
+
+
 class CognitiveAimModel(nn.Module):
     """Drop-in for the reference `CognitiveAimModel` (inference only)."""
 
@@ -203,6 +223,7 @@ class CognitiveAimModel(nn.Module):
             t = torch.tensor(0) if kind == "buf_long" else torch.zeros(shape)
             _register(self, name, t, buffer=kind.startswith("buf"))
         reference_init_(dict(self.state_dict(keep_vars=True)), cfg)
+        self._weights_version = 0  # bumped whenever the packed weights change: a Scene records it
         self._packed = None       # device-side packed weights (bf16 GEMM operands etc.)
         self._packed_key = None
         self._tables: Dict = {}   # per-grid tables (pos-embed, PE, centre bias, masks)
@@ -233,6 +254,7 @@ class CognitiveAimModel(nn.Module):
         return super().load_state_dict(state_dict, strict=strict, assign=assign)
 
     def _invalidate(self):
+        self._weights_version = getattr(self, "_weights_version", 0) + 1  # scenes encoded before are stale
         self._packed = None
         self._tables = {}
         self._ws = {}
@@ -292,6 +314,7 @@ class CognitiveAimModel(nn.Module):
         pk = self._pack()
         for i, (A, Bm) in adapters.items():
             self._write_lora(pk["layers"][i], A, Bm)
+        self._weights_version += 1
 
     def _device(self) -> torch.device:
         return self.backbone.layernorm.weight.device
@@ -482,6 +505,8 @@ class CognitiveAimModel(nn.Module):
                 # LayerNorm folding: per (row, 128-column span) (sum, M2) of the residual row; `h` then holds the raw rows
                 "ln_stats": torch.empty(B * T, _D // 128, 2, **fl),
                 "heat": torch.empty(B, N, **fl), "argmax": torch.empty(B, device=dev, dtype=torch.int32),
+                # per-image tickets of ops.guide_tail: zero here, and every launch leaves them at zero
+                "tail_ticket": torch.zeros(B, device=dev, dtype=torch.int32),
                 "pool": torch.empty(B, _POOL_SPLITS, _D, **fl), "pool_pe": torch.empty(B, _POOL_SPLITS, _D, **fl),
                 "pooled": torch.empty(B, _D, **fl), "feats": torch.empty(B, self.cfg.num_iterations, 64, **fl),
                 "focal_feat": torch.empty(B, 64, **fl), "fused": torch.empty(B, 192, **fl),
@@ -673,14 +698,17 @@ class CognitiveAimModel(nn.Module):
             ops.layernorm(x, pk["lnw"], pk["lnb"], ws["tokens"].view(B * T, _D))
         return ws["tokens"]
 
-    def _run(self, ws, key, fn):
+    def _run(self, ws, key, fn, graphs=None):
         """Run `fn` (a fixed sequence of launches on fixed buffers): eagerly, or — with `use_cuda_graphs` — captured
         once per key and replayed.  The first call runs eagerly as well: it performs the library's one-time
-        allocations and attribute settings, which are illegal during capture."""
+        allocations and attribute settings, which are illegal during capture.  `graphs`: the store of the graphs
+        (default: the workspace's)."""
         if not self.use_cuda_graphs or ops.tracing_events():
             fn()
             return
-        graph = ws["graphs"].get(key)
+        if graphs is None:
+            graphs = ws["graphs"]
+        graph = graphs.get(key)
         if graph is None:
             fn()
             graph = torch.cuda.CUDAGraph()
@@ -688,9 +716,10 @@ class CognitiveAimModel(nn.Module):
                 n0 = ops.launch_count()
                 fn()
                 launches = ops.launch_count() - n0
-            ws["graphs"][key] = (graph, launches)
-            if len(ws["graphs"]) > 8:
-                ws["graphs"].pop(next(iter(ws["graphs"])))
+            # a graph kept outside the workspace (a Scene's) keeps the workspace buffers it reads alive
+            graphs[key] = (graph, launches) if graphs is ws["graphs"] else (graph, launches, ws)
+            if len(graphs) > 8:
+                graphs.pop(next(iter(graphs)))
             return  # the eager run above produced this call's results
         graph[0].replay()
         ops.count_launches(graph[1])
@@ -976,6 +1005,71 @@ class CognitiveAimModel(nn.Module):
         for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb"), bufs):
             ops.fetch_pinned(sw[dst], buf)
 
+    @staticmethod
+    def _check_guidances(guidances):
+        """K of an instruction sweep's guidance list (checked before anything is drawn or launched)."""
+        if not isinstance(guidances, (list, tuple)):
+            raise ValueError("guidances must be a list of K instructions / guidance tensors / per-image lists")
+        K = len(guidances)
+        if not 1 <= K <= _SWEEP_MAX_K:
+            raise ValueError(f"an instruction sweep takes 1..{_SWEEP_MAX_K} guidances, got {K}")
+        if any(gd is None for gd in guidances):
+            raise ValueError("a None guidance runs the un-guided focal path (src/model.py:1206-1212): use "
+                             "forward_with_guidance for it")
+        return K
+
+    def _sweep_masks(self, guidances, B: int, g: int) -> torch.Tensor:
+        """[K, B, N] masks of a sweep: strings and [N] guidance broadcast over the batch."""
+        N = g * g
+        masks = []
+        for gd in guidances:
+            m = self._mask(gd, g)
+            if m.dim() == 2 and m.shape[0] != B:
+                raise ValueError(f"{m.shape[0]} per-image instructions for a batch of {B}")
+            masks.append(m.expand(B, N))
+        return torch.stack(masks)
+
+    def _stage_sweep_call(self, ws, mask, B: int, S: int, K: int):
+        """The K calls' random draws (in the reference's order) and masks -> the sweep buffers; returns them."""
+        draws = self._sweep_draws(B, K)
+        sw = self._sweep_buffers(ws, B, S, K)
+        slot = self._pinned_slot()
+        self._stage_sweep(sw, slot, draws, B, K)
+        slot["event"].record()
+        sw["mask_in"].copy_(mask, non_blocking=True)
+        return sw
+
+    def _sweep_device(self, sw, B: int, g: int, K: int, base, exif, cam):
+        """Device side of a sweep after the backbone: the K CuriosityModule runs, the focal pass (`base` [B, N] when it
+        is shared; with curiosity-guided attention one pass per call on sw['tokens']), then the sweep's softmax, pool
+        and heads.  Shared by `forward_with_guidance_sweep` and `guide_sweep` (which reads a Scene's tokens)."""
+        pk = self._packed
+        N, T = g * g, g * g + 1
+        self._curiosity_runs(sw, B, T, ("guided",) * K)
+        if self.cfg.curiosity_guided:
+            # each call's focal attention is modulated by its own curiosity score (src/model.py:264-276)
+            for k in range(K):
+                sw["base"][k].copy_(self._focal_iterations(sw, B, g, want_features=False, cur_weight=sw["cur_weight"][k]))
+            base, base_k_stride = sw["base"], B * N
+        else:
+            base, base_k_stride = (self._focal_iterations(sw, B, g, want_features=False) if base is None else base), 0
+        ops.guided_softmax_sweep(base, base_k_stride, sw["mask_in"], sw["heat"], sw["argmax"], K, B, N)
+        ops.weighted_pool_sweep(sw["tokens"], T * _D, 1, sw["heat"], sw["pool"], K, B, N, _D, _POOL_SPLITS)
+        ops.heads(pk["heads"], tokens=sw["tokens"], tokens_per_img=T, depth=sw["depth"], conf=sw["conf"], B=K * B,
+                  pool_partial=sw["pool"], pool_splits=_POOL_SPLITS, tmp_w=sw["tmpw"], tmp_b=sw["tmpb"],
+                  exif=exif, camera_idx=cam, num_cameras=self.cfg.num_cameras,
+                  fault_ptr=self._fault_word().data_ptr(), sweep_images=B)
+        self._curiosity_join()
+
+    def _sweep_results(self, sw, K: int, return_attention: bool):
+        heat = sw["heat"].clone()
+        # what the last of the K calls leaves behind
+        self._last_attention_weights = heat[K - 1]
+        self._last_argmax = sw["argmax"][K - 1].clone()
+        self._last_curiosity = sw["cur_reward"][K - 1]
+        depth, conf = sw["depth"].clone().unsqueeze(-1), sw["conf"].clone().unsqueeze(-1)
+        return (depth, conf, heat) if return_attention else (depth, conf)
+
     @torch.no_grad()
     @_on_own_device
     def forward_with_guidance_sweep(self, images, exif_data, guidances, return_attention=False):
@@ -986,14 +1080,7 @@ class CognitiveAimModel(nn.Module):
         accepts: an instruction string or alias, a guidance tensor [N'], or a list of B per-image instructions.
         Returns depth [K, B, 1], confidence [K, B, 1] (and the heat maps [K, B, N] with `return_attention`)."""
         self._raise_on_fault()
-        if not isinstance(guidances, (list, tuple)):
-            raise ValueError("guidances must be a list of K instructions / guidance tensors / per-image lists")
-        K = len(guidances)
-        if not 1 <= K <= _SWEEP_MAX_K:
-            raise ValueError(f"an instruction sweep takes 1..{_SWEEP_MAX_K} guidances, got {K}")
-        if any(gd is None for gd in guidances):
-            raise ValueError("a None guidance runs the un-guided focal path (src/model.py:1206-1212): use "
-                             "forward_with_guidance for it")
+        K = self._check_guidances(guidances)
         if exif_data is None or not self.use_exif:
             raise ValueError("an instruction sweep needs EXIF data and a model with the EXIF prior (otherwise the "
                              "reference falls back to forward(): use forward_with_guidance)")
@@ -1001,57 +1088,184 @@ class CognitiveAimModel(nn.Module):
         for gd in guidances:
             self._check_per_image(gd, B)
         self._check_exif(exif_data, B)
-        pk = self._pack()
+        self._pack()
         g = S // 14
-        N, T = g * g, g * g + 1
-        masks = []
-        for gd in guidances:
-            m = self._mask(gd, g)
-            if m.dim() == 2 and m.shape[0] != B:
-                raise ValueError(f"{m.shape[0]} per-image instructions for a batch of {B}")
-            masks.append(m.expand(B, N))
-        mask = torch.stack(masks)  # [K, B, N]: strings and [N] guidance broadcast over the batch
+        mask = self._sweep_masks(guidances, B, g)
         exif, cam = self._exif_tensors(exif_data, B)
-        draws = self._sweep_draws(B, K)
         ws = self._workspace(B, S)
-        sw = self._sweep_buffers(ws, B, S, K)
-        slot = self._pinned_slot()
-        self._stage_sweep(sw, slot, draws, B, K)
-        slot["event"].record()
-        sw["mask_in"].copy_(mask, non_blocking=True)
+        sw = self._stage_sweep_call(ws, mask, B, S, K)
         ws["exif_in"].copy_(exif, non_blocking=True)
         ws["cam_in"].copy_(cam, non_blocking=True)
+        self._grid_tables(g)
+        patches, images = self._patch_rows(images, ws, S)
+
+        def device_pass():
+            self._backbone_layers(ws, patches, B, S)
+            self._sweep_device(sw, B, g, K, None, ws["exif_in"], ws["cam_in"])
+
+        self._run(ws, ("sweep", K, self._curiosity_key()), device_pass)
+        self._keepalive = (exif, cam, mask, images)
+        return self._sweep_results(sw, K, return_attention)
+
+    # -- scenes: encode a batch once, guide it any number of times ---------------------------------------
+    @torch.no_grad()
+    @_on_own_device
+    def encode(self, images, exif_data) -> Scene:
+        """The instruction-independent part of `forward_with_guidance` — the backbone and (unless curiosity-guided
+        attention is enabled) the focal iterations — run once and kept in a `Scene` for `guide` / `guide_sweep`.
+        Takes the images `forward_with_guidance` takes.  Draws nothing from the global generator and leaves the
+        CuriosityModule state and every `_last_*` attribute as they are."""
+        self._raise_on_fault()
+        if exif_data is None or not self.use_exif:
+            raise ValueError("a scene needs EXIF data and a model with the EXIF prior (otherwise the reference falls "
+                             "back to forward(): use forward_with_guidance)")
+        B, S = self._check_images(images)
+        self._check_exif(exif_data, B)
+        self._pack()
+        dev = self._device()
+        g = S // 14
+        N, T = g * g, g * g + 1
+        exif, cam = self._exif_tensors(exif_data, B)
+        ws = self._workspace(B, S)
         self._grid_tables(g)
         patches, images = self._patch_rows(images, ws, S)
         cg = self.cfg.curiosity_guided
 
         def device_pass():
             self._backbone_layers(ws, patches, B, S)
-            self._curiosity_runs(sw, B, T, ("guided",) * K)
-            if cg:
-                # each call's focal attention is modulated by its own curiosity score (src/model.py:264-276)
-                for k in range(K):
-                    sw["base"][k].copy_(self._focal_iterations(ws, B, g, want_features=False, cur_weight=sw["cur_weight"][k]))
-                base, base_k_stride = sw["base"], B * N
+            if not cg:
+                self._focal_iterations(ws, B, g, want_features=False)
+
+        self._run(ws, ("encode", patches.data_ptr(), cg), device_pass)
+        tokens = torch.empty(B, T, _D, device=dev, dtype=torch.float32)
+        base = None if cg else torch.empty(B, N, device=dev, dtype=torch.float32)
+        if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
+            for t in (tokens, base):
+                if t is not None:
+                    t.fill_(float("nan"))
+        tokens.copy_(ws["tokens"])
+        if base is not None:
+            base.copy_(ws["attn"][self.cfg.num_iterations - 1])
+        # cloned: the scene owns its EXIF even when the caller's tensors were already contiguous device tensors
+        scene = Scene(self, B, S, tokens, base, exif.clone(), cam.clone())
+        self._keepalive = (exif, cam, images)  # until the next call, like the forwards (the copies are enqueued)
+        return scene
+
+    def _check_scene(self, scene):
+        if not isinstance(scene, Scene):
+            raise ValueError("expected a Scene from model.encode")
+        if scene._model() is not self:
+            raise ValueError("the scene was encoded by another model")
+        if scene.device != self._device():
+            raise ValueError(f"the scene lives on {scene.device}, the model on {self._device()}")
+        if scene._stamp != self._weights_version:
+            scene._graphs.clear()  # their workspace is no longer the model's: do not keep it alive
+            raise ValueError("stale scene: the model's weights changed after it was encoded (encode the images again)")
+
+    def _scene_ws(self, scene):
+        """The (B, S) workspace for a guide call: its scratch buffers, with the scene's tokens in place of the
+        workspace's (nothing is copied)."""
+        self._pack()
+        self._grid_tables(scene.S // 14)
+        ws = self._workspace(scene.B, scene.S)
+        return ws, {**ws, "tokens": scene.tokens}
+
+    def _run_scene(self, scene, ws, key, fn):
+        """Eager at a scene's first guide call; from the second on captured (once, on the scene's own buffers and this
+        workspace) and replayed.  The graphs go with the scene."""
+        first = scene._guided == 0
+        scene._guided += 1
+        if first:
+            fn()
+        else:
+            for k in [k for k, v in scene._graphs.items() if v[2] is not ws]:
+                del scene._graphs[k]  # captured on a workspace the model has since replaced: release it
+            self._run(ws, key + (id(ws), self._curiosity_key()), fn, graphs=scene._graphs)
+
+    @torch.no_grad()
+    @_on_own_device
+    def guide(self, scene: Scene, attention_guidance, return_attention=False):
+        """`forward_with_guidance(images, exif_data, attention_guidance, return_attention)` for the images and EXIF of
+        `scene`, bit for bit — outputs, global generator draws, CuriosityModule ring buffer and pointer, `_last_*` —
+        without re-running the backbone (nor, unless curiosity-guided attention is enabled, the focal iterations).
+        The tail (guided softmax, pool, heads) is one kernel (ops.guide_tail)."""
+        self._raise_on_fault()
+        self._check_scene(scene)
+        if attention_guidance is None:
+            raise ValueError("a None guidance runs the un-guided focal path (src/model.py:1206-1212): use "
+                             "forward_with_guidance for it")
+        B, S = scene.B, scene.S
+        self._check_per_image(attention_guidance, B)
+        pk = self._pack()
+        g = S // 14
+        N, T = g * g, g * g + 1
+        mask = self._mask(attention_guidance, g)
+        if mask.dim() == 2 and mask.shape[0] != B:
+            raise ValueError(f"{mask.shape[0]} per-image instructions for a batch of {B}")
+        draws = [self._curiosity_draw(B)]  # :1185
+        tmp = nn.Linear(_D, 64)  # :1421
+        ws, wsx = self._scene_ws(scene)
+        slot = self._pinned_slot()
+        slot["w"].copy_(tmp.weight.detach())
+        slot["b"].copy_(tmp.bias.detach())
+        self._stage_draws(ws, slot, draws)
+        ws["mask_in"].copy_(mask, non_blocking=True)
+        ops.fetch_pinned(ws["tmpw"], slot["w"])
+        ops.fetch_pinned(ws["tmpb"], slot["b"])
+        slot["event"].record()
+        cg = self.cfg.curiosity_guided
+
+        def device_pass():
+            self._curiosity_runs(wsx, B, T, ("guided",))
+            base = (self._focal_iterations(wsx, B, g, want_features=False, cur_weight=ws["cur_weight"][0]) if cg
+                    else scene.base)
+            heads_in = dict(tmp_w=ws["tmpw"], tmp_b=ws["tmpb"], exif=scene.exif, camera_idx=scene.camera_idx,
+                            num_cameras=self.cfg.num_cameras, fault_ptr=self._fault_word().data_ptr())
+            if B <= _GUIDE_TAIL_MAX_B:  # one launch (include/cogaim_b200.h CA_GUIDE_TAIL_MAX_B)
+                ops.guide_tail(pk["heads"], base=base, mask=ws["mask_in"], heat=ws["heat"], argmax=ws["argmax"],
+                               ticket=ws["tail_ticket"], tokens=scene.tokens, depth=ws["depth"], conf=ws["conf"], B=B,
+                               N=N, pool_partial=ws["pool"], **heads_in)
             else:
-                base, base_k_stride = self._focal_iterations(ws, B, g, want_features=False), 0
-            ops.guided_softmax_sweep(base, base_k_stride, sw["mask_in"], sw["heat"], sw["argmax"], K, B, N)
-            ops.weighted_pool_sweep(ws["tokens"], T * _D, 1, sw["heat"], sw["pool"], K, B, N, _D, _POOL_SPLITS)
-            ops.heads(pk["heads"], tokens=ws["tokens"], tokens_per_img=T, depth=sw["depth"], conf=sw["conf"], B=K * B,
-                      pool_partial=sw["pool"], pool_splits=_POOL_SPLITS, tmp_w=sw["tmpw"], tmp_b=sw["tmpb"],
-                      exif=ws["exif_in"], camera_idx=ws["cam_in"], num_cameras=self.cfg.num_cameras,
-                      fault_ptr=self._fault_word().data_ptr(), sweep_images=B)
+                ops.guided_softmax(base, ws["mask_in"], ws["heat"], ws["argmax"], B, N)
+                ops.weighted_pool(scene.tokens, T * _D, 1, ws["heat"], None, ws["pool"], B, N, _D, _POOL_SPLITS)
+                ops.heads(pk["heads"], tokens=scene.tokens, tokens_per_img=T, depth=ws["depth"], conf=ws["conf"], B=B,
+                          pool_partial=ws["pool"], pool_splits=_POOL_SPLITS, **heads_in)
             self._curiosity_join()
 
-        self._run(ws, ("sweep", K, self._curiosity_key()), device_pass)
-        self._keepalive = (exif, cam, mask, images)
-        heat = sw["heat"].clone()
-        # what the last of the K calls leaves behind
-        self._last_attention_weights = heat[K - 1]
-        self._last_argmax = sw["argmax"][K - 1].clone()
-        self._last_curiosity = sw["cur_reward"][K - 1]
-        depth, conf = sw["depth"].clone().unsqueeze(-1), sw["conf"].clone().unsqueeze(-1)
+        self._run_scene(scene, ws, ("guide",), device_pass)
+        self._keepalive = (mask,)
+        heat = ws["heat"].clone()
+        self._last_attention_weights = heat  # :1212
+        self._last_argmax = ws["argmax"].clone()
+        self._last_curiosity = ws["cur_reward"][0]
+        depth, conf = ws["depth"].clone().unsqueeze(1), ws["conf"].clone().unsqueeze(1)
         return (depth, conf, heat) if return_attention else (depth, conf)
+
+    @torch.no_grad()
+    @_on_own_device
+    def guide_sweep(self, scene: Scene, guidances, return_attention=False):
+        """`forward_with_guidance_sweep(images, exif_data, guidances, return_attention)` for the images and EXIF of
+        `scene`, bit for bit, without re-running the backbone (nor, unless curiosity-guided attention is enabled, the
+        focal iterations)."""
+        self._raise_on_fault()
+        self._check_scene(scene)
+        K = self._check_guidances(guidances)
+        B, S = scene.B, scene.S
+        for gd in guidances:
+            self._check_per_image(gd, B)
+        self._pack()
+        g = S // 14
+        mask = self._sweep_masks(guidances, B, g)
+        ws, _ = self._scene_ws(scene)
+        sw = self._stage_sweep_call(ws, mask, B, S, K)
+        sw["tokens"] = scene.tokens
+
+        def device_pass():
+            self._sweep_device(sw, B, g, K, scene.base, scene.exif, scene.camera_idx)
+
+        self._run_scene(scene, ws, ("sweep", K), device_pass)
+        self._keepalive = (mask,)
+        return self._sweep_results(sw, K, return_attention)
 
     @torch.no_grad()
     @_on_own_device

@@ -294,5 +294,98 @@ class NativeModel:
         self._held = [images]
         return tokens
 
+    @torch.no_grad()
+    def encode(self, images, exif, S=None) -> "NativeScene":
+        """ca_encode: the backbone and the focal pass of the batch, once, kept in a scene for `guide` / `guide_sweep`.
+        Draws nothing from the global generator."""
+        if exif is None:
+            raise ValueError("a scene needs EXIF data (without it the reference falls back to forward())")
+        c, held, B, S = self._call(images, exif, S)
+        out = C.c_void_p()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ca_encode(self._h, C.byref(c), C.byref(out), self._stream()), "ca_encode")
+        self._held = held
+        return NativeScene(self.lib, out, B, S, self.device)
+
+    @torch.no_grad()
+    def guide(self, scene: "NativeScene", guidance):
+        """ca_guide: `forward_with_guidance` on the encoded images (same draws, same results, same order of draws)."""
+        if guidance is None:
+            raise ValueError("guide needs an instruction or a guidance tensor")
+        B, N = scene.B, (scene.S // 14) ** 2
+        c = _lib.GuideCall()
+        held = []
+        if isinstance(guidance, str):
+            c.instruction = guidance.encode()
+        else:
+            m = guidance.to(self.device, torch.float32).contiguous()
+            held.append(m)
+            c.mask, c.mask_batch_stride = m.data_ptr(), (N if m.dim() == 2 else 0)
+        eps, noise = torch.randn(B, 192), torch.randn(B, _D)       # :609, :744
+        tmp = nn.Linear(_D, 64)                                    # :1421
+        tw, tb = tmp.weight.detach().contiguous(), tmp.bias.detach().contiguous()
+        held += [eps, noise, tw, tb]
+        c.tmp_w, c.tmp_b, c.eps, c.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
+        out = {"depth": torch.empty(B, device=self.device), "conf": torch.empty(B, device=self.device),
+               "heat": torch.empty(B, N, device=self.device),
+               "argmax": torch.empty(B, device=self.device, dtype=torch.int32)}
+        c.depth, c.conf, c.attention, c.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ca_guide(self._h, scene.ptr, C.byref(c), self._stream()), "ca_guide")
+        self._held = held
+        return out["depth"].unsqueeze(1), out["conf"].unsqueeze(1), out["heat"], out["argmax"]
+
+    @torch.no_grad()
+    def guide_sweep(self, scene: "NativeScene", guidances):
+        """ca_guide_sweep: `forward_with_guidance_sweep` on the encoded images."""
+        K = len(guidances)
+        if not 1 <= K <= _lib.SWEEP_MAX_K:
+            raise ValueError(f"an instruction sweep takes 1..{_lib.SWEEP_MAX_K} guidances, got {K}")
+        B, N = scene.B, (scene.S // 14) ** 2
+        s = _lib.SweepCall()
+        s.K = K
+        held = []
+        if all(isinstance(g, str) for g in guidances):
+            names = (C.c_char_p * K)(*[g.encode() for g in guidances])
+            held.append(names)
+            s.instructions = C.cast(names, C.POINTER(C.c_char_p))
+        elif all(torch.is_tensor(g) and g.dim() == 1 and g.numel() == N for g in guidances):
+            m = torch.stack([g.to(self.device, torch.float32) for g in guidances]).contiguous()
+            held.append(m)
+            s.masks = m.data_ptr()
+        else:
+            raise ValueError(f"guidances must be K instruction strings or K guidance tensors of length {N}")
+        draws = []
+        for _ in range(K):
+            eps, noise = torch.randn(B, 192), torch.randn(B, _D)
+            tmp = nn.Linear(_D, 64)
+            draws.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
+        eps, noise, tw, tb = (torch.stack([d[i] for d in draws]).contiguous() for i in range(4))
+        held += [eps, noise, tw, tb]
+        s.tmp_w, s.tmp_b, s.eps, s.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
+        out = {"depth": torch.empty(K, B, device=self.device), "conf": torch.empty(K, B, device=self.device),
+               "heat": torch.empty(K, B, N, device=self.device),
+               "argmax": torch.empty(K, B, device=self.device, dtype=torch.int32)}
+        s.depth, s.conf, s.attention, s.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ca_guide_sweep(self._h, scene.ptr, C.byref(s), self._stream()), "ca_guide_sweep")
+        self._held = held
+        return out["depth"].unsqueeze(-1), out["conf"].unsqueeze(-1), out["heat"], out["argmax"]
+
     def launch_count(self) -> int:
         return int(self.lib.ca_last_launch_count(self._h))
+
+
+class NativeScene:
+    """A ca_scene: released by `close()` or when dropped."""
+
+    def __init__(self, lib, ptr, B: int, S: int, device):
+        self.lib, self.ptr, self.B, self.S, self.device = lib, ptr, B, S, device
+
+    def close(self):
+        if self.ptr is not None and self.ptr.value:
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.ca_scene_destroy(self.ptr), "ca_scene_destroy")
+        self.ptr = None
+
+    __del__ = close

@@ -473,6 +473,39 @@ def heads(weights, *, tokens, tokens_per_img, depth, conf, B, focal_feat=None, p
     _end(e0, "heads", 1)
 
 
+def guide_tail(weights, *, base, mask, heat, argmax, ticket, tokens, depth, conf, B, N, pool_partial, tmp_w, tmp_b,
+               exif=None, camera_idx=None, num_cameras=0, fault_ptr=None, pooled_out=None, alpha=0.7, temperature=0.05):
+    """`guided_softmax` -> `weighted_pool` (pool_partial [B, splits, 768], rows 1..N of each image's tokens) -> `heads`
+    of one guided call in ONE launch, bit for bit.  mask: [N] or [B, N]; ticket: int32 [B], zero before the first call
+    (every call leaves it at zero)."""
+    import ctypes as C
+    _req(base, torch.float32, "base")
+    _req(mask, torch.float32, "mask")
+    _req(heat, torch.float32, "heat")
+    _req(ticket, torch.int32, "ticket")
+    _req(pool_partial, torch.float32, "pool_partial")
+    _req(tokens, torch.float32, "tokens")
+    if tuple(tokens.shape) != (B, N + 1, 768) or not tokens.is_contiguous() or tokens.data_ptr() % 16:
+        raise ValueError(f"guide_tail: tokens must be a contiguous, 16-byte aligned [B, N + 1, 768] = [{B}, {N + 1}, 768] "
+                         f"tensor, got {tuple(tokens.shape)}")
+    if not pool_partial.is_contiguous() or pool_partial.data_ptr() % 16:
+        raise ValueError("guide_tail: pool_partial must be contiguous and 16-byte aligned")
+    if argmax is not None:
+        _req(argmax, torch.int32, "argmax")
+    if mask.dim() == 2 and mask.shape[0] != B:
+        raise ValueError(f"per-image mask has {mask.shape[0]} rows for a batch of {B}")
+    if ticket.numel() < B or pool_partial.dim() != 3 or pool_partial.shape[0] < B or pool_partial.shape[2] != 768:
+        raise ValueError("guide_tail: ticket needs B entries and pool_partial must be [B, splits, 768]")
+    stride = mask.stride(0) if mask.dim() == 2 else 0
+    inp = _lib.HeadsInputs(_dp(tokens), N + 1, None, _dp(pool_partial), pool_partial.shape[1], _dp(tmp_w), _dp(tmp_b),
+                           _dp(pooled_out), _dp(exif), _dp(camera_idx), int(num_cameras), fault_ptr, 0)
+    e0 = _begin()
+    check(_lib.load().ca_guide_tail(C.byref(weights), C.byref(inp), ptr(base), ptr(mask), stride, ptr(heat), ptr(argmax),
+                                    ptr(ticket), ptr(depth), ptr(conf), B, N, alpha, temperature, stream_ptr()),
+          "ca_guide_tail")
+    _end(e0, "tail", 1, float(B * N * 768 * 4))
+
+
 def make_curiosity_weights(named):
     """named: dict field -> fp32 CUDA tensor or None for the four local_curiosity fields (kept alive by the caller)."""
     w = _lib.CuriosityWeights()

@@ -2,6 +2,7 @@
 
     python examples/predict_like_demo.py IMAGE.jpg [--instruction center] [--image-size 224] [--overlay out.npy]
     python examples/predict_like_demo.py --image-dir DIR [--instruction center] [--image-size 224]
+    python examples/predict_like_demo.py IMAGE.jpg --interactive < instructions.txt
 
 What demo.py does per image and what runs here instead:
     Image.open(path).convert('RGB')                    -> nvJPEG decode on the GPU              (model.preprocess_jpeg)
@@ -14,6 +15,9 @@ What demo.py does per image and what runs here instead:
 (`Predictor.predict_all`, model.forward_with_guidance_sweep) instead of nine calls, with the same printed results.
 `--image-dir` (demo.py:406-432 `predict_batch`, one call per file there) decodes every JPEG of the folder in one batched
 nvJPEG call and runs the photographs, whatever their sizes, through ONE forward (`Predictor.predict_batch`).
+`--interactive` encodes the photograph once (`Predictor.encode`, model.encode: decode, backbone, focal stream) and then
+reads instructions from stdin, one per line, printing for each the line `predict` prints (`Predictor.predict_scene`,
+model.guide); the results equal successive `predict` calls on the same photograph.
 Weights: random init (seed 0, the reference's own construction order) unless --checkpoint names a reference state_dict.
 """
 from __future__ import annotations
@@ -127,10 +131,34 @@ class Predictor:
             out.append((float(depth[i].squeeze()), float(conf[i].squeeze()), meta))
         return out
 
+    @torch.no_grad()
+    def encode(self, jpeg_bytes: bytes, exif=None):
+        """Decode and encode one photograph for any number of later instructions (`predict_scene`)."""
+        x = self.model.preprocess_jpeg([jpeg_bytes], self.image_size)
+        return self.model.encode(x, exif if exif is not None else self.default_exif(1))
+
+    @torch.no_grad()
+    def predict_scene(self, scene, instruction, overlay_size=None):
+        """`predict(jpeg_bytes, instruction, exif, overlay_size)` for the photograph `scene` was encoded from, bit for bit
+        (the backbone and the focal stream are not run again)."""
+        depth, conf, heat = self.model.guide(scene, instruction, return_attention=True)
+        g = self.image_size // 14
+        cell = int(heat[0].argmax())
+        meta = {"processed_size": (self.image_size, self.image_size), "instruction": instruction,
+                "attention_cell": (cell // g, cell % g),
+                "model_status": {"ambient": self.model.use_ambient, "focal": self.model.use_focal, "exif": self.model.use_exif}}
+        if overlay_size is not None:
+            meta["overlay"] = self.model.focus_map(overlay_size, attention=heat)[0]
+        return float(depth.squeeze()), float(conf.squeeze()), meta
+
     def model_images(self, jpeg_files):
         """JPEG files (bytes) -> list of decoded uint8 [H_i, W_i, 3] CUDA tensors (one nvjpegDecodeBatched call)."""
         with torch.cuda.device(self.device):
             return ops.jpeg_decode_batch(list(jpeg_files), self.device)
+
+
+def result_line(ins, depth, conf, meta):
+    return f"{str(ins):13s} depth {depth:.4f}  confidence {conf:.4f}  attention cell {meta['attention_cell']}"
 
 
 def main():
@@ -141,6 +169,8 @@ def main():
     ap.add_argument("--image-size", type=int, default=224)  # configs/experiment_B.yaml:87
     ap.add_argument("--checkpoint", default=None)
     ap.add_argument("--overlay", default=None, help="write the overlay heat map of the last instruction as .npy")
+    ap.add_argument("--interactive", action="store_true",
+                    help="encode IMAGE once, then read instructions from stdin, one per line")
     args = ap.parse_args()
     if (args.image is None) == (args.image_dir is None):
         ap.error("give IMAGE or --image-dir DIR")
@@ -157,17 +187,25 @@ def main():
             ap.error(f"no JPEG files in {args.image_dir}")
         files = [open(os.path.join(args.image_dir, f), "rb").read() for f in names]
         for depth, conf, meta in p.predict_batch(files, args.instruction):  # one line per file, sorted by name
-            print(f"{str(args.instruction):13s} depth {depth:.4f}  confidence {conf:.4f}  "
-                  f"attention cell {meta['attention_cell']}")
+            print(result_line(args.instruction, depth, conf, meta))
         return
     data = open(args.image, "rb").read()
+    if args.interactive:
+        if args.instruction or args.overlay:
+            ap.error("--interactive reads its instructions from stdin and takes no --overlay")
+        scene = p.encode(data)
+        for line in sys.stdin:
+            ins = line.strip()
+            if ins:
+                print(result_line(ins, *p.predict_scene(scene, ins)), flush=True)
+        return
     overlay_size = (480, 640) if args.overlay else None
     if args.instruction == "all":  # every instruction in one sweep (backbone and focal pass once)
         results = zip(INSTRUCTIONS, p.predict_all(data, INSTRUCTIONS, overlay_size=overlay_size))
     else:
         results = [(args.instruction, p.predict(data, args.instruction, overlay_size=overlay_size))]
     for ins, (depth, conf, meta) in results:
-        print(f"{str(ins):13s} depth {depth:.4f}  confidence {conf:.4f}  attention cell {meta['attention_cell']}")
+        print(result_line(ins, depth, conf, meta))
     if args.overlay:
         import numpy as np
         np.save(args.overlay, meta["overlay"].cpu().numpy())

@@ -196,6 +196,20 @@ typedef struct ca_heads_inputs {
  * `w` and `in` are HOST pointers to the structs above.  src/model.py:1195-1230. */
 int ca_heads(const ca_heads_weights* w, const ca_heads_inputs* in, float* depth, float* conf, float* fused_out, int B,
              void* stream);
+/* The guided tail of one call in ONE launch: ca_guided_softmax(base, mask) -> ca_weighted_pool(tokens, heat,
+ * in->pool_splits splits) -> ca_heads(in), with results bit-identical to that chain.  Grid (in->pool_splits, B); every CTA
+ * recomputes its image's softmax, pools its split into in->pool_partial (a [B, pool_splits, 768] scratch this call
+ * overwrites) and the image's last CTA runs the heads.  in->focal_feat must be NULL and in->sweep_images 0;
+ * in->tokens_per_img must be N + 1.  ticket: [B] device counters, zero before the first launch; every launch leaves them
+ * at zero (no clearing between launches).  argmax may be NULL.  N <= 8192. */
+/* Largest batch for which guide calls (Python `guide`, handle `ca_guide`) use ca_guide_tail; larger batches run the
+ * three-kernel chain.  A single image is launch-bound, and one launch replaces three.  A batch is bandwidth-bound: a
+ * ca_guide_tail CTA of 1024 threads fills an SM's register file, and only 6 of its warps stream tokens, while several
+ * 192-thread pool CTAs of the chain share an SM.  tools/bench_scene.py times both at B = 1 and B = 32. */
+#define CA_GUIDE_TAIL_MAX_B 1
+int ca_guide_tail(const ca_heads_weights* w, const ca_heads_inputs* in, const float* base, const float* mask,
+                  long long mask_batch_stride, float* heat, int32_t* argmax, uint32_t* ticket, float* depth, float* conf,
+                  int B, int N, float alpha, float temperature, void* stream);
 
 typedef struct ca_focal_value_args {
   const float* tok_partial;  /* [B, splits, 768] partial sums of c_j * rowscale_j * tokens_j */
@@ -418,6 +432,38 @@ int ca_backbone_list(ca_handle* h, const uint8_t* const* image_list, const int* 
                      void* stream);
 /* kernels launched by the last ca_forward* / ca_backbone call of this handle (the launch-count claim of bench.py). */
 int ca_last_launch_count(const ca_handle* h);
+
+/* Scenes: encode a batch once, guide it any number of times.  A scene owns the backbone tokens [B, 1+N, 768], the last
+ * focal iteration's attention [B, N], the EXIF and camera indices of the batch, and the graphs captured on them; it
+ * belongs to the handle that encoded it.  A scene of a destroyed handle (or of another handle) is refused with
+ * CA_STATUS_INVALID and never dereferenced through its handle; so is a scene already destroyed. */
+typedef struct ca_scene ca_scene;
+/* The instruction-independent part of ca_forward_guided: `call` supplies images (or image_list / image_hw), images_u8,
+ * B, S, exif, camera_idx (both required), fault (used by the scene's guide calls) and use_graph; its per-call fields
+ * (instruction, mask, tmp_w, tmp_b, eps, noise, depth, conf, attention, argmax, fused) must be NULL. */
+int ca_encode(ca_handle* h, const ca_forward_call* call, ca_scene** out, void* stream);
+/* One guided call on a scene: HOST pointers where marked, device otherwise. */
+typedef struct ca_guide_call {
+  const char* instruction;      /* HOST instruction string / alias, or NULL when `mask` is given */
+  const float* mask;            /* explicit guidance [N] (mask_batch_stride 0) or per image [B, N] (stride N) */
+  long long mask_batch_stride;
+  const float* tmp_w;           /* HOST [64, 768]: per-call projection weight   src/model.py:1421 */
+  const float* tmp_b;           /* HOST [64] */
+  const float* eps;             /* HOST [B, 192]: CuriosityModule draw of :609 */
+  const float* noise;           /* HOST [B, 768]: draw of :744 */
+  float* depth;                 /* out [B] */
+  float* conf;                  /* out [B] */
+  float* attention;             /* out [B, N] heat map */
+  int* argmax;                  /* out [B] or NULL */
+} ca_guide_call;
+/* ca_forward_guided on the encoded images, bit for bit given the same draws, without the backbone and the focal pass:
+ * the CuriosityModule run and the fused tail (ca_guide_tail).  With use_graph the launches are captured on the scene's
+ * buffers at its second guide call and replayed after. */
+int ca_guide(ca_handle* h, ca_scene* scene, const ca_guide_call* call, void* stream);
+/* ca_forward_guided_sweep on the encoded images, bit for bit given the same draws (ca_sweep_call as there). */
+int ca_guide_sweep(ca_handle* h, ca_scene* scene, const ca_sweep_call* sweep, void* stream);
+/* Release a scene's memory and graphs (waits for the device).  NULL is a no-op. */
+int ca_scene_destroy(ca_scene* scene);
 
 #ifdef __cplusplus
 }
