@@ -112,6 +112,12 @@ class GuideCall(C.Structure):
                 ("depth", C.c_void_p), ("conf", C.c_void_p), ("attention", C.c_void_p), ("argmax", C.c_void_p)]
 
 
+class DepthFieldCall(C.Structure):
+    """ca_depth_field_call (include/cogaim_b200.h)."""
+    _fields_ = [("tmp_w", C.c_void_p), ("tmp_b", C.c_void_p), ("eps", C.c_void_p), ("noise", C.c_void_p),
+                ("depth", C.c_void_p), ("conf", C.c_void_p)]
+
+
 # name -> (argtypes); every function returns int status except where noted in _RESTYPES
 _SIGNATURES = {
     "ca_version": [],
@@ -157,6 +163,9 @@ _SIGNATURES = {
     "ca_heads": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, c_ptr, C.c_int, c_ptr],
     "ca_guide_tail": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, C.c_longlong, c_ptr, c_ptr, c_ptr,
                       c_ptr, c_ptr, C.c_int, C.c_int, C.c_float, C.c_float, c_ptr],
+    "ca_token_project": [c_ptr, C.c_longlong, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, c_ptr],
+    "ca_depth_field_cells": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int,
+                             C.c_int, C.c_float, C.c_float, c_ptr],
     "ca_focal_value": [C.POINTER(FocalValueArgs), C.c_int, c_ptr],
     "ca_focal_fusion": [c_ptr, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, c_ptr],
     "ca_create": [C.POINTER(C.c_void_p), C.POINTER(ModelWeights), C.c_int],
@@ -170,6 +179,7 @@ _SIGNATURES = {
     "ca_encode": [c_ptr, C.POINTER(ForwardCall), C.POINTER(C.c_void_p), c_ptr],
     "ca_guide": [c_ptr, c_ptr, C.POINTER(GuideCall), c_ptr],
     "ca_guide_sweep": [c_ptr, c_ptr, C.POINTER(SweepCall), c_ptr],
+    "ca_depth_field": [c_ptr, c_ptr, C.POINTER(DepthFieldCall), c_ptr],
     "ca_scene_destroy": [c_ptr],
 }
 

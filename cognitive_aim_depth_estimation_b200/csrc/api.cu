@@ -3,6 +3,7 @@
 
 #include "attention.cuh"
 #include "curiosity.cuh"
+#include "field.cuh"
 #include "focal.cuh"
 #include "gemm.cuh"
 #include "heads.cuh"
@@ -212,6 +213,19 @@ int ca_guide_tail(const ca_heads_weights* w, const ca_heads_inputs* in, const fl
   if (!w || !in) return ca::invalid("guide_tail: null argument struct");
   return ca::guide_tail_launch(*w, *in, base, mask, mask_batch_stride, heat, argmax, ticket, depth, conf, B, N, alpha,
                                temperature, static_cast<cudaStream_t>(stream));
+}
+
+int ca_token_project(const float* src, long long src_batch_stride, int row_offset, const float* tmp_w, float* P, int B,
+                     int N, void* stream) {
+  return ca::token_project_launch(src, src_batch_stride, row_offset, tmp_w, P, B, N, static_cast<cudaStream_t>(stream));
+}
+
+int ca_depth_field_cells(const ca_heads_weights* w, const ca_heads_inputs* in, const float* base, const float* P,
+                         float* cst, float* depth, float* conf, int B, int g, float alpha, float temperature,
+                         void* stream) {
+  if (!w || !in) return ca::invalid("depth_field_cells: null argument struct");
+  return ca::depth_field_cells_launch(*w, *in, base, P, cst, depth, conf, B, g, alpha, temperature,
+                                      static_cast<cudaStream_t>(stream));
 }
 
 int ca_focal_value(const ca_focal_value_args* a, int B, void* stream) {

@@ -28,6 +28,7 @@
 
 #include "attention.cuh"
 #include "curiosity.cuh"
+#include "field.cuh"
 #include "focal.cuh"
 #include "gemm.cuh"
 #include "heads.cuh"
@@ -69,11 +70,16 @@ struct Workspace {
     int* argmax;
   };
   std::map<int, Sweep> sweeps;  // K -> buffers
+  // depth fields (allocated at the first ca_depth_field on this workspace): projected tokens [B, N, 64], the per-image
+  // fusion constant [B, 192], the field [B, N] x 2
+  void* field_arena = nullptr;
+  float *field_P = nullptr, *field_cst = nullptr, *field_depth = nullptr, *field_conf = nullptr;
 };
 
 void free_workspace(Workspace& w) {
   for (auto& g : w.graphs) cudaGraphExecDestroy(g.second.first);
   for (auto& s : w.sweeps) cudaFree(s.second.arena);
+  cudaFree(w.field_arena);
   cudaFree(w.arena);
 }
 
@@ -392,6 +398,21 @@ int get_sweep(Workspace& w, int K, Workspace::Sweep** out) {
     it = w.sweeps.emplace(K, s).first;
   }
   *out = &it->second;
+  return 0;
+}
+
+int get_field(Workspace& w) {
+  if (w.field_arena) return 0;
+  const int g = w.S / 14;
+  const size_t BN = static_cast<size_t>(w.B) * g * g;
+  const size_t o_cst = BN * 64 * 4, o_depth = o_cst + ((static_cast<size_t>(w.B) * 192 * 4 + 255) & ~size_t(255));
+  const size_t o_conf = o_depth + ((BN * 4 + 255) & ~size_t(255));
+  CA_CUDA(cudaMalloc(&w.field_arena, o_conf + BN * 4));
+  char* a = static_cast<char*>(w.field_arena);
+  w.field_P = reinterpret_cast<float*>(a);
+  w.field_cst = reinterpret_cast<float*>(a + o_cst);
+  w.field_depth = reinterpret_cast<float*>(a + o_depth);
+  w.field_conf = reinterpret_cast<float*>(a + o_conf);
   return 0;
 }
 
@@ -1257,6 +1278,49 @@ int ca_guide_sweep(ca_handle* h, ca_scene* sc, const ca_sweep_call* sw, void* st
   CA_CUDA(cudaMemcpyAsync(sw->conf, s.conf, KB * 4, cudaMemcpyDeviceToDevice, st));
   CA_CUDA(cudaMemcpyAsync(sw->attention, s.heat, KB * N * 4, cudaMemcpyDeviceToDevice, st));
   if (sw->argmax) CA_CUDA(cudaMemcpyAsync(sw->argmax, s.argmax, KB * 4, cudaMemcpyDeviceToDevice, st));
+  h->last_launches = h->launches;
+  return 0;
+}
+
+int ca_depth_field(ca_handle* h, ca_scene* sc, const ca_depth_field_call* c, void* stream) {
+  CA_TRY(check_scene(h, sc));
+  CA_REQUIRE(c, "depth_field: null call");
+  CA_REQUIRE(c->tmp_w && c->tmp_b && c->eps && c->noise,
+             "depth_field: null per-call projection or CuriosityModule draws (HOST pointers, src/model.py:609,744,1421)");
+  CA_REQUIRE(c->depth && c->conf, "depth_field: null output");
+  DeviceGuard guard(h->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int B = sc->B, g = sc->S / 14, N = g * g, T = N + 1;
+  Workspace* wp = nullptr;
+  Tables* tb = nullptr;
+  CA_TRY(scene_workspace(h, sc, &wp, &tb));
+  Workspace& w = *wp;
+  CA_TRY(get_field(w));
+  h->launches = 0;
+  ca_forward_call staged{};
+  staged.tmp_w = c->tmp_w;
+  staged.tmp_b = c->tmp_b;
+  staged.eps = c->eps;
+  staged.noise = c->noise;
+  CA_TRY(stage_host_inputs(h, w, staged, true, 1, st));
+  CA_TRY(run_captured(h, sc->graphs, sc->seen, 200, sc->use_graph, st, [&]() -> int {
+    CA_TRY(curiosity_fork(h, w, 1, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st, sc->tokens));
+    LAUNCH(ca::token_project_launch(sc->tokens, static_cast<long long>(T) * kD, 1, w.tmpw, w.field_P, B, N, st));
+    ca_heads_inputs in{};
+    in.tokens = sc->tokens;
+    in.tokens_per_img = T;
+    in.tmp_b = w.tmpb;
+    in.exif = sc->exif;
+    in.camera_idx = sc->cam;
+    in.num_cameras = h->w.num_cameras;
+    in.fault = sc->fault;
+    CA_TRY(ca::depth_field_cells_launch(h->w.heads, in, sc->base, w.field_P, w.field_cst, w.field_depth, w.field_conf, B,
+                                        g, 0.7f, 0.05f, st));
+    h->launches += 2;
+    return curiosity_join(h, st);
+  }));
+  CA_CUDA(cudaMemcpyAsync(c->depth, w.field_depth, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c->conf, w.field_conf, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
   h->last_launches = h->launches;
   return 0;
 }

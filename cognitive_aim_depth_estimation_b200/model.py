@@ -1267,6 +1267,65 @@ class CognitiveAimModel(nn.Module):
         self._keepalive = (mask,)
         return self._sweep_results(sw, K, return_attention)
 
+    def _field_buffers(self, ws, B: int, N: int):
+        """The depth-field buffers of a (B, S) workspace, added at its first field: the projected tokens [B, N, 64], the
+        per-image fusion constant [B, 192] and the field itself."""
+        if "field_P" not in ws:
+            fl = dict(device=self._device(), dtype=torch.float32)
+            ws.update(field_P=torch.empty(B, N, 64, **fl), field_cst=torch.empty(B, 192, **fl),
+                      field_depth=torch.empty(B, N, **fl), field_conf=torch.empty(B, N, **fl))
+            if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
+                for k in ("field_P", "field_cst", "field_depth", "field_conf"):
+                    ws[k].fill_(float("nan"))
+        return ws
+
+    @torch.no_grad()
+    @_on_own_device
+    def depth_field(self, scene: Scene):
+        """The guided depth and confidence with the focus on every cell of the g x g patch grid (g = S / 14): returns
+        depth, confidence [B, g, g] fp32.  Cell (y, x) of image b is what `guide(scene, tables.focus_mask(y, x, g))` gives
+        for image b with the same draws, within fp32 rounding (the field projects the tokens before pooling them and sums
+        each cell's softmax over its focus disk, where all but < N e^-36 of the weight lies).  So cell (g//4, g//4) is the
+        "top-left" prediction, and likewise for the other off-centre instructions; "center" has its own mask, and cell
+        (g//2, g//2) is not its prediction.
+        One call draws what one `guide` call draws, in its order (the CuriosityModule's randn(B, 192), randn(B, 768),
+        then nn.Linear(768, 64)); every cell uses that one projection, and the CuriosityModule runs once (B ring
+        entries).  `_last_curiosity` is set as `guide` sets it; `_last_attention_weights` and `_last_argmax` are left as
+        they are (there is no single heat map)."""
+        self._raise_on_fault()
+        self._check_scene(scene)
+        B, S = scene.B, scene.S
+        pk = self._pack()
+        g = S // 14
+        N, T = g * g, g * g + 1
+        draws = [self._curiosity_draw(B)]  # :1185
+        tmp = nn.Linear(_D, 64)  # :1421
+        ws, wsx = self._scene_ws(scene)
+        self._field_buffers(ws, B, N)
+        slot = self._pinned_slot()
+        slot["w"].copy_(tmp.weight.detach())
+        slot["b"].copy_(tmp.bias.detach())
+        self._stage_draws(ws, slot, draws)
+        ops.fetch_pinned(ws["tmpw"], slot["w"])
+        ops.fetch_pinned(ws["tmpb"], slot["b"])
+        slot["event"].record()
+        cg = self.cfg.curiosity_guided
+
+        def device_pass():
+            self._curiosity_runs(wsx, B, T, ("guided",))
+            base = (self._focal_iterations(wsx, B, g, want_features=False, cur_weight=ws["cur_weight"][0]) if cg
+                    else scene.base)
+            ops.token_project(scene.tokens, T * _D, 1, ws["tmpw"], ws["field_P"], B, N)
+            ops.depth_field_cells(pk["heads"], base=base, P=ws["field_P"], cst=ws["field_cst"], depth=ws["field_depth"],
+                                  conf=ws["field_conf"], tokens=scene.tokens, tmp_b=ws["tmpb"], B=B, g=g,
+                                  exif=scene.exif, camera_idx=scene.camera_idx, num_cameras=self.cfg.num_cameras,
+                                  fault_ptr=self._fault_word().data_ptr())
+            self._curiosity_join()
+
+        self._run_scene(scene, ws, ("field",), device_pass)
+        self._last_curiosity = ws["cur_reward"][0]
+        return ws["field_depth"].clone().view(B, g, g), ws["field_conf"].clone().view(B, g, g)
+
     @torch.no_grad()
     @_on_own_device
     def forward(self, images, exif_data=None, return_attention=False):

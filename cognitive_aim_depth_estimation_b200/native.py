@@ -372,6 +372,23 @@ class NativeModel:
         self._held = held
         return out["depth"].unsqueeze(-1), out["conf"].unsqueeze(-1), out["heat"], out["argmax"]
 
+    @torch.no_grad()
+    def depth_field(self, scene: "NativeScene"):
+        """ca_depth_field: `CognitiveAimModel.depth_field` on the encoded images (the draws of one guide call, in its
+        order).  Returns depth, confidence [B, g, g]."""
+        B, g = scene.B, scene.S // 14
+        eps, noise = torch.randn(B, 192), torch.randn(B, _D)       # :609, :744
+        tmp = nn.Linear(_D, 64)                                    # :1421
+        tw, tb = tmp.weight.detach().contiguous(), tmp.bias.detach().contiguous()
+        c = _lib.DepthFieldCall()
+        c.tmp_w, c.tmp_b, c.eps, c.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
+        depth, conf = torch.empty(B, g, g, device=self.device), torch.empty(B, g, g, device=self.device)
+        c.depth, c.conf = depth.data_ptr(), conf.data_ptr()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ca_depth_field(self._h, scene.ptr, C.byref(c), self._stream()), "ca_depth_field")
+        self._held = [eps, noise, tw, tb]
+        return depth, conf
+
     def launch_count(self) -> int:
         return int(self.lib.ca_last_launch_count(self._h))
 

@@ -506,6 +506,52 @@ def guide_tail(weights, *, base, mask, heat, argmax, ticket, tokens, depth, conf
     _end(e0, "tail", 1, float(B * N * 768 * 4))
 
 
+def token_project(src, src_batch_stride, row_offset, tmp_w, P, B, N):
+    """P [B, N, 64] = rows row_offset .. row_offset + N - 1 of each image of `src` (fp32, 768 wide, images
+    `src_batch_stride` floats apart) times tmp_w [64, 768] transposed: the per-call projection of every patch token."""
+    _req(src, torch.float32, "src")
+    _req(tmp_w, torch.float32, "tmp_w")
+    _req(P, torch.float32, "P")
+    if tuple(tmp_w.shape) != (64, 768) or not tmp_w.is_contiguous():
+        raise ValueError("token_project: tmp_w must be a contiguous [64, 768] tensor")
+    if P.numel() < B * N * 64 or not P.is_contiguous():
+        raise ValueError("token_project: P must be a contiguous tensor of at least B * N * 64 floats")
+    if src.numel() < (B - 1) * src_batch_stride + (row_offset + N) * 768:
+        raise ValueError("token_project: src is smaller than B images of row_offset + N rows")
+    e0 = _begin()
+    check(_lib.load().ca_token_project(ptr(src), src_batch_stride, row_offset, ptr(tmp_w), ptr(P), B, N, stream_ptr()),
+          "ca_token_project")
+    _end(e0, "token_project", 1, float(B * N * 768 * 4))
+
+
+def depth_field_cells(weights, *, base, P, cst, depth, conf, tokens, tmp_b, B, g, exif=None, camera_idx=None,
+                      num_cameras=0, fault_ptr=None, alpha=0.7, temperature=0.05):
+    """depth, conf [B, g * g]: for every cell c, the guided call whose mask is `tables.focus_mask` at c, from the
+    projected tokens P [B, g * g, 64] (`token_project`), the focal attention `base` [B, g * g], the CLS rows of `tokens`
+    [B, g * g + 1, 768], the projection bias tmp_b [64] and the EXIF inputs as `heads` takes them.  cst: [B, 192]
+    scratch.  Two launches (the per-image fusion constant, then the cells)."""
+    import ctypes as C
+    N = g * g
+    for t, name in ((base, "base"), (P, "P"), (cst, "cst"), (depth, "depth"), (conf, "conf"), (tokens, "tokens"),
+                    (tmp_b, "tmp_b")):
+        _req(t, torch.float32, name)
+        if not t.is_contiguous():
+            raise ValueError(f"depth_field_cells: {name} must be contiguous")
+    if tuple(tokens.shape) != (B, N + 1, 768):
+        raise ValueError(f"depth_field_cells: tokens must be [B, N + 1, 768] = [{B}, {N + 1}, 768], got "
+                         f"{tuple(tokens.shape)}")
+    if (base.numel() < B * N or P.numel() < B * N * 64 or cst.numel() < B * 192 or depth.numel() < B * N
+            or conf.numel() < B * N or tmp_b.numel() != 64):
+        raise ValueError("depth_field_cells: base / depth / conf need B * g * g floats, P B * g * g * 64, cst B * 192 "
+                         "and tmp_b 64")
+    inp = _lib.HeadsInputs(_dp(tokens), N + 1, None, None, 0, None, _dp(tmp_b), None, _dp(exif), _dp(camera_idx),
+                           int(num_cameras), fault_ptr, 0)
+    e0 = _begin()
+    check(_lib.load().ca_depth_field_cells(C.byref(weights), C.byref(inp), ptr(base), ptr(P), ptr(cst), ptr(depth),
+                                           ptr(conf), B, g, alpha, temperature, stream_ptr()), "ca_depth_field_cells")
+    _end(e0, "field_cells", 2, float(B * N * 64 * 4))
+
+
 def make_curiosity_weights(named):
     """named: dict field -> fp32 CUDA tensor or None for the four local_curiosity fields (kept alive by the caller)."""
     w = _lib.CuriosityWeights()

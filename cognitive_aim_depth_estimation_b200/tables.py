@@ -20,31 +20,44 @@ def canonical_instruction(s: str) -> str:
     return _ALIASES.get(s, s)
 
 
-def _focus(name: str, g: int):
-    """(y, x, radius, inner weight, outer weight) of an instruction (src/model.py:1270-1376) or None."""
+def focus_cell(name: str, g: int):
+    """(y, x) of an off-centre instruction's focus cell (src/model.py:1282-1376), or None for "center" and unknown
+    strings."""
     q, h, t = g // 4, g // 2, g * 3 // 4
-    if name == "center":
-        return h, h, max(1, g // 4), 3.0, 1.5
-    table = {"left": (h, q), "right": (h, t), "top": (q, h), "bottom": (t, h), "top-left": (q, q),
-             "top-right": (q, t), "bottom-left": (t, q), "bottom-right": (t, t)}
-    if name in table:
-        y, x = table[name]
-        return y, x, max(1, g // 6), 5.0, 2.0
-    return None
+    return {"left": (h, q), "right": (h, t), "top": (q, h), "bottom": (t, h), "top-left": (q, q), "top-right": (q, t),
+            "bottom-left": (t, q), "bottom-right": (t, t)}.get(name)
 
 
-def instruction_mask(instruction: str, g: int) -> torch.Tensor:
-    """Flattened g x g spatial mask of a textual instruction; unknown strings give all ones (reference behaviour)."""
-    f = _focus(canonical_instruction(instruction), g)
+def _disk_mask(fy: int, fx: int, g: int, r: int, hi: float, lo: float) -> torch.Tensor:
+    """hi where the distance to (fy, fx) is <= r, lo where it is <= 2r, 1 elsewhere."""
     mask = torch.ones(g, g, dtype=torch.float32)
-    if f is None:
-        return mask.flatten()
-    fy, fx, r, hi, lo = f
     y, x = torch.meshgrid(torch.arange(g), torch.arange(g), indexing="ij")
     dist = torch.sqrt(((y - fy) ** 2 + (x - fx) ** 2).double())  # math.sqrt on Python ints == exact fp64
     mask[dist <= 2 * r] = lo
     mask[dist <= r] = hi
     return mask.flatten()
+
+
+def focus_mask(y: int, x: int, g: int) -> torch.Tensor:
+    """Flattened g x g mask of the off-centre instructions with the focus moved to cell (y, x): 5.0 where
+    dy^2 + dx^2 <= r^2, 2.0 where dy^2 + dx^2 <= 4 r^2, 1.0 elsewhere, r = max(1, g // 6) (src/model.py:1282-1376).
+    Each of the eight off-centre instructions is this mask at its `focus_cell`; "center" is not (it has its own radius
+    and weights).  Cell (y, x) of `CognitiveAimModel.depth_field` is the guided call with this mask."""
+    if not (0 <= y < g and 0 <= x < g):
+        raise ValueError(f"focus cell ({y}, {x}) lies outside the {g} x {g} grid")
+    return _disk_mask(y, x, g, max(1, g // 6), 5.0, 2.0)
+
+
+def instruction_mask(instruction: str, g: int) -> torch.Tensor:
+    """Flattened g x g spatial mask of a textual instruction; unknown strings give all ones (reference behaviour)."""
+    name = canonical_instruction(instruction)
+    if name == "center":
+        h = g // 2
+        return _disk_mask(h, h, g, max(1, g // 4), 3.0, 1.5)
+    cell = focus_cell(name, g)
+    if cell is None:
+        return torch.ones(g * g, dtype=torch.float32)
+    return focus_mask(*cell, g)
 
 
 def resolve_guidance(guidance, n: int) -> torch.Tensor:

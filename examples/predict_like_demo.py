@@ -3,6 +3,7 @@
     python examples/predict_like_demo.py IMAGE.jpg [--instruction center] [--image-size 224] [--overlay out.npy]
     python examples/predict_like_demo.py --image-dir DIR [--instruction center] [--image-size 224]
     python examples/predict_like_demo.py IMAGE.jpg --interactive < instructions.txt
+    python examples/predict_like_demo.py IMAGE.jpg --depth-field OUT.npz
 
 What demo.py does per image and what runs here instead:
     Image.open(path).convert('RGB')                    -> nvJPEG decode on the GPU              (model.preprocess_jpeg)
@@ -18,6 +19,9 @@ nvJPEG call and runs the photographs, whatever their sizes, through ONE forward 
 `--interactive` encodes the photograph once (`Predictor.encode`, model.encode: decode, backbone, focal stream) and then
 reads instructions from stdin, one per line, printing for each the line `predict` prints (`Predictor.predict_scene`,
 model.guide); the results equal successive `predict` calls on the same photograph.
+`--depth-field OUT.npz` encodes the photograph once and saves the guided depth and confidence with the focus on every
+cell of the g x g patch grid (`Predictor.depth_field`, model.depth_field) as `depth` and `confidence` [g, g]: cell
+(y, x) is the prediction of a guided call focused there (cell (g//4, g//4) is the "top-left" prediction).
 Weights: random init (seed 0, the reference's own construction order) unless --checkpoint names a reference state_dict.
 """
 from __future__ import annotations
@@ -151,6 +155,13 @@ class Predictor:
             meta["overlay"] = self.model.focus_map(overlay_size, attention=heat)[0]
         return float(depth.squeeze()), float(conf.squeeze()), meta
 
+    @torch.no_grad()
+    def depth_field(self, jpeg_bytes: bytes, exif=None):
+        """-> (depth, confidence) [g, g] CPU tensors: the guided prediction with the focus on every cell of the patch grid,
+        from one encode and one depth-field call."""
+        depth, conf = self.model.depth_field(self.encode(jpeg_bytes, exif))
+        return depth[0].cpu(), conf[0].cpu()
+
     def model_images(self, jpeg_files):
         """JPEG files (bytes) -> list of decoded uint8 [H_i, W_i, 3] CUDA tensors (one nvjpegDecodeBatched call)."""
         with torch.cuda.device(self.device):
@@ -171,6 +182,8 @@ def main():
     ap.add_argument("--overlay", default=None, help="write the overlay heat map of the last instruction as .npy")
     ap.add_argument("--interactive", action="store_true",
                     help="encode IMAGE once, then read instructions from stdin, one per line")
+    ap.add_argument("--depth-field", default=None, metavar="OUT.npz",
+                    help="save the guided depth and confidence with the focus on every patch cell as [g, g] arrays")
     args = ap.parse_args()
     if (args.image is None) == (args.image_dir is None):
         ap.error("give IMAGE or --image-dir DIR")
@@ -190,6 +203,16 @@ def main():
             print(result_line(args.instruction, depth, conf, meta))
         return
     data = open(args.image, "rb").read()
+    if args.depth_field:
+        if args.instruction or args.overlay or args.interactive:
+            ap.error("--depth-field takes no --instruction, --overlay or --interactive")
+        import numpy as np
+        depth, conf = p.depth_field(data)
+        np.savez(args.depth_field, depth=depth.numpy(), confidence=conf.numpy())
+        g = depth.shape[0]
+        print(f"depth field {g} x {g}: depth {float(depth.min()):.4f} .. {float(depth.max()):.4f}  confidence "
+              f"{float(conf.min()):.4f} .. {float(conf.max()):.4f}  -> {args.depth_field}")
+        return
     if args.interactive:
         if args.instruction or args.overlay:
             ap.error("--interactive reads its instructions from stdin and takes no --overlay")

@@ -211,6 +211,23 @@ int ca_guide_tail(const ca_heads_weights* w, const ca_heads_inputs* in, const fl
                   long long mask_batch_stride, float* heat, int32_t* argmax, uint32_t* ticket, float* depth, float* conf,
                   int B, int N, float alpha, float temperature, void* stream);
 
+/* Depth fields (CognitiveAimModel.depth_field): the guided call with the focus on every cell of the g x g grid.
+ * P[b, n, :] = src[b * src_batch_stride + (row_offset + n) * 768 + :] . tmp_w^T for n < N: [B, N, 64] fp32, the per-call
+ * projection tmp_w [64, 768] applied to every patch token once.  src, tmp_w and P 16-byte aligned. */
+int ca_token_project(const float* src, long long src_batch_stride, int row_offset, const float* tmp_w, float* P, int B,
+                     int N, void* stream);
+/* depth[b, c], conf[b, c] for every cell c = y * g + x of the g x g grid: the guided call (ca_guided_softmax ->
+ * ca_weighted_pool -> ca_heads) whose mask is 5 on the disk dy^2 + dx^2 <= r^2 around (y, x), 2 out to 2r and 1 elsewhere,
+ * r = max(1, g / 6).  base [B, g * g] is the focal attention, a probability vector per image (0 <= base <= 1): then the
+ * disk's logits exceed all others by (4 alpha - 1) / temperature = 36 at the reference's 0.7 / 0.05, and the softmax is
+ * taken over the disk alone (the rest weighs < N e^-36).  Other alpha / temperature are refused when that gap is below 36.
+ * P [B, g * g, 64] from ca_token_project; tmp_b [64] the projection bias (in->tmp_b).  `in` supplies tokens (the CLS rows,
+ * tokens_per_img), tmp_b, exif, camera_idx, num_cameras and fault as for ca_heads; its other members are not read.
+ * cst: [B, 192] scratch (the fusion layer's per-image part).  Two launches; no atomics in any reduction. */
+int ca_depth_field_cells(const ca_heads_weights* w, const ca_heads_inputs* in, const float* base, const float* P,
+                         float* cst, float* depth, float* conf, int B, int g, float alpha, float temperature,
+                         void* stream);
+
 typedef struct ca_focal_value_args {
   const float* tok_partial;  /* [B, splits, 768] partial sums of c_j * rowscale_j * tokens_j */
   const float* pe_partial;   /* [B, splits, 768] partial sums of c_j * PE_j */
@@ -462,6 +479,19 @@ typedef struct ca_guide_call {
 int ca_guide(ca_handle* h, ca_scene* scene, const ca_guide_call* call, void* stream);
 /* ca_forward_guided_sweep on the encoded images, bit for bit given the same draws (ca_sweep_call as there). */
 int ca_guide_sweep(ca_handle* h, ca_scene* scene, const ca_sweep_call* sweep, void* stream);
+/* A depth field of a scene: HOST pointers where marked, device otherwise. */
+typedef struct ca_depth_field_call {
+  const float* tmp_w;           /* HOST [64, 768]: per-call projection weight   src/model.py:1421 */
+  const float* tmp_b;           /* HOST [64] */
+  const float* eps;             /* HOST [B, 192]: CuriosityModule draw of :609 */
+  const float* noise;           /* HOST [B, 768]: draw of :744 */
+  float* depth;                 /* out [B, N]: cell c = y * g + x */
+  float* conf;                  /* out [B, N] */
+} ca_depth_field_call;
+/* The guided depth and confidence with the focus mask of every cell of the grid (ca_depth_field_cells), from one call's
+ * draws: one projection for every cell and one CuriosityModule run (B ring entries).  The scene graph policy and the
+ * refusals are those of ca_guide. */
+int ca_depth_field(ca_handle* h, ca_scene* scene, const ca_depth_field_call* call, void* stream);
 /* Release a scene's memory and graphs (waits for the device).  NULL is a no-op. */
 int ca_scene_destroy(ca_scene* scene);
 
