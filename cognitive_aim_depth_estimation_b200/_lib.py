@@ -93,7 +93,7 @@ class ForwardCall(C.Structure):
 
 
 SWEEP_MAX_K = 16  # CA_SWEEP_MAX_K (include/cogaim_b200.h)
-GUIDE_TAIL_MAX_B = 1  # CA_GUIDE_TAIL_MAX_B: guide calls of larger batches run the three-kernel chain
+GUIDE_TAIL_MAX_B = 1  # CA_GUIDE_TAIL_MAX_B: single guided calls of larger batches (and sweeps) run the three-kernel chain
 RESIZE_MAX_SIDE = 16384  # CA_RESIZE_MAX_SIDE
 RESIZE_LIST_CHUNK = 128  # CA_RESIZE_LIST_CHUNK
 

@@ -178,27 +178,27 @@ int ca_focal_finalize(const float* pc, const float* cbias, float* attn, const fl
 
 int ca_guided_softmax(const float* base, const float* mask, long long mask_batch_stride, float* heat, int32_t* argmax,
                       int B, int N, float alpha, float temperature, void* stream) {
-  return ca::guided_softmax_launch(base, mask, mask_batch_stride, heat, argmax, B, N, alpha, temperature,
+  return ca::guided_softmax_launch(base, 0, mask, 0, mask_batch_stride, heat, argmax, 1, B, N, alpha, temperature,
                                    static_cast<cudaStream_t>(stream));
 }
 
 int ca_weighted_pool(const float* src, long long src_batch_stride, int row_offset, const float* w, const float* w2,
                      float* partial, int B, int N, int D, int splits, void* stream) {
-  return ca::weighted_pool_launch(src, src_batch_stride, row_offset, w, w2, partial, B, N, D, splits,
+  return ca::weighted_pool_launch(src, src_batch_stride, row_offset, w, w2, partial, 1, B, N, D, splits,
                                   static_cast<cudaStream_t>(stream));
 }
 
 int ca_guided_softmax_sweep(const float* base, long long base_k_stride, const float* mask, long long mask_k_stride,
                             long long mask_batch_stride, float* heat, int32_t* argmax, int K, int B, int N, float alpha,
                             float temperature, void* stream) {
-  return ca::guided_softmax_sweep_launch(base, base_k_stride, mask, mask_k_stride, mask_batch_stride, heat, argmax, K, B, N,
-                                         alpha, temperature, static_cast<cudaStream_t>(stream));
+  return ca::guided_softmax_launch(base, base_k_stride, mask, mask_k_stride, mask_batch_stride, heat, argmax, K, B, N,
+                                   alpha, temperature, static_cast<cudaStream_t>(stream));
 }
 
 int ca_weighted_pool_sweep(const float* src, long long src_batch_stride, int row_offset, const float* w, float* partial,
                            int K, int B, int N, int D, int splits, void* stream) {
-  return ca::weighted_pool_sweep_launch(src, src_batch_stride, row_offset, w, partial, K, B, N, D, splits,
-                                        static_cast<cudaStream_t>(stream));
+  return ca::weighted_pool_launch(src, src_batch_stride, row_offset, w, nullptr, partial, K, B, N, D, splits,
+                                  static_cast<cudaStream_t>(stream));
 }
 
 int ca_heads(const ca_heads_weights* w, const ca_heads_inputs* in, float* depth, float* conf, float* fused_out, int B,

@@ -269,12 +269,18 @@ __global__ void __launch_bounds__(256) guided_softmax_kernel(const float* __rest
   if (threadIdx.x == 0 && argmax) argmax[r] = mi;
 }
 
-// partial[b, split, :] = sum_{n in split} w[b, n] * (w2 ? w2[b, n] : 1) * src[b*src_batch_stride + (row_offset+n)*D + :]
-// D = 768: 192 threads x float4.  grid = (splits, B).
+// partial[k * B + b, split, :] = sum_{n in split} w[k, b, n] * (w2 ? w2[b, n] : 1) * src[b*src_batch_stride + (row_offset+n)*D + :]
+// for K <= KMAX weight vectors w [K, B, N] (K = 1: a single vector; K > 1: an instruction sweep).  D = 768: 192 threads x
+// float4.  grid = (splits, B).  A CTA reads its rows of image b's tokens ONCE and keeps one float4 accumulator per vector.
+// Every accumulator goes through the same sequence — same rows per split, same batches of 8 rows with the same zero padding
+// in the tail, same fmaf chain — so partial row k * B + b is bit for bit the KMAX = 1 result for weight vector k alone.
+// KMAX accumulators live in registers (16 x 4 at the largest instantiation, no spills).  w2 (the focal value path's second
+// factor) is read by the KMAX = 1 instantiation only, whose loads and FMAs are those of a plain one-vector pool.
+template <int KMAX>
 __global__ void __launch_bounds__(192) weighted_pool_kernel(const float* __restrict__ src, long long src_batch_stride,
                                                              int row_offset, const float* __restrict__ w,
                                                              const float* __restrict__ w2, float* __restrict__ partial,
-                                                             int N, int D, int rows_per_split) {
+                                                             int K, int B, int N, int D, int rows_per_split) {
   griddep_sync();  // PDL: nothing before this line reads or writes global memory
   const int b = blockIdx.y;
   const int split = blockIdx.x;
@@ -284,8 +290,11 @@ __global__ void __launch_bounds__(192) weighted_pool_kernel(const float* __restr
                                                      static_cast<size_t>(row_offset) * D);
   const float* wb = w + static_cast<size_t>(b) * N;
   const float* w2b = w2 ? w2 + static_cast<size_t>(b) * N : nullptr;
+  const size_t w_k_stride = static_cast<size_t>(B) * N;
   const int dv = D / 4;
-  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  float4 acc[KMAX];
+#pragma unroll
+  for (int k = 0; k < KMAX; ++k) acc[k] = make_float4(0.f, 0.f, 0.f, 0.f);
   constexpr int kBatch = 8;  // loads of a batch issued together (memory-level parallelism), then the FMAs in row order
   for (int n = n0; n < n1; n += kBatch) {
     float4 t[kBatch];
@@ -294,55 +303,16 @@ __global__ void __launch_bounds__(192) weighted_pool_kernel(const float* __restr
     for (int u = 0; u < kBatch; ++u) {
       const bool in = n + u < n1;
       t[u] = in ? s4[static_cast<size_t>(n + u) * dv + threadIdx.x] : make_float4(0.f, 0.f, 0.f, 0.f);
-      g[u] = in ? (w2b ? wb[n + u] * w2b[n + u] : wb[n + u]) : 0.f;
+      if (KMAX == 1) g[u] = in ? (w2b ? wb[n + u] * w2b[n + u] : wb[n + u]) : 0.f;  // one vector: loaded with the tokens
     }
-#pragma unroll
-    for (int u = 0; u < kBatch; ++u) {
-      acc.x = fmaf(g[u], t[u].x, acc.x);
-      acc.y = fmaf(g[u], t[u].y, acc.y);
-      acc.z = fmaf(g[u], t[u].z, acc.z);
-      acc.w = fmaf(g[u], t[u].w, acc.w);
-    }
-  }
-  reinterpret_cast<float4*>(partial + (static_cast<size_t>(b) * gridDim.x + split) * D)[threadIdx.x] = acc;
-}
-
-// weighted_pool_kernel for K weight vectors at once (an instruction sweep): w is [K, B, N] (row k * B + b), partial is
-// [K * B, splits, D].  A CTA reads its rows of image b's tokens ONCE and keeps one float4 accumulator per vector.  Each
-// accumulator goes through weighted_pool_kernel's exact sequence — same rows per split, same batches of 8 rows with the
-// same zero padding in the tail, same fmaf chain — so partial row k * B + b is bit for bit what weighted_pool_kernel
-// writes for weight vector k.  KMAX accumulators live in registers (16 x 4 at the largest instantiation, no spills).
-template <int KMAX>
-__global__ void __launch_bounds__(192) weighted_pool_sweep_kernel(const float* __restrict__ src, long long src_batch_stride,
-                                                                   int row_offset, const float* __restrict__ w,
-                                                                   float* __restrict__ partial, int K, int B, int N, int D,
-                                                                   int rows_per_split) {
-  griddep_sync();  // PDL: nothing before this line reads or writes global memory
-  const int b = blockIdx.y;
-  const int split = blockIdx.x;
-  const int n0 = split * rows_per_split;
-  const int n1 = min(N, n0 + rows_per_split);
-  const float4* s4 = reinterpret_cast<const float4*>(src + static_cast<size_t>(b) * src_batch_stride +
-                                                     static_cast<size_t>(row_offset) * D);
-  const float* wb = w + static_cast<size_t>(b) * N;
-  const size_t w_k_stride = static_cast<size_t>(B) * N;
-  const int dv = D / 4;
-  float4 acc[KMAX];
-#pragma unroll
-  for (int k = 0; k < KMAX; ++k) acc[k] = make_float4(0.f, 0.f, 0.f, 0.f);
-  constexpr int kBatch = 8;
-  for (int n = n0; n < n1; n += kBatch) {
-    float4 t[kBatch];
-#pragma unroll
-    for (int u = 0; u < kBatch; ++u)
-      t[u] = (n + u < n1) ? s4[static_cast<size_t>(n + u) * dv + threadIdx.x] : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
     for (int k = 0; k < KMAX; ++k) {
-      if (k < K) {
-        const float* wk = wb + k * w_k_stride;
-        float g[kBatch];
+      if (KMAX == 1 || k < K) {
+        if (KMAX > 1) {
+          const float* wk = wb + k * w_k_stride;
 #pragma unroll
-        for (int u = 0; u < kBatch; ++u) g[u] = (n + u < n1) ? wk[n + u] : 0.f;
+          for (int u = 0; u < kBatch; ++u) g[u] = (n + u < n1) ? wk[n + u] : 0.f;
+        }
 #pragma unroll
         for (int u = 0; u < kBatch; ++u) {
           acc[k].x = fmaf(g[u], t[u].x, acc[k].x);
@@ -355,7 +325,7 @@ __global__ void __launch_bounds__(192) weighted_pool_sweep_kernel(const float* _
   }
 #pragma unroll
   for (int k = 0; k < KMAX; ++k)
-    if (k < K)
+    if (KMAX == 1 || k < K)
       reinterpret_cast<float4*>(partial + ((static_cast<size_t>(k) * B + b) * gridDim.x + split) * D)[threadIdx.x] = acc[k];
 }
 
@@ -524,25 +494,15 @@ int focal_finalize_launch(const float* pc, const float* cbias, float* attn, cons
   return 0;
 }
 
-int guided_softmax_launch(const float* base, const float* mask, long long mask_batch_stride, float* heat, int* argmax,
-                          int B, int N, float alpha, float temperature, cudaStream_t stream) {
+int guided_softmax_launch(const float* base, long long base_k_stride, const float* mask, long long mask_k_stride,
+                          long long mask_batch_stride, float* heat, int* argmax, int K, int B, int N, float alpha,
+                          float temperature, cudaStream_t stream) {
   CA_REQUIRE(base && mask && heat, "guided_softmax: null pointer");
-  CA_REQUIRE(mask_batch_stride == 0 || mask_batch_stride >= N, "guided_softmax: mask batch stride must be 0 or >= N");
-  CA_TRY(launch_kernel(guided_softmax_kernel, dim3(B), dim3(256), 0, stream, base, 0LL, mask, 0LL, mask_batch_stride, heat,
-                       argmax, B, N, alpha, temperature));
-  CA_CUDA(cudaGetLastError());
-  return 0;
-}
-
-int guided_softmax_sweep_launch(const float* base, long long base_k_stride, const float* mask, long long mask_k_stride,
-                                long long mask_batch_stride, float* heat, int* argmax, int K, int B, int N, float alpha,
-                                float temperature, cudaStream_t stream) {
-  CA_REQUIRE(base && mask && heat, "guided_softmax_sweep: null pointer");
-  CA_REQUIRE(K >= 1 && K <= kSweepMaxK && B > 0 && N > 0, "guided_softmax_sweep: 1..16 instructions, B > 0, N > 0");
+  CA_REQUIRE(K >= 1 && K <= kSweepMaxK && B > 0 && N > 0, "guided_softmax: 1..16 instructions, B > 0, N > 0");
   CA_REQUIRE(base_k_stride == 0 || base_k_stride >= static_cast<long long>(B) * N,
-             "guided_softmax_sweep: base stride per instruction must be 0 or >= B * N");
-  CA_REQUIRE(mask_batch_stride == 0 || mask_batch_stride >= N, "guided_softmax_sweep: mask batch stride must be 0 or >= N");
-  CA_REQUIRE(mask_k_stride == 0 || mask_k_stride >= N, "guided_softmax_sweep: mask stride per instruction must be 0 or >= N");
+             "guided_softmax: base stride per instruction must be 0 or >= B * N");
+  CA_REQUIRE(mask_batch_stride == 0 || mask_batch_stride >= N, "guided_softmax: mask batch stride must be 0 or >= N");
+  CA_REQUIRE(mask_k_stride == 0 || mask_k_stride >= N, "guided_softmax: mask stride per instruction must be 0 or >= N");
   CA_TRY(launch_kernel(guided_softmax_kernel, dim3(K * B), dim3(256), 0, stream, base, base_k_stride, mask, mask_k_stride,
                        mask_batch_stride, heat, argmax, B, N, alpha, temperature));
   CA_CUDA(cudaGetLastError());
@@ -550,34 +510,27 @@ int guided_softmax_sweep_launch(const float* base, long long base_k_stride, cons
 }
 
 int weighted_pool_launch(const float* src, long long src_batch_stride, int row_offset, const float* w, const float* w2,
-                         float* partial, int B, int N, int D, int splits, cudaStream_t stream) {
+                         float* partial, int K, int B, int N, int D, int splits, cudaStream_t stream) {
   CA_REQUIRE(src && w && partial, "weighted_pool: null pointer");
   CA_REQUIRE(D == 768, "weighted_pool: only D = 768 is instantiated");
-  CA_REQUIRE(splits > 0, "weighted_pool: splits must be positive");
+  CA_REQUIRE(splits > 0 && B > 0 && N > 0, "weighted_pool: splits, B and N must be positive");
+  CA_REQUIRE(K >= 1 && K <= kSweepMaxK, "weighted_pool: 1..16 weight vectors");
+  CA_REQUIRE(w2 == nullptr || K == 1, "weighted_pool: w2 only with a single weight vector");
   const int rps = (N + splits - 1) / splits;
-  CA_TRY(launch_kernel(weighted_pool_kernel, dim3(dim3(splits, B)), dim3(192), 0, stream, src, src_batch_stride, row_offset, w, w2, partial, N, D, rps));
-  CA_CUDA(cudaGetLastError());
-  return 0;
-}
-
-int weighted_pool_sweep_launch(const float* src, long long src_batch_stride, int row_offset, const float* w, float* partial,
-                               int K, int B, int N, int D, int splits, cudaStream_t stream) {
-  CA_REQUIRE(src && w && partial, "weighted_pool_sweep: null pointer");
-  CA_REQUIRE(D == 768, "weighted_pool_sweep: only D = 768 is instantiated");
-  CA_REQUIRE(splits > 0 && B > 0 && N > 0, "weighted_pool_sweep: splits, B and N must be positive");
-  CA_REQUIRE(K >= 1 && K <= kSweepMaxK, "weighted_pool_sweep: 1..16 weight vectors");
-  const int rps = (N + splits - 1) / splits;  // the split of weighted_pool_launch: the partials must line up with it
   const dim3 grid(splits, B);
   // the smallest instantiation that holds K accumulators: registers (and so occupancy) follow K
-  if (K <= 4)
-    CA_TRY(launch_kernel(weighted_pool_sweep_kernel<4>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w,
+  if (K == 1)
+    CA_TRY(launch_kernel(weighted_pool_kernel<1>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w, w2,
+                         partial, K, B, N, D, rps));
+  else if (K <= 4)
+    CA_TRY(launch_kernel(weighted_pool_kernel<4>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w, w2,
                          partial, K, B, N, D, rps));
   else if (K <= 8)
-    CA_TRY(launch_kernel(weighted_pool_sweep_kernel<8>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w,
+    CA_TRY(launch_kernel(weighted_pool_kernel<8>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w, w2,
                          partial, K, B, N, D, rps));
   else
-    CA_TRY(launch_kernel(weighted_pool_sweep_kernel<kSweepMaxK>, grid, dim3(192), 0, stream, src, src_batch_stride,
-                         row_offset, w, partial, K, B, N, D, rps));
+    CA_TRY(launch_kernel(weighted_pool_kernel<kSweepMaxK>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset,
+                         w, w2, partial, K, B, N, D, rps));
   CA_CUDA(cudaGetLastError());
   return 0;
 }

@@ -53,21 +53,20 @@ struct Workspace {
   unsigned long long gen = 0;  // unique per allocation: a scene's graphs captured on another workspace are not replayed
   void* arena = nullptr;
   __nv_bfloat16 *patches, *h, *qkv, *att, *mlp, *xin, *qk;
-  float *x, *tokens, *pm, *ps, *pc, *wtab, *attn, *cvec, *rowscale, *heat, *pool, *pool_pe, *pooled, *feats, *focal_feat,
-      *fused, *depth, *conf, *mask_in, *tmpw, *tmpb, *exif_in, *cur_eps, *cur_noise, *cur_raw, *cur_reward, *ln_stats;
+  float *x, *tokens, *pm, *ps, *pc, *wtab, *attn, *cvec, *rowscale, *pool, *pool_pe, *feats, *focal_feat, *fused, *depth,
+      *conf, *exif_in, *cur_eps, *cur_noise, *cur_raw, *cur_reward, *ln_stats;
   void* E;
-  int* argmax;
-  int* tail_ticket;  // [B] per-image tickets of the fused guide tail, zero when idle
   long long* cam_in;
   int P = 0, lde = 0;
   std::map<int, std::pair<cudaGraphExec_t, int>> graphs;  // path key -> (executable graph, launches)
   std::map<int, int> seen;                                // path key -> calls so far
-  // instruction sweeps: the per-call buffers of K calls (rows k * B + b), one arena per K; the backbone and focal
-  // buffers above are shared with the single-call paths
+  // guided calls: the per-call buffers of K calls (rows k * B + b; K = 1 for a single call), one arena per K; the
+  // backbone and focal buffers above are shared with the un-guided forward
   struct Sweep {
     void* arena = nullptr;
     float *mask_in, *heat, *pool, *depth, *conf, *tmpw, *tmpb, *cur_eps, *cur_noise, *cur_raw, *cur_reward;
     int* argmax;
+    int* tail_ticket;  // [B] per-image tickets of the fused guide tail, zero when idle
   };
   std::map<int, Sweep> sweeps;  // K -> buffers
   // depth fields (allocated at the first ca_depth_field on this workspace): projected tokens [B, N, 64], the per-image
@@ -338,22 +337,15 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   want(&w.attn, iters * BN * 4);
   want(&w.cvec, BN * 4);
   want(&w.rowscale, 2 * BN * 4);
-  want(&w.heat, BN * 4);
-  want(&w.argmax, B * 4);
   want(&w.pool, static_cast<size_t>(B) * kPoolSplits * kD * 4);
   want(&w.pool_pe, static_cast<size_t>(B) * kPoolSplits * kD * 4);
-  want(&w.pooled, static_cast<size_t>(B) * kD * 4);
   want(&w.feats, static_cast<size_t>(B) * iters * 64 * 4);
   want(&w.focal_feat, static_cast<size_t>(B) * 64 * 4);
   want(&w.fused, static_cast<size_t>(B) * 192 * 4);
   want(&w.depth, B * 4);
   want(&w.conf, B * 4);
-  want(&w.mask_in, BN * 4);
-  want(&w.tmpw, 64 * kD * 4);
-  want(&w.tmpb, 64 * 4);
   want(&w.exif_in, B * 3 * 4);
   want(&w.cam_in, B * 8);
-  want(&w.tail_ticket, B * 4);
   want(&w.cur_eps, static_cast<size_t>(kMaxRuns) * B * 192 * 4);
   want(&w.cur_noise, static_cast<size_t>(kMaxRuns) * B * kD * 4);
   want(&w.cur_raw, static_cast<size_t>(kMaxRuns) * B * 4);
@@ -362,7 +354,6 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   for (auto& s : slots) *s.p = static_cast<char*>(w.arena) + s.o;
   CA_CUDA(cudaMemset(w.exif_in, 0, B * 3 * 4));
   CA_CUDA(cudaMemset(w.cam_in, 0, B * 8));
-  CA_CUDA(cudaMemset(w.tail_ticket, 0, B * 4));
   static std::atomic<unsigned long long> next_gen{1};
   w.gen = next_gen.fetch_add(1);
   *out = &h->ws.emplace(key, w).first->second;
@@ -381,7 +372,7 @@ int get_sweep(Workspace& w, int K, Workspace::Sweep** out) {
       slots.push_back({reinterpret_cast<void**>(p), off});
       off += (bytes + 255) & ~static_cast<size_t>(255);
     };
-    want(&s.mask_in, K * N * 4);
+    want(&s.mask_in, KB * N * 4);  // a mask row per image and call at most
     want(&s.heat, KB * N * 4);
     want(&s.argmax, KB * 4);
     want(&s.pool, KB * kPoolSplits * kD * 4);
@@ -393,8 +384,10 @@ int get_sweep(Workspace& w, int K, Workspace::Sweep** out) {
     want(&s.cur_noise, KB * kD * 4);
     want(&s.cur_raw, KB * 4);
     want(&s.cur_reward, KB * 4);
+    want(&s.tail_ticket, static_cast<size_t>(w.B) * 4);
     CA_CUDA(cudaMalloc(&s.arena, off));
     for (auto& sl : slots) *sl.first = static_cast<char*>(s.arena) + sl.second;
+    CA_CUDA(cudaMemset(s.tail_ticket, 0, static_cast<size_t>(w.B) * 4));
     it = w.sweeps.emplace(K, s).first;
   }
   *out = &it->second;
@@ -549,8 +542,8 @@ int focal_iterations(ca_handle* h, Workspace& w, const Tables& tb, bool want_fea
       LAUNCH(ca::rowstats_merge_launch(w.pm, w.ps, attn, nullptr, nullptr, w.wtab, B * N, N, w.P, st));
       LAUNCH(ca::colsum_e_launch(w.E, w.lde, static_cast<long long>(N) * w.lde, w.wtab, w.pc, B, N, w.P, st));
       LAUNCH(ca::focal_finalize_launch(w.pc, nullptr, w.cvec, nullptr, nullptr, B, N, w.P, 0.0f, 1, nullptr, 0.5f, st));
-      LAUNCH(ca::weighted_pool_launch(w.tokens, static_cast<long long>(T) * kD, 1, w.cvec, rs, w.pool, B, N, kD, kPoolSplits, st));
-      LAUNCH(ca::weighted_pool_launch(tb.pe, 0, 0, w.cvec, nullptr, w.pool_pe, B, N, kD, kPoolSplits, st));
+      LAUNCH(ca::weighted_pool_launch(w.tokens, static_cast<long long>(T) * kD, 1, w.cvec, rs, w.pool, 1, B, N, kD, kPoolSplits, st));
+      LAUNCH(ca::weighted_pool_launch(tb.pe, 0, 0, w.cvec, nullptr, w.pool_pe, 1, B, N, kD, kPoolSplits, st));
       ca_focal_value_args v{};
       v.tok_partial = w.pool;
       v.pe_partial = w.pool_pe;
@@ -599,25 +592,17 @@ int curiosity_join(ca_handle* h, cudaStream_t st) {
   return 0;
 }
 
-int heads(ca_handle* h, Workspace& w, bool guided, bool has_exif, int* fault, cudaStream_t st) {
+int heads(ca_handle* h, Workspace& w, bool has_exif, int* fault, cudaStream_t st) {
   const int g = w.S / 14, T = g * g + 1;
   ca_heads_inputs in{};
   in.tokens = w.tokens;
   in.tokens_per_img = T;
-  if (guided) {
-    in.pool_partial = w.pool;
-    in.pool_splits = kPoolSplits;
-    in.tmp_w = w.tmpw;
-    in.tmp_b = w.tmpb;
-    in.pooled_out = w.pooled;
-  } else {
-    in.focal_feat = w.focal_feat;
-  }
+  in.focal_feat = w.focal_feat;
   in.exif = has_exif ? w.exif_in : nullptr;
   in.camera_idx = has_exif ? w.cam_in : nullptr;
   in.num_cameras = h->w.num_cameras;
   in.fault = fault;
-  LAUNCH(ca::heads_launch(h->w.heads, in, w.depth, w.conf, guided ? nullptr : w.fused, w.B, st));
+  LAUNCH(ca::heads_launch(h->w.heads, in, w.depth, w.conf, w.fused, w.B, st));
   return 0;
 }
 
@@ -637,22 +622,12 @@ int pinned_slot(ca_handle* h, size_t need, PinnedSlot** out) {
   return 0;
 }
 
-int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, bool guided, int runs, cudaStream_t st) {
+int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, int runs, cudaStream_t st) {
   const size_t B = w.B;
-  const size_t n_w = guided ? 64 * kD + 64 : 0;
-  const size_t need = n_w + static_cast<size_t>(runs) * B * (192 + kD);
   PinnedSlot* sp = nullptr;
-  CA_TRY(pinned_slot(h, need, &sp));
+  CA_TRY(pinned_slot(h, static_cast<size_t>(runs) * B * (192 + kD), &sp));
   PinnedSlot& s = *sp;
   float* p = s.buf;
-  if (guided) {
-    memcpy(p, c.tmp_w, 64 * kD * sizeof(float));
-    memcpy(p + 64 * kD, c.tmp_b, 64 * sizeof(float));
-    CA_TRY(ca::fetch_pinned_launch(w.tmpw, p, 64 * kD, st));
-    CA_TRY(ca::fetch_pinned_launch(w.tmpb, p + 64 * kD, 64, st));
-    h->launches += 2;
-    p += n_w;
-  }
   memcpy(p, c.eps, static_cast<size_t>(runs) * B * 192 * sizeof(float));
   memcpy(p + static_cast<size_t>(runs) * B * 192, c.noise, static_cast<size_t>(runs) * B * kD * sizeof(float));
   CA_TRY(ca::fetch_pinned_launch(w.cur_eps, p, static_cast<size_t>(runs) * B * 192, st));
@@ -662,17 +637,18 @@ int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, bool
   return 0;
 }
 
-// the K calls' projections and curiosity draws (HOST) -> one pinned slot sized for K -> the sweep's device buffers
-int stage_sweep_inputs(ca_handle* h, Workspace& w, Workspace::Sweep& s, const ca_sweep_call& c, cudaStream_t st) {
-  const size_t K = c.K, B = w.B;
+// the K guided calls' projections and curiosity draws (HOST) -> one pinned slot sized for K -> the device buffers of K
+int stage_guided_draws(ca_handle* h, Workspace& w, Workspace::Sweep& s, size_t K, const float* tmp_w, const float* tmp_b,
+                       const float* eps, const float* noise, cudaStream_t st) {
+  const size_t B = w.B;
   const size_t n_tw = K * 64 * kD, n_tb = K * 64, n_eps = K * B * 192, n_noise = K * B * kD;
   PinnedSlot* slot = nullptr;
   CA_TRY(pinned_slot(h, n_tw + n_tb + n_eps + n_noise, &slot));
   float* p = slot->buf;
-  memcpy(p, c.tmp_w, n_tw * sizeof(float));
-  memcpy(p + n_tw, c.tmp_b, n_tb * sizeof(float));
-  memcpy(p + n_tw + n_tb, c.eps, n_eps * sizeof(float));
-  memcpy(p + n_tw + n_tb + n_eps, c.noise, n_noise * sizeof(float));
+  memcpy(p, tmp_w, n_tw * sizeof(float));
+  memcpy(p + n_tw, tmp_b, n_tb * sizeof(float));
+  memcpy(p + n_tw + n_tb, eps, n_eps * sizeof(float));
+  memcpy(p + n_tw + n_tb + n_eps, noise, n_noise * sizeof(float));
   CA_TRY(ca::fetch_pinned_launch(s.tmpw, p, n_tw, st));
   CA_TRY(ca::fetch_pinned_launch(s.tmpb, p + n_tw, n_tb, st));
   CA_TRY(ca::fetch_pinned_launch(s.cur_eps, p + n_tw + n_tb, n_eps, st));
@@ -797,11 +773,31 @@ int scene_workspace(ca_handle* h, ca_scene* sc, Workspace** out, Tables** tb) {
   return 0;
 }
 
-int check_call(const ca_handle* h, const ca_forward_call* c) {
-  CA_REQUIRE(h && c, "null handle / call");
-  CA_REQUIRE(c->B > 0, "forward: empty batch");
+// The batch of a call (its images and side) and, with `exif_for`, its EXIF inputs: what every entry point that takes a
+// batch checks.  The error texts start with the entry point's name.
+int check_batch(const ca_forward_call* c, const std::string& who, const char* exif_for = nullptr) {
+  if (c->B <= 0) return invalid((who + ": empty batch").c_str());
   CA_TRY(check_images(images_of(*c)));
-  CA_REQUIRE(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260, "forward: image side must be a multiple of 14 in [56, 1260]");
+  if (!(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260))
+    return invalid((who + ": image side must be a multiple of 14 in [56, 1260]").c_str());
+  if (exif_for && !(c->exif && c->camera_idx))
+    return invalid((std::string(exif_for) + ": EXIF inputs are required (without them the reference falls back to "
+                                            "forward(): call ca_forward)").c_str());
+  return 0;
+}
+
+// A sweep or a scene takes the per-call fields elsewhere (`where`): in the ca_forward_call they must be NULL.
+int check_batch_only(const ca_forward_call* c, const std::string& who, const char* where) {
+  CA_TRY(check_batch(c, who, who.c_str()));
+  if (c->instruction || c->mask || c->tmp_w || c->tmp_b || c->eps || c->noise || c->depth || c->conf || c->attention ||
+      c->argmax || c->fused)
+    return invalid((who + ": the per-call fields of ca_forward_call must be NULL (they go in " + where + ")").c_str());
+  return 0;
+}
+
+int check_call(const ca_handle* h, const ca_forward_call* c, const char* exif_for = nullptr) {
+  CA_REQUIRE(h && c, "null handle / call");
+  CA_TRY(check_batch(c, "forward", exif_for));
   CA_REQUIRE(c->depth && c->conf, "forward: null output");
   CA_REQUIRE(c->eps && c->noise, "forward: null CuriosityModule draws (HOST pointers, src/model.py:609,744)");
   return 0;
@@ -818,6 +814,125 @@ struct DeviceGuard {
     if (prev >= 0) cudaSetDevice(prev);
   }
 };
+
+// K guided calls over one batch (K = 1: a single call).  Their instructions (K strings) or masks ([K, N] shared by the
+// batch, or [K, B, N] with mask_batch_stride = N), per-call projections and CuriosityModule draws (HOST), and outputs
+// ([K, B], heat maps [K, B, N]).
+struct GuidedCall {
+  int K;
+  const char* const* instructions;
+  const float* masks;
+  long long mask_batch_stride;
+  const float *tmp_w, *tmp_b, *eps, *noise;
+  float *depth, *conf, *attention;
+  int* argmax;
+};
+
+// Every guided entry point: the tokens and the base attention come from a scene `sc`, or (sc = nullptr) from the
+// backbone and the focal pass over the images of `call`.  The tail of K = 1 and B <= CA_GUIDE_TAIL_MAX_B is
+// ca_guide_tail (one launch); any other runs guided_softmax -> weighted_pool -> heads over the K * B rows.
+int run_guided(ca_handle* h, const ca_forward_call* call, ca_scene* sc, const GuidedCall& c, cudaStream_t st) {
+  DeviceGuard guard(h->device);
+  const int K = c.K, B = sc ? sc->B : call->B, S = sc ? sc->S : call->S, g = S / 14, N = g * g, T = N + 1;
+  Workspace* wp = nullptr;
+  Tables* tb = nullptr;
+  if (sc) {
+    CA_TRY(scene_workspace(h, sc, &wp, &tb));
+  } else {
+    CA_TRY(get_workspace(h, B, S, &wp));
+    CA_TRY(get_tables(h, g, &tb));
+  }
+  Workspace& w = *wp;
+  Workspace::Sweep* sp = nullptr;
+  CA_TRY(get_sweep(w, K, &sp));
+  Workspace::Sweep& s = *sp;
+  h->launches = 0;
+  // the mask rows of call k start at k * rows: one row shared by the batch, or one per image
+  const long long mbs = c.instructions ? 0 : c.mask_batch_stride;
+  const size_t rows = static_cast<size_t>(mbs ? B : 1) * N;
+  if (c.instructions) {
+    for (int k = 0; k < K; ++k) {
+      float* m = nullptr;
+      CA_TRY(get_mask(tb, c.instructions[k], g, &m));
+      CA_CUDA(cudaMemcpyAsync(s.mask_in + static_cast<size_t>(k) * N, m, static_cast<size_t>(N) * 4, cudaMemcpyDeviceToDevice, st));
+    }
+  } else {
+    CA_CUDA(cudaMemcpyAsync(s.mask_in, c.masks, K * rows * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  CA_TRY(stage_guided_draws(h, w, s, K, c.tmp_w, c.tmp_b, c.eps, c.noise, st));
+  ca_heads_inputs in{};
+  in.tokens_per_img = T;
+  in.pool_partial = s.pool;
+  in.pool_splits = kPoolSplits;
+  in.tmp_w = s.tmpw;
+  in.tmp_b = s.tmpb;
+  in.num_cameras = h->w.num_cameras;
+  if (sc) {
+    in.tokens = sc->tokens;
+    in.exif = sc->exif;
+    in.camera_idx = sc->cam;
+    in.fault = sc->fault;
+  } else {
+    CA_CUDA(cudaMemcpyAsync(w.exif_in, call->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
+    CA_CUDA(cudaMemcpyAsync(w.cam_in, call->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
+    CA_TRY(patch_rows(h, w, images_of(*call), st));
+    in.tokens = w.tokens;
+    in.exif = w.exif_in;
+    in.camera_idx = w.cam_in;
+    in.fault = call->fault;
+  }
+  auto seq = [&]() -> int {
+    if (!sc) CA_TRY(backbone_layers(h, w, *tb, st));
+    CA_TRY(curiosity_fork(h, w, K, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st, in.tokens));
+    float* base = sc ? sc->base : nullptr;
+    if (!sc) CA_TRY(focal_iterations(h, w, *tb, false, st, &base));  // shared by the K calls: it does not read the instruction
+    if (K == 1 && B <= CA_GUIDE_TAIL_MAX_B) {
+      LAUNCH(ca::guide_tail_launch(h->w.heads, in, base, s.mask_in, mbs ? N : 0, s.heat, s.argmax,
+                                   reinterpret_cast<unsigned int*>(s.tail_ticket), s.depth, s.conf, B, N, 0.7f, 0.05f, st));
+    } else {
+      LAUNCH(ca::guided_softmax_launch(base, 0, s.mask_in, static_cast<long long>(rows), mbs ? N : 0, s.heat, s.argmax, K, B,
+                                       N, 0.7f, 0.05f, st));
+      LAUNCH(ca::weighted_pool_launch(in.tokens, static_cast<long long>(T) * kD, 1, s.heat, nullptr, s.pool, K, B, N, kD,
+                                      kPoolSplits, st));
+      ca_heads_inputs sweep_in = in;
+      sweep_in.sweep_images = B;
+      LAUNCH(ca::heads_launch(h->w.heads, sweep_in, s.depth, s.conf, nullptr, K * B, st));
+    }
+    return curiosity_join(h, st);
+  };
+  const int key = 2 * K + (mbs ? 1 : 0);
+  if (sc)
+    CA_TRY(run_captured(h, sc->graphs, sc->seen, 100 + key, sc->use_graph, st, seq));
+  else
+    CA_TRY(run_sequence(h, w, 300 + key, call->use_graph != 0, st, seq));
+  const size_t KB = static_cast<size_t>(K) * B;
+  CA_CUDA(cudaMemcpyAsync(c.depth, s.depth, KB * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c.conf, s.conf, KB * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c.attention, s.heat, KB * N * 4, cudaMemcpyDeviceToDevice, st));
+  if (c.argmax) CA_CUDA(cudaMemcpyAsync(c.argmax, s.argmax, KB * 4, cudaMemcpyDeviceToDevice, st));
+  h->last_launches = h->launches;
+  return 0;
+}
+
+// The checks of a sweep's instructions / masks, draws and outputs; the texts start with `who`.
+int check_sweep(const ca_sweep_call* sw, const std::string& who) {
+  const int K = sw->K;
+  if (!(K >= 1 && K <= CA_SWEEP_MAX_K)) return invalid((who + ": K must be in 1..CA_SWEEP_MAX_K (16)").c_str());
+  if ((sw->instructions != nullptr) == (sw->masks != nullptr))
+    return invalid((who + ": give instructions OR masks").c_str());
+  if (sw->instructions)
+    for (int k = 0; k < K; ++k)
+      if (!sw->instructions[k]) return invalid((who + ": null instruction string").c_str());
+  if (!(sw->tmp_w && sw->tmp_b && sw->eps && sw->noise))
+    return invalid((who + ": null per-call projections or CuriosityModule draws (HOST pointers)").c_str());
+  if (!(sw->depth && sw->conf && sw->attention)) return invalid((who + ": null output").c_str());
+  return 0;
+}
+
+GuidedCall sweep_call(const ca_sweep_call& sw) {
+  return {sw.K, sw.instructions, sw.masks, 0, sw.tmp_w, sw.tmp_b, sw.eps, sw.noise, sw.depth, sw.conf, sw.attention,
+          sw.argmax};
+}
 
 }  // namespace
 
@@ -917,133 +1032,23 @@ int ca_backbone_list(ca_handle* h, const uint8_t* const* image_list, const int* 
 }
 
 int ca_forward_guided(ca_handle* h, const ca_forward_call* c, void* stream) {
-  CA_TRY(check_call(h, c));
-  CA_REQUIRE(c->exif && c->camera_idx, "forward_guided: EXIF inputs are required (without them the reference falls back "
-                                       "to forward(): call ca_forward)");
+  CA_TRY(check_call(h, c, "forward_guided"));
   CA_REQUIRE(c->tmp_w && c->tmp_b, "forward_guided: null per-call projection (HOST pointers, src/model.py:1421)");
   CA_REQUIRE((c->instruction != nullptr) != (c->mask != nullptr), "forward_guided: give an instruction OR a mask");
   CA_REQUIRE(c->attention, "forward_guided: null heat-map output");
-  DeviceGuard guard(h->device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int B = c->B, S = c->S, g = S / 14, N = g * g, T = N + 1;
-  Workspace* wp = nullptr;
-  Tables* tb = nullptr;
-  CA_TRY(get_workspace(h, B, S, &wp));
-  CA_TRY(get_tables(h, g, &tb));
-  Workspace& w = *wp;
-  h->launches = 0;
-  const float* mask = c->mask;
-  long long mstride = c->mask_batch_stride;
-  if (c->instruction) {
-    float* m = nullptr;
-    CA_TRY(get_mask(tb, c->instruction, g, &m));
-    mask = m;
-    mstride = 0;
-  }
-  CA_REQUIRE(mstride == 0 || mstride == N, "forward_guided: mask batch stride must be 0 or N");
-  CA_TRY(stage_host_inputs(h, w, *c, true, 1, st));
-  CA_CUDA(cudaMemcpyAsync(w.mask_in, mask, static_cast<size_t>(mstride ? B : 1) * N * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
-  CA_TRY(patch_rows(h, w, images_of(*c), st));
-  int* fault = c->fault;
-  const int key = 100 + (mstride ? 1 : 0);
-  CA_TRY(run_sequence(h, w, key, c->use_graph != 0, st, [&]() -> int {
-    CA_TRY(backbone_layers(h, w, *tb, st));
-    CA_TRY(curiosity_fork(h, w, 1, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st));
-    float* base = nullptr;
-    CA_TRY(focal_iterations(h, w, *tb, false, st, &base));
-    LAUNCH(ca::guided_softmax_launch(base, w.mask_in, mstride ? N : 0, w.heat, w.argmax, B, N, 0.7f, 0.05f, st));
-    LAUNCH(ca::weighted_pool_launch(w.tokens, static_cast<long long>(T) * kD, 1, w.heat, nullptr, w.pool, B, N, kD, kPoolSplits, st));
-    CA_TRY(heads(h, w, true, true, fault, st));
-    CA_TRY(curiosity_join(h, st));
-    return 0;
-  }));
-  CA_CUDA(cudaMemcpyAsync(c->depth, w.depth, B * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(c->conf, w.conf, B * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(c->attention, w.heat, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
-  if (c->argmax) CA_CUDA(cudaMemcpyAsync(c->argmax, w.argmax, B * 4, cudaMemcpyDeviceToDevice, st));
-  h->last_launches = h->launches;
-  return 0;
+  const int g = c->S / 14;
+  CA_REQUIRE(c->instruction || c->mask_batch_stride == 0 || c->mask_batch_stride == g * g,
+             "forward_guided: mask batch stride must be 0 or N");
+  const GuidedCall gc{1, c->instruction ? &c->instruction : nullptr, c->mask, c->mask_batch_stride, c->tmp_w, c->tmp_b,
+                      c->eps, c->noise, c->depth, c->conf, c->attention, c->argmax};
+  return run_guided(h, c, nullptr, gc, static_cast<cudaStream_t>(stream));
 }
 
 int ca_forward_guided_sweep(ca_handle* h, const ca_forward_call* c, const ca_sweep_call* sw, void* stream) {
   CA_REQUIRE(h && c && sw, "forward_guided_sweep: null handle / call / sweep");
-  CA_REQUIRE(c->B > 0, "forward_guided_sweep: empty batch");
-  CA_TRY(check_images(images_of(*c)));
-  CA_REQUIRE(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260,
-             "forward_guided_sweep: image side must be a multiple of 14 in [56, 1260]");
-  CA_REQUIRE(c->exif && c->camera_idx, "forward_guided_sweep: EXIF inputs are required (without them the reference falls "
-                                       "back to forward(): call ca_forward)");
-  CA_REQUIRE(!c->instruction && !c->mask && !c->tmp_w && !c->tmp_b && !c->eps && !c->noise && !c->depth && !c->conf &&
-                 !c->attention && !c->argmax && !c->fused,
-             "forward_guided_sweep: the per-call fields of ca_forward_call must be NULL (they go in ca_sweep_call)");
-  const int K = sw->K;
-  CA_REQUIRE(K >= 1 && K <= CA_SWEEP_MAX_K, "forward_guided_sweep: K must be in 1..CA_SWEEP_MAX_K (16)");
-  CA_REQUIRE((sw->instructions != nullptr) != (sw->masks != nullptr), "forward_guided_sweep: give instructions OR masks");
-  if (sw->instructions)
-    for (int k = 0; k < K; ++k) CA_REQUIRE(sw->instructions[k], "forward_guided_sweep: null instruction string");
-  CA_REQUIRE(sw->tmp_w && sw->tmp_b && sw->eps && sw->noise,
-             "forward_guided_sweep: null per-call projections or CuriosityModule draws (HOST pointers)");
-  CA_REQUIRE(sw->depth && sw->conf && sw->attention, "forward_guided_sweep: null output");
-  DeviceGuard guard(h->device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int B = c->B, S = c->S, g = S / 14, N = g * g, T = N + 1;
-  Workspace* wp = nullptr;
-  Tables* tb = nullptr;
-  Workspace::Sweep* sp = nullptr;
-  CA_TRY(get_workspace(h, B, S, &wp));
-  CA_TRY(get_tables(h, g, &tb));
-  Workspace& w = *wp;
-  CA_TRY(get_sweep(w, K, &sp));
-  Workspace::Sweep& s = *sp;
-  h->launches = 0;
-  // mask set [K, N], one row per call, shared by the batch (mask stride per image 0)
-  if (sw->instructions) {
-    for (int k = 0; k < K; ++k) {
-      float* m = nullptr;
-      CA_TRY(get_mask(tb, sw->instructions[k], g, &m));
-      CA_CUDA(cudaMemcpyAsync(s.mask_in + static_cast<size_t>(k) * N, m, static_cast<size_t>(N) * 4, cudaMemcpyDeviceToDevice, st));
-    }
-  } else {
-    CA_CUDA(cudaMemcpyAsync(s.mask_in, sw->masks, static_cast<size_t>(K) * N * 4, cudaMemcpyDeviceToDevice, st));
-  }
-  CA_TRY(stage_sweep_inputs(h, w, s, *sw, st));
-  CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
-  CA_TRY(patch_rows(h, w, images_of(*c), st));
-  int* fault = c->fault;
-  CA_TRY(run_sequence(h, w, 300 + K, c->use_graph != 0, st, [&]() -> int {
-    CA_TRY(backbone_layers(h, w, *tb, st));
-    CA_TRY(curiosity_fork(h, w, K, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st));
-    float* base = nullptr;
-    CA_TRY(focal_iterations(h, w, *tb, false, st, &base));  // shared by the K calls: it does not read the instruction
-    LAUNCH(ca::guided_softmax_sweep_launch(base, 0, s.mask_in, N, 0, s.heat, s.argmax, K, B, N, 0.7f, 0.05f, st));
-    LAUNCH(ca::weighted_pool_sweep_launch(w.tokens, static_cast<long long>(T) * kD, 1, s.heat, s.pool, K, B, N, kD,
-                                          kPoolSplits, st));
-    ca_heads_inputs in{};
-    in.tokens = w.tokens;
-    in.tokens_per_img = T;
-    in.pool_partial = s.pool;
-    in.pool_splits = kPoolSplits;
-    in.tmp_w = s.tmpw;
-    in.tmp_b = s.tmpb;
-    in.exif = w.exif_in;
-    in.camera_idx = w.cam_in;
-    in.num_cameras = h->w.num_cameras;
-    in.fault = fault;
-    in.sweep_images = B;
-    LAUNCH(ca::heads_launch(h->w.heads, in, s.depth, s.conf, nullptr, K * B, st));
-    CA_TRY(curiosity_join(h, st));
-    return 0;
-  }));
-  const size_t KB = static_cast<size_t>(K) * B;
-  CA_CUDA(cudaMemcpyAsync(sw->depth, s.depth, KB * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(sw->conf, s.conf, KB * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(sw->attention, s.heat, KB * N * 4, cudaMemcpyDeviceToDevice, st));
-  if (sw->argmax) CA_CUDA(cudaMemcpyAsync(sw->argmax, s.argmax, KB * 4, cudaMemcpyDeviceToDevice, st));
-  h->last_launches = h->launches;
-  return 0;
+  CA_TRY(check_batch_only(c, "forward_guided_sweep", "ca_sweep_call"));
+  CA_TRY(check_sweep(sw, "forward_guided_sweep"));
+  return run_guided(h, c, nullptr, sweep_call(*sw), static_cast<cudaStream_t>(stream));
 }
 
 int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
@@ -1061,7 +1066,7 @@ int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
   h->launches = 0;
   const bool has_exif = c->exif != nullptr && h->w.num_cameras > 0;
   const int runs = c->curiosity_runs;
-  CA_TRY(stage_host_inputs(h, w, *c, false, runs, st));
+  CA_TRY(stage_host_inputs(h, w, *c, runs, st));
   if (has_exif) {
     CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
     CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
@@ -1074,7 +1079,7 @@ int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
     CA_TRY(backbone_layers(h, w, *tb, st));
     CA_TRY(curiosity_fork(h, w, runs, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st));
     CA_TRY(focal_iterations(h, w, *tb, true, st, &att));
-    CA_TRY(heads(h, w, false, has_exif, fault, st));
+    CA_TRY(heads(h, w, has_exif, fault, st));
     CA_TRY(curiosity_join(h, st));
     return 0;
   }));
@@ -1094,14 +1099,7 @@ int ca_encode(ca_handle* h, const ca_forward_call* c, ca_scene** out, void* stre
     std::lock_guard<std::mutex> lock(g_live_mu);
     CA_REQUIRE(g_live_handles.count(h) != 0, "encode: the handle has been destroyed");
   }
-  CA_REQUIRE(c->B > 0, "encode: empty batch");
-  CA_TRY(check_images(images_of(*c)));
-  CA_REQUIRE(c->S >= 56 && c->S % 14 == 0 && c->S <= 1260, "encode: image side must be a multiple of 14 in [56, 1260]");
-  CA_REQUIRE(c->exif && c->camera_idx, "encode: EXIF inputs are required (without them the reference falls back to "
-                                       "forward(): call ca_forward)");
-  CA_REQUIRE(!c->instruction && !c->mask && !c->tmp_w && !c->tmp_b && !c->eps && !c->noise && !c->depth && !c->conf &&
-                 !c->attention && !c->argmax && !c->fused,
-             "encode: the per-call fields of ca_forward_call must be NULL (they go in ca_guide_call / ca_sweep_call)");
+  CA_TRY(check_batch_only(c, "encode", "ca_guide_call / ca_sweep_call"));
   DeviceGuard guard(h->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int B = c->B, S = c->S, g = S / 14, N = g * g, T = N + 1;
@@ -1165,121 +1163,19 @@ int ca_guide(ca_handle* h, ca_scene* sc, const ca_guide_call* c, void* stream) {
   CA_REQUIRE(c->tmp_w && c->tmp_b && c->eps && c->noise,
              "guide: null per-call projection or CuriosityModule draws (HOST pointers, src/model.py:609,744,1421)");
   CA_REQUIRE(c->depth && c->conf && c->attention, "guide: null output");
-  DeviceGuard guard(h->device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int B = sc->B, g = sc->S / 14, N = g * g, T = N + 1;
-  Workspace* wp = nullptr;
-  Tables* tb = nullptr;
-  CA_TRY(scene_workspace(h, sc, &wp, &tb));
-  Workspace& w = *wp;
-  h->launches = 0;
-  const float* mask = c->mask;
-  long long mstride = c->mask_batch_stride;
-  if (c->instruction) {
-    float* m = nullptr;
-    CA_TRY(get_mask(tb, c->instruction, g, &m));
-    mask = m;
-    mstride = 0;
-  }
-  CA_REQUIRE(mstride == 0 || mstride == N, "guide: mask batch stride must be 0 or N");
-  ca_forward_call staged{};
-  staged.tmp_w = c->tmp_w;
-  staged.tmp_b = c->tmp_b;
-  staged.eps = c->eps;
-  staged.noise = c->noise;
-  CA_TRY(stage_host_inputs(h, w, staged, true, 1, st));
-  CA_CUDA(cudaMemcpyAsync(w.mask_in, mask, static_cast<size_t>(mstride ? B : 1) * N * 4, cudaMemcpyDeviceToDevice, st));
-  CA_TRY(run_captured(h, sc->graphs, sc->seen, 1 + (mstride ? 1 : 0), sc->use_graph, st, [&]() -> int {
-    CA_TRY(curiosity_fork(h, w, 1, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st, sc->tokens));
-    ca_heads_inputs in{};
-    in.tokens = sc->tokens;
-    in.tokens_per_img = T;
-    in.pool_partial = w.pool;
-    in.pool_splits = kPoolSplits;
-    in.tmp_w = w.tmpw;
-    in.tmp_b = w.tmpb;
-    in.exif = sc->exif;
-    in.camera_idx = sc->cam;
-    in.num_cameras = h->w.num_cameras;
-    in.fault = sc->fault;
-    if (B <= CA_GUIDE_TAIL_MAX_B) {
-      LAUNCH(ca::guide_tail_launch(h->w.heads, in, sc->base, w.mask_in, mstride ? N : 0, w.heat, w.argmax, reinterpret_cast<unsigned int*>(w.tail_ticket),
-                                   w.depth, w.conf, B, N, 0.7f, 0.05f, st));
-    } else {
-      LAUNCH(ca::guided_softmax_launch(sc->base, w.mask_in, mstride ? N : 0, w.heat, w.argmax, B, N, 0.7f, 0.05f, st));
-      LAUNCH(ca::weighted_pool_launch(sc->tokens, static_cast<long long>(T) * kD, 1, w.heat, nullptr, w.pool, B, N, kD,
-                                      kPoolSplits, st));
-      LAUNCH(ca::heads_launch(h->w.heads, in, w.depth, w.conf, nullptr, B, st));
-    }
-    return curiosity_join(h, st);
-  }));
-  CA_CUDA(cudaMemcpyAsync(c->depth, w.depth, B * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(c->conf, w.conf, B * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(c->attention, w.heat, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
-  if (c->argmax) CA_CUDA(cudaMemcpyAsync(c->argmax, w.argmax, B * 4, cudaMemcpyDeviceToDevice, st));
-  h->last_launches = h->launches;
-  return 0;
+  const int g = sc->S / 14;
+  CA_REQUIRE(c->instruction || c->mask_batch_stride == 0 || c->mask_batch_stride == g * g,
+             "guide: mask batch stride must be 0 or N");
+  const GuidedCall gc{1, c->instruction ? &c->instruction : nullptr, c->mask, c->mask_batch_stride, c->tmp_w, c->tmp_b,
+                      c->eps, c->noise, c->depth, c->conf, c->attention, c->argmax};
+  return run_guided(h, nullptr, sc, gc, static_cast<cudaStream_t>(stream));
 }
 
 int ca_guide_sweep(ca_handle* h, ca_scene* sc, const ca_sweep_call* sw, void* stream) {
   CA_TRY(check_scene(h, sc));
   CA_REQUIRE(sw, "guide_sweep: null sweep");
-  const int K = sw->K;
-  CA_REQUIRE(K >= 1 && K <= CA_SWEEP_MAX_K, "guide_sweep: K must be in 1..CA_SWEEP_MAX_K (16)");
-  CA_REQUIRE((sw->instructions != nullptr) != (sw->masks != nullptr), "guide_sweep: give instructions OR masks");
-  if (sw->instructions)
-    for (int k = 0; k < K; ++k) CA_REQUIRE(sw->instructions[k], "guide_sweep: null instruction string");
-  CA_REQUIRE(sw->tmp_w && sw->tmp_b && sw->eps && sw->noise,
-             "guide_sweep: null per-call projections or CuriosityModule draws (HOST pointers)");
-  CA_REQUIRE(sw->depth && sw->conf && sw->attention, "guide_sweep: null output");
-  DeviceGuard guard(h->device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int B = sc->B, g = sc->S / 14, N = g * g, T = N + 1;
-  Workspace* wp = nullptr;
-  Tables* tb = nullptr;
-  CA_TRY(scene_workspace(h, sc, &wp, &tb));
-  Workspace& w = *wp;
-  Workspace::Sweep* sp = nullptr;
-  CA_TRY(get_sweep(w, K, &sp));
-  Workspace::Sweep& s = *sp;
-  h->launches = 0;
-  if (sw->instructions) {
-    for (int k = 0; k < K; ++k) {
-      float* m = nullptr;
-      CA_TRY(get_mask(tb, sw->instructions[k], g, &m));
-      CA_CUDA(cudaMemcpyAsync(s.mask_in + static_cast<size_t>(k) * N, m, static_cast<size_t>(N) * 4, cudaMemcpyDeviceToDevice, st));
-    }
-  } else {
-    CA_CUDA(cudaMemcpyAsync(s.mask_in, sw->masks, static_cast<size_t>(K) * N * 4, cudaMemcpyDeviceToDevice, st));
-  }
-  CA_TRY(stage_sweep_inputs(h, w, s, *sw, st));
-  CA_TRY(run_captured(h, sc->graphs, sc->seen, 100 + K, sc->use_graph, st, [&]() -> int {
-    CA_TRY(curiosity_fork(h, w, K, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st, sc->tokens));
-    LAUNCH(ca::guided_softmax_sweep_launch(sc->base, 0, s.mask_in, N, 0, s.heat, s.argmax, K, B, N, 0.7f, 0.05f, st));
-    LAUNCH(ca::weighted_pool_sweep_launch(sc->tokens, static_cast<long long>(T) * kD, 1, s.heat, s.pool, K, B, N, kD,
-                                          kPoolSplits, st));
-    ca_heads_inputs in{};
-    in.tokens = sc->tokens;
-    in.tokens_per_img = T;
-    in.pool_partial = s.pool;
-    in.pool_splits = kPoolSplits;
-    in.tmp_w = s.tmpw;
-    in.tmp_b = s.tmpb;
-    in.exif = sc->exif;
-    in.camera_idx = sc->cam;
-    in.num_cameras = h->w.num_cameras;
-    in.fault = sc->fault;
-    in.sweep_images = B;
-    LAUNCH(ca::heads_launch(h->w.heads, in, s.depth, s.conf, nullptr, K * B, st));
-    return curiosity_join(h, st);
-  }));
-  const size_t KB = static_cast<size_t>(K) * B;
-  CA_CUDA(cudaMemcpyAsync(sw->depth, s.depth, KB * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(sw->conf, s.conf, KB * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(sw->attention, s.heat, KB * N * 4, cudaMemcpyDeviceToDevice, st));
-  if (sw->argmax) CA_CUDA(cudaMemcpyAsync(sw->argmax, s.argmax, KB * 4, cudaMemcpyDeviceToDevice, st));
-  h->last_launches = h->launches;
-  return 0;
+  CA_TRY(check_sweep(sw, "guide_sweep"));
+  return run_guided(h, nullptr, sc, sweep_call(*sw), static_cast<cudaStream_t>(stream));
 }
 
 int ca_depth_field(ca_handle* h, ca_scene* sc, const ca_depth_field_call* c, void* stream) {
@@ -1296,20 +1192,18 @@ int ca_depth_field(ca_handle* h, ca_scene* sc, const ca_depth_field_call* c, voi
   CA_TRY(scene_workspace(h, sc, &wp, &tb));
   Workspace& w = *wp;
   CA_TRY(get_field(w));
+  Workspace::Sweep* sp = nullptr;
+  CA_TRY(get_sweep(w, 1, &sp));  // the buffers of one guided call
+  Workspace::Sweep& s = *sp;
   h->launches = 0;
-  ca_forward_call staged{};
-  staged.tmp_w = c->tmp_w;
-  staged.tmp_b = c->tmp_b;
-  staged.eps = c->eps;
-  staged.noise = c->noise;
-  CA_TRY(stage_host_inputs(h, w, staged, true, 1, st));
+  CA_TRY(stage_guided_draws(h, w, s, 1, c->tmp_w, c->tmp_b, c->eps, c->noise, st));
   CA_TRY(run_captured(h, sc->graphs, sc->seen, 200, sc->use_graph, st, [&]() -> int {
-    CA_TRY(curiosity_fork(h, w, 1, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st, sc->tokens));
-    LAUNCH(ca::token_project_launch(sc->tokens, static_cast<long long>(T) * kD, 1, w.tmpw, w.field_P, B, N, st));
+    CA_TRY(curiosity_fork(h, w, 1, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st, sc->tokens));
+    LAUNCH(ca::token_project_launch(sc->tokens, static_cast<long long>(T) * kD, 1, s.tmpw, w.field_P, B, N, st));
     ca_heads_inputs in{};
     in.tokens = sc->tokens;
     in.tokens_per_img = T;
-    in.tmp_b = w.tmpb;
+    in.tmp_b = s.tmpb;
     in.exif = sc->exif;
     in.camera_idx = sc->cam;
     in.num_cameras = h->w.num_cameras;

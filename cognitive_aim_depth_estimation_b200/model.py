@@ -31,7 +31,7 @@ import torch.nn as nn
 
 from . import ops, tables
 from ._lib import RESIZE_MAX_SIDE as _RESIZE_MAX_SIDE  # largest photograph side the resize stages in shared memory
-from ._lib import GUIDE_TAIL_MAX_B as _GUIDE_TAIL_MAX_B  # guide calls of larger batches run the three-kernel tail
+from ._lib import GUIDE_TAIL_MAX_B as _GUIDE_TAIL_MAX_B  # single guided calls of larger batches run the three-kernel tail
 from ._lib import SWEEP_MAX_K as _SWEEP_MAX_K  # instructions per sweep: the sweep pool keeps one accumulator each
 from .config import DEFAULT_COGNITIVE_MODULES, EffectiveConfig, effective_config
 from .init import reference_init_
@@ -505,14 +505,12 @@ class CognitiveAimModel(nn.Module):
                 # LayerNorm folding: per (row, 128-column span) (sum, M2) of the residual row; `h` then holds the raw rows
                 "ln_stats": torch.empty(B * T, _D // 128, 2, **fl),
                 "heat": torch.empty(B, N, **fl), "argmax": torch.empty(B, device=dev, dtype=torch.int32),
-                # per-image tickets of ops.guide_tail: zero here, and every launch leaves them at zero
-                "tail_ticket": torch.zeros(B, device=dev, dtype=torch.int32),
                 "pool": torch.empty(B, _POOL_SPLITS, _D, **fl), "pool_pe": torch.empty(B, _POOL_SPLITS, _D, **fl),
-                "pooled": torch.empty(B, _D, **fl), "feats": torch.empty(B, self.cfg.num_iterations, 64, **fl),
+                "feats": torch.empty(B, self.cfg.num_iterations, 64, **fl),
                 "focal_feat": torch.empty(B, 64, **fl), "fused": torch.empty(B, 192, **fl),
                 "depth": torch.empty(B, **fl), "conf": torch.empty(B, **fl),
                 # per-call inputs, at fixed addresses so that captured graphs can be replayed
-                "mask_in": torch.empty(B, N, **fl), "tmpw": torch.empty(64, _D, **fl), "tmpb": torch.empty(64, **fl),
+                "mask_in": torch.empty(B, N, **fl),
                 "exif_in": torch.zeros(B, 3, **fl), "cam_in": torch.zeros(B, device=dev, dtype=torch.int64),
                 # CuriosityModule: up to _MAX_CURIOSITY_RUNS runs per call (src/model.py:992,1104,1138,1185), each with
                 # its own pair of Gaussian draws; rewards per run; modulation weights per (run, iteration)
@@ -543,8 +541,7 @@ class CognitiveAimModel(nn.Module):
         completed."""
         ring = getattr(self, "_pinned_ring", None)
         if ring is None:
-            ring = {"slots": [{"w": torch.empty(64, _D).pin_memory(), "b": torch.empty(64).pin_memory(),
-                               "draws": {}, "event": torch.cuda.Event()} for _ in range(4)], "next": 0}
+            ring = {"slots": [{"draws": {}, "sweep": {}, "event": torch.cuda.Event()} for _ in range(4)], "next": 0}
             self._pinned_ring = ring
         slot = ring["slots"][ring["next"]]
         ring["next"] = (ring["next"] + 1) % len(ring["slots"])
@@ -890,7 +887,8 @@ class CognitiveAimModel(nn.Module):
     @torch.no_grad()
     @_on_own_device
     def forward_with_guidance(self, images, exif_data=None, attention_guidance=None, return_attention=False):
-        """reference src/model.py:1157-1240.  Returns (depth [B,1], confidence [B,1][, attention [B,N]])."""
+        """reference src/model.py:1157-1240.  Returns (depth [B,1], confidence [B,1][, attention [B,N]]).  With EXIF and a
+        guidance this is the sweep of one instruction, `forward_with_guidance_sweep(images, exif_data, [guidance])`."""
         self._raise_on_fault()
         if attention_guidance is None and exif_data is not None and self.use_exif:
             # guidance None -> plain focal-stream features and attention (:1206-1212)
@@ -900,57 +898,9 @@ class CognitiveAimModel(nn.Module):
             # (:1237-1240) AFTER the guided attention was stored at :1212 — reproduce exactly that end state.
             return self._forward_impl(images, exif_data, return_attention, mode="guided_fallback",
                                       guidance=attention_guidance)
-        B, S = self._check_images(images)
-        self._check_per_image(attention_guidance, B)
-        self._check_exif(exif_data, B)
-        pk = self._pack()
-        dev = self._device()
-        g = S // 14
-        N, T = g * g, g * g + 1
-        mask = self._mask(attention_guidance, g)
-        if mask.dim() == 2 and mask.shape[0] != B:
-            raise ValueError(f"{mask.shape[0]} per-image instructions for a batch of {B}")
-        exif, cam = self._exif_tensors(exif_data, B)
-        draws = [self._curiosity_draw(B)]  # :1185
-        tmp = nn.Linear(_D, 64)  # same constructor => same CPU-generator draws as src/model.py:1421
-        ws = self._workspace(B, S)
-        # The projection travels through a small ring of PINNED staging buffers: a copy from pageable memory would block
-        # the host until the stream has drained, i.e. serialise host-side launch work with the previous step.
-        slot = self._pinned_slot()
-        slot["w"].copy_(tmp.weight.detach())
-        slot["b"].copy_(tmp.bias.detach())
-        self._stage_draws(ws, slot, draws)
-        ws["mask_in"].copy_(mask, non_blocking=True)
-        ops.fetch_pinned(ws["tmpw"], slot["w"])
-        ops.fetch_pinned(ws["tmpb"], slot["b"])
-        slot["event"].record()
-        ws["exif_in"].copy_(exif, non_blocking=True)
-        ws["cam_in"].copy_(cam, non_blocking=True)
-        self._grid_tables(g)
-        patches, images = self._patch_rows(images, ws, S)
-        cur_weight = ws["cur_weight"][0] if self.cfg.curiosity_guided else None
-
-        def device_pass():
-            self._backbone_layers(ws, patches, B, S)
-            self._curiosity_runs(ws, B, T, ("guided",))
-            base = self._focal_iterations(ws, B, g, want_features=False, cur_weight=cur_weight)
-            ops.guided_softmax(base, ws["mask_in"], ws["heat"], ws["argmax"], B, N)
-            ops.weighted_pool(ws["tokens"], T * _D, 1, ws["heat"], None, ws["pool"], B, N, _D, _POOL_SPLITS)
-            ops.heads(pk["heads"], tokens=ws["tokens"], tokens_per_img=T, depth=ws["depth"], conf=ws["conf"], B=B,
-                      pool_partial=ws["pool"], pool_splits=_POOL_SPLITS, tmp_w=ws["tmpw"], tmp_b=ws["tmpb"],
-                      pooled_out=ws["pooled"], exif=ws["exif_in"], camera_idx=ws["cam_in"],
-                      num_cameras=self.cfg.num_cameras, fault_ptr=self._fault_word().data_ptr())
-            self._curiosity_join()
-
-        self._run(ws, ("guided", self._curiosity_key()), device_pass)
-        # keep the temporaries referenced until the next call (their copies are enqueued, not finished)
-        self._keepalive = (exif, cam, mask, images)
-        heat = ws["heat"].clone()
-        self._last_attention_weights = heat  # :1212
-        self._last_argmax = ws["argmax"].clone()
-        self._last_curiosity = ws["cur_reward"][0]
-        depth, conf = ws["depth"].clone().unsqueeze(1), ws["conf"].clone().unsqueeze(1)
-        return (depth, conf, heat) if return_attention else (depth, conf)
+        depth, conf, _ = self.forward_with_guidance_sweep(images, exif_data, [attention_guidance], return_attention=True)
+        heat = self._last_attention_weights  # :1212
+        return (depth[0], conf[0], heat) if return_attention else (depth[0], conf[0])
 
     def _sweep_draws(self, B: int, K: int):
         """The host-side random draws of K successive guided calls, in the reference's order per call: the
@@ -964,8 +914,8 @@ class CognitiveAimModel(nn.Module):
         return out
 
     def _sweep_buffers(self, ws, B: int, S: int, K: int):
-        """Per-call buffers of a K-instruction sweep (rows k * B + b), kept with the (B, S) workspace whose backbone and
-        focal buffers the sweep shares."""
+        """Per-call buffers of K guided calls (rows k * B + b; K = 1 for a single call), kept with the (B, S) workspace
+        whose backbone and focal buffers the calls share."""
         sweeps = ws.setdefault("sweeps", {})
         sw = sweeps.get(K)
         if sw is None:
@@ -983,7 +933,9 @@ class CognitiveAimModel(nn.Module):
                 "cur_raw": torch.empty(K, B, **fl), "cur_reward": torch.empty(K, B, **fl),
                 "cur_weight": torch.empty(K, iters, B, **fl),
                 # curiosity-guided attention: one focal pass per call, its last-iteration attention kept per call
-                "base": torch.empty(K, B, N, **fl) if self.cfg.curiosity_guided else None,
+                "base": torch.empty(K, B, N, **fl) if self.cfg.curiosity_guided and K > 1 else None,
+                # per-image tickets of ops.guide_tail: zero here, and every launch leaves them at zero
+                "tail_ticket": torch.zeros(B, device=dev, dtype=torch.int32),
             }
             if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
                 for t in sw.values():
@@ -992,18 +944,6 @@ class CognitiveAimModel(nn.Module):
             sweeps[K] = sw
         # the single-call buffers (tokens, focal workspace, EXIF, graphs) come from ws; the per-call ones from sw
         return {**ws, **sw}
-
-    def _stage_sweep(self, sw, slot, draws, B: int, K: int):
-        """The K calls' draws -> pinned staging sized for (B, K) -> the sweep's device buffers (as _stage_draws)."""
-        bufs = slot.setdefault("sweep", {}).get((B, K))
-        if bufs is None:
-            bufs = slot["sweep"][(B, K)] = tuple(torch.empty(*s).pin_memory() for s in
-                                                 ((K, B, 192), (K, B, _D), (K, 64, _D), (K, 64)))
-        for k, d in enumerate(draws):
-            for buf, t in zip(bufs, d):
-                buf[k].copy_(t)
-        for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb"), bufs):
-            ops.fetch_pinned(sw[dst], buf)
 
     @staticmethod
     def _check_guidances(guidances):
@@ -1018,8 +958,8 @@ class CognitiveAimModel(nn.Module):
                              "forward_with_guidance for it")
         return K
 
-    def _sweep_masks(self, guidances, B: int, g: int) -> torch.Tensor:
-        """[K, B, N] masks of a sweep: strings and [N] guidance broadcast over the batch."""
+    def _sweep_masks(self, guidances, B: int, g: int):
+        """The K [B, N] masks of a sweep (views: strings and [N] guidance broadcast over the batch)."""
         N = g * g
         masks = []
         for gd in guidances:
@@ -1027,38 +967,58 @@ class CognitiveAimModel(nn.Module):
             if m.dim() == 2 and m.shape[0] != B:
                 raise ValueError(f"{m.shape[0]} per-image instructions for a batch of {B}")
             masks.append(m.expand(B, N))
-        return torch.stack(masks)
+        return masks
 
-    def _stage_sweep_call(self, ws, mask, B: int, S: int, K: int):
-        """The K calls' random draws (in the reference's order) and masks -> the sweep buffers; returns them."""
-        draws = self._sweep_draws(B, K)
+    def _stage_sweep_call(self, ws, mask, draws, B: int, S: int):
+        """The K calls' random draws (`_sweep_draws`, made before any buffer is looked up) -> pinned staging sized for
+        (B, K) -> the sweep buffers, and the K masks (or None) stacked into sw['mask_in']; returns the buffers."""
+        K = len(draws)
         sw = self._sweep_buffers(ws, B, S, K)
         slot = self._pinned_slot()
-        self._stage_sweep(sw, slot, draws, B, K)
+        bufs = slot["sweep"].get((B, K))
+        if bufs is None:
+            bufs = slot["sweep"][(B, K)] = tuple(torch.empty(*s).pin_memory() for s in
+                                                 ((K, B, 192), (K, B, _D), (K, 64, _D), (K, 64)))
+        for k, d in enumerate(draws):
+            for buf, t in zip(bufs, d):
+                buf[k].copy_(t)
+        for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb"), bufs):
+            ops.fetch_pinned(sw[dst], buf)  # SM-side reads of the pinned staging area, as in _stage_draws
         slot["event"].record()
-        sw["mask_in"].copy_(mask, non_blocking=True)
+        if mask is not None:
+            torch.stack(mask, out=sw["mask_in"])
         return sw
 
     def _sweep_device(self, sw, B: int, g: int, K: int, base, exif, cam):
-        """Device side of a sweep after the backbone: the K CuriosityModule runs, the focal pass (`base` [B, N] when it
-        is shared; with curiosity-guided attention one pass per call on sw['tokens']), then the sweep's softmax, pool
-        and heads.  Shared by `forward_with_guidance_sweep` and `guide_sweep` (which reads a Scene's tokens)."""
+        """Device side of K guided calls after the backbone: the K CuriosityModule runs, the focal pass (`base` [B, N]
+        when it is shared; with curiosity-guided attention one pass per call on sw['tokens']), then the tail: for one call
+        of at most _GUIDE_TAIL_MAX_B images ops.guide_tail (one launch), else the softmax, pool and heads of the K * B
+        rows.  Shared by every guided entry point (`guide_sweep` reads a Scene's tokens)."""
         pk = self._packed
         N, T = g * g, g * g + 1
         self._curiosity_runs(sw, B, T, ("guided",) * K)
-        if self.cfg.curiosity_guided:
+        base_k_stride = 0
+        if self.cfg.curiosity_guided and K == 1:
+            base = self._focal_iterations(sw, B, g, want_features=False, cur_weight=sw["cur_weight"][0])
+        elif self.cfg.curiosity_guided:
             # each call's focal attention is modulated by its own curiosity score (src/model.py:264-276)
             for k in range(K):
                 sw["base"][k].copy_(self._focal_iterations(sw, B, g, want_features=False, cur_weight=sw["cur_weight"][k]))
             base, base_k_stride = sw["base"], B * N
+        elif base is None:
+            base = self._focal_iterations(sw, B, g, want_features=False)
+        heads_in = dict(exif=exif, camera_idx=cam, num_cameras=self.cfg.num_cameras,
+                        fault_ptr=self._fault_word().data_ptr())
+        if K == 1 and B <= _GUIDE_TAIL_MAX_B:  # one launch (include/cogaim_b200.h CA_GUIDE_TAIL_MAX_B)
+            ops.guide_tail(pk["heads"], base=base, mask=sw["mask_in"][0], heat=sw["heat"][0], argmax=sw["argmax"][0],
+                           ticket=sw["tail_ticket"], tokens=sw["tokens"], depth=sw["depth"][0], conf=sw["conf"][0], B=B,
+                           N=N, pool_partial=sw["pool"], tmp_w=sw["tmpw"][0], tmp_b=sw["tmpb"][0], **heads_in)
         else:
-            base, base_k_stride = (self._focal_iterations(sw, B, g, want_features=False) if base is None else base), 0
-        ops.guided_softmax_sweep(base, base_k_stride, sw["mask_in"], sw["heat"], sw["argmax"], K, B, N)
-        ops.weighted_pool_sweep(sw["tokens"], T * _D, 1, sw["heat"], sw["pool"], K, B, N, _D, _POOL_SPLITS)
-        ops.heads(pk["heads"], tokens=sw["tokens"], tokens_per_img=T, depth=sw["depth"], conf=sw["conf"], B=K * B,
-                  pool_partial=sw["pool"], pool_splits=_POOL_SPLITS, tmp_w=sw["tmpw"], tmp_b=sw["tmpb"],
-                  exif=exif, camera_idx=cam, num_cameras=self.cfg.num_cameras,
-                  fault_ptr=self._fault_word().data_ptr(), sweep_images=B)
+            ops.guided_softmax_sweep(base, base_k_stride, sw["mask_in"], sw["heat"], sw["argmax"], K, B, N)
+            ops.weighted_pool_sweep(sw["tokens"], T * _D, 1, sw["heat"], sw["pool"], K, B, N, _D, _POOL_SPLITS)
+            ops.heads(pk["heads"], tokens=sw["tokens"], tokens_per_img=T, depth=sw["depth"], conf=sw["conf"], B=K * B,
+                      pool_partial=sw["pool"], pool_splits=_POOL_SPLITS, tmp_w=sw["tmpw"], tmp_b=sw["tmpb"],
+                      sweep_images=B, **heads_in)
         self._curiosity_join()
 
     def _sweep_results(self, sw, K: int, return_attention: bool):
@@ -1092,8 +1052,9 @@ class CognitiveAimModel(nn.Module):
         g = S // 14
         mask = self._sweep_masks(guidances, B, g)
         exif, cam = self._exif_tensors(exif_data, B)
+        draws = self._sweep_draws(B, K)
         ws = self._workspace(B, S)
-        sw = self._stage_sweep_call(ws, mask, B, S, K)
+        sw = self._stage_sweep_call(ws, mask, draws, B, S)
         ws["exif_in"].copy_(exif, non_blocking=True)
         ws["cam_in"].copy_(cam, non_blocking=True)
         self._grid_tables(g)
@@ -1182,64 +1143,14 @@ class CognitiveAimModel(nn.Module):
                 del scene._graphs[k]  # captured on a workspace the model has since replaced: release it
             self._run(ws, key + (id(ws), self._curiosity_key()), fn, graphs=scene._graphs)
 
-    @torch.no_grad()
-    @_on_own_device
     def guide(self, scene: Scene, attention_guidance, return_attention=False):
         """`forward_with_guidance(images, exif_data, attention_guidance, return_attention)` for the images and EXIF of
         `scene`, bit for bit — outputs, global generator draws, CuriosityModule ring buffer and pointer, `_last_*` —
-        without re-running the backbone (nor, unless curiosity-guided attention is enabled, the focal iterations).
-        The tail (guided softmax, pool, heads) is one kernel (ops.guide_tail)."""
-        self._raise_on_fault()
-        self._check_scene(scene)
-        if attention_guidance is None:
-            raise ValueError("a None guidance runs the un-guided focal path (src/model.py:1206-1212): use "
-                             "forward_with_guidance for it")
-        B, S = scene.B, scene.S
-        self._check_per_image(attention_guidance, B)
-        pk = self._pack()
-        g = S // 14
-        N, T = g * g, g * g + 1
-        mask = self._mask(attention_guidance, g)
-        if mask.dim() == 2 and mask.shape[0] != B:
-            raise ValueError(f"{mask.shape[0]} per-image instructions for a batch of {B}")
-        draws = [self._curiosity_draw(B)]  # :1185
-        tmp = nn.Linear(_D, 64)  # :1421
-        ws, wsx = self._scene_ws(scene)
-        slot = self._pinned_slot()
-        slot["w"].copy_(tmp.weight.detach())
-        slot["b"].copy_(tmp.bias.detach())
-        self._stage_draws(ws, slot, draws)
-        ws["mask_in"].copy_(mask, non_blocking=True)
-        ops.fetch_pinned(ws["tmpw"], slot["w"])
-        ops.fetch_pinned(ws["tmpb"], slot["b"])
-        slot["event"].record()
-        cg = self.cfg.curiosity_guided
-
-        def device_pass():
-            self._curiosity_runs(wsx, B, T, ("guided",))
-            base = (self._focal_iterations(wsx, B, g, want_features=False, cur_weight=ws["cur_weight"][0]) if cg
-                    else scene.base)
-            heads_in = dict(tmp_w=ws["tmpw"], tmp_b=ws["tmpb"], exif=scene.exif, camera_idx=scene.camera_idx,
-                            num_cameras=self.cfg.num_cameras, fault_ptr=self._fault_word().data_ptr())
-            if B <= _GUIDE_TAIL_MAX_B:  # one launch (include/cogaim_b200.h CA_GUIDE_TAIL_MAX_B)
-                ops.guide_tail(pk["heads"], base=base, mask=ws["mask_in"], heat=ws["heat"], argmax=ws["argmax"],
-                               ticket=ws["tail_ticket"], tokens=scene.tokens, depth=ws["depth"], conf=ws["conf"], B=B,
-                               N=N, pool_partial=ws["pool"], **heads_in)
-            else:
-                ops.guided_softmax(base, ws["mask_in"], ws["heat"], ws["argmax"], B, N)
-                ops.weighted_pool(scene.tokens, T * _D, 1, ws["heat"], None, ws["pool"], B, N, _D, _POOL_SPLITS)
-                ops.heads(pk["heads"], tokens=scene.tokens, tokens_per_img=T, depth=ws["depth"], conf=ws["conf"], B=B,
-                          pool_partial=ws["pool"], pool_splits=_POOL_SPLITS, **heads_in)
-            self._curiosity_join()
-
-        self._run_scene(scene, ws, ("guide",), device_pass)
-        self._keepalive = (mask,)
-        heat = ws["heat"].clone()
-        self._last_attention_weights = heat  # :1212
-        self._last_argmax = ws["argmax"].clone()
-        self._last_curiosity = ws["cur_reward"][0]
-        depth, conf = ws["depth"].clone().unsqueeze(1), ws["conf"].clone().unsqueeze(1)
-        return (depth, conf, heat) if return_attention else (depth, conf)
+        without re-running the backbone (nor, unless curiosity-guided attention is enabled, the focal iterations):
+        `guide_sweep(scene, [attention_guidance])`."""
+        depth, conf, _ = self.guide_sweep(scene, [attention_guidance], return_attention=True)
+        heat = self._last_attention_weights  # :1212
+        return (depth[0], conf[0], heat) if return_attention else (depth[0], conf[0])
 
     @torch.no_grad()
     @_on_own_device
@@ -1256,8 +1167,9 @@ class CognitiveAimModel(nn.Module):
         self._pack()
         g = S // 14
         mask = self._sweep_masks(guidances, B, g)
+        draws = self._sweep_draws(B, K)
         ws, _ = self._scene_ws(scene)
-        sw = self._stage_sweep_call(ws, mask, B, S, K)
+        sw = self._stage_sweep_call(ws, mask, draws, B, S)
         sw["tokens"] = scene.tokens
 
         def device_pass():
@@ -1298,32 +1210,26 @@ class CognitiveAimModel(nn.Module):
         pk = self._pack()
         g = S // 14
         N, T = g * g, g * g + 1
-        draws = [self._curiosity_draw(B)]  # :1185
-        tmp = nn.Linear(_D, 64)  # :1421
-        ws, wsx = self._scene_ws(scene)
+        draws = self._sweep_draws(B, 1)  # :1185, :1421
+        ws, _ = self._scene_ws(scene)
         self._field_buffers(ws, B, N)
-        slot = self._pinned_slot()
-        slot["w"].copy_(tmp.weight.detach())
-        slot["b"].copy_(tmp.bias.detach())
-        self._stage_draws(ws, slot, draws)
-        ops.fetch_pinned(ws["tmpw"], slot["w"])
-        ops.fetch_pinned(ws["tmpb"], slot["b"])
-        slot["event"].record()
+        sw = self._stage_sweep_call(ws, None, draws, B, S)
+        sw["tokens"] = scene.tokens
         cg = self.cfg.curiosity_guided
 
         def device_pass():
-            self._curiosity_runs(wsx, B, T, ("guided",))
-            base = (self._focal_iterations(wsx, B, g, want_features=False, cur_weight=ws["cur_weight"][0]) if cg
+            self._curiosity_runs(sw, B, T, ("guided",))
+            base = (self._focal_iterations(sw, B, g, want_features=False, cur_weight=sw["cur_weight"][0]) if cg
                     else scene.base)
-            ops.token_project(scene.tokens, T * _D, 1, ws["tmpw"], ws["field_P"], B, N)
+            ops.token_project(scene.tokens, T * _D, 1, sw["tmpw"][0], ws["field_P"], B, N)
             ops.depth_field_cells(pk["heads"], base=base, P=ws["field_P"], cst=ws["field_cst"], depth=ws["field_depth"],
-                                  conf=ws["field_conf"], tokens=scene.tokens, tmp_b=ws["tmpb"], B=B, g=g,
+                                  conf=ws["field_conf"], tokens=scene.tokens, tmp_b=sw["tmpb"][0], B=B, g=g,
                                   exif=scene.exif, camera_idx=scene.camera_idx, num_cameras=self.cfg.num_cameras,
                                   fault_ptr=self._fault_word().data_ptr())
             self._curiosity_join()
 
         self._run_scene(scene, ws, ("field",), device_pass)
-        self._last_curiosity = ws["cur_reward"][0]
+        self._last_curiosity = sw["cur_reward"][0]
         return ws["field_depth"].clone().view(B, g, g), ws["field_conf"].clone().view(B, g, g)
 
     @torch.no_grad()

@@ -188,43 +188,43 @@ class NativeModel:
         c.use_graph = int(self.use_graph)
         return c, held, B, S
 
-    @torch.no_grad()
-    def forward_with_guidance(self, images, exif, guidance, S=None):
-        """-> depth [B,1], confidence [B,1], heat map [B,N], arg-max cell [B] (reference src/model.py:1157-1240).
-        `images` may be a list of uint8 [H_i, W_i, 3] photographs of individual sizes: the library resizes them to S."""
-        c, held, B, S = self._call(images, exif, S)
-        N = (S // 14) ** 2
-        eps, noise = torch.randn(B, 192), torch.randn(B, _D)       # :609, :744 (CuriosityModule, before the projection)
-        tmp = nn.Linear(_D, 64)                                    # :1421: same constructor => same generator draws
-        tw, tb = tmp.weight.detach().contiguous(), tmp.bias.detach().contiguous()
+    @staticmethod
+    def _draws(c, B: int, K: int, held):
+        """The HOST draws of K guided calls, in the reference's order per call: the CuriosityModule's randn(B, 192),
+        randn(B, 768) (:609, :744), then nn.Linear(768, 64) (:1421: same constructor => same generator draws); stacked
+        over the calls and set in the call struct `c`."""
+        draws = []
+        for _ in range(K):
+            eps, noise = torch.randn(B, 192), torch.randn(B, _D)
+            tmp = nn.Linear(_D, 64)
+            draws.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
+        eps, noise, tw, tb = (torch.stack([d[i] for d in draws]).contiguous() for i in range(4))
+        held += [eps, noise, tw, tb]
+        c.tmp_w, c.tmp_b, c.eps, c.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
+
+    def _outputs(self, c, K: int, B: int, N: int):
+        """The outputs of K guided calls — depth, confidence [K, B], heat maps [K, B, N], arg-max cells [K, B] — with
+        their pointers set in the call struct `c`."""
+        out = {"depth": torch.empty(K, B, device=self.device), "conf": torch.empty(K, B, device=self.device),
+               "heat": torch.empty(K, B, N, device=self.device),
+               "argmax": torch.empty(K, B, device=self.device, dtype=torch.int32)}
+        c.depth, c.conf, c.attention, c.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
+        return out
+
+    def _guidance(self, c, guidance, N: int, held):
+        """One call's instruction string, or guidance tensor [N] / [B, N], into the call struct `c`."""
         if isinstance(guidance, str):
             c.instruction = guidance.encode()
         else:
             m = guidance.to(self.device, torch.float32).contiguous()
             held.append(m)
             c.mask, c.mask_batch_stride = m.data_ptr(), (N if m.dim() == 2 else 0)
-        c.tmp_w, c.tmp_b, c.eps, c.noise, c.curiosity_runs = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr(), 1
-        out = {"depth": torch.empty(B, device=self.device), "conf": torch.empty(B, device=self.device),
-               "heat": torch.empty(B, N, device=self.device),
-               "argmax": torch.empty(B, device=self.device, dtype=torch.int32)}
-        c.depth, c.conf, c.attention, c.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
-        with torch.cuda.device(self.device):
-            _lib.check(self.lib.ca_forward_guided(self._h, C.byref(c), self._stream()), "ca_forward_guided")
-        self._held = held  # inputs stay referenced until the next call (their reads are enqueued, not finished)
-        return out["depth"].unsqueeze(1), out["conf"].unsqueeze(1), out["heat"], out["argmax"]
 
-    @torch.no_grad()
-    def forward_with_guidance_sweep(self, images, exif, guidances, S=None):
-        """K = len(guidances) `forward_with_guidance` calls in one native call (ca_forward_guided_sweep): the backbone and
-        the focal pass run once.  `guidances`: K instruction strings, or K guidance tensors [N].  Draws the K calls'
-        random numbers in the reference's order per call.  -> depth [K,B,1], confidence [K,B,1], heat maps [K,B,N],
-        arg-max cells [K,B]."""
+    def _guidances(self, s, guidances, N: int, held):
+        """A sweep's K instruction strings, or K guidance tensors [N], into the sweep struct `s`."""
         K = len(guidances)
         if not 1 <= K <= _lib.SWEEP_MAX_K:
             raise ValueError(f"an instruction sweep takes 1..{_lib.SWEEP_MAX_K} guidances, got {K}")
-        c, held, B, S = self._call(images, exif, S)
-        N = (S // 14) ** 2
-        s = _lib.SweepCall()
         s.K = K
         if all(isinstance(g, str) for g in guidances):
             names = (C.c_char_p * K)(*[g.encode() for g in guidances])
@@ -236,18 +236,35 @@ class NativeModel:
             s.masks = m.data_ptr()
         else:
             raise ValueError(f"guidances must be K instruction strings or K guidance tensors of length {N}")
-        draws = []
-        for _ in range(K):
-            eps, noise = torch.randn(B, 192), torch.randn(B, _D)   # :609, :744 of call k
-            tmp = nn.Linear(_D, 64)                                # :1421 of call k
-            draws.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
-        eps, noise, tw, tb = (torch.stack([d[i] for d in draws]).contiguous() for i in range(4))
-        held += [eps, noise, tw, tb]
-        s.tmp_w, s.tmp_b, s.eps, s.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
-        out = {"depth": torch.empty(K, B, device=self.device), "conf": torch.empty(K, B, device=self.device),
-               "heat": torch.empty(K, B, N, device=self.device),
-               "argmax": torch.empty(K, B, device=self.device, dtype=torch.int32)}
-        s.depth, s.conf, s.attention, s.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
+        return K
+
+    @torch.no_grad()
+    def forward_with_guidance(self, images, exif, guidance, S=None):
+        """-> depth [B,1], confidence [B,1], heat map [B,N], arg-max cell [B] (reference src/model.py:1157-1240).
+        `images` may be a list of uint8 [H_i, W_i, 3] photographs of individual sizes: the library resizes them to S."""
+        c, held, B, S = self._call(images, exif, S)
+        N = (S // 14) ** 2
+        self._draws(c, B, 1, held)
+        c.curiosity_runs = 1
+        self._guidance(c, guidance, N, held)
+        out = self._outputs(c, 1, B, N)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ca_forward_guided(self._h, C.byref(c), self._stream()), "ca_forward_guided")
+        self._held = held  # inputs stay referenced until the next call (their reads are enqueued, not finished)
+        return out["depth"][0].unsqueeze(1), out["conf"][0].unsqueeze(1), out["heat"][0], out["argmax"][0]
+
+    @torch.no_grad()
+    def forward_with_guidance_sweep(self, images, exif, guidances, S=None):
+        """K = len(guidances) `forward_with_guidance` calls in one native call (ca_forward_guided_sweep): the backbone and
+        the focal pass run once.  `guidances`: K instruction strings, or K guidance tensors [N].  Draws the K calls'
+        random numbers in the reference's order per call.  -> depth [K,B,1], confidence [K,B,1], heat maps [K,B,N],
+        arg-max cells [K,B]."""
+        c, held, B, S = self._call(images, exif, S)
+        N = (S // 14) ** 2
+        s = _lib.SweepCall()
+        K = self._guidances(s, guidances, N, held)
+        self._draws(s, B, K, held)
+        out = self._outputs(s, K, B, N)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.ca_forward_guided_sweep(self._h, C.byref(c), C.byref(s), self._stream()),
                        "ca_forward_guided_sweep")
@@ -315,58 +332,23 @@ class NativeModel:
         B, N = scene.B, (scene.S // 14) ** 2
         c = _lib.GuideCall()
         held = []
-        if isinstance(guidance, str):
-            c.instruction = guidance.encode()
-        else:
-            m = guidance.to(self.device, torch.float32).contiguous()
-            held.append(m)
-            c.mask, c.mask_batch_stride = m.data_ptr(), (N if m.dim() == 2 else 0)
-        eps, noise = torch.randn(B, 192), torch.randn(B, _D)       # :609, :744
-        tmp = nn.Linear(_D, 64)                                    # :1421
-        tw, tb = tmp.weight.detach().contiguous(), tmp.bias.detach().contiguous()
-        held += [eps, noise, tw, tb]
-        c.tmp_w, c.tmp_b, c.eps, c.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
-        out = {"depth": torch.empty(B, device=self.device), "conf": torch.empty(B, device=self.device),
-               "heat": torch.empty(B, N, device=self.device),
-               "argmax": torch.empty(B, device=self.device, dtype=torch.int32)}
-        c.depth, c.conf, c.attention, c.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
+        self._guidance(c, guidance, N, held)
+        self._draws(c, B, 1, held)
+        out = self._outputs(c, 1, B, N)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.ca_guide(self._h, scene.ptr, C.byref(c), self._stream()), "ca_guide")
         self._held = held
-        return out["depth"].unsqueeze(1), out["conf"].unsqueeze(1), out["heat"], out["argmax"]
+        return out["depth"][0].unsqueeze(1), out["conf"][0].unsqueeze(1), out["heat"][0], out["argmax"][0]
 
     @torch.no_grad()
     def guide_sweep(self, scene: "NativeScene", guidances):
         """ca_guide_sweep: `forward_with_guidance_sweep` on the encoded images."""
-        K = len(guidances)
-        if not 1 <= K <= _lib.SWEEP_MAX_K:
-            raise ValueError(f"an instruction sweep takes 1..{_lib.SWEEP_MAX_K} guidances, got {K}")
         B, N = scene.B, (scene.S // 14) ** 2
         s = _lib.SweepCall()
-        s.K = K
         held = []
-        if all(isinstance(g, str) for g in guidances):
-            names = (C.c_char_p * K)(*[g.encode() for g in guidances])
-            held.append(names)
-            s.instructions = C.cast(names, C.POINTER(C.c_char_p))
-        elif all(torch.is_tensor(g) and g.dim() == 1 and g.numel() == N for g in guidances):
-            m = torch.stack([g.to(self.device, torch.float32) for g in guidances]).contiguous()
-            held.append(m)
-            s.masks = m.data_ptr()
-        else:
-            raise ValueError(f"guidances must be K instruction strings or K guidance tensors of length {N}")
-        draws = []
-        for _ in range(K):
-            eps, noise = torch.randn(B, 192), torch.randn(B, _D)
-            tmp = nn.Linear(_D, 64)
-            draws.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
-        eps, noise, tw, tb = (torch.stack([d[i] for d in draws]).contiguous() for i in range(4))
-        held += [eps, noise, tw, tb]
-        s.tmp_w, s.tmp_b, s.eps, s.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
-        out = {"depth": torch.empty(K, B, device=self.device), "conf": torch.empty(K, B, device=self.device),
-               "heat": torch.empty(K, B, N, device=self.device),
-               "argmax": torch.empty(K, B, device=self.device, dtype=torch.int32)}
-        s.depth, s.conf, s.attention, s.argmax = (out[k].data_ptr() for k in ("depth", "conf", "heat", "argmax"))
+        K = self._guidances(s, guidances, N, held)
+        self._draws(s, B, K, held)
+        out = self._outputs(s, K, B, N)
         with torch.cuda.device(self.device):
             _lib.check(self.lib.ca_guide_sweep(self._h, scene.ptr, C.byref(s), self._stream()), "ca_guide_sweep")
         self._held = held
@@ -377,16 +359,14 @@ class NativeModel:
         """ca_depth_field: `CognitiveAimModel.depth_field` on the encoded images (the draws of one guide call, in its
         order).  Returns depth, confidence [B, g, g]."""
         B, g = scene.B, scene.S // 14
-        eps, noise = torch.randn(B, 192), torch.randn(B, _D)       # :609, :744
-        tmp = nn.Linear(_D, 64)                                    # :1421
-        tw, tb = tmp.weight.detach().contiguous(), tmp.bias.detach().contiguous()
         c = _lib.DepthFieldCall()
-        c.tmp_w, c.tmp_b, c.eps, c.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
+        held = []
+        self._draws(c, B, 1, held)
         depth, conf = torch.empty(B, g, g, device=self.device), torch.empty(B, g, g, device=self.device)
         c.depth, c.conf = depth.data_ptr(), conf.data_ptr()
         with torch.cuda.device(self.device):
             _lib.check(self.lib.ca_depth_field(self._h, scene.ptr, C.byref(c), self._stream()), "ca_depth_field")
-        self._held = [eps, noise, tw, tb]
+        self._held = held
         return depth, conf
 
     def launch_count(self) -> int:

@@ -202,7 +202,8 @@ int ca_heads(const ca_heads_weights* w, const ca_heads_inputs* in, float* depth,
  * overwrites) and the image's last CTA runs the heads.  in->focal_feat must be NULL and in->sweep_images 0;
  * in->tokens_per_img must be N + 1.  ticket: [B] device counters, zero before the first launch; every launch leaves them
  * at zero (no clearing between launches).  argmax may be NULL.  N <= 8192. */
-/* Largest batch for which guide calls (Python `guide`, handle `ca_guide`) use ca_guide_tail; larger batches run the
+/* Largest batch for which a single guided call (K = 1: forward_with_guidance, guide and sweeps of one instruction;
+ * ca_forward_guided, ca_guide and their sweeps) uses ca_guide_tail; larger batches and sweeps of K > 1 run the
  * three-kernel chain.  A single image is launch-bound, and one launch replaces three.  A batch is bandwidth-bound: a
  * ca_guide_tail CTA of 1024 threads fills an SM's register file, and only 6 of its warps stream tokens, while several
  * 192-thread pool CTAs of the chain share an SM.  tools/bench_scene.py times both at B = 1 and B = 32. */

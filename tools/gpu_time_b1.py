@@ -15,7 +15,7 @@ for B, S in ((1, 518), (1, 224), (8, 518)):
         model.forward_with_guidance(x, ex, "center", return_attention=True)
     torch.cuda.synchronize()
     ws = model._workspace(B, S)
-    (graph, n), = [v for k, v in ws["graphs"].items() if k[0] == "guided"]
+    (graph, n), = [v for k, v in ws["graphs"].items() if k[:2] == ("sweep", 1)]  # a guided call is a sweep of one
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(50):
