@@ -6,7 +6,7 @@
 //     37 x 37 grid, bicubic align_corners=False otherwise), the focal 2-D sinusoidal position encoding
 //     (src/model.py:140-166), the Gaussian centre bias (:208-231) and the instruction masks (:1270-1376);
 //   * one activation workspace per (batch, resolution), carved out of a single device allocation;
-//   * a ring of pinned staging buffers for the per-call HOST inputs (per-call projection, curiosity draws), pulled to the
+//   * a ring of pinned staging buffers for the per-call HOST inputs (curiosity draws, per-call projections), pulled to the
 //     device by SM-side reads so they never queue on the H2D copy engine behind the application's image upload;
 //   * the launch sequence itself (the same kernels, in the same order, as cognitive_aim_depth_estimation_b200/model.py),
 //     the CuriosityModule on a forked side stream, and one CUDA graph per (path, batch, resolution).
@@ -53,22 +53,23 @@ struct Workspace {
   unsigned long long gen = 0;  // unique per allocation: a scene's graphs captured on another workspace are not replayed
   void* arena = nullptr;
   __nv_bfloat16 *patches, *h, *qkv, *att, *mlp, *xin, *qk;
-  float *x, *tokens, *pm, *ps, *pc, *wtab, *attn, *cvec, *rowscale, *pool, *pool_pe, *feats, *focal_feat, *fused, *depth,
-      *conf, *exif_in, *cur_eps, *cur_noise, *cur_raw, *cur_reward, *ln_stats;
+  float *x, *tokens, *pm, *ps, *pc, *wtab, *attn, *cvec, *rowscale, *pool, *pool_pe, *feats, *focal_feat, *fused,
+      *exif_in, *ln_stats;
   void* E;
   long long* cam_in;
   int P = 0, lde = 0;
   std::map<int, std::pair<cudaGraphExec_t, int>> graphs;  // path key -> (executable graph, launches)
   std::map<int, int> seen;                                // path key -> calls so far
-  // guided calls: the per-call buffers of K calls (rows k * B + b; K = 1 for a single call), one arena per K; the
-  // backbone and focal buffers above are shared with the un-guided forward
+  // The per-call ("sweep") buffers of a call with R CuriosityModule runs (rows r * B + b), one arena per R: R guided calls of a
+  // sweep (R = 1: a single guided call or a depth field), or an un-guided forward's runs, whose heads write rows 0..B-1.
+  // The backbone and focal buffers above are shared by every call.
   struct Sweep {
     void* arena = nullptr;
     float *mask_in, *heat, *pool, *depth, *conf, *tmpw, *tmpb, *cur_eps, *cur_noise, *cur_raw, *cur_reward;
     int* argmax;
     int* tail_ticket;  // [B] per-image tickets of the fused guide tail, zero when idle
   };
-  std::map<int, Sweep> sweeps;  // K -> buffers
+  std::map<int, Sweep> sweeps;  // R -> buffers
   // depth fields (allocated at the first ca_depth_field on this workspace): projected tokens [B, N, 64], the per-image
   // fusion constant [B, 192], the field [B, N] x 2
   void* field_arena = nullptr;
@@ -290,6 +291,22 @@ int get_mask(Tables* t, const char* instruction, int g, float** out) {
 // ------------------------------------------------------------------------------------------------------------------
 // workspace
 // ------------------------------------------------------------------------------------------------------------------
+// Buffers carved out of one device allocation, each at a 256-byte-aligned offset: add() them, then alloc().
+struct Layout {
+  std::vector<std::pair<void**, size_t>> slots;
+  size_t bytes = 0;
+  template <class T>
+  void add(T** p, size_t n) {
+    slots.push_back({reinterpret_cast<void**>(p), bytes});
+    bytes += (n + 255) & ~static_cast<size_t>(255);
+  }
+  int alloc(void** arena) {
+    CA_CUDA(cudaMalloc(arena, bytes));
+    for (auto& s : slots) *s.first = static_cast<char*>(*arena) + s.second;
+    return 0;
+  }
+};
+
 int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   const auto key = std::make_pair(B, S);
   auto it = h->ws.find(key);
@@ -310,48 +327,33 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   w.P = ca::gemm_stats_partials(static_cast<int>(N));
   w.lde = 64 * static_cast<int>((N + 63) / 64);
   const int iters = h->w.n_focal;
-  size_t off = 0;
-  auto take = [&](size_t bytes) {
-    const size_t o = off;
-    off += (bytes + 255) & ~static_cast<size_t>(255);
-    return o;
-  };
-  struct Slot { void** p; size_t o; };
-  std::vector<Slot> slots;
-  auto want = [&](auto** p, size_t bytes) { slots.push_back({reinterpret_cast<void**>(p), take(bytes)}); };
-  want(&w.patches, BN * ca::kPatchRowStride * 2);
-  want(&w.x, M * kD * 4);
-  want(&w.h, M * kD * 2);
-  want(&w.ln_stats, M * (kD / 128) * 2 * 4);
-  want(&w.qkv, M * 3 * kD * 2);
-  want(&w.att, M * kD * 2);
-  want(&w.mlp, M * kMlp * 2);
-  want(&w.tokens, M * kD * 4);
-  want(&w.xin, BN * kD * 2);
-  want(&w.qk, BN * 2 * kD * 2);
-  want(&w.pm, BN * w.P * 4);
-  want(&w.ps, BN * w.P * 4);
-  want(&w.pc, BN * w.P * 4);
-  want(&w.wtab, BN * w.P * 4);
-  want(&w.E, BN * w.lde * 2);
-  want(&w.attn, iters * BN * 4);
-  want(&w.cvec, BN * 4);
-  want(&w.rowscale, 2 * BN * 4);
-  want(&w.pool, static_cast<size_t>(B) * kPoolSplits * kD * 4);
-  want(&w.pool_pe, static_cast<size_t>(B) * kPoolSplits * kD * 4);
-  want(&w.feats, static_cast<size_t>(B) * iters * 64 * 4);
-  want(&w.focal_feat, static_cast<size_t>(B) * 64 * 4);
-  want(&w.fused, static_cast<size_t>(B) * 192 * 4);
-  want(&w.depth, B * 4);
-  want(&w.conf, B * 4);
-  want(&w.exif_in, B * 3 * 4);
-  want(&w.cam_in, B * 8);
-  want(&w.cur_eps, static_cast<size_t>(kMaxRuns) * B * 192 * 4);
-  want(&w.cur_noise, static_cast<size_t>(kMaxRuns) * B * kD * 4);
-  want(&w.cur_raw, static_cast<size_t>(kMaxRuns) * B * 4);
-  want(&w.cur_reward, static_cast<size_t>(kMaxRuns) * B * 4);
-  CA_CUDA(cudaMalloc(&w.arena, off));
-  for (auto& s : slots) *s.p = static_cast<char*>(w.arena) + s.o;
+  Layout l;
+  l.add(&w.patches, BN * ca::kPatchRowStride * 2);
+  l.add(&w.x, M * kD * 4);
+  l.add(&w.h, M * kD * 2);
+  l.add(&w.ln_stats, M * (kD / 128) * 2 * 4);
+  l.add(&w.qkv, M * 3 * kD * 2);
+  l.add(&w.att, M * kD * 2);
+  l.add(&w.mlp, M * kMlp * 2);
+  l.add(&w.tokens, M * kD * 4);
+  l.add(&w.xin, BN * kD * 2);
+  l.add(&w.qk, BN * 2 * kD * 2);
+  l.add(&w.pm, BN * w.P * 4);
+  l.add(&w.ps, BN * w.P * 4);
+  l.add(&w.pc, BN * w.P * 4);
+  l.add(&w.wtab, BN * w.P * 4);
+  l.add(&w.E, BN * w.lde * 2);
+  l.add(&w.attn, iters * BN * 4);
+  l.add(&w.cvec, BN * 4);
+  l.add(&w.rowscale, 2 * BN * 4);
+  l.add(&w.pool, static_cast<size_t>(B) * kPoolSplits * kD * 4);
+  l.add(&w.pool_pe, static_cast<size_t>(B) * kPoolSplits * kD * 4);
+  l.add(&w.feats, static_cast<size_t>(B) * iters * 64 * 4);
+  l.add(&w.focal_feat, static_cast<size_t>(B) * 64 * 4);
+  l.add(&w.fused, static_cast<size_t>(B) * 192 * 4);
+  l.add(&w.exif_in, B * 3 * 4);
+  l.add(&w.cam_in, B * 8);
+  CA_TRY(l.alloc(&w.arena));
   CA_CUDA(cudaMemset(w.exif_in, 0, B * 3 * 4));
   CA_CUDA(cudaMemset(w.cam_in, 0, B * 8));
   static std::atomic<unsigned long long> next_gen{1};
@@ -360,35 +362,29 @@ int get_workspace(ca_handle* h, int B, int S, Workspace** out) {
   return 0;
 }
 
-int get_sweep(Workspace& w, int K, Workspace::Sweep** out) {
-  auto it = w.sweeps.find(K);
+int get_sweep(Workspace& w, int R, Workspace::Sweep** out) {
+  auto it = w.sweeps.find(R);
   if (it == w.sweeps.end()) {
     const int g = w.S / 14;
-    const size_t N = static_cast<size_t>(g) * g, KB = static_cast<size_t>(K) * w.B;
-    size_t off = 0;
-    std::vector<std::pair<void**, size_t>> slots;
+    const size_t N = static_cast<size_t>(g) * g, RB = static_cast<size_t>(R) * w.B;
     Workspace::Sweep s;
-    auto want = [&](auto** p, size_t bytes) {
-      slots.push_back({reinterpret_cast<void**>(p), off});
-      off += (bytes + 255) & ~static_cast<size_t>(255);
-    };
-    want(&s.mask_in, KB * N * 4);  // a mask row per image and call at most
-    want(&s.heat, KB * N * 4);
-    want(&s.argmax, KB * 4);
-    want(&s.pool, KB * kPoolSplits * kD * 4);
-    want(&s.depth, KB * 4);
-    want(&s.conf, KB * 4);
-    want(&s.tmpw, static_cast<size_t>(K) * 64 * kD * 4);
-    want(&s.tmpb, static_cast<size_t>(K) * 64 * 4);
-    want(&s.cur_eps, KB * 192 * 4);
-    want(&s.cur_noise, KB * kD * 4);
-    want(&s.cur_raw, KB * 4);
-    want(&s.cur_reward, KB * 4);
-    want(&s.tail_ticket, static_cast<size_t>(w.B) * 4);
-    CA_CUDA(cudaMalloc(&s.arena, off));
-    for (auto& sl : slots) *sl.first = static_cast<char*>(s.arena) + sl.second;
+    Layout l;
+    l.add(&s.mask_in, RB * N * 4);  // a mask row per image and call at most
+    l.add(&s.heat, RB * N * 4);
+    l.add(&s.argmax, RB * 4);
+    l.add(&s.pool, RB * kPoolSplits * kD * 4);
+    l.add(&s.depth, RB * 4);
+    l.add(&s.conf, RB * 4);
+    l.add(&s.tmpw, static_cast<size_t>(R) * 64 * kD * 4);
+    l.add(&s.tmpb, static_cast<size_t>(R) * 64 * 4);
+    l.add(&s.cur_eps, RB * 192 * 4);
+    l.add(&s.cur_noise, RB * kD * 4);
+    l.add(&s.cur_raw, RB * 4);
+    l.add(&s.cur_reward, RB * 4);
+    l.add(&s.tail_ticket, static_cast<size_t>(w.B) * 4);
+    CA_TRY(l.alloc(&s.arena));
     CA_CUDA(cudaMemset(s.tail_ticket, 0, static_cast<size_t>(w.B) * 4));
-    it = w.sweeps.emplace(K, s).first;
+    it = w.sweeps.emplace(R, s).first;
   }
   *out = &it->second;
   return 0;
@@ -398,15 +394,12 @@ int get_field(Workspace& w) {
   if (w.field_arena) return 0;
   const int g = w.S / 14;
   const size_t BN = static_cast<size_t>(w.B) * g * g;
-  const size_t o_cst = BN * 64 * 4, o_depth = o_cst + ((static_cast<size_t>(w.B) * 192 * 4 + 255) & ~size_t(255));
-  const size_t o_conf = o_depth + ((BN * 4 + 255) & ~size_t(255));
-  CA_CUDA(cudaMalloc(&w.field_arena, o_conf + BN * 4));
-  char* a = static_cast<char*>(w.field_arena);
-  w.field_P = reinterpret_cast<float*>(a);
-  w.field_cst = reinterpret_cast<float*>(a + o_cst);
-  w.field_depth = reinterpret_cast<float*>(a + o_depth);
-  w.field_conf = reinterpret_cast<float*>(a + o_conf);
-  return 0;
+  Layout l;
+  l.add(&w.field_P, BN * 64 * 4);
+  l.add(&w.field_cst, static_cast<size_t>(w.B) * 192 * 4);
+  l.add(&w.field_depth, BN * 4);
+  l.add(&w.field_conf, BN * 4);
+  return l.alloc(&w.field_arena);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -570,7 +563,7 @@ int focal_iterations(ca_handle* h, Workspace& w, const Tables& tb, bool want_fea
 // CuriosityModule runs of one call on the side stream (forked here, joined by curiosity_join): output-dead under the
 // shipped configurations and latency-bound, so it runs under the focal stream's GEMMs.  The fork / join are stream
 // dependencies: during capture they become a parallel branch of the graph.
-// eps / noise / raw / reward: [runs, B, ...] buffers of the runs (the workspace's, or an instruction sweep's).
+// eps / noise / raw / reward: [runs, B, ...] buffers of the runs, in the call's sweep buffers.
 int curiosity_fork(ca_handle* h, Workspace& w, int runs, const float* eps, const float* noise, float* raw, float* reward,
                    cudaStream_t st, const float* tokens = nullptr) {
   const int B = w.B, g = w.S / 14, T = g * g + 1;
@@ -592,7 +585,7 @@ int curiosity_join(ca_handle* h, cudaStream_t st) {
   return 0;
 }
 
-int heads(ca_handle* h, Workspace& w, bool has_exif, int* fault, cudaStream_t st) {
+int heads(ca_handle* h, Workspace& w, Workspace::Sweep& s, bool has_exif, int* fault, cudaStream_t st) {
   const int g = w.S / 14, T = g * g + 1;
   ca_heads_inputs in{};
   in.tokens = w.tokens;
@@ -602,7 +595,7 @@ int heads(ca_handle* h, Workspace& w, bool has_exif, int* fault, cudaStream_t st
   in.camera_idx = has_exif ? w.cam_in : nullptr;
   in.num_cameras = h->w.num_cameras;
   in.fault = fault;
-  LAUNCH(ca::heads_launch(h->w.heads, in, w.depth, w.conf, w.fused, w.B, st));
+  LAUNCH(ca::heads_launch(h->w.heads, in, s.depth, s.conf, w.fused, w.B, st));
   return 0;
 }
 
@@ -622,38 +615,25 @@ int pinned_slot(ca_handle* h, size_t need, PinnedSlot** out) {
   return 0;
 }
 
-int stage_host_inputs(ca_handle* h, Workspace& w, const ca_forward_call& c, int runs, cudaStream_t st) {
-  const size_t B = w.B;
-  PinnedSlot* sp = nullptr;
-  CA_TRY(pinned_slot(h, static_cast<size_t>(runs) * B * (192 + kD), &sp));
-  PinnedSlot& s = *sp;
-  float* p = s.buf;
-  memcpy(p, c.eps, static_cast<size_t>(runs) * B * 192 * sizeof(float));
-  memcpy(p + static_cast<size_t>(runs) * B * 192, c.noise, static_cast<size_t>(runs) * B * kD * sizeof(float));
-  CA_TRY(ca::fetch_pinned_launch(w.cur_eps, p, static_cast<size_t>(runs) * B * 192, st));
-  CA_TRY(ca::fetch_pinned_launch(w.cur_noise, p + static_cast<size_t>(runs) * B * 192, static_cast<size_t>(runs) * B * kD, st));
-  h->launches += 2;
-  CA_CUDA(cudaEventRecord(s.done, st));
-  return 0;
-}
-
-// the K guided calls' projections and curiosity draws (HOST) -> one pinned slot sized for K -> the device buffers of K
-int stage_guided_draws(ca_handle* h, Workspace& w, Workspace::Sweep& s, size_t K, const float* tmp_w, const float* tmp_b,
-                       const float* eps, const float* noise, cudaStream_t st) {
-  const size_t B = w.B;
-  const size_t n_tw = K * 64 * kD, n_tb = K * 64, n_eps = K * B * 192, n_noise = K * B * kD;
+// The HOST draws of R CuriosityModule runs, and for guided calls their projections (tmp_w / tmp_b, or none) -> one pinned
+// slot -> the call's sweep buffers
+int stage_draws(ca_handle* h, int B, Workspace::Sweep& s, int R, const float* eps, const float* noise, cudaStream_t st,
+                const float* tmp_w = nullptr, const float* tmp_b = nullptr) {
+  const size_t r = R, n_proj = tmp_w ? r * 64 * kD : 0, n_bias = tmp_w ? r * 64 : 0;
+  const struct { float* dst; const float* src; size_t n; } parts[] = {
+      {s.tmpw, tmp_w, n_proj}, {s.tmpb, tmp_b, n_bias}, {s.cur_eps, eps, r * B * 192}, {s.cur_noise, noise, r * B * kD}};
+  size_t need = 0;
+  for (const auto& q : parts) need += q.n;
   PinnedSlot* slot = nullptr;
-  CA_TRY(pinned_slot(h, n_tw + n_tb + n_eps + n_noise, &slot));
+  CA_TRY(pinned_slot(h, need, &slot));
   float* p = slot->buf;
-  memcpy(p, tmp_w, n_tw * sizeof(float));
-  memcpy(p + n_tw, tmp_b, n_tb * sizeof(float));
-  memcpy(p + n_tw + n_tb, eps, n_eps * sizeof(float));
-  memcpy(p + n_tw + n_tb + n_eps, noise, n_noise * sizeof(float));
-  CA_TRY(ca::fetch_pinned_launch(s.tmpw, p, n_tw, st));
-  CA_TRY(ca::fetch_pinned_launch(s.tmpb, p + n_tw, n_tb, st));
-  CA_TRY(ca::fetch_pinned_launch(s.cur_eps, p + n_tw + n_tb, n_eps, st));
-  CA_TRY(ca::fetch_pinned_launch(s.cur_noise, p + n_tw + n_tb + n_eps, n_noise, st));
-  h->launches += 4;
+  for (const auto& q : parts) {
+    if (q.n == 0) continue;
+    memcpy(p, q.src, q.n * sizeof(float));
+    CA_TRY(ca::fetch_pinned_launch(q.dst, p, q.n, st));
+    ++h->launches;
+    p += q.n;
+  }
   CA_CUDA(cudaEventRecord(slot->done, st));
   return 0;
 }
@@ -859,7 +839,7 @@ int run_guided(ca_handle* h, const ca_forward_call* call, ca_scene* sc, const Gu
   } else {
     CA_CUDA(cudaMemcpyAsync(s.mask_in, c.masks, K * rows * 4, cudaMemcpyDeviceToDevice, st));
   }
-  CA_TRY(stage_guided_draws(h, w, s, K, c.tmp_w, c.tmp_b, c.eps, c.noise, st));
+  CA_TRY(stage_draws(h, B, s, K, c.eps, c.noise, st, c.tmp_w, c.tmp_b));
   ca_heads_inputs in{};
   in.tokens_per_img = T;
   in.pool_partial = s.pool;
@@ -1066,7 +1046,10 @@ int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
   h->launches = 0;
   const bool has_exif = c->exif != nullptr && h->w.num_cameras > 0;
   const int runs = c->curiosity_runs;
-  CA_TRY(stage_host_inputs(h, w, *c, runs, st));
+  Workspace::Sweep* sp = nullptr;
+  CA_TRY(get_sweep(w, runs, &sp));
+  Workspace::Sweep& s = *sp;
+  CA_TRY(stage_draws(h, B, s, runs, c->eps, c->noise, st));
   if (has_exif) {
     CA_CUDA(cudaMemcpyAsync(w.exif_in, c->exif, static_cast<size_t>(B) * 3 * 4, cudaMemcpyDeviceToDevice, st));
     CA_CUDA(cudaMemcpyAsync(w.cam_in, c->camera_idx, static_cast<size_t>(B) * 8, cudaMemcpyDeviceToDevice, st));
@@ -1077,15 +1060,15 @@ int ca_forward(ca_handle* h, const ca_forward_call* c, void* stream) {
   const int key = 200 + (has_exif ? 1 : 0) + 2 * runs;
   CA_TRY(run_sequence(h, w, key, c->use_graph != 0, st, [&]() -> int {
     CA_TRY(backbone_layers(h, w, *tb, st));
-    CA_TRY(curiosity_fork(h, w, runs, w.cur_eps, w.cur_noise, w.cur_raw, w.cur_reward, st));
+    CA_TRY(curiosity_fork(h, w, runs, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st));
     CA_TRY(focal_iterations(h, w, *tb, true, st, &att));
-    CA_TRY(heads(h, w, has_exif, fault, st));
+    CA_TRY(heads(h, w, s, has_exif, fault, st));
     CA_TRY(curiosity_join(h, st));
     return 0;
   }));
   att = w.attn + static_cast<size_t>(h->w.n_focal - 1) * B * N;
-  CA_CUDA(cudaMemcpyAsync(c->depth, w.depth, B * 4, cudaMemcpyDeviceToDevice, st));
-  CA_CUDA(cudaMemcpyAsync(c->conf, w.conf, B * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c->depth, s.depth, B * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c->conf, s.conf, B * 4, cudaMemcpyDeviceToDevice, st));
   if (c->attention) CA_CUDA(cudaMemcpyAsync(c->attention, att, static_cast<size_t>(B) * N * 4, cudaMemcpyDeviceToDevice, st));
   if (c->fused) CA_CUDA(cudaMemcpyAsync(c->fused, w.fused, static_cast<size_t>(B) * 192 * 4, cudaMemcpyDeviceToDevice, st));
   h->last_launches = h->launches;
@@ -1117,18 +1100,16 @@ int ca_encode(ca_handle* h, const ca_forward_call* c, ca_scene** out, void* stre
   }));
   base = w.attn + static_cast<size_t>(h->w.n_focal - 1) * B * N;
   const size_t tok = static_cast<size_t>(B) * T * kD * 4, bn = static_cast<size_t>(B) * N * 4;
-  const size_t o_base = (tok + 255) & ~size_t(255), o_exif = o_base + ((bn + 255) & ~size_t(255));
-  const size_t o_cam = o_exif + 256 * ((static_cast<size_t>(B) * 12 + 255) / 256);
   ca_scene* sc = new ca_scene();
-  if (cudaMalloc(&sc->arena, o_cam + static_cast<size_t>(B) * 8) != cudaSuccess) {
+  Layout l;
+  l.add(&sc->tokens, tok);
+  l.add(&sc->base, bn);
+  l.add(&sc->exif, static_cast<size_t>(B) * 12);
+  l.add(&sc->cam, static_cast<size_t>(B) * 8);
+  if (const int status = l.alloc(&sc->arena)) {
     delete sc;
-    return ca::cuda_fail(cudaGetLastError(), "encode: scene allocation", __FILE__, __LINE__);
+    return status;
   }
-  char* a = static_cast<char*>(sc->arena);
-  sc->tokens = reinterpret_cast<float*>(a);
-  sc->base = reinterpret_cast<float*>(a + o_base);
-  sc->exif = reinterpret_cast<float*>(a + o_exif);
-  sc->cam = reinterpret_cast<long long*>(a + o_cam);
   sc->handle_id = h->id;
   sc->device = h->device;
   sc->B = B;
@@ -1196,7 +1177,7 @@ int ca_depth_field(ca_handle* h, ca_scene* sc, const ca_depth_field_call* c, voi
   CA_TRY(get_sweep(w, 1, &sp));  // the buffers of one guided call
   Workspace::Sweep& s = *sp;
   h->launches = 0;
-  CA_TRY(stage_guided_draws(h, w, s, 1, c->tmp_w, c->tmp_b, c->eps, c->noise, st));
+  CA_TRY(stage_draws(h, B, s, 1, c->eps, c->noise, st, c->tmp_w, c->tmp_b));
   CA_TRY(run_captured(h, sc->graphs, sc->seen, 200, sc->use_graph, st, [&]() -> int {
     CA_TRY(curiosity_fork(h, w, 1, s.cur_eps, s.cur_noise, s.cur_raw, s.cur_reward, st, sc->tokens));
     LAUNCH(ca::token_project_launch(sc->tokens, static_cast<long long>(T) * kD, 1, s.tmpw, w.field_P, B, N, st));

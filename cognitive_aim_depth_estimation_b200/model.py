@@ -41,9 +41,17 @@ _HEADS = 12
 _LAYERS = 12
 _MLP = 3072
 _POOL_SPLITS = 32  # 1024 CTAs at B = 32: the 8-way split (256 CTAs) reached 39 % of the HBM rate (profiles/r01e_bw_kernels.md)
-_MAX_CURIOSITY_RUNS = 3
 _LORA_PAD = 64  # fused LoRA: the rank is padded to one 64-wide K block of the tcgen05 GEMM (K = 768 + 64 = 13 blocks)
 _MAX_SIDE = 1260  # 90 x 90 patch tokens: the focal vector stages keep an image's N <= 8192 columns in one CTA (csrc/focal.cu)
+
+
+def _poison(tensors):
+    """Test aid (CA_POISON_WS): fresh floating-point buffers start as NaN, so a kernel that reads a slot nobody wrote
+    (e.g. an unwritten partial-sum column) produces NaN instead of plausible stale data."""
+    if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
+        for t in tensors:
+            if torch.is_tensor(t) and t.is_floating_point():
+                t.fill_(float("nan"))
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -504,31 +512,17 @@ class CognitiveAimModel(nn.Module):
                 "rowscale": torch.empty(2, B, N, **fl),
                 # LayerNorm folding: per (row, 128-column span) (sum, M2) of the residual row; `h` then holds the raw rows
                 "ln_stats": torch.empty(B * T, _D // 128, 2, **fl),
-                "heat": torch.empty(B, N, **fl), "argmax": torch.empty(B, device=dev, dtype=torch.int32),
                 "pool": torch.empty(B, _POOL_SPLITS, _D, **fl), "pool_pe": torch.empty(B, _POOL_SPLITS, _D, **fl),
                 "feats": torch.empty(B, self.cfg.num_iterations, 64, **fl),
                 "focal_feat": torch.empty(B, 64, **fl), "fused": torch.empty(B, 192, **fl),
-                "depth": torch.empty(B, **fl), "conf": torch.empty(B, **fl),
                 # per-call inputs, at fixed addresses so that captured graphs can be replayed
-                "mask_in": torch.empty(B, N, **fl),
                 "exif_in": torch.zeros(B, 3, **fl), "cam_in": torch.zeros(B, device=dev, dtype=torch.int64),
-                # CuriosityModule: up to _MAX_CURIOSITY_RUNS runs per call (src/model.py:992,1104,1138,1185), each with
-                # its own pair of Gaussian draws; rewards per run; modulation weights per (run, iteration)
-                "cur_eps": torch.zeros(_MAX_CURIOSITY_RUNS, B, 192, **fl),
-                "cur_noise": torch.zeros(_MAX_CURIOSITY_RUNS, B, _D, **fl),
-                "cur_raw": torch.empty(_MAX_CURIOSITY_RUNS, B, **fl),
-                "cur_reward": torch.empty(_MAX_CURIOSITY_RUNS, B, **fl),
-                "cur_weight": torch.empty(_MAX_CURIOSITY_RUNS, self.cfg.num_iterations, B, **fl),
-                "att_run": torch.empty(_MAX_CURIOSITY_RUNS, B, N, **fl),
                 "graphs": {},
+                # the per-call buffers, one set per number of CuriosityModule runs (_sweep_buffers)
+                "sweeps": {},
             }
             ws["h"], ws["att"] = ws["h_ext"][:, :_D], ws["att_ext"][:, :_D]
-            if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
-                # test aid: every floating-point workspace starts as NaN, so a kernel that reads a slot nobody wrote
-                # (e.g. an unwritten partial-sum column) produces NaN instead of plausible stale data
-                for k, t in ws.items():
-                    if torch.is_tensor(t) and t.is_floating_point() and k not in ("exif_in",):
-                        t.fill_(float("nan"))
+            _poison(t for k, t in ws.items() if k != "exif_in")
             if len(self._ws) >= 4:  # keep the cache bounded
                 self._ws.pop(next(iter(self._ws)))
             self._ws[key] = ws
@@ -541,30 +535,33 @@ class CognitiveAimModel(nn.Module):
         completed."""
         ring = getattr(self, "_pinned_ring", None)
         if ring is None:
-            ring = {"slots": [{"draws": {}, "sweep": {}, "event": torch.cuda.Event()} for _ in range(4)], "next": 0}
+            ring = {"slots": [{"draws": {}, "event": torch.cuda.Event()} for _ in range(4)], "next": 0}
             self._pinned_ring = ring
         slot = ring["slots"][ring["next"]]
         ring["next"] = (ring["next"] + 1) % len(ring["slots"])
         slot["event"].synchronize()
         return slot
 
-    def _stage_draws(self, ws, slot, draws):
-        """Curiosity draws [(eps [B,192], noise [B,768]), ...] -> pinned staging -> the fixed device buffers the
-        (possibly graph-captured) curiosity kernel reads."""
-        k, B = len(draws), draws[0][0].shape[0]
-        # one pinned pair per batch size, kept for the life of the model: a kernel reads them asynchronously, so they
-        # must never go back to the host allocator while a read may be in flight (the slot's event guards their REUSE)
-        bufs = slot["draws"].get(B)
+    def _stage_runs(self, cs, draws):
+        """The host draws of R CuriosityModule runs, made before any buffer is looked up — R tuples (eps [B,192],
+        noise [B,768]) of an un-guided forward, or `_sweep_draws`' (eps, noise, projection weight, bias) of R guided calls
+        — through the pinned staging of one ring slot into the sweep buffers' cur_eps, cur_noise (and tmpw, tmpb)."""
+        R, B = len(draws), draws[0][0].shape[0]
+        slot = self._pinned_slot()
+        # pinned buffers per (B, R), kept for the life of the model: a kernel reads them asynchronously, so they must
+        # never go back to the host allocator while a read may be in flight (the slot's event guards their REUSE)
+        bufs = slot["draws"].get((B, R))
         if bufs is None:
-            bufs = slot["draws"][B] = (torch.empty(_MAX_CURIOSITY_RUNS, B, 192).pin_memory(),
-                                       torch.empty(_MAX_CURIOSITY_RUNS, B, _D).pin_memory())
-        for j, (eps, noise) in enumerate(draws):
-            bufs[0][j].copy_(eps)
-            bufs[1][j].copy_(noise)
+            bufs = slot["draws"][(B, R)] = tuple(torch.empty(*s).pin_memory() for s in
+                                                 ((R, B, 192), (R, B, _D), (R, 64, _D), (R, 64)))
+        for k, d in enumerate(draws):
+            for buf, t in zip(bufs, d):
+                buf[k].copy_(t)
         # SM-side reads of the pinned staging area (ops.fetch_pinned), not cudaMemcpyAsync: these few hundred KB must not
         # wait on the H2D copy engine behind the application's upload of the next image batch
-        ops.fetch_pinned(ws["cur_eps"][:k], bufs[0][:k])
-        ops.fetch_pinned(ws["cur_noise"][:k], bufs[1][:k])
+        for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb")[:len(draws[0])], bufs):
+            ops.fetch_pinned(cs[dst], buf)
+        slot["event"].record()
 
     @staticmethod
     def _check_side(S):
@@ -721,23 +718,25 @@ class CognitiveAimModel(nn.Module):
         graph[0].replay()
         ops.count_launches(graph[1])
 
-    def _focal_iterations(self, ws, B: int, g: int, want_features: bool, cur_weight=None):
-        """IterativeFocalStream (src/model.py:391-455): per iteration Q|K projection, one tensor-core pass over Q K^T
-        (row statistics + stored exponentials), the column sums as a bandwidth pass, and the vector epilogue.
-        `cur_weight` [n_iters, B]: curiosity modulation (only with curiosity_guided_attention.enabled, :264-276).
-        Returns the last iteration's attention [B, N]; fills ws['focal_feat'] when `want_features`."""
+    def _focal_iterations(self, ws, B: int, g: int, want_features: bool, cur_weight=None, tokens=None):
+        """IterativeFocalStream (src/model.py:391-455) on `tokens` [B, 1+N, 768] (default: the workspace's; a scene's
+        for a guide call): per iteration Q|K projection, one tensor-core pass over Q K^T (row statistics + stored exponentials), the column sums
+        as a bandwidth pass, and the vector epilogue.  `cur_weight` [n_iters, B]: curiosity modulation (only with
+        curiosity_guided_attention.enabled, :264-276).  Returns the last iteration's attention [B, N]; fills
+        ws['focal_feat'] when `want_features`."""
         pk = self._pack()
         tb = self._grid_tables(g)
         N = g * g
         scale_log2 = ops.LOG2E / math.sqrt(_D // 8)  # src/model.py:69 (single head, sqrt(768 // 8))
         iters = self.cfg.num_iterations
+        tokens = ws["tokens"] if tokens is None else tokens
         qk = ws["qk"]
         q, k = qk[:, :_D], qk[:, _D:]
         rs = None
         for i in range(iters):
           with _nvtx(f"cogaim.focal{i}"):
             F_ = pk["focal"][i]
-            ops.focal_input(ws["tokens"], tb["pe"], rs, ws["xin"], B, N, _D)
+            ops.focal_input(tokens, tb["pe"], rs, ws["xin"], B, N, _D)
             ops.gemm(ws["xin"], F_["wqk"], ops.EPI_BIAS_BF16, qk, bias=F_["bqk"])
             common = dict(M=N, N=N, K=_D, lda=2 * _D, ldw=2 * _D, batch=B, a_batch_stride=N * 2 * _D,
                           w_batch_stride=N * 2 * _D, scale_log2=scale_log2)
@@ -757,7 +756,7 @@ class CognitiveAimModel(nn.Module):
                 ops.colsum_e(E, ws["wtab"], ws["pc"], B, N)
                 ops.focal_finalize(ws["pc"], None, ws["cvec"], None, None, B, N, 0.0, 1)
                 T = N + 1
-                ops.weighted_pool(ws["tokens"], T * _D, 1, ws["cvec"], rs, ws["pool"], B, N, _D, _POOL_SPLITS)
+                ops.weighted_pool(tokens, T * _D, 1, ws["cvec"], rs, ws["pool"], B, N, _D, _POOL_SPLITS)
                 ops.weighted_pool(tb["pe"], 0, 0, ws["cvec"], None, ws["pool_pe"], B, N, _D, _POOL_SPLITS)
                 ops.focal_value(tok_partial=ws["pool"], pe_partial=ws["pool_pe"], splits=_POOL_SPLITS, wv=F_["wv"],
                                 bv=F_["bv"], proj_w0=F_["pw0"], proj_b0=F_["pb0"], proj_w1=F_["pw1"], proj_b1=F_["pb1"],
@@ -845,10 +844,11 @@ class CognitiveAimModel(nn.Module):
         noise = torch.randn(Bg, 768)
         return eps[lo:lo + B], noise[lo:lo + B]
 
-    def _curiosity_runs(self, ws, B: int, T: int, roles):
-        """Device side of the CuriosityModule runs of one call, in the reference's order: rewards, ring-buffer update,
-        and (curiosity-guided configuration only) the attention modulation weights of each run.  The score of the
-        un-guided attention runs is clamped to [0.5, 1] (src/model.py:1107, :1141); the others are not."""
+    def _curiosity_runs(self, cs, tokens, B: int, T: int, roles):
+        """Device side of the CuriosityModule runs of one call on `tokens`, in the reference's order: rewards, ring-buffer
+        update, and (curiosity-guided configuration only) the attention modulation weights of each run, in the sweep
+        buffers `cs`.  The score of the un-guided attention runs is clamped to [0.5, 1] (src/model.py:1107, :1141); the others
+        are not."""
         pk = self._packed
         cm = self.curiosity_module
         # Output-dead under the shipped configurations and latency-bound (one CTA per image through ten small dense
@@ -862,21 +862,21 @@ class CognitiveAimModel(nn.Module):
             side.wait_stream(torch.cuda.current_stream())
         self._curiosity_side = side
         with torch.cuda.stream(side) if side is not None else contextlib.nullcontext():
-            self._curiosity_launches(ws, B, T, roles, pk, cm)
+            self._curiosity_launches(cs, tokens, B, T, roles, pk, cm)
 
     def _curiosity_join(self):
         side, self._curiosity_side = getattr(self, "_curiosity_side", None), None
         if side is not None:
             torch.cuda.current_stream().wait_stream(side)
 
-    def _curiosity_launches(self, ws, B, T, roles, pk, cm):
+    def _curiosity_launches(self, cs, tokens, B, T, roles, pk, cm):
         for j, role in enumerate(roles):
-            ops.curiosity(pk["curiosity"], tokens=ws["tokens"], tokens_per_img=T, eps=ws["cur_eps"][j],
-                          noise=ws["cur_noise"][j], reward_raw=ws["cur_raw"][j], reward=ws["cur_reward"][j],
+            ops.curiosity(pk["curiosity"], tokens=tokens, tokens_per_img=T, eps=cs["cur_eps"][j],
+                          noise=cs["cur_noise"][j], reward_raw=cs["cur_raw"][j], reward=cs["cur_reward"][j],
                           history=cm.exploration_history, history_pointer=cm.history_pointer, B=B)
             if self.cfg.curiosity_guided:
                 lo, hi = (0.5, 1.0) if role in ("last", "ret") else (1.0, 0.0)
-                ops.curiosity_modulation(pk["curiosity_mod"], ws["cur_reward"][j], lo, hi, ws["cur_weight"][j], B,
+                ops.curiosity_modulation(pk["curiosity_mod"], cs["cur_reward"][j], lo, hi, cs["cur_weight"][j], B,
                                          self.cfg.num_iterations, self.cfg.focal_hidden_dim // 8)
 
     def _curiosity_key(self):
@@ -913,37 +913,38 @@ class CognitiveAimModel(nn.Module):
             out.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
         return out
 
-    def _sweep_buffers(self, ws, B: int, S: int, K: int):
-        """Per-call buffers of K guided calls (rows k * B + b; K = 1 for a single call), kept with the (B, S) workspace
-        whose backbone and focal buffers the calls share."""
-        sweeps = ws.setdefault("sweeps", {})
-        sw = sweeps.get(K)
-        if sw is None:
+    def _sweep_buffers(self, ws, B: int, S: int, R: int):
+        """The per-call buffers ("sweep" buffers) of a call with R CuriosityModule runs (rows r * B + b), kept with the
+        (B, S) workspace whose backbone, focal and value-path buffers every call shares.  R guided calls of a sweep (R = 1: a single
+        guided call or a depth field) use every row; an un-guided forward's heads write rows 0..B-1 of depth / conf and
+        its `guided_fallback` softmax uses row 0 of mask_in / heat / argmax.  An un-guided forward of one run and a single
+        guided call share a set: both write it before they read it, on one stream."""
+        cs = ws["sweeps"].get(R)
+        if cs is None:
             dev = self._device()
             N = (S // 14) ** 2
             fl = dict(device=dev, dtype=torch.float32)
-            iters = self.cfg.num_iterations
-            sw = {
-                "mask_in": torch.empty(K, B, N, **fl), "heat": torch.empty(K, B, N, **fl),
-                "argmax": torch.empty(K, B, device=dev, dtype=torch.int32),
-                "pool": torch.empty(K * B, _POOL_SPLITS, _D, **fl),
-                "depth": torch.empty(K, B, **fl), "conf": torch.empty(K, B, **fl),
-                "tmpw": torch.empty(K, 64, _D, **fl), "tmpb": torch.empty(K, 64, **fl),
-                "cur_eps": torch.zeros(K, B, 192, **fl), "cur_noise": torch.zeros(K, B, _D, **fl),
-                "cur_raw": torch.empty(K, B, **fl), "cur_reward": torch.empty(K, B, **fl),
-                "cur_weight": torch.empty(K, iters, B, **fl),
-                # curiosity-guided attention: one focal pass per call, its last-iteration attention kept per call
-                "base": torch.empty(K, B, N, **fl) if self.cfg.curiosity_guided and K > 1 else None,
+            cs = {
+                # the host draws (_stage_runs): a Gaussian pair per run, and the fresh projection of each guided call
+                "cur_eps": torch.zeros(R, B, 192, **fl), "cur_noise": torch.zeros(R, B, _D, **fl),
+                "tmpw": torch.empty(R, 64, _D, **fl), "tmpb": torch.empty(R, 64, **fl),
+                # rewards per run; modulation weights per (run, iteration)
+                "cur_raw": torch.empty(R, B, **fl), "cur_reward": torch.empty(R, B, **fl),
+                "cur_weight": torch.empty(R, self.cfg.num_iterations, B, **fl),
+                # curiosity-guided attention: each run's focal attention, modulated by its own score
+                "base": torch.empty(R, B, N, **fl) if self.cfg.curiosity_guided and R > 1 else None,
+                "mask_in": torch.empty(R, B, N, **fl), "heat": torch.empty(R, B, N, **fl),
+                "argmax": torch.empty(R, B, device=dev, dtype=torch.int32),
+                "tail_pool": torch.empty(R * B, _POOL_SPLITS, _D, **fl),
                 # per-image tickets of ops.guide_tail: zero here, and every launch leaves them at zero
                 "tail_ticket": torch.zeros(B, device=dev, dtype=torch.int32),
+                "depth": torch.empty(R, B, **fl), "conf": torch.empty(R, B, **fl),
             }
-            if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
-                for t in sw.values():
-                    if torch.is_tensor(t) and t.is_floating_point():
-                        t.fill_(float("nan"))
-            sweeps[K] = sw
-        # the single-call buffers (tokens, focal workspace, EXIF, graphs) come from ws; the per-call ones from sw
-        return {**ws, **sw}
+            # a function is handed the workspace and the sweep buffers separately: no name may mean two buffers
+            assert ws.keys().isdisjoint(cs), sorted(ws.keys() & cs.keys())
+            _poison(cs.values())
+            ws["sweeps"][R] = cs
+        return cs
 
     @staticmethod
     def _check_guidances(guidances):
@@ -969,65 +970,46 @@ class CognitiveAimModel(nn.Module):
             masks.append(m.expand(B, N))
         return masks
 
-    def _stage_sweep_call(self, ws, mask, draws, B: int, S: int):
-        """The K calls' random draws (`_sweep_draws`, made before any buffer is looked up) -> pinned staging sized for
-        (B, K) -> the sweep buffers, and the K masks (or None) stacked into sw['mask_in']; returns the buffers."""
-        K = len(draws)
-        sw = self._sweep_buffers(ws, B, S, K)
-        slot = self._pinned_slot()
-        bufs = slot["sweep"].get((B, K))
-        if bufs is None:
-            bufs = slot["sweep"][(B, K)] = tuple(torch.empty(*s).pin_memory() for s in
-                                                 ((K, B, 192), (K, B, _D), (K, 64, _D), (K, 64)))
-        for k, d in enumerate(draws):
-            for buf, t in zip(bufs, d):
-                buf[k].copy_(t)
-        for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb"), bufs):
-            ops.fetch_pinned(sw[dst], buf)  # SM-side reads of the pinned staging area, as in _stage_draws
-        slot["event"].record()
-        if mask is not None:
-            torch.stack(mask, out=sw["mask_in"])
-        return sw
-
-    def _sweep_device(self, sw, B: int, g: int, K: int, base, exif, cam):
-        """Device side of K guided calls after the backbone: the K CuriosityModule runs, the focal pass (`base` [B, N]
-        when it is shared; with curiosity-guided attention one pass per call on sw['tokens']), then the tail: for one call
-        of at most _GUIDE_TAIL_MAX_B images ops.guide_tail (one launch), else the softmax, pool and heads of the K * B
-        rows.  Shared by every guided entry point (`guide_sweep` reads a Scene's tokens)."""
+    def _guided_device(self, ws, cs, tokens, B: int, g: int, K: int, base, exif, cam):
+        """Device side of K guided calls after the backbone, on `tokens` (the workspace's, or a Scene's for `guide_sweep`):
+        the K CuriosityModule runs, the focal pass (`base` [B, N] when it is shared; with curiosity-guided attention one
+        pass per call), then the tail: for one call of at most _GUIDE_TAIL_MAX_B images ops.guide_tail (one launch), else
+        the softmax, pool and heads of the K * B rows.  Shared by every guided entry point."""
         pk = self._packed
         N, T = g * g, g * g + 1
-        self._curiosity_runs(sw, B, T, ("guided",) * K)
+        self._curiosity_runs(cs, tokens, B, T, ("guided",) * K)
         base_k_stride = 0
         if self.cfg.curiosity_guided and K == 1:
-            base = self._focal_iterations(sw, B, g, want_features=False, cur_weight=sw["cur_weight"][0])
+            base = self._focal_iterations(ws, B, g, want_features=False, cur_weight=cs["cur_weight"][0], tokens=tokens)
         elif self.cfg.curiosity_guided:
             # each call's focal attention is modulated by its own curiosity score (src/model.py:264-276)
             for k in range(K):
-                sw["base"][k].copy_(self._focal_iterations(sw, B, g, want_features=False, cur_weight=sw["cur_weight"][k]))
-            base, base_k_stride = sw["base"], B * N
+                cs["base"][k].copy_(self._focal_iterations(ws, B, g, want_features=False, cur_weight=cs["cur_weight"][k],
+                                                           tokens=tokens))
+            base, base_k_stride = cs["base"], B * N
         elif base is None:
-            base = self._focal_iterations(sw, B, g, want_features=False)
+            base = self._focal_iterations(ws, B, g, want_features=False, tokens=tokens)
         heads_in = dict(exif=exif, camera_idx=cam, num_cameras=self.cfg.num_cameras,
                         fault_ptr=self._fault_word().data_ptr())
         if K == 1 and B <= _GUIDE_TAIL_MAX_B:  # one launch (include/cogaim_b200.h CA_GUIDE_TAIL_MAX_B)
-            ops.guide_tail(pk["heads"], base=base, mask=sw["mask_in"][0], heat=sw["heat"][0], argmax=sw["argmax"][0],
-                           ticket=sw["tail_ticket"], tokens=sw["tokens"], depth=sw["depth"][0], conf=sw["conf"][0], B=B,
-                           N=N, pool_partial=sw["pool"], tmp_w=sw["tmpw"][0], tmp_b=sw["tmpb"][0], **heads_in)
+            ops.guide_tail(pk["heads"], base=base, mask=cs["mask_in"][0], heat=cs["heat"][0], argmax=cs["argmax"][0],
+                           ticket=cs["tail_ticket"], tokens=tokens, depth=cs["depth"][0], conf=cs["conf"][0], B=B,
+                           N=N, pool_partial=cs["tail_pool"], tmp_w=cs["tmpw"][0], tmp_b=cs["tmpb"][0], **heads_in)
         else:
-            ops.guided_softmax_sweep(base, base_k_stride, sw["mask_in"], sw["heat"], sw["argmax"], K, B, N)
-            ops.weighted_pool_sweep(sw["tokens"], T * _D, 1, sw["heat"], sw["pool"], K, B, N, _D, _POOL_SPLITS)
-            ops.heads(pk["heads"], tokens=sw["tokens"], tokens_per_img=T, depth=sw["depth"], conf=sw["conf"], B=K * B,
-                      pool_partial=sw["pool"], pool_splits=_POOL_SPLITS, tmp_w=sw["tmpw"], tmp_b=sw["tmpb"],
+            ops.guided_softmax_sweep(base, base_k_stride, cs["mask_in"], cs["heat"], cs["argmax"], K, B, N)
+            ops.weighted_pool_sweep(tokens, T * _D, 1, cs["heat"], cs["tail_pool"], K, B, N, _D, _POOL_SPLITS)
+            ops.heads(pk["heads"], tokens=tokens, tokens_per_img=T, depth=cs["depth"], conf=cs["conf"], B=K * B,
+                      pool_partial=cs["tail_pool"], pool_splits=_POOL_SPLITS, tmp_w=cs["tmpw"], tmp_b=cs["tmpb"],
                       sweep_images=B, **heads_in)
         self._curiosity_join()
 
-    def _sweep_results(self, sw, K: int, return_attention: bool):
-        heat = sw["heat"].clone()
+    def _sweep_results(self, cs, K: int, return_attention: bool):
+        heat = cs["heat"].clone()
         # what the last of the K calls leaves behind
         self._last_attention_weights = heat[K - 1]
-        self._last_argmax = sw["argmax"][K - 1].clone()
-        self._last_curiosity = sw["cur_reward"][K - 1]
-        depth, conf = sw["depth"].clone().unsqueeze(-1), sw["conf"].clone().unsqueeze(-1)
+        self._last_argmax = cs["argmax"][K - 1].clone()
+        self._last_curiosity = cs["cur_reward"][K - 1]
+        depth, conf = cs["depth"].clone().unsqueeze(-1), cs["conf"].clone().unsqueeze(-1)
         return (depth, conf, heat) if return_attention else (depth, conf)
 
     @torch.no_grad()
@@ -1054,7 +1036,9 @@ class CognitiveAimModel(nn.Module):
         exif, cam = self._exif_tensors(exif_data, B)
         draws = self._sweep_draws(B, K)
         ws = self._workspace(B, S)
-        sw = self._stage_sweep_call(ws, mask, draws, B, S)
+        cs = self._sweep_buffers(ws, B, S, K)
+        self._stage_runs(cs, draws)
+        torch.stack(mask, out=cs["mask_in"])
         ws["exif_in"].copy_(exif, non_blocking=True)
         ws["cam_in"].copy_(cam, non_blocking=True)
         self._grid_tables(g)
@@ -1062,11 +1046,11 @@ class CognitiveAimModel(nn.Module):
 
         def device_pass():
             self._backbone_layers(ws, patches, B, S)
-            self._sweep_device(sw, B, g, K, None, ws["exif_in"], ws["cam_in"])
+            self._guided_device(ws, cs, ws["tokens"], B, g, K, None, ws["exif_in"], ws["cam_in"])
 
         self._run(ws, ("sweep", K, self._curiosity_key()), device_pass)
         self._keepalive = (exif, cam, mask, images)
-        return self._sweep_results(sw, K, return_attention)
+        return self._sweep_results(cs, K, return_attention)
 
     # -- scenes: encode a batch once, guide it any number of times ---------------------------------------
     @torch.no_grad()
@@ -1100,10 +1084,7 @@ class CognitiveAimModel(nn.Module):
         self._run(ws, ("encode", patches.data_ptr(), cg), device_pass)
         tokens = torch.empty(B, T, _D, device=dev, dtype=torch.float32)
         base = None if cg else torch.empty(B, N, device=dev, dtype=torch.float32)
-        if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
-            for t in (tokens, base):
-                if t is not None:
-                    t.fill_(float("nan"))
+        _poison((tokens, base))
         tokens.copy_(ws["tokens"])
         if base is not None:
             base.copy_(ws["attn"][self.cfg.num_iterations - 1])
@@ -1124,12 +1105,11 @@ class CognitiveAimModel(nn.Module):
             raise ValueError("stale scene: the model's weights changed after it was encoded (encode the images again)")
 
     def _scene_ws(self, scene):
-        """The (B, S) workspace for a guide call: its scratch buffers, with the scene's tokens in place of the
-        workspace's (nothing is copied)."""
+        """The (B, S) workspace whose scratch buffers a guide call on `scene` uses; the scene's tokens are passed on
+        separately (nothing is copied)."""
         self._pack()
         self._grid_tables(scene.S // 14)
-        ws = self._workspace(scene.B, scene.S)
-        return ws, {**ws, "tokens": scene.tokens}
+        return self._workspace(scene.B, scene.S)
 
     def _run_scene(self, scene, ws, key, fn):
         """Eager at a scene's first guide call; from the second on captured (once, on the scene's own buffers and this
@@ -1168,16 +1148,17 @@ class CognitiveAimModel(nn.Module):
         g = S // 14
         mask = self._sweep_masks(guidances, B, g)
         draws = self._sweep_draws(B, K)
-        ws, _ = self._scene_ws(scene)
-        sw = self._stage_sweep_call(ws, mask, draws, B, S)
-        sw["tokens"] = scene.tokens
+        ws = self._scene_ws(scene)
+        cs = self._sweep_buffers(ws, B, S, K)
+        self._stage_runs(cs, draws)
+        torch.stack(mask, out=cs["mask_in"])
 
         def device_pass():
-            self._sweep_device(sw, B, g, K, scene.base, scene.exif, scene.camera_idx)
+            self._guided_device(ws, cs, scene.tokens, B, g, K, scene.base, scene.exif, scene.camera_idx)
 
         self._run_scene(scene, ws, ("sweep", K), device_pass)
         self._keepalive = (mask,)
-        return self._sweep_results(sw, K, return_attention)
+        return self._sweep_results(cs, K, return_attention)
 
     def _field_buffers(self, ws, B: int, N: int):
         """The depth-field buffers of a (B, S) workspace, added at its first field: the projected tokens [B, N, 64], the
@@ -1186,9 +1167,7 @@ class CognitiveAimModel(nn.Module):
             fl = dict(device=self._device(), dtype=torch.float32)
             ws.update(field_P=torch.empty(B, N, 64, **fl), field_cst=torch.empty(B, 192, **fl),
                       field_depth=torch.empty(B, N, **fl), field_conf=torch.empty(B, N, **fl))
-            if os.environ.get("CA_POISON_WS", "0") not in ("", "0"):
-                for k in ("field_P", "field_cst", "field_depth", "field_conf"):
-                    ws[k].fill_(float("nan"))
+            _poison(ws[k] for k in ("field_P", "field_cst", "field_depth", "field_conf"))
         return ws
 
     @torch.no_grad()
@@ -1211,25 +1190,25 @@ class CognitiveAimModel(nn.Module):
         g = S // 14
         N, T = g * g, g * g + 1
         draws = self._sweep_draws(B, 1)  # :1185, :1421
-        ws, _ = self._scene_ws(scene)
+        ws = self._scene_ws(scene)
         self._field_buffers(ws, B, N)
-        sw = self._stage_sweep_call(ws, None, draws, B, S)
-        sw["tokens"] = scene.tokens
+        cs = self._sweep_buffers(ws, B, S, 1)
+        self._stage_runs(cs, draws)
         cg = self.cfg.curiosity_guided
 
         def device_pass():
-            self._curiosity_runs(sw, B, T, ("guided",))
-            base = (self._focal_iterations(sw, B, g, want_features=False, cur_weight=sw["cur_weight"][0]) if cg
-                    else scene.base)
-            ops.token_project(scene.tokens, T * _D, 1, sw["tmpw"][0], ws["field_P"], B, N)
+            self._curiosity_runs(cs, scene.tokens, B, T, ("guided",))
+            base = (self._focal_iterations(ws, B, g, want_features=False, cur_weight=cs["cur_weight"][0],
+                                           tokens=scene.tokens) if cg else scene.base)
+            ops.token_project(scene.tokens, T * _D, 1, cs["tmpw"][0], ws["field_P"], B, N)
             ops.depth_field_cells(pk["heads"], base=base, P=ws["field_P"], cst=ws["field_cst"], depth=ws["field_depth"],
-                                  conf=ws["field_conf"], tokens=scene.tokens, tmp_b=sw["tmpb"][0], B=B, g=g,
+                                  conf=ws["field_conf"], tokens=scene.tokens, tmp_b=cs["tmpb"][0], B=B, g=g,
                                   exif=scene.exif, camera_idx=scene.camera_idx, num_cameras=self.cfg.num_cameras,
                                   fault_ptr=self._fault_word().data_ptr())
             self._curiosity_join()
 
         self._run_scene(scene, ws, ("field",), device_pass)
-        self._last_curiosity = sw["cur_reward"][0]
+        self._last_curiosity = cs["cur_reward"][0]
         return ws["field_depth"].clone().view(B, g, g), ws["field_conf"].clone().view(B, g, g)
 
     @torch.no_grad()
@@ -1272,15 +1251,14 @@ class CognitiveAimModel(nn.Module):
                 mask = self._mask(guidance, g)
                 nn.Linear(_D, 64)  # :1421 is reached (and draws) before the 128-wide concat fails in `fusion`
         ws = self._workspace(B, S)
-        slot = self._pinned_slot()
-        self._stage_draws(ws, slot, draws)
-        slot["event"].record()
+        cs = self._sweep_buffers(ws, B, S, len(roles))
+        self._stage_runs(cs, draws)
         has_exif = exif is not None
         if has_exif:
             ws["exif_in"].copy_(exif, non_blocking=True)
             ws["cam_in"].copy_(cam, non_blocking=True)
         if mask is not None:
-            ws["mask_in"].copy_(mask, non_blocking=True)
+            cs["mask_in"][0].copy_(mask, non_blocking=True)
         self._grid_tables(g)
         patches, images = self._patch_rows(images, ws, S)
         cg = self.cfg.curiosity_guided
@@ -1288,18 +1266,19 @@ class CognitiveAimModel(nn.Module):
 
         def device_pass():
             self._backbone_layers(ws, patches, B, S)
-            self._curiosity_runs(ws, B, T, roles)
+            tokens = ws["tokens"]
+            self._curiosity_runs(cs, tokens, B, T, roles)
             if cg:
                 # the attention-only calls of the reference see their own run's (clamped) score: separate passes
                 for j, role in enumerate(roles):
                     if role != "features":
-                        att_j = self._focal_iterations(ws, B, g, want_features=False, cur_weight=ws["cur_weight"][j])
-                        ws["att_run"][j].copy_(att_j)
-            att_f = self._focal_iterations(ws, B, g, want_features=True, cur_weight=ws["cur_weight"][jf] if cg else None)
+                        att_j = self._focal_iterations(ws, B, g, want_features=False, cur_weight=cs["cur_weight"][j])
+                        cs["base"][j].copy_(att_j)
+            att_f = self._focal_iterations(ws, B, g, want_features=True, cur_weight=cs["cur_weight"][jf] if cg else None)
             if mask is not None:
-                base = ws["att_run"][roles.index("guided")] if cg else att_f
-                ops.guided_softmax(base, ws["mask_in"], ws["heat"], ws["argmax"], B, N)
-            ops.heads(pk["heads"], tokens=ws["tokens"], tokens_per_img=T, depth=ws["depth"], conf=ws["conf"], B=B,
+                base = cs["base"][roles.index("guided")] if cg else att_f
+                ops.guided_softmax(base, cs["mask_in"][0], cs["heat"][0], cs["argmax"][0], B, N)
+            ops.heads(pk["heads"], tokens=tokens, tokens_per_img=T, depth=cs["depth"][0], conf=cs["conf"][0], B=B,
                       focal_feat=ws["focal_feat"], exif=ws["exif_in"] if has_exif else None,
                       camera_idx=ws["cam_in"] if has_exif else None, fused_out=ws["fused"],
                       num_cameras=self.cfg.num_cameras, fault_ptr=self._fault_word().data_ptr())
@@ -1310,18 +1289,18 @@ class CognitiveAimModel(nn.Module):
         att_feat = ws["attn"][self.cfg.num_iterations - 1]
 
         def att_of(role):
-            return (ws["att_run"][roles.index(role)] if cg and role != "features" else att_feat).clone()
+            return (cs["base"][roles.index(role)] if cg and role != "features" else att_feat).clone()
 
         self.fusion_features = ws["fused"].clone()  # :1089
-        self._last_curiosity = ws["cur_reward"][jf]
+        self._last_curiosity = cs["cur_reward"][jf]
         if mode == "forward":
             if not has_last:  # :1093-1113 only set when absent
                 self._last_attention_weights = att_of("last")
         elif mode == "guided_none":
             self._last_attention_weights = att_of("features")  # :1212 always stores
         elif mode == "guided_fallback":
-            self._last_attention_weights = ws["heat"].clone() if mask is not None else att_of("guided")  # :1212
-        depth, conf = ws["depth"].clone().unsqueeze(1), ws["conf"].clone().unsqueeze(1)
+            self._last_attention_weights = cs["heat"][0].clone() if mask is not None else att_of("guided")  # :1212
+        depth, conf = cs["depth"][0].clone().unsqueeze(1), cs["conf"][0].clone().unsqueeze(1)
         if not return_attention:
             return depth, conf
         return depth, conf, att_of("ret" if "ret" in roles else "features")

@@ -189,18 +189,19 @@ class NativeModel:
         return c, held, B, S
 
     @staticmethod
-    def _draws(c, B: int, K: int, held):
-        """The HOST draws of K guided calls, in the reference's order per call: the CuriosityModule's randn(B, 192),
-        randn(B, 768) (:609, :744), then nn.Linear(768, 64) (:1421: same constructor => same generator draws); stacked
-        over the calls and set in the call struct `c`."""
+    def _draws(c, B: int, R: int, held, projections: bool = True):
+        """The HOST draws of R CuriosityModule runs, in the reference's order per run: randn(B, 192), randn(B, 768)
+        (:609, :744), then for a guided call nn.Linear(768, 64) (:1421: same constructor => same generator draws);
+        stacked over the runs and set in the call struct `c`."""
         draws = []
-        for _ in range(K):
+        for _ in range(R):
             eps, noise = torch.randn(B, 192), torch.randn(B, _D)
-            tmp = nn.Linear(_D, 64)
-            draws.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
-        eps, noise, tw, tb = (torch.stack([d[i] for d in draws]).contiguous() for i in range(4))
-        held += [eps, noise, tw, tb]
-        c.tmp_w, c.tmp_b, c.eps, c.noise = tw.data_ptr(), tb.data_ptr(), eps.data_ptr(), noise.data_ptr()
+            tmp = nn.Linear(_D, 64) if projections else None
+            draws.append((eps, noise) + ((tmp.weight.detach(), tmp.bias.detach()) if projections else ()))
+        stacked = [torch.stack(t).contiguous() for t in zip(*draws)]
+        held += stacked
+        for field, t in zip(("eps", "noise", "tmp_w", "tmp_b"), stacked):
+            setattr(c, field, t.data_ptr())
 
     def _outputs(self, c, K: int, B: int, N: int):
         """The outputs of K guided calls — depth, confidence [K, B], heat maps [K, B, N], arg-max cells [K, B] — with
@@ -277,10 +278,8 @@ class NativeModel:
         `runs`: how often the reference would run its CuriosityModule in this call (1..3, :992, :1104, :1138)."""
         c, held, B, S = self._call(images, exif, S)
         N = (S // 14) ** 2
-        draws = [(torch.randn(B, 192), torch.randn(B, _D)) for _ in range(runs)]
-        eps = torch.stack([d[0] for d in draws]).contiguous()
-        noise = torch.stack([d[1] for d in draws]).contiguous()
-        c.eps, c.noise, c.curiosity_runs = eps.data_ptr(), noise.data_ptr(), runs
+        self._draws(c, B, runs, held, projections=False)
+        c.curiosity_runs = runs
         out = {"depth": torch.empty(B, device=self.device), "conf": torch.empty(B, device=self.device),
                "att": torch.empty(B, N, device=self.device), "fused": torch.empty(B, 192, device=self.device)}
         c.depth, c.conf, c.attention, c.fused = (out[k].data_ptr() for k in ("depth", "conf", "att", "fused"))
