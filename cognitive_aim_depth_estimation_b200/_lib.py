@@ -36,7 +36,7 @@ class HeadsInputs(C.Structure):
     _fields_ = [("tokens", C.c_void_p), ("tokens_per_img", C.c_int), ("focal_feat", C.c_void_p),
                 ("pool_partial", C.c_void_p), ("pool_splits", C.c_int), ("tmp_w", C.c_void_p), ("tmp_b", C.c_void_p),
                 ("pooled_out", C.c_void_p), ("exif", C.c_void_p), ("camera_idx", C.c_void_p),
-                ("num_cameras", C.c_int), ("fault", C.c_void_p), ("sweep_images", C.c_int)]
+                ("num_cameras", C.c_int), ("fault", C.c_void_p), ("sweep_images", C.c_int), ("call_of_row", C.c_void_p)]
 
 
 class FocalValueArgs(C.Structure):
@@ -94,6 +94,9 @@ class ForwardCall(C.Structure):
 
 SWEEP_MAX_K = 16  # CA_SWEEP_MAX_K (include/cogaim_b200.h)
 GUIDE_TAIL_MAX_B = 1  # CA_GUIDE_TAIL_MAX_B: single guided calls of larger batches (and sweeps) run the three-kernel chain
+GUIDE_MANY_MAX_CALLS = 64  # CA_GUIDE_MANY_MAX_CALLS: guide calls per guide_many
+GUIDE_MANY_MAX_ROWS = 256  # CA_GUIDE_MANY_MAX_ROWS: images of all calls of one guide_many
+GUIDE_MANY_ROW_WORDS = 6  # ca_guide_many_row: five device pointers and the call index, 8 bytes each
 RESIZE_MAX_SIDE = 16384  # CA_RESIZE_MAX_SIDE
 RESIZE_LIST_CHUNK = 128  # CA_RESIZE_LIST_CHUNK
 
@@ -110,6 +113,14 @@ class GuideCall(C.Structure):
     _fields_ = [("instruction", C.c_char_p), ("mask", C.c_void_p), ("mask_batch_stride", C.c_longlong),
                 ("tmp_w", C.c_void_p), ("tmp_b", C.c_void_p), ("eps", C.c_void_p), ("noise", C.c_void_p),
                 ("depth", C.c_void_p), ("conf", C.c_void_p), ("attention", C.c_void_p), ("argmax", C.c_void_p)]
+
+
+class GuideManyCall(C.Structure):
+    """ca_guide_many_call (include/cogaim_b200.h)."""
+    _fields_ = [("m", C.c_int), ("scenes", C.POINTER(C.c_void_p)), ("instructions", C.POINTER(C.c_char_p)),
+                ("masks", C.c_void_p), ("tmp_w", C.c_void_p), ("tmp_b", C.c_void_p), ("eps", C.c_void_p),
+                ("noise", C.c_void_p), ("depth", C.c_void_p), ("conf", C.c_void_p), ("attention", C.c_void_p),
+                ("argmax", C.c_void_p), ("use_graph", C.c_int)]
 
 
 class DepthFieldCall(C.Structure):
@@ -160,6 +171,8 @@ _SIGNATURES = {
                                 C.c_int, C.c_float, C.c_float, c_ptr],
     "ca_weighted_pool_sweep": [c_ptr, C.c_longlong, C.c_int, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                c_ptr],
+    "ca_gather_rows": [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr],
+    "ca_weighted_pool_rows": [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr],
     "ca_heads": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, c_ptr, C.c_int, c_ptr],
     "ca_guide_tail": [C.POINTER(HeadsWeights), C.POINTER(HeadsInputs), c_ptr, c_ptr, C.c_longlong, c_ptr, c_ptr, c_ptr,
                       c_ptr, c_ptr, C.c_int, C.c_int, C.c_float, C.c_float, c_ptr],
@@ -180,6 +193,7 @@ _SIGNATURES = {
     "ca_guide": [c_ptr, c_ptr, C.POINTER(GuideCall), c_ptr],
     "ca_guide_sweep": [c_ptr, c_ptr, C.POINTER(SweepCall), c_ptr],
     "ca_depth_field": [c_ptr, c_ptr, C.POINTER(DepthFieldCall), c_ptr],
+    "ca_guide_many": [c_ptr, C.POINTER(GuideManyCall), c_ptr],
     "ca_scene_destroy": [c_ptr],
 }
 

@@ -201,6 +201,17 @@ int ca_weighted_pool_sweep(const float* src, long long src_batch_stride, int row
                                   static_cast<cudaStream_t>(stream));
 }
 
+int ca_gather_rows(const ca_guide_many_row* rows, int R, int N, int num_cameras, float* cls, float* base, float* exif,
+                   long long* camera_idx, int32_t* call_of_row, void* stream) {
+  return ca::gather_rows_launch(rows, R, N, num_cameras, cls, base, exif, camera_idx, call_of_row,
+                                static_cast<cudaStream_t>(stream));
+}
+
+int ca_weighted_pool_rows(const ca_guide_many_row* rows, const float* w, float* partial, int R, int N, int D, int splits,
+                          void* stream) {
+  return ca::weighted_pool_rows_launch(rows, w, partial, R, N, D, splits, static_cast<cudaStream_t>(stream));
+}
+
 int ca_heads(const ca_heads_weights* w, const ca_heads_inputs* in, float* depth, float* conf, float* fused_out, int B,
              void* stream) {
   if (!w || !in) return ca::invalid("heads: null argument struct");

@@ -276,18 +276,22 @@ __global__ void __launch_bounds__(256) guided_softmax_kernel(const float* __rest
 // in the tail, same fmaf chain — so partial row k * B + b is bit for bit the KMAX = 1 result for weight vector k alone.
 // KMAX accumulators live in registers (16 x 4 at the largest instantiation, no spills).  w2 (the focal value path's second
 // factor) is read by the KMAX = 1 instantiation only, whose loads and FMAs are those of a plain one-vector pool.
-template <int KMAX>
+// ROWS (KMAX = 1 only): row b's tokens start at rows[b].tokens instead of src + b * src_batch_stride (rows of several
+// scenes, ca_guide_many); everything after that pointer is the one-vector pool.
+template <int KMAX, bool ROWS = false>
 __global__ void __launch_bounds__(192) weighted_pool_kernel(const float* __restrict__ src, long long src_batch_stride,
                                                              int row_offset, const float* __restrict__ w,
                                                              const float* __restrict__ w2, float* __restrict__ partial,
-                                                             int K, int B, int N, int D, int rows_per_split) {
+                                                             int K, int B, int N, int D, int rows_per_split,
+                                                             const ca_guide_many_row* __restrict__ rows) {
+  static_assert(!ROWS || KMAX == 1, "the row-table pool pools one weight vector per row");
   griddep_sync();  // PDL: nothing before this line reads or writes global memory
   const int b = blockIdx.y;
   const int split = blockIdx.x;
   const int n0 = split * rows_per_split;
   const int n1 = min(N, n0 + rows_per_split);
-  const float4* s4 = reinterpret_cast<const float4*>(src + static_cast<size_t>(b) * src_batch_stride +
-                                                     static_cast<size_t>(row_offset) * D);
+  const float* img = ROWS ? rows[b].tokens : src + static_cast<size_t>(b) * src_batch_stride;
+  const float4* s4 = reinterpret_cast<const float4*>(img + static_cast<size_t>(row_offset) * D);
   const float* wb = w + static_cast<size_t>(b) * N;
   const float* w2b = w2 ? w2 + static_cast<size_t>(b) * N : nullptr;
   const size_t w_k_stride = static_cast<size_t>(B) * N;
@@ -327,6 +331,34 @@ __global__ void __launch_bounds__(192) weighted_pool_kernel(const float* __restr
   for (int k = 0; k < KMAX; ++k)
     if (KMAX == 1 || k < K)
       reinterpret_cast<float4*>(partial + ((static_cast<size_t>(k) * B + b) * gridDim.x + split) * D)[threadIdx.x] = acc[k];
+}
+
+// The per-row inputs of the rows of several scenes, gathered through the row table into the call's buffers (one CTA per
+// row): the CLS token, the focal attention row, the EXIF and camera index, and the call index.  About 3 KB + 4 N bytes
+// per row; the patch tokens stay where they are.
+constexpr int kGatherThreads = 256;
+__global__ void __launch_bounds__(kGatherThreads) gather_rows_kernel(const ca_guide_many_row* __restrict__ rows, int N,
+                                                                     int num_cameras, float* __restrict__ cls,
+                                                                     float* __restrict__ base,
+                                                                     float* __restrict__ exif,
+                                                                     long long* __restrict__ camera_idx,
+                                                                     int* __restrict__ call_of_row) {
+  griddep_sync();  // PDL: nothing before this line reads or writes global memory
+  const int r = blockIdx.x, tid = threadIdx.x;
+  const ca_guide_many_row row = rows[r];
+  const float4* c4 = reinterpret_cast<const float4*>(row.tokens);
+  float4* o4 = reinterpret_cast<float4*>(cls + static_cast<size_t>(r) * 768);
+  if (tid < 192) o4[tid] = c4[tid];
+  float* ob = base + static_cast<size_t>(r) * N;
+  for (int j = tid; j < N; j += kGatherThreads) ob[j] = row.base[j];
+  if (tid < 3) exif[static_cast<size_t>(r) * 3 + tid] = row.exif[tid];
+  if (tid == 0) {
+    const long long cam = *row.camera_idx;
+    camera_idx[r] = cam;
+    call_of_row[r] = static_cast<int>(row.call);
+    // reported in the row's own fault word (the scenes of one call may report to different words); the heads clamp it
+    if (num_cameras > 0 && (cam < 0 || cam >= num_cameras) && row.fault) atomicOr(row.fault, 1);
+  }
 }
 
 // The guided tail of one call in one launch: guided_softmax -> weighted_pool -> heads, bit for bit.
@@ -521,16 +553,39 @@ int weighted_pool_launch(const float* src, long long src_batch_stride, int row_o
   // the smallest instantiation that holds K accumulators: registers (and so occupancy) follow K
   if (K == 1)
     CA_TRY(launch_kernel(weighted_pool_kernel<1>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w, w2,
-                         partial, K, B, N, D, rps));
+                         partial, K, B, N, D, rps, nullptr));
   else if (K <= 4)
     CA_TRY(launch_kernel(weighted_pool_kernel<4>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w, w2,
-                         partial, K, B, N, D, rps));
+                         partial, K, B, N, D, rps, nullptr));
   else if (K <= 8)
     CA_TRY(launch_kernel(weighted_pool_kernel<8>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset, w, w2,
-                         partial, K, B, N, D, rps));
+                         partial, K, B, N, D, rps, nullptr));
   else
     CA_TRY(launch_kernel(weighted_pool_kernel<kSweepMaxK>, grid, dim3(192), 0, stream, src, src_batch_stride, row_offset,
-                         w, w2, partial, K, B, N, D, rps));
+                         w, w2, partial, K, B, N, D, rps, nullptr));
+  CA_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int weighted_pool_rows_launch(const ca_guide_many_row* rows, const float* w, float* partial, int R, int N, int D,
+                              int splits, cudaStream_t stream) {
+  CA_REQUIRE(rows && w && partial, "weighted_pool_rows: null pointer");
+  CA_REQUIRE(D == 768, "weighted_pool_rows: only D = 768 is instantiated");
+  CA_REQUIRE(splits > 0 && R > 0 && N > 0, "weighted_pool_rows: splits, R and N must be positive");
+  const int rps = (N + splits - 1) / splits;  // as weighted_pool_launch: the same rows per split, so the same bits
+  CA_TRY(launch_kernel(weighted_pool_kernel<1, true>, dim3(splits, R), dim3(192), 0, stream, nullptr, 0LL, 1, w, nullptr,
+                       partial, 1, R, N, D, rps, rows));
+  CA_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int gather_rows_launch(const ca_guide_many_row* rows, int R, int N, int num_cameras, float* cls, float* base,
+                       float* exif, long long* camera_idx, int* call_of_row, cudaStream_t stream) {
+  CA_REQUIRE(rows && cls && base && exif && camera_idx && call_of_row, "gather_rows: null pointer");
+  CA_REQUIRE(R > 0 && N > 0, "gather_rows: R and N must be positive");
+  CA_REQUIRE((reinterpret_cast<uintptr_t>(cls) & 15) == 0, "gather_rows: cls must be 16-byte aligned");
+  CA_TRY(launch_kernel(gather_rows_kernel, dim3(R), dim3(kGatherThreads), 0, stream, rows, N, num_cameras, cls, base, exif, camera_idx,
+                       call_of_row));
   CA_CUDA(cudaGetLastError());
   return 0;
 }
@@ -539,7 +594,8 @@ int guide_tail_launch(const HeadsWeights& w, const HeadsInputs& in, const float*
                       long long mask_batch_stride, float* heat, int* argmax, unsigned int* ticket, float* depth,
                       float* conf, int B, int N, float alpha, float temperature, cudaStream_t stream) {
   CA_REQUIRE(base && mask && heat && ticket && depth && conf && in.tokens, "guide_tail: null pointer");
-  CA_REQUIRE(in.focal_feat == nullptr && in.sweep_images == 0, "guide_tail: guided single calls only (no focal_feat, no sweep)");
+  CA_REQUIRE(in.focal_feat == nullptr && in.sweep_images == 0 && in.call_of_row == nullptr,
+             "guide_tail: guided single calls only (no focal_feat, no sweep, no call_of_row)");
   CA_REQUIRE(in.pool_partial && in.tmp_w && in.tmp_b && in.pool_splits > 0, "guide_tail: pool partials and projection needed");
   CA_REQUIRE(in.exif == nullptr || in.camera_idx != nullptr, "guide_tail: EXIF given without camera_idx");
   CA_REQUIRE(B > 0 && N > 0 && N <= kTailMaxN, "guide_tail: B > 0 and 0 < N <= 8192");

@@ -22,6 +22,11 @@ int guided_softmax_launch(const float* base, long long base_k_stride, const floa
 // w: [K, B, N], partial: [K * B, splits, D]; w2 ([B, N], optional) with K = 1 only
 int weighted_pool_launch(const float* src, long long src_batch_stride, int row_offset, const float* w, const float* w2,
                          float* partial, int K, int B, int N, int D, int splits, cudaStream_t stream);
+// rows of several scenes (ca_guide_many): the pool of row r reads rows[r].tokens; gather_rows copies the per-row inputs
+int weighted_pool_rows_launch(const ca_guide_many_row* rows, const float* w, float* partial, int R, int N, int D,
+                              int splits, cudaStream_t stream);
+int gather_rows_launch(const ca_guide_many_row* rows, int R, int N, int num_cameras, float* cls, float* base,
+                       float* exif, long long* camera_idx, int* call_of_row, cudaStream_t stream);
 // guided_softmax -> weighted_pool (in.pool_splits splits) -> heads in one launch, bit for bit; ticket: [B] zero-initialised
 // counters, left at zero by every launch.
 int guide_tail_launch(const HeadsWeights& w, const HeadsInputs& in, const float* base, const float* mask,

@@ -73,6 +73,8 @@ int heads_launch(const HeadsWeights& w, const HeadsInputs& in, float* depth, flo
   CA_REQUIRE(in.exif == nullptr || in.camera_idx != nullptr, "heads: EXIF given without camera_idx");
   CA_REQUIRE(in.sweep_images >= 0 && (in.sweep_images == 0 || (in.focal_feat == nullptr && B % in.sweep_images == 0)),
              "heads: an instruction sweep is guided only and needs B = K * sweep_images rows");
+  CA_REQUIRE(in.call_of_row == nullptr || (in.focal_feat == nullptr && in.sweep_images == 0),
+             "heads: call_of_row is guided only and excludes sweep_images");
   CA_TRY(launch_kernel(heads_kernel, dim3(B), dim3(kHeadsThreads), 0, stream, w, in, depth, conf, fused_out));
   CA_CUDA(cudaGetLastError());
   return 0;

@@ -12,7 +12,8 @@
 namespace ca {
 namespace {
 
-// r: output row; b = r % nb: image; k = r / nb: instruction of a sweep (0 otherwise).
+// r: output row; b = r % nb: image; k = r / nb: instruction of a sweep (0 otherwise), or in.call_of_row[r] (the rows of
+// several guide calls).
 __device__ __forceinline__ void heads_row(const HeadsWeights& wt, const HeadsInputs& in, float* __restrict__ depth,
                                           float* __restrict__ conf, float* __restrict__ fused_out, int r, int nb) {
   __shared__ __align__(16) float s_in[768];
@@ -21,7 +22,6 @@ __device__ __forceinline__ void heads_row(const HeadsWeights& wt, const HeadsInp
   __shared__ __align__(16) float s_cat[192];
   __shared__ __align__(16) float s_f[192];
   const int b = r % nb;
-  const size_t k = r / nb;
   const int tid = threadIdx.x;
 
   // ---- ambient stream on the CLS token ----
@@ -46,6 +46,7 @@ __device__ __forceinline__ void heads_row(const HeadsWeights& wt, const HeadsInp
       if (in.pooled_out) in.pooled_out[static_cast<size_t>(r) * 768 + i] = acc;
     }
     __syncthreads();
+    const size_t k = in.call_of_row ? static_cast<size_t>(in.call_of_row[r]) : static_cast<size_t>(r / nb);
     dense(in.tmp_w + k * 64 * 768, in.tmp_b + k * 64, s_in, s_cat + 64, 768, 64, false);
   }
 

@@ -83,6 +83,18 @@ void free_workspace(Workspace& w) {
   cudaFree(w.arena);
 }
 
+// The buffers of ca_guide_many at one side S, sized at the caps (CA_GUIDE_MANY_MAX_ROWS rows, CA_GUIDE_MANY_MAX_CALLS
+// calls): a call of R rows and m calls uses the first R / m of each.  Graphs per (R, m).
+struct ManyBufs {
+  void* arena = nullptr;
+  ca_guide_many_row* rows;
+  float *cls, *base, *exif, *eps, *noise, *raw, *reward, *tmpw, *tmpb, *mask_in, *heat, *pool, *depth, *conf;
+  long long* cam;
+  int *call, *argmax;
+  std::map<int, std::pair<cudaGraphExec_t, int>> graphs;
+  std::map<int, int> seen;
+};
+
 struct PinnedSlot {
   float* buf = nullptr;
   size_t cap = 0;
@@ -108,6 +120,7 @@ struct ca_handle {
   uint8_t* resize_buf = nullptr;
   size_t resize_cap = 0;
   unsigned long long id = 0;  // unique per handle: scenes record it (a later handle may reuse the address)
+  std::map<int, ManyBufs> many;  // ca_guide_many buffers per side S
 };
 
 // A scene (ca_encode): buffers it owns in one device allocation, the handle it belongs to (by id, never dereferenced
@@ -272,6 +285,16 @@ int get_tables(ca_handle* h, int g, Tables** out) {
   }
   *out = &it->second;
   return 0;
+}
+
+// one of the nine instructions or an alias, in any case (ca_guide_many refuses other strings)
+bool known_instruction(const char* instruction) {
+  std::string s(instruction);
+  for (auto& ch : s) ch = static_cast<char>(tolower(ch));
+  for (const char* k : {"center", "left", "right", "top", "bottom", "top-left", "top-right", "bottom-left", "bottom-right",
+                        "topleft", "topright", "bottomleft", "bottomright"})
+    if (s == k) return true;
+  return false;
 }
 
 int get_mask(Tables* t, const char* instruction, int g, float** out) {
@@ -914,6 +937,45 @@ GuidedCall sweep_call(const ca_sweep_call& sw) {
           sw.argmax};
 }
 
+int get_many(ca_handle* h, int S, ManyBufs** out) {
+  auto it = h->many.find(S);
+  if (it == h->many.end()) {
+    if (h->many.size() >= 4) {  // keep the cache bounded: drop the oldest side
+      auto old = h->many.begin();
+      CA_CUDA(cudaDeviceSynchronize());
+      for (auto& g : old->second.graphs) cudaGraphExecDestroy(g.second.first);
+      cudaFree(old->second.arena);
+      h->many.erase(old);
+    }
+    const int g = S / 14;
+    const size_t N = static_cast<size_t>(g) * g, R = CA_GUIDE_MANY_MAX_ROWS, m = CA_GUIDE_MANY_MAX_CALLS;
+    ManyBufs b;
+    Layout l;
+    l.add(&b.rows, R * sizeof(ca_guide_many_row));
+    l.add(&b.cls, R * kD * 4);
+    l.add(&b.base, R * N * 4);
+    l.add(&b.exif, R * 3 * 4);
+    l.add(&b.cam, R * 8);
+    l.add(&b.call, R * 4);
+    l.add(&b.eps, R * 192 * 4);
+    l.add(&b.noise, R * kD * 4);
+    l.add(&b.raw, R * 4);
+    l.add(&b.reward, R * 4);
+    l.add(&b.tmpw, m * 64 * kD * 4);
+    l.add(&b.tmpb, m * 64 * 4);
+    l.add(&b.mask_in, R * N * 4);
+    l.add(&b.heat, R * N * 4);
+    l.add(&b.argmax, R * 4);
+    l.add(&b.pool, R * kPoolSplits * kD * 4);
+    l.add(&b.depth, R * 4);
+    l.add(&b.conf, R * 4);
+    CA_TRY(l.alloc(&b.arena));
+    it = h->many.emplace(S, b).first;
+  }
+  *out = &it->second;
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -968,6 +1030,10 @@ int ca_destroy(ca_handle* h) {
     if (s.done) cudaEventDestroy(s.done);
   }
   if (h->resize_buf) cudaFree(h->resize_buf);
+  for (auto& kv : h->many) {
+    for (auto& g : kv.second.graphs) cudaGraphExecDestroy(g.second.first);
+    cudaFree(kv.second.arena);
+  }
   cudaStreamDestroy(h->side);
   cudaEventDestroy(h->fork);
   cudaEventDestroy(h->join);
@@ -1157,6 +1223,109 @@ int ca_guide_sweep(ca_handle* h, ca_scene* sc, const ca_sweep_call* sw, void* st
   CA_REQUIRE(sw, "guide_sweep: null sweep");
   CA_TRY(check_sweep(sw, "guide_sweep"));
   return run_guided(h, nullptr, sc, sweep_call(*sw), static_cast<cudaStream_t>(stream));
+}
+
+int ca_guide_many(ca_handle* h, const ca_guide_many_call* c, void* stream) {
+  CA_REQUIRE(h && c, "guide_many: null handle / call");
+  const int m = c->m;
+  CA_REQUIRE(m >= 1 && m <= CA_GUIDE_MANY_MAX_CALLS, "guide_many: m must be in 1..CA_GUIDE_MANY_MAX_CALLS (64)");
+  CA_REQUIRE(c->scenes, "guide_many: null scene array");
+  // every scene is checked before anything is enqueued
+  int R = 0;
+  for (int j = 0; j < m; ++j) {
+    CA_TRY(check_scene(h, c->scenes[j]));
+    CA_REQUIRE(c->scenes[j]->S == c->scenes[0]->S, "guide_many: the scenes must share the image side S");
+    R += c->scenes[j]->B;
+  }
+  CA_REQUIRE(R <= CA_GUIDE_MANY_MAX_ROWS, "guide_many: more than CA_GUIDE_MANY_MAX_ROWS (256) images in all");
+  CA_REQUIRE((c->instructions != nullptr) != (c->masks != nullptr), "guide_many: give instructions OR masks");
+  CA_REQUIRE(c->tmp_w && c->tmp_b && c->eps && c->noise,
+             "guide_many: null per-call projections or CuriosityModule draws (HOST pointers, src/model.py:609,744,1421)");
+  CA_REQUIRE(c->depth && c->conf && c->attention, "guide_many: null output");
+  DeviceGuard guard(h->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int S = c->scenes[0]->S, g = S / 14, N = g * g;
+  Tables* tb = nullptr;
+  CA_TRY(get_tables(h, g, &tb));
+  std::vector<float*> masks;
+  if (c->instructions)
+    for (int j = 0; j < m; ++j) {
+      CA_REQUIRE(c->instructions[j], "guide_many: null instruction string");
+      CA_REQUIRE(known_instruction(c->instructions[j]), "guide_many: unknown instruction");
+      float* mk = nullptr;
+      CA_TRY(get_mask(tb, c->instructions[j], g, &mk));
+      masks.push_back(mk);
+    }
+  ManyBufs* bp = nullptr;
+  CA_TRY(get_many(h, S, &bp));
+  ManyBufs& b = *bp;
+  h->launches = 0;
+  if (c->instructions) {
+    int r = 0;
+    for (int j = 0; j < m; ++j)
+      for (int i = 0; i < c->scenes[j]->B; ++i, ++r)
+        CA_CUDA(cudaMemcpyAsync(b.mask_in + static_cast<size_t>(r) * N, masks[j], static_cast<size_t>(N) * 4,
+                                cudaMemcpyDeviceToDevice, st));
+  } else {
+    CA_CUDA(cudaMemcpyAsync(b.mask_in, c->masks, static_cast<size_t>(R) * N * 4, cudaMemcpyDeviceToDevice, st));
+  }
+  // the row table, staged with the draws through one pinned slot
+  std::vector<ca_guide_many_row> table;
+  table.reserve(R);
+  const size_t T = static_cast<size_t>(N) + 1;
+  for (int j = 0; j < m; ++j) {
+    const ca_scene* sc = c->scenes[j];
+    for (int i = 0; i < sc->B; ++i)
+      table.push_back({sc->tokens + i * T * kD, sc->base + static_cast<size_t>(i) * N, sc->exif + i * 3, sc->cam + i,
+                       sc->fault, j});
+  }
+  const size_t words = table.size() * sizeof(ca_guide_many_row) / 4;
+  const struct { float* dst; const float* src; size_t n; } parts[] = {
+      {b.tmpw, c->tmp_w, static_cast<size_t>(m) * 64 * kD}, {b.tmpb, c->tmp_b, static_cast<size_t>(m) * 64},
+      {b.eps, c->eps, static_cast<size_t>(R) * 192}, {b.noise, c->noise, static_cast<size_t>(R) * kD},
+      {reinterpret_cast<float*>(b.rows), reinterpret_cast<const float*>(table.data()), words}};
+  size_t need = 0;
+  for (const auto& q : parts) need += q.n;
+  PinnedSlot* slot = nullptr;
+  CA_TRY(pinned_slot(h, need, &slot));
+  float* p = slot->buf;
+  for (const auto& q : parts) {
+    memcpy(p, q.src, q.n * sizeof(float));
+    CA_TRY(ca::fetch_pinned_launch(q.dst, p, q.n, st));
+    ++h->launches;
+    p += q.n;
+  }
+  CA_CUDA(cudaEventRecord(slot->done, st));
+  auto seq = [&]() -> int {
+    LAUNCH(ca::gather_rows_launch(b.rows, R, N, h->w.num_cameras, b.cls, b.base, b.exif, b.cam, b.call, st));
+    CA_CUDA(cudaEventRecord(h->fork, st));
+    CA_CUDA(cudaStreamWaitEvent(h->side, h->fork, 0));
+    CA_TRY(ca::curiosity_launch(h->w.curiosity, b.cls, 1, b.eps, b.noise, b.raw, b.reward, h->w.exploration_history,
+                                h->w.history_len, h->w.history_pointer, R, h->side));
+    h->launches += h->w.exploration_history ? 2 : 1;
+    LAUNCH(ca::guided_softmax_launch(b.base, 0, b.mask_in, 0, N, b.heat, b.argmax, 1, R, N, 0.7f, 0.05f, st));
+    LAUNCH(ca::weighted_pool_rows_launch(b.rows, b.heat, b.pool, R, N, kD, kPoolSplits, st));
+    ca_heads_inputs in{};
+    in.tokens = b.cls;
+    in.tokens_per_img = 1;
+    in.pool_partial = b.pool;
+    in.pool_splits = kPoolSplits;
+    in.tmp_w = b.tmpw;
+    in.tmp_b = b.tmpb;
+    in.exif = b.exif;
+    in.camera_idx = b.cam;
+    in.num_cameras = h->w.num_cameras;
+    in.call_of_row = b.call;  // a bad camera index was reported by gather_rows, in its scene's fault word
+    LAUNCH(ca::heads_launch(h->w.heads, in, b.depth, b.conf, nullptr, R, st));
+    return curiosity_join(h, st);
+  };
+  CA_TRY(run_captured(h, b.graphs, b.seen, R * (CA_GUIDE_MANY_MAX_CALLS + 1) + m, c->use_graph != 0, st, seq));
+  CA_CUDA(cudaMemcpyAsync(c->depth, b.depth, static_cast<size_t>(R) * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c->conf, b.conf, static_cast<size_t>(R) * 4, cudaMemcpyDeviceToDevice, st));
+  CA_CUDA(cudaMemcpyAsync(c->attention, b.heat, static_cast<size_t>(R) * N * 4, cudaMemcpyDeviceToDevice, st));
+  if (c->argmax) CA_CUDA(cudaMemcpyAsync(c->argmax, b.argmax, static_cast<size_t>(R) * 4, cudaMemcpyDeviceToDevice, st));
+  h->last_launches = h->launches;
+  return 0;
 }
 
 int ca_depth_field(ca_handle* h, ca_scene* sc, const ca_depth_field_call* c, void* stream) {

@@ -33,6 +33,8 @@ from . import ops, tables
 from ._lib import RESIZE_MAX_SIDE as _RESIZE_MAX_SIDE  # largest photograph side the resize stages in shared memory
 from ._lib import GUIDE_TAIL_MAX_B as _GUIDE_TAIL_MAX_B  # single guided calls of larger batches run the three-kernel tail
 from ._lib import SWEEP_MAX_K as _SWEEP_MAX_K  # instructions per sweep: the sweep pool keeps one accumulator each
+from ._lib import GUIDE_MANY_MAX_CALLS as _GUIDE_MANY_MAX_CALLS, GUIDE_MANY_MAX_ROWS as _GUIDE_MANY_MAX_ROWS
+from ._lib import GUIDE_MANY_ROW_WORDS as _GUIDE_MANY_ROW_WORDS
 from .config import DEFAULT_COGNITIVE_MODULES, EffectiveConfig, effective_config
 from .init import reference_init_
 
@@ -236,6 +238,7 @@ class CognitiveAimModel(nn.Module):
         self._packed_key = None
         self._tables: Dict = {}   # per-grid tables (pos-embed, PE, centre bias, masks)
         self._ws: Dict = {}       # workspaces keyed by (B, S)
+        self._many: Dict = {}     # guide_many buffers keyed by (S, R, m)
         self.input_size = None        # side uint8 [B, H, W, 3] inputs are resized to (demo.py's dataset.image_size); None = as given
         self.validate_inputs = True   # camera_idx range faults (checked on the device) are raised at the next call
         self._fault = None            # pinned int32 the heads kernel flags input faults in
@@ -266,6 +269,7 @@ class CognitiveAimModel(nn.Module):
         self._packed = None
         self._tables = {}
         self._ws = {}
+        self._many = {}
 
     def _sd(self) -> Dict[str, torch.Tensor]:
         return dict(self.state_dict(keep_vars=True))
@@ -547,20 +551,29 @@ class CognitiveAimModel(nn.Module):
         noise [B,768]) of an un-guided forward, or `_sweep_draws`' (eps, noise, projection weight, bias) of R guided calls
         — through the pinned staging of one ring slot into the sweep buffers' cur_eps, cur_noise (and tmpw, tmpb)."""
         R, B = len(draws), draws[0][0].shape[0]
+
+        def fill(bufs):
+            for k, d in enumerate(draws):
+                for buf, t in zip(bufs, d):
+                    buf[k].copy_(t)
+            return [(cs[dst], buf) for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb")[:len(draws[0])], bufs)]
+
+        self._stage_pinned((B, R), ((R, B, 192), (R, B, _D), (R, 64, _D), (R, 64)), fill)
+
+    def _stage_pinned(self, key, shapes, fill):
+        """Per-call host inputs through the pinned staging of one ring slot: `fill` writes the slot's fp32 buffers of
+        `shapes` (kept per `key`) and returns the (device destination, pinned source) pairs to read, in order."""
         slot = self._pinned_slot()
-        # pinned buffers per (B, R), kept for the life of the model: a kernel reads them asynchronously, so they must
+        # pinned buffers per key, kept for the life of the model: a kernel reads them asynchronously, so they must
         # never go back to the host allocator while a read may be in flight (the slot's event guards their REUSE)
-        bufs = slot["draws"].get((B, R))
+        bufs = slot["draws"].get(key)
         if bufs is None:
-            bufs = slot["draws"][(B, R)] = tuple(torch.empty(*s).pin_memory() for s in
-                                                 ((R, B, 192), (R, B, _D), (R, 64, _D), (R, 64)))
-        for k, d in enumerate(draws):
-            for buf, t in zip(bufs, d):
-                buf[k].copy_(t)
+            bufs = slot["draws"][key] = tuple(torch.empty(*s).pin_memory() for s in shapes)
+        pairs = fill(bufs)
         # SM-side reads of the pinned staging area (ops.fetch_pinned), not cudaMemcpyAsync: these few hundred KB must not
         # wait on the H2D copy engine behind the application's upload of the next image batch
-        for dst, buf in zip(("cur_eps", "cur_noise", "tmpw", "tmpb")[:len(draws[0])], bufs):
-            ops.fetch_pinned(cs[dst], buf)
+        for dst, buf in pairs:
+            ops.fetch_pinned(dst, buf)
         slot["event"].record()
 
     @staticmethod
@@ -1159,6 +1172,168 @@ class CognitiveAimModel(nn.Module):
         self._run_scene(scene, ws, ("sweep", K), device_pass)
         self._keepalive = (mask,)
         return self._sweep_results(cs, K, return_attention)
+
+    # -- many scenes: one guide call on each of m scenes, answered together -----------------------------------
+    def _check_many(self, scenes, guidances):
+        """(S, R) of a guide_many call, R = the images of all its scenes; checked before anything is drawn or launched."""
+        if not isinstance(scenes, (list, tuple)) or not isinstance(guidances, (list, tuple)):
+            raise ValueError("guide_many takes a list of scenes and a list of guidances")
+        m = len(scenes)
+        if m == 0 or len(guidances) != m:
+            raise ValueError(f"guide_many takes m >= 1 scenes and one guidance per scene (got {m} scenes and "
+                             f"{len(guidances)} guidances)")
+        if m > _GUIDE_MANY_MAX_CALLS:
+            raise ValueError(f"guide_many takes at most {_GUIDE_MANY_MAX_CALLS} scenes, got {m}")
+        if any(gd is None for gd in guidances):
+            raise ValueError("a None guidance runs the un-guided focal path (src/model.py:1206-1212): use "
+                             "forward_with_guidance for it")
+        for scene in scenes:
+            self._check_scene(scene)
+        S = scenes[0].S
+        if any(scene.S != S for scene in scenes):
+            raise ValueError(f"the scenes of one guide_many call must share the image side (got "
+                             f"{sorted({scene.S for scene in scenes})})")
+        for scene, gd in zip(scenes, guidances):
+            self._check_per_image(gd, scene.B)
+            for one in (gd if isinstance(gd, (list, tuple)) else [gd]):
+                if isinstance(one, str) and tables.canonical_instruction(one) not in tables.INSTRUCTIONS:
+                    raise ValueError(f"unknown instruction {one!r} (one of {', '.join(tables.INSTRUCTIONS)} or an alias)")
+        R = sum(scene.B for scene in scenes)
+        if R > _GUIDE_MANY_MAX_ROWS:
+            raise ValueError(f"guide_many takes at most {_GUIDE_MANY_MAX_ROWS} images over all scenes, got {R}")
+        return S, R
+
+    def _many_buffers(self, S: int):
+        """The buffers of guide_many calls at side S, sized at the caps (CA_GUIDE_MANY_MAX_ROWS rows,
+        CA_GUIDE_MANY_MAX_CALLS calls): a call of R rows and m calls uses the first R rows / m projections of each, and
+        its graph is kept per (R, m).  Nothing here is per (B, S): no backbone workspace is needed."""
+        cs = self._many.get(S)
+        if cs is None:
+            dev = self._device()
+            N = (S // 14) ** 2
+            R, m = _GUIDE_MANY_MAX_ROWS, _GUIDE_MANY_MAX_CALLS
+            fl = dict(device=dev, dtype=torch.float32)
+            cs = {
+                # ca_guide_many_row [R] as fp32 words, staged with the draws (ops.fetch_pinned reads fp32)
+                "rows": torch.empty(R, 2 * _GUIDE_MANY_ROW_WORDS, **fl),
+                "cls": torch.empty(R, _D, **fl), "base": torch.empty(R, N, **fl), "exif": torch.empty(R, 3, **fl),
+                "cam": torch.empty(R, device=dev, dtype=torch.int64),
+                "call": torch.empty(R, device=dev, dtype=torch.int32),
+                # one CuriosityModule run over the R rows: the ring receives them in call order
+                "cur_eps": torch.zeros(1, R, 192, **fl), "cur_noise": torch.zeros(1, R, _D, **fl),
+                "cur_raw": torch.empty(1, R, **fl), "cur_reward": torch.empty(1, R, **fl),
+                "tmpw": torch.empty(m, 64, _D, **fl), "tmpb": torch.empty(m, 64, **fl),
+                "mask_in": torch.empty(R, N, **fl), "heat": torch.empty(R, N, **fl),
+                "argmax": torch.empty(R, device=dev, dtype=torch.int32),
+                "tail_pool": torch.empty(R, _POOL_SPLITS, _D, **fl),
+                "depth": torch.empty(R, **fl), "conf": torch.empty(R, **fl),
+                "graphs": {}, "calls": {},
+            }
+            _poison(cs.values())
+            if len(self._many) >= 4:  # keep the cache bounded
+                self._many.pop(next(iter(self._many)))
+            self._many[S] = cs
+        return cs
+
+    @staticmethod
+    def _many_rows(cs, R: int, m: int):
+        """The views of the first R rows / m calls of a guide_many buffer set (leading slices: contiguous)."""
+        per_call = ("tmpw", "tmpb")
+        rows = {k: (v[:m] if k in per_call else v[:, :R] if k.startswith("cur_") else v[:R])
+                for k, v in cs.items() if torch.is_tensor(v)}
+        rows["graphs"] = cs["graphs"]
+        return rows
+
+    @staticmethod
+    def _row_table(scenes, N: int, fault: int):
+        """ca_guide_many_row [R] as int64 words: per image of each scene in call order, the addresses of its tokens,
+        focal attention, EXIF and camera index in the scene, the fault word a bad camera index is reported in, and its
+        call index."""
+        words = []
+        for j, scene in enumerate(scenes):
+            tok, base, exif, cam = (t.data_ptr() for t in (scene.tokens, scene.base, scene.exif, scene.camera_idx))
+            for b in range(scene.B):
+                words += [tok + b * (N + 1) * _D * 4, base + b * N * 4, exif + b * 12, cam + b * 8, fault, j]
+        return torch.tensor(words, dtype=torch.int64)
+
+    @torch.no_grad()
+    @_on_own_device
+    def guide_many(self, scenes, guidances, return_attention=False):
+        """One guide call on each of m scenes, answered together: returns the list of m tuples
+        `[guide(scenes[j], guidances[j], return_attention) for j in range(m)]`, bit for bit, and leaves the global
+        generator, the CuriosityModule ring buffer and pointer and `_last_*` (from call m) as that loop would.  The
+        scenes may differ in batch size and repeat; they share the model, the device and the image side S.  A guidance
+        is what `guide` takes, except that an unknown instruction string is refused.  At most
+        CA_GUIDE_MANY_MAX_CALLS scenes of CA_GUIDE_MANY_MAX_ROWS images in all (include/cogaim_b200.h).
+        The R images of all calls run as one batch: the CLS tokens, focal attention rows and EXIF are gathered through
+        a row table (the patch tokens are read where the scenes keep them), then one CuriosityModule run, one guided
+        softmax, pool and heads pass.  With curiosity-guided attention every call needs its own focal pass, and the m
+        calls run one after another."""
+        self._raise_on_fault()
+        S, R = self._check_many(scenes, guidances)
+        self._pack()
+        g = S // 14
+        N = g * g
+        masks = [self._sweep_masks([gd], scene.B, g)[0] for scene, gd in zip(scenes, guidances)]
+        if self.cfg.curiosity_guided:
+            return [self.guide(scene, gd, return_attention) for scene, gd in zip(scenes, guidances)]
+        m = len(scenes)
+        draws = [self._sweep_draws(scene.B, 1)[0] for scene in scenes]  # call order: :609, :744, :1421 per call
+        full = self._many_buffers(S)
+        cs = self._many_rows(full, R, m)
+        table = self._row_table(scenes, N, self._fault_word().data_ptr())
+        caps = (_GUIDE_MANY_MAX_ROWS, _GUIDE_MANY_MAX_CALLS)
+
+        def fill(bufs):
+            eps, noise, tmpw, tmpb, rows = bufs
+            r = 0
+            for j, (scene, d) in enumerate(zip(scenes, draws)):
+                eps[r:r + scene.B].copy_(d[0])
+                noise[r:r + scene.B].copy_(d[1])
+                tmpw[j].copy_(d[2])
+                tmpb[j].copy_(d[3])
+                r += scene.B
+            rows[:R].view(torch.int64).copy_(table.view(R, _GUIDE_MANY_ROW_WORDS))
+            return [(cs["cur_eps"][0], eps[:R]), (cs["cur_noise"][0], noise[:R]), (cs["tmpw"], tmpw[:m]),
+                    (cs["tmpb"], tmpb[:m]), (cs["rows"], rows[:R])]
+
+        # one pinned set per ring slot, at the caps: the staging memory does not grow with the (R, m) seen
+        self._stage_pinned("many", ((caps[0], 192), (caps[0], _D), (caps[1], 64, _D), (caps[1], 64),
+                                    (caps[0], 2 * _GUIDE_MANY_ROW_WORDS)), fill)
+        torch.cat(masks, out=cs["mask_in"])
+        pk = self._packed
+
+        def device_pass():
+            ops.gather_rows(cs["rows"], R, N, cs["cls"], cs["base"], cs["exif"], cs["cam"], cs["call"],
+                            num_cameras=self.cfg.num_cameras)  # reports a bad camera index in the row's fault word
+            self._curiosity_runs(cs, cs["cls"], R, 1, ("guided",))
+            ops.guided_softmax(cs["base"], cs["mask_in"], cs["heat"], cs["argmax"], R, N)
+            ops.weighted_pool_rows(cs["rows"], cs["heat"], cs["tail_pool"], R, N, _D, _POOL_SPLITS)
+            ops.heads(pk["heads"], tokens=cs["cls"], tokens_per_img=1, depth=cs["depth"], conf=cs["conf"], B=R,
+                      pool_partial=cs["tail_pool"], pool_splits=_POOL_SPLITS, tmp_w=cs["tmpw"], tmp_b=cs["tmpb"],
+                      exif=cs["exif"], camera_idx=cs["cam"], num_cameras=self.cfg.num_cameras, call_of_row=cs["call"])
+            self._curiosity_join()
+
+        # eager at the first call of this (R, m), captured at the second, replayed after — with any scenes: the row
+        # table is data
+        calls = full["calls"][(R, m)] = full["calls"].get((R, m), 0) + 1
+        if calls == 1:
+            device_pass()
+        else:
+            self._run(cs, ("many", R, m, self._curiosity_key()), device_pass)
+        self._keepalive = (tuple(scenes), masks)
+        heat = cs["heat"].clone()
+        depth, conf = cs["depth"].clone().unsqueeze(-1), cs["conf"].clone().unsqueeze(-1)
+        out, r = [], 0
+        for scene in scenes:
+            rows = slice(r, r + scene.B)
+            out.append((depth[rows], conf[rows], heat[rows]) if return_attention else (depth[rows], conf[rows]))
+            r += scene.B
+        last = slice(R - scenes[-1].B, R)  # what call m leaves behind
+        self._last_attention_weights = heat[last]
+        self._last_argmax = cs["argmax"][last].clone()
+        self._last_curiosity = cs["cur_reward"][0, last].clone()
+        return out
 
     def _field_buffers(self, ws, B: int, N: int):
         """The depth-field buffers of a (B, S) workspace, added at its first field: the projected tokens [B, N, 64], the

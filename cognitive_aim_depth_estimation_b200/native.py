@@ -311,12 +311,16 @@ class NativeModel:
         return tokens
 
     @torch.no_grad()
-    def encode(self, images, exif, S=None) -> "NativeScene":
+    def encode(self, images, exif, S=None, fault=None) -> "NativeScene":
         """ca_encode: the backbone and the focal pass of the batch, once, kept in a scene for `guide` / `guide_sweep`.
-        Draws nothing from the global generator."""
+        Draws nothing from the global generator.  `fault`: an optional pinned int32 tensor in which the scene's guide
+        calls report a camera index outside the embedding table (bit 0)."""
         if exif is None:
             raise ValueError("a scene needs EXIF data (without it the reference falls back to forward())")
         c, held, B, S = self._call(images, exif, S)
+        if fault is not None:
+            c.fault = fault.data_ptr()
+            held.append(fault)
         out = C.c_void_p()
         with torch.cuda.device(self.device):
             _lib.check(self.lib.ca_encode(self._h, C.byref(c), C.byref(out), self._stream()), "ca_encode")
@@ -352,6 +356,56 @@ class NativeModel:
             _lib.check(self.lib.ca_guide_sweep(self._h, scene.ptr, C.byref(s), self._stream()), "ca_guide_sweep")
         self._held = held
         return out["depth"].unsqueeze(-1), out["conf"].unsqueeze(-1), out["heat"], out["argmax"]
+
+    @torch.no_grad()
+    def guide_many(self, scenes, guidances):
+        """ca_guide_many: one `guide` call on each of m scenes of one side S in one native call, bit for bit what the m
+        `guide` calls return, with their draws made in the same order.  `guidances`: m instruction strings, or m guidance
+        tensors ([N] or [B_j, N]).  -> a list of m (depth [B_j,1], confidence [B_j,1], heat map [B_j,N], arg-max
+        cell [B_j])."""
+        m = len(scenes)
+        if m == 0 or len(guidances) != m:
+            raise ValueError("guide_many takes m >= 1 scenes and one guidance per scene")
+        S = scenes[0].S
+        N = (S // 14) ** 2
+        R = sum(sc.B for sc in scenes)
+        c = _lib.GuideManyCall()
+        c.m = m
+        ptrs = (C.c_void_p * m)(*[sc.ptr.value if sc.ptr is not None else None for sc in scenes])
+        c.scenes = C.cast(ptrs, C.POINTER(C.c_void_p))
+        held = [ptrs]
+        if all(isinstance(g, str) for g in guidances):
+            names = (C.c_char_p * m)(*[g.encode() for g in guidances])
+            held.append(names)
+            c.instructions = C.cast(names, C.POINTER(C.c_char_p))
+        elif all(torch.is_tensor(g) for g in guidances):
+            rows = [g.to(self.device, torch.float32).reshape(-1, N).expand(sc.B, N) for sc, g in zip(scenes, guidances)]
+            masks = torch.cat(rows).contiguous()
+            held.append(masks)
+            c.masks = masks.data_ptr()
+        else:
+            raise ValueError("guidances must be m instruction strings or m guidance tensors")
+        draws = []
+        for sc in scenes:  # per call in order: randn(B_j, 192), randn(B_j, 768), nn.Linear(768, 64)
+            eps, noise = torch.randn(sc.B, 192), torch.randn(sc.B, _D)
+            tmp = nn.Linear(_D, 64)
+            draws.append((eps, noise, tmp.weight.detach(), tmp.bias.detach()))
+        eps, noise = torch.cat([d[0] for d in draws]), torch.cat([d[1] for d in draws])
+        tmp_w, tmp_b = torch.stack([d[2] for d in draws]).contiguous(), torch.stack([d[3] for d in draws]).contiguous()
+        held += [eps, noise, tmp_w, tmp_b]
+        c.eps, c.noise, c.tmp_w, c.tmp_b = eps.data_ptr(), noise.data_ptr(), tmp_w.data_ptr(), tmp_b.data_ptr()
+        out = self._outputs(c, 1, R, N)
+        c.use_graph = int(self.use_graph)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.ca_guide_many(self._h, C.byref(c), self._stream()), "ca_guide_many")
+        self._held = held
+        res, r = [], 0
+        for sc in scenes:
+            rows = slice(r, r + sc.B)
+            res.append((out["depth"][0, rows].unsqueeze(1), out["conf"][0, rows].unsqueeze(1), out["heat"][0, rows],
+                        out["argmax"][0, rows]))
+            r += sc.B
+        return res
 
     @torch.no_grad()
     def depth_field(self, scene: "NativeScene"):

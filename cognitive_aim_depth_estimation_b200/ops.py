@@ -323,6 +323,46 @@ def weighted_pool_sweep(src, src_batch_stride, row_offset, w, partial, K, B, N, 
     _end(e0, "pool", 1, float(B * N * D * 4))
 
 
+def _row_table(rows, R):
+    """A device row table (`ca_guide_many_row` [R]) held as int64 [R, GUIDE_MANY_ROW_WORDS] or fp32 [R, 2 * words]."""
+    if not rows.is_cuda or rows.dtype not in (torch.int64, torch.float32) or not rows.is_contiguous():
+        raise ValueError("rows must be a contiguous CUDA tensor (int64 or fp32 words of ca_guide_many_row)")
+    if rows.numel() * rows.element_size() != R * _lib.GUIDE_MANY_ROW_WORDS * 8:
+        raise ValueError(f"rows must hold {R} ca_guide_many_row entries")
+
+
+def gather_rows(rows, R, N, cls, base, exif, camera_idx, call_of_row, num_cameras=0):
+    """Through the row table `rows` (ca_guide_many_row [R]): cls [R, 768], base [R, N], exif [R, 3], camera_idx [R]
+    (int64) and call_of_row [R] (int32), one launch (csrc/focal.cu).  A camera index outside [0, num_cameras) sets bit 0
+    of the row's fault word."""
+    _row_table(rows, R)
+    for t, n in ((cls, "cls"), (base, "base"), (exif, "exif")):
+        _req(t, torch.float32, n)
+    _req(camera_idx, torch.int64, "camera_idx")
+    _req(call_of_row, torch.int32, "call_of_row")
+    if cls.numel() < R * 768 or base.numel() < R * N or exif.numel() < R * 3 or camera_idx.numel() < R \
+            or call_of_row.numel() < R:
+        raise ValueError("gather_rows: the outputs are smaller than R rows")
+    e0 = _begin()
+    check(_lib.load().ca_gather_rows(ptr(rows), R, N, int(num_cameras), ptr(cls), ptr(base), ptr(exif), ptr(camera_idx),
+                                     ptr(call_of_row), stream_ptr()), "ca_gather_rows")
+    _end(e0, "small", 1)
+
+
+def weighted_pool_rows(rows, w, partial, R, N, D, splits):
+    """`weighted_pool` over R rows of several scenes: row r pools w [R, N] against the tokens the row table points to
+    (rows 1..N of that image); partial [R, splits, D]."""
+    _row_table(rows, R)
+    _req(w, torch.float32, "w")
+    _req(partial, torch.float32, "partial")
+    if w.numel() < R * N or partial.numel() < R * splits * D:
+        raise ValueError("weighted_pool_rows: w needs R * N and partial R * splits * D floats")
+    e0 = _begin()
+    check(_lib.load().ca_weighted_pool_rows(ptr(rows), ptr(w), ptr(partial), R, N, D, splits, stream_ptr()),
+          "ca_weighted_pool_rows")
+    _end(e0, "pool", 1, float(R * N * D * 4))
+
+
 def resize_u8(src, out_h, out_w):
     """uint8 [B, H0, W0, 3] -> uint8 [B, out_h, out_w, 3], bit-exact PIL.Image.resize(..., BILINEAR) (csrc/resize.cu)."""
     _req(src, torch.uint8, "src")
@@ -458,15 +498,17 @@ def make_heads_weights(named):
 
 def heads(weights, *, tokens, tokens_per_img, depth, conf, B, focal_feat=None, pool_partial=None, pool_splits=0,
           tmp_w=None, tmp_b=None, pooled_out=None, exif=None, camera_idx=None, fused_out=None, num_cameras=0,
-          fault_ptr=None, sweep_images=0):
+          fault_ptr=None, sweep_images=0, call_of_row=None):
     """`fault_ptr`: address of a device-visible int32 (pinned host memory) that receives bit 0 when a camera index lies
     outside [0, num_cameras) — the range check of the embedding lookup, done on the device so the call never syncs.
     `sweep_images` > 0: an instruction sweep of B / sweep_images calls over `sweep_images` images (rows k * images + b,
-    tmp_w [K, 64, 768], tmp_b [K, 64]; include/cogaim_b200.h ca_heads_inputs)."""
+    tmp_w [K, 64, 768], tmp_b [K, 64]; include/cogaim_b200.h ca_heads_inputs).  `call_of_row` (int32 [B]): row r uses
+    projection call_of_row[r] of tmp_w [m, 64, 768] / tmp_b [m, 64] (the rows of several guide calls)."""
     import ctypes as C
+    _req(call_of_row, torch.int32, "call_of_row")
     inp = _lib.HeadsInputs(_dp(tokens), tokens_per_img, _dp(focal_feat), _dp(pool_partial), pool_splits, _dp(tmp_w),
                            _dp(tmp_b), _dp(pooled_out), _dp(exif), _dp(camera_idx), int(num_cameras), fault_ptr,
-                           int(sweep_images))
+                           int(sweep_images), _dp(call_of_row))
     e0 = _begin()
     check(_lib.load().ca_heads(C.byref(weights), C.byref(inp), ptr(depth), ptr(conf), ptr(fused_out), B, stream_ptr()),
           "ca_heads")

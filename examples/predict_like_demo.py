@@ -3,6 +3,7 @@
     python examples/predict_like_demo.py IMAGE.jpg [--instruction center] [--image-size 224] [--overlay out.npy]
     python examples/predict_like_demo.py --image-dir DIR [--instruction center] [--image-size 224]
     python examples/predict_like_demo.py IMAGE.jpg --interactive < instructions.txt
+    python examples/predict_like_demo.py A.jpg B.jpg C.jpg --interactive < lines.txt
     python examples/predict_like_demo.py IMAGE.jpg --depth-field OUT.npz
 
 What demo.py does per image and what runs here instead:
@@ -18,7 +19,10 @@ What demo.py does per image and what runs here instead:
 nvJPEG call and runs the photographs, whatever their sizes, through ONE forward (`Predictor.predict_batch`).
 `--interactive` encodes the photograph once (`Predictor.encode`, model.encode: decode, backbone, focal stream) and then
 reads instructions from stdin, one per line, printing for each the line `predict` prints (`Predictor.predict_scene`,
-model.guide); the results equal successive `predict` calls on the same photograph.
+model.guide); the results equal successive `predict` calls on the same photograph.  With several IMAGEs each is
+encoded once and each stdin line gives one instruction per photograph, in order (`-` skips one); the line is answered by
+ONE `guide_many` call over the photographs it names (`Predictor.predict_scenes`), printing `NAME: ` and the `predict`
+line per answered photograph — the results of successive `predict` calls in that order.
 `--depth-field OUT.npz` encodes the photograph once and saves the guided depth and confidence with the focus on every
 cell of the g x g patch grid (`Predictor.depth_field`, model.depth_field) as `depth` and `confidence` [g, g]: cell
 (y, x) is the prediction of a guided call focused there (cell (g//4, g//4) is the "top-left" prediction).
@@ -156,6 +160,22 @@ class Predictor:
         return float(depth.squeeze()), float(conf.squeeze()), meta
 
     @torch.no_grad()
+    def predict_scenes(self, scenes, instructions):
+        """`[predict_scene(s, ins) for s, ins in zip(scenes, instructions)]` in ONE call (model.guide_many): one guided
+        pass over the photographs of all scenes, bit for bit the same results and model state."""
+        g = self.image_size // 14
+        out = []
+        for ins, (depth, conf, heat) in zip(instructions, self.model.guide_many(list(scenes), list(instructions),
+                                                                                return_attention=True)):
+            cell = int(heat[0].argmax())
+            meta = {"processed_size": (self.image_size, self.image_size), "instruction": ins,
+                    "attention_cell": (cell // g, cell % g),
+                    "model_status": {"ambient": self.model.use_ambient, "focal": self.model.use_focal,
+                                     "exif": self.model.use_exif}}
+            out.append((float(depth.squeeze()), float(conf.squeeze()), meta))
+        return out
+
+    @torch.no_grad()
     def depth_field(self, jpeg_bytes: bytes, exif=None):
         """-> (depth, confidence) [g, g] CPU tensors: the guided prediction with the focus on every cell of the patch grid,
         from one encode and one depth-field call."""
@@ -174,19 +194,22 @@ def result_line(ins, depth, conf, meta):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("image", nargs="?")
+    ap.add_argument("image", nargs="*", help="one photograph (several with --interactive)")
     ap.add_argument("--image-dir", default=None, help="predict every .jpg / .jpeg of DIR in one batched call")
     ap.add_argument("--instruction", default=None, help="one of %s, or 'all'" % ", ".join(INSTRUCTIONS))
     ap.add_argument("--image-size", type=int, default=224)  # configs/experiment_B.yaml:87
     ap.add_argument("--checkpoint", default=None)
     ap.add_argument("--overlay", default=None, help="write the overlay heat map of the last instruction as .npy")
     ap.add_argument("--interactive", action="store_true",
-                    help="encode IMAGE once, then read instructions from stdin, one per line")
+                    help="encode each IMAGE once, then read instructions from stdin, one line per step with one "
+                         "instruction per IMAGE ('-' skips one)")
     ap.add_argument("--depth-field", default=None, metavar="OUT.npz",
                     help="save the guided depth and confidence with the focus on every patch cell as [g, g] arrays")
     args = ap.parse_args()
-    if (args.image is None) == (args.image_dir is None):
+    if bool(args.image) == (args.image_dir is not None):
         ap.error("give IMAGE or --image-dir DIR")
+    if len(args.image) > 1 and not args.interactive:
+        ap.error("several IMAGEs are taken with --interactive only")
     # without a checkpoint: the reference's own random init (demo.py:148-150 "continuing with randomly initialized
     # weights") — create_model draws it from the global generator exactly like the reference's constructor
     sd = torch.load(args.checkpoint, map_location="cpu") if args.checkpoint else None
@@ -202,7 +225,7 @@ def main():
         for depth, conf, meta in p.predict_batch(files, args.instruction):  # one line per file, sorted by name
             print(result_line(args.instruction, depth, conf, meta))
         return
-    data = open(args.image, "rb").read()
+    data = open(args.image[0], "rb").read()
     if args.depth_field:
         if args.instruction or args.overlay or args.interactive:
             ap.error("--depth-field takes no --instruction, --overlay or --interactive")
@@ -216,11 +239,26 @@ def main():
     if args.interactive:
         if args.instruction or args.overlay:
             ap.error("--interactive reads its instructions from stdin and takes no --overlay")
-        scene = p.encode(data)
+        if len(args.image) == 1:
+            scene = p.encode(data)
+            for line in sys.stdin:
+                ins = line.strip()
+                if ins:
+                    print(result_line(ins, *p.predict_scene(scene, ins)), flush=True)
+            return
+        scenes = [p.encode(open(path, "rb").read()) for path in args.image]
+        names = [os.path.basename(path) for path in args.image]
         for line in sys.stdin:
-            ins = line.strip()
-            if ins:
-                print(result_line(ins, *p.predict_scene(scene, ins)), flush=True)
+            words = line.split()
+            if not words:
+                continue
+            if len(words) != len(scenes):
+                print(f"expected {len(scenes)} instructions ('-' to skip one), got {len(words)}", file=sys.stderr)
+                continue
+            picked = [j for j, w in enumerate(words) if w != "-"]
+            if picked:
+                for j, res in zip(picked, p.predict_scenes([scenes[j] for j in picked], [words[j] for j in picked])):
+                    print(f"{names[j]}: " + result_line(words[j], *res), flush=True)
         return
     overlay_size = (480, 640) if args.overlay else None
     if args.instruction == "all":  # every instruction in one sweep (backbone and focal pass once)

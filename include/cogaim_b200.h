@@ -161,6 +161,30 @@ int ca_guided_softmax_sweep(const float* base, long long base_k_stride, const fl
 int ca_weighted_pool_sweep(const float* src, long long src_batch_stride, int row_offset, const float* w, float* partial,
                            int K, int B, int N, int D, int splits, void* stream);
 
+/* Rows of several scenes: m guide calls answered together (ca_guide_many, CognitiveAimModel.guide_many).  Row r of the
+ * batch is one image of one call's scene, r in call order; the row table holds, per row, DEVICE pointers into the scene
+ * that owns the image.  Nothing of a scene is copied but the few values below. */
+#define CA_GUIDE_MANY_MAX_CALLS 64 /* guide calls per ca_guide_many */
+#define CA_GUIDE_MANY_MAX_ROWS 256 /* rows (the images of all calls) per ca_guide_many */
+typedef struct ca_guide_many_row {
+  const float* tokens;          /* the image's tokens [1 + N, 768] fp32 (row 0: CLS), 16-byte aligned */
+  const float* base;            /* its focal attention [N] */
+  const float* exif;            /* its EXIF [3] */
+  const long long* camera_idx;  /* its camera index */
+  int* fault;                   /* the fault word a bad camera index of this image is reported in (bit 0), or NULL */
+  long long call;               /* j: the guide call the row belongs to */
+} ca_guide_many_row;
+/* One launch: cls[r, :] = rows[r].tokens[0, :] ([R, 768]), base[r, :] = rows[r].base ([R, N]), exif[r, :] ([R, 3]),
+ * camera_idx[r] ([R] int64) and call_of_row[r] = rows[r].call ([R] int32).  A camera index outside [0, num_cameras)
+ * sets bit 0 of rows[r].fault (the heads clamp it).  `rows` is a DEVICE array of R entries. */
+int ca_gather_rows(const ca_guide_many_row* rows, int R, int N, int num_cameras, float* cls, float* base, float* exif,
+                   long long* camera_idx, int32_t* call_of_row, void* stream);
+/* ca_weighted_pool with the tokens of row r read through the row table: partial[r, s, :] = sum_{n in split s} w[r, n] *
+ * rows[r].tokens[(1 + n) * 768 + :].  Partial r is bit for bit what ca_weighted_pool writes for that image alone with
+ * the same `splits`.  `rows`: DEVICE [R]; w: [R, N]; D must be 768. */
+int ca_weighted_pool_rows(const ca_guide_many_row* rows, const float* w, float* partial, int R, int N, int D, int splits,
+                          void* stream);
+
 /* Heads ------------------------------------------------------------------------------------------ */
 /* All members are DEVICE pointers to fp32 row-major [out, in] weights / [out] biases of the reference modules. */
 typedef struct ca_heads_weights {
@@ -190,6 +214,9 @@ typedef struct ca_heads_inputs {
                                  K * sweep_images; CTA r reads image b = r % sweep_images (CLS token, EXIF, camera index),
                                  projection k = r / sweep_images of tmp_w [K, 64, 768] / tmp_b [K, 64], pool_partial row r,
                                  and writes depth[r], conf[r] */
+  const int32_t* call_of_row; /* guided only, with sweep_images 0: [B] device; row r uses projection call_of_row[r] of
+                                 tmp_w [m, 64, 768] / tmp_b [m, 64] (rows of several guide calls, ca_guide_many).  NULL:
+                                 the projection follows sweep_images as above */
 } ca_heads_inputs;
 
 /* depth[B], conf[B] (and optionally fused_out[B,192]) from the backbone tokens + focal slot + EXIF.
@@ -493,6 +520,30 @@ typedef struct ca_depth_field_call {
  * draws: one projection for every cell and one CuriosityModule run (B ring entries).  The scene graph policy and the
  * refusals are those of ca_guide. */
 int ca_depth_field(ca_handle* h, ca_scene* scene, const ca_depth_field_call* call, void* stream);
+/* One guide call on each of m scenes in one: HOST pointers where marked, device otherwise.  Rows r = 0..R-1 are the
+ * images of the calls in call order, R = sum of the scenes' B. */
+typedef struct ca_guide_many_call {
+  int m;                           /* 1..CA_GUIDE_MANY_MAX_CALLS; R at most CA_GUIDE_MANY_MAX_ROWS */
+  ca_scene* const* scenes;         /* HOST [m]: scenes of this handle, all of one side S; a scene may repeat */
+  const char* const* instructions; /* HOST [m] instruction strings / aliases, or NULL when `masks` is given */
+  const float* masks;              /* [R, N] explicit guidance, one row per image; or NULL */
+  const float* tmp_w;              /* HOST [m, 64, 768]: the per-call projections, in call order  src/model.py:1421 */
+  const float* tmp_b;              /* HOST [m, 64] */
+  const float* eps;                /* HOST [R, 192]: the CuriosityModule draw of :609 of each call, rows in call order */
+  const float* noise;              /* HOST [R, 768]: the draw of :744 */
+  float* depth;                    /* out [R] */
+  float* conf;                     /* out [R] */
+  float* attention;                /* out [R, N] heat maps */
+  int* argmax;                     /* out [R] or NULL */
+  int use_graph;                   /* 1: capture the launches at the second call of this (S, R, m) and replay them after,
+                                      for any scenes */
+} ca_guide_many_call;
+/* m ca_guide calls, one per scene, bit for bit given the same draws, in ONE pass over the R rows: the row inputs
+ * gathered through a row table (ca_gather_rows), one CuriosityModule run over the R CLS rows (the ring receives them in
+ * call order), the guided softmax, ca_weighted_pool_rows and the heads with call_of_row.  Each scene's graphs are left
+ * alone.  Every scene is checked as ca_guide checks it before anything is enqueued; a bad camera index of scene j is
+ * reported in scene j's fault word. */
+int ca_guide_many(ca_handle* h, const ca_guide_many_call* call, void* stream);
 /* Release a scene's memory and graphs (waits for the device).  NULL is a no-op. */
 int ca_scene_destroy(ca_scene* scene);
 
